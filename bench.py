@@ -8,6 +8,7 @@ replicated, no data-path collective => weak scaling).
   value  : edge-world validity checks/s, inputs resident in HBM, kernel launched through porrt_edge_validity_dev
   e2e    : the same metric through the host-buffer C-ABI call porrt_edge_validity (pinned host buffers, H2D + D2H inside)
   --impl reference : the reference's CPU path (oracle restatement; the Rust crate cannot be built here) on host cores
+  --dump-outputs DIR : the per-edge results of the last timed step as DIR/*.npy (dump_outputs), to compare two builds
 """
 import argparse
 import ctypes as C
@@ -38,7 +39,13 @@ def parse_args():
     ap.add_argument("--map-size", type=int, default=8192)
     ap.add_argument("--cpu-sample", type=int, default=2_000_000, help="edges in the CPU-baseline sample")
     ap.add_argument("--no-extras", action="store_true", help="skip the kNN / PRM-build side measurements")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last timed step as DIR/<name>.npy (rank 0's edges; "
+                         "see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    return args
 
 
 def workload_config(args):
@@ -47,6 +54,24 @@ def workload_config(args):
             "edges_per_gpu_per_step": args.edges, "map_seed": 1, "edge_seed": "2+rank",
             "l2": "edge streams (32 B in + 12 B out per edge, %.0f MB per step) exceed L2; the 64 MiB fused grid is meant to stay L2-resident"
                   % (args.edges * 44 / 1e6)}
+
+
+DUMP_EDGES = 1 << 20   # edges written by --dump-outputs: 4 B + 16 B each = 20 MiB
+
+
+def dump_outputs(out_dir, vid, mask=None):
+    """Writes the per-edge results of the timed path's last step, so that two builds can be compared output for output:
+    validity_id.npy (float32, the validity id or panic code of each edge) and, where the path returns them, world_mask.npy
+    (float64 [low 32 bits, high 32 bits] of each edge's 64-bit world mask; both halves are exact in float64).  Batches of more
+    than DUMP_EDGES edges are sampled: the same ascending edge indices every run (numpy default_rng(0)) for a given batch size."""
+    n = len(vid)
+    idx = np.arange(n) if n <= DUMP_EDGES else np.sort(np.random.default_rng(0).choice(n, DUMP_EDGES, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "validity_id.npy"), np.asarray(vid)[idx].astype(np.float32))
+    if mask is not None:
+        m = np.ascontiguousarray(np.asarray(mask)[idx]).view(np.uint64)
+        words = np.stack([m & np.uint64(0xFFFFFFFF), m >> np.uint64(32)], axis=1)
+        np.save(os.path.join(out_dir, "world_mask.npy"), words.astype(np.float64))
 
 
 def make_inputs(args, rank):
@@ -175,8 +200,10 @@ def run_reference(args):
         omap.edge_validity_timed(sa[: n // 4], sb[: n // 4], threads)
     t = 0.0
     for _ in range(args.steps):
-        _, dt = omap.edge_validity_timed(sa, sb, threads)
+        out, dt = omap.edge_validity_timed(sa, sb, threads)
         t += dt
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, out)
     value = n * N_WORLDS * args.steps / t
     line = {"impl": "reference", "metric": METRIC, "value": value, "unit": UNIT, "n_gpus": args.gpus, "steps": args.steps,
             "warmup": args.warmup, "ms_per_step": 1e3 * t / args.steps, "higher_is_better": True, "scaling": "weak",
@@ -755,6 +782,8 @@ def main():
     h_ti = torch.arange(E, 2 * E, dtype=torch.int32).pin_memory()
     want_vid = d_vid.cpu()
     want_mask = d_mask.cpu()
+    if args.dump_outputs and rank == 0:      # nothing after the timed loop has written d_vid / d_mask: the last step's results
+        dump_outputs(args.dump_outputs, want_vid.numpy(), want_mask.numpy())
     del d_a, d_b, d_vid, d_mask
     torch.cuda.empty_cache()
     tree = P.KdTree(ctx, np.concatenate([a, b]), cell_size=0.01)        # the vertex set: 2E node states, resident
