@@ -68,6 +68,9 @@ const char* porrt_last_error(porrt_ctx* ctx);
 #define PORRT_OPT_FORCE_GLOBAL_SWEEPS 2   /* value != 0: porrt_sssp_worlds / porrt_belief_vi run the thread-per-(node, column) sweeps over
                                              the table in global memory (used by itself for roadmaps whose column of V doubles does not
                                              fit in shared memory, V > ~29000) although the on-chip column solver would fit */
+#define PORRT_OPT_FORCE_THREAD_PER_QUERY_NN 3  /* value != 0: radius / 1-NN / k-NN queries skip the tile kernels and run the
+                                             thread-per-query ring search (used by itself for batches < 2048 queries and for
+                                             the queries the tiles cannot serve) */
 int32_t porrt_ctx_set_option(porrt_ctx* ctx, int32_t option, int64_t value);
 /* number of kernels this ctx has launched so far (bench.py's gpu_launches) */
 int64_t porrt_ctx_launch_count(porrt_ctx* ctx);

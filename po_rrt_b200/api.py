@@ -22,6 +22,7 @@ NODE_UNKNOWN, NODE_ACTION, NODE_OBSERVATION = 0, 1, 2
 ERR_CAPACITY = 4
 OPT_FORCE_LARGE_MAP_PATH = 1
 OPT_FORCE_GLOBAL_SWEEPS = 2
+OPT_FORCE_THREAD_PER_QUERY_NN = 3
 
 
 class PorrtError(RuntimeError):

@@ -108,6 +108,7 @@ struct porrt_ctx {
   DevBuf d_grid, d_coarse, d_validities, d_zone_pos, d_plane, d_bits;
   bool force_large_map_path = false;   // PORRT_OPT_FORCE_LARGE_MAP_PATH (tests): run map.cu's kernel although edge3.cu's would fit
   bool force_global_sweeps = false;    // PORRT_OPT_FORCE_GLOBAL_SWEEPS (tests): value backups by graph.cu's sweeps although colsolve.cu would fit
+  bool force_thread_per_query_nn = false;  // PORRT_OPT_FORCE_THREAD_PER_QUERY_NN (tests): nn.cu's kernels although nn_tile.cu's would serve
   // host copies of the raw images are NOT kept: the product never walks pixels on the CPU.
 
   // ---- vertices / cell grid (nn.cu)

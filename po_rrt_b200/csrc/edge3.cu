@@ -16,11 +16,13 @@
 //   * pixel k of the line is a + k*U + floor(k*dy/dx)*V (closed form, A5) and floor(k*dy/dx) = hi32(k*S + 2^16) with
 //     S = min(floor(dy*2^32/dx), 2^32-1): ONE integer multiply-add, exact for dx < 2^15 (proof in DESIGN.md 3.1,
 //     exhaustive check in tests/test_oracle_golden.py).
-// Work is flattened as in v2: the strips of a warp's 32 edges form one sequence, lanes take consecutive groups of
-// four strips, undecided strips are queued in shared memory and resolved by full warps afterwards; strips of edges
-// already known to be blocked are dropped.  Blocks containing gray pixels (door zones: zone ids and the reference's
-// panics matter) go to a per-pixel pass over the fused byte grid; whenever the ORDER of events along the line could
-// matter the edge is re-walked sequentially (walk_sequential), which is what makes the panic codes bit-exact.
+// Work is flattened as in v2: the strips of a warp's 32 edges are cut into items of E3_G consecutive strips of one edge.
+// Pass 1 runs in two phases: every lane first takes its own edge's first item, then the remaining items of the edges not
+// yet blocked form one sequence that the lanes take in turn.  Items with undecided strips are queued in shared memory and
+// resolved strip by strip by full warps afterwards; strips of edges already known to be blocked are dropped.  Blocks
+// containing gray pixels (door zones: zone ids and the reference's panics matter) go to a per-pixel pass over the fused
+// byte grid; whenever the ORDER of events along the line could matter the edge is re-walked sequentially
+// (walk_sequential), which is what makes the panic codes bit-exact.
 #include "edge_common.cuh"
 
 // Per-edge record in shared memory, three 16-byte chunks.  The minor axis is MIRRORED for edges whose minor step is
@@ -48,7 +50,7 @@ struct WarpMem {
   uint4 rec[3][32];         // Rec3 chunks, chunk-major (conflict-free 16-byte accesses)
   uint32_t obst[32];        // != 0: a blocking pixel is on the line
   uint32_t zmin[32], zmax[32];
-  uint32_t qb[E3_QB];       // E3_ITEM_QUEUE: pairs (e | first strip << 5, want mask: bit 4g = strip g); else e | strip << 5
+  uint32_t qb[E3_QB];       // items (e | first strip << 5, want mask: bit 4g = strip g) in [0, 2 * E3_QI), strip scratch after
   uint32_t qg[E3_QG];       // e | strip << 5
 };
 
@@ -92,26 +94,6 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
   // ---- resolution of the queued strips
   auto drain = [&]() {
     __syncwarp();
-#if !E3_ITEM_QUEUE
-    // (1) bitmap strips: drop those of edges already blocked, then one lane per strip
-    int live_n = 0;
-    for (int q0 = 0; q0 < qb_n; q0 += 32) {
-      const int q = q0 + lane;
-      uint32_t ent = 0;
-      bool live = false;
-      if (q < qb_n) { ent = wm.qb[q]; live = wm.obst[ent & 31] == 0; }
-      const unsigned lv = __ballot_sync(0xffffffffu, live);
-      __syncwarp();
-      if (live) wm.qb[live_n + __popc(lv & lt_mask)] = ent;
-      live_n += __popc(lv);
-      __syncwarp();
-    }
-    for (int q0 = 0; q0 < live_n; q0 += 32) {
-      const int q = q0 + lane;
-      if (q < live_n) {
-        const uint32_t ent = wm.qb[q];
-        const int e = ent & 31, ts = (int)(ent >> 5);
-#else
     // (1) bitmap strips.  The queue holds ITEMS (edge, first strip, mask of the strips that need their bitmaps) in
     // qb[0 .. 2 * E3_QI); per group of 32 items the strips are written out to qb[2 * E3_QI ..) -- prefix sums of the mask
     // popcounts, every lane expands its own item -- so that every lane of a round tests one strip.  Items of edges already
@@ -134,63 +116,51 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
       for (int pos = i_incl - i_cnt; i_want; i_want &= i_want - 1)
         qs[pos++] = i_ent + ((uint32_t)((__ffs(i_want) - 1) >> 2) << 5);
       __syncwarp();
-    for (int q0 = 0; q0 < live_n; q0 += 32) {
-      const int q = q0 + lane;
-      if (q < live_n) {
-        const uint32_t ent = qs[q];
-        const int e = ent & 31, ts = (int)(ent >> 5);
-#endif
-        if (wm.obst[e] == 0) {
-          const uint4 r0 = wm.rec[0][e], r1 = wm.rec[1][e];
-          const int dirs = (int)wm.rec[2][e].z;
-          const int dxo = (int)r1.y, n0m = (int)r1.x;
-          const uint32_t S = r1.z;
-          const int lo_raw = (int)r0.x + ts * E3_BS;
-          const int k_lo = max(0, lo_raw), k_hi = min(dxo, lo_raw + E3_BS - 1);
-          const bool neg_major = (dirs & 2) != 0;
-          const int bn_a = minor_m((uint32_t)k_lo, S, n0m) >> E3_LOG_BS;
-          const int bn_b = minor_m((uint32_t)k_hi, S, n0m) >> E3_LOG_BS;
-          const int blk_a = (int)r0.y - m.plane_guard + ts * (int)r0.z + bn_a * (int)r0.w;
-          const uint32_t* tiles = m.bits + (size_t)(((dirs & 1) << 1) | ((dirs >> 2) & 1)) * (size_t)m.bits_var_words;
-          uint32_t A[8], B[8];
+      for (int q0 = 0; q0 < live_n; q0 += 32) {
+        const int q = q0 + lane;
+        if (q < live_n) {
+          const uint32_t ent = qs[q];
+          const int e = ent & 31, ts = (int)(ent >> 5);
+          if (wm.obst[e] == 0) {
+            const uint4 r0 = wm.rec[0][e], r1 = wm.rec[1][e];
+            const int dirs = (int)wm.rec[2][e].z;
+            const int dxo = (int)r1.y, n0m = (int)r1.x;
+            const uint32_t S = r1.z;
+            const int lo_raw = (int)r0.x + ts * E3_BS;
+            const int k_lo = max(0, lo_raw), k_hi = min(dxo, lo_raw + E3_BS - 1);
+            const bool neg_major = (dirs & 2) != 0;
+            const int bn_a = minor_m((uint32_t)k_lo, S, n0m) >> E3_LOG_BS;
+            const int bn_b = minor_m((uint32_t)k_hi, S, n0m) >> E3_LOG_BS;
+            const int blk_a = (int)r0.y - m.plane_guard + ts * (int)r0.z + bn_a * (int)r0.w;
+            const uint32_t* tiles = m.bits + (size_t)(((dirs & 1) << 1) | ((dirs >> 2) & 1)) * (size_t)m.bits_var_words;
+            uint32_t A[8], B[8];
 #pragma unroll
-          for (int w = 0; w < 8; ++w) B[w] = 0;
-          ld256(A, tiles + (size_t)blk_a * 8);
-          if (bn_b != bn_a) ld256(B, tiles + (size_t)(blk_a + (int)r0.w) * 8);
-          // u_t = minor offset (walking direction) of the pixel at major position t, counted from block a's first
-          // row: 0..15 in block a, 16..31 in block b.  hi32(Y_t) = u_t - t, Y linear in t.
-          const int k0 = neg_major ? lo_raw + E3_BS - 1 : lo_raw;          // k at t = 0
-          const int c_hi = n0m - (bn_a << E3_LOG_BS);
-          const int t_lo = neg_major ? lo_raw + E3_BS - 1 - k_hi : k_lo - lo_raw;
-          const int t_hi = neg_major ? lo_raw + E3_BS - 1 - k_lo : k_hi - lo_raw;
-          const uint32_t Vm = ((2u << t_hi) - 1u) & ~((1u << t_lo) - 1u);  // positions that are pixels of this edge
-          uint32_t acc = 0;
-#if !E3_FINE_MODE
-          uint64_t Y = ((uint64_t)(uint32_t)c_hi << 32) + (uint64_t)((int64_t)k0 * (int64_t)(uint64_t)S) + E3_BIAS;
-          const uint64_t D = (neg_major ? (uint64_t)0 - (uint64_t)S : (uint64_t)S) - (1ull << 32);
-#endif
+            for (int w = 0; w < 8; ++w) B[w] = 0;
+            ld256(A, tiles + (size_t)blk_a * 8);
+            if (bn_b != bn_a) ld256(B, tiles + (size_t)(blk_a + (int)r0.w) * 8);
+            // u_t = minor offset (walking direction) of the pixel at major position t, counted from block a's first
+            // row: 0..15 in block a, 16..31 in block b.  hi32(Y_t) = u_t - t, Y linear in t.
+            const int k0 = neg_major ? lo_raw + E3_BS - 1 : lo_raw;          // k at t = 0
+            const int c_hi = n0m - (bn_a << E3_LOG_BS);
+            const int t_lo = neg_major ? lo_raw + E3_BS - 1 - k_hi : k_lo - lo_raw;
+            const int t_hi = neg_major ? lo_raw + E3_BS - 1 - k_lo : k_hi - lo_raw;
+            const uint32_t Vm = ((2u << t_hi) - 1u) & ~((1u << t_lo) - 1u);  // positions that are pixels of this edge
+            uint32_t acc = 0;
+            uint64_t Y = ((uint64_t)(uint32_t)c_hi << 32) + (uint64_t)((int64_t)k0 * (int64_t)(uint64_t)S) + E3_BIAS;
+            const uint64_t D = (neg_major ? (uint64_t)0 - (uint64_t)S : (uint64_t)S) - (1ull << 32);
 #pragma unroll
-          for (int t = 0; t < E3_BS; ++t) {
-            const uint32_t V = (t & 1) ? __byte_perm(A[t >> 1], B[t >> 1], 0x7632) : __byte_perm(A[t >> 1], B[t >> 1], 0x5410);
-#if E3_FINE_MODE
-            int kt;   // k at major position t; IMAD keeps the add off the ALU pipe
-            asm("mad.lo.s32 %0, %1, %2, %3;" : "=r"(kt) : "r"(neg_major ? -1 : 1), "r"(t), "r"(k0));
-            const int u = minor_m((uint32_t)kt, S, c_hi);               // garbage where Vm is 0
-            if (Vm & (1u << t)) acc |= (1u << u) & V;
-#else
-            const uint32_t x = Vm & (1u << t);
-            acc |= __funnelshift_l(x, x, (uint32_t)(Y >> 32)) & V;     // bit t rotated to bit u_t; hi32(Y_t) = u_t - t
-            Y += D;
-#endif
+            for (int t = 0; t < E3_BS; ++t) {
+              const uint32_t V = (t & 1) ? __byte_perm(A[t >> 1], B[t >> 1], 0x7632) : __byte_perm(A[t >> 1], B[t >> 1], 0x5410);
+              const uint32_t x = Vm & (1u << t);
+              acc |= __funnelshift_l(x, x, (uint32_t)(Y >> 32)) & V;     // bit t rotated to bit u_t; hi32(Y_t) = u_t - t
+              Y += D;
+            }
+            if (acc) wm.obst[e] = 1;
           }
-          if (acc) wm.obst[e] = 1;
         }
+        __syncwarp();
       }
-      __syncwarp();
     }
-#if E3_ITEM_QUEUE
-    }
-#endif
     // (2) strips through blocks with gray pixels: per pixel on the fused byte grid, 16 lanes per strip
     for (int q0 = 0; q0 < qg_n; q0 += 2) {
       const int q = q0 + (lane >> 4);
@@ -259,14 +229,8 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
       dirs = (major_i ? 1 : 0) | (d_major < 0 ? 2 : 0) | (d_minor < 0 ? 4 : 0);
       if (!my_flags) {  // the start pixel blocks: Obstacle at k = 0, nothing to walk (the reference returns at the first pixel)
         const int sb = m.plane_guard + ((int)ai >> E3_LOG_BS) * cw + ((int)aj >> E3_LOG_BS);
-        const uint32_t sc = plane_class<false>(smem, (uint32_t)sb);
+        const uint32_t sc = plane_class(smem, (uint32_t)sb);
         pre_blocked = sc == K_BLOCKED ? 1u : 0u;
-#if E3_START_PIXEL
-        if (sc == K_MIXED || sc == K_SPECIAL) {   // one byte of the fused grid settles the edges that start inside an obstacle
-          const uint32_t code = __ldg(m.grid + tile_addr((int)ai, (int)aj, m.tiles_x));
-          pre_blocked = (KIND == PORRT_DOMAIN_SHELF ? code != 255 : code == 0) ? 1u : 0u;
-        }
-#endif
       }
       if (!my_flags && !pre_blocked) {
         if (dxo > 0) S = slope_fixed_point(dyo, dxo);
@@ -305,14 +269,12 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
         int idx_m = (int)q0.y + ts0 * sm_;
 #pragma unroll
         for (int g = 0; g < E3_G; ++g) {
-          // only an edge's first strip starts before k = 0; k_lo past the end (masked strips) stays inside the guards.
-          // Shifts by constants are written as multiply-high so that they issue on the FMA pipe: the ALU pipe is the
-          // kernel's bound (ncu: math-pipe throttle).
+          // only an edge's first strip starts before k = 0; k_lo past the end (masked strips) stays inside the guards
           const int k_lo = g == 0 ? max(0, lo_raw) : lo_raw, k_hi = min(e_dxo, lo_raw + E3_BS - 1);
           const uint32_t na = (uint32_t)minor_m((uint32_t)k_lo, e_S, e_n0m), nb = (uint32_t)minor_m((uint32_t)k_hi, e_S, e_n0m);
-          const uint32_t ia = (uint32_t)idx_m + shr_c<E3_SHR_FMA != 0>(na, E3_LOG_BS) * (uint32_t)sn_;
-          const uint32_t ib = (uint32_t)idx_m + shr_c<E3_SHR_FMA != 0>(nb, E3_LOG_BS) * (uint32_t)sn_;
-          const uint32_t ca = plane_class<(E3_ADDR_MODE & 1) != 0>(smem, ia), cb = plane_class<(E3_ADDR_MODE & 2) != 0>(smem, ib);
+          const uint32_t ia = (uint32_t)idx_m + (na >> E3_LOG_BS) * (uint32_t)sn_;
+          const uint32_t ib = (uint32_t)idx_m + (nb >> E3_LOG_BS) * (uint32_t)sn_;
+          const uint32_t ca = plane_class(smem, ia), cb = plane_class(smem, ib);
           cls += ((1u << ca) | (1u << cb)) * (1u << (4 * g));
           lo_raw += E3_BS; idx_m += sm_;
         }
@@ -321,7 +283,6 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
       const uint32_t blocked = cls & 0x44444444u, special = (cls >> 3) & 0x11111111u;
       if (blocked) wm.obst[e] = 1;                                 // the bitmaps cannot change the outcome any more
       const uint32_t want = blocked ? 0u : ((cls >> 1) & 0x11111111u & ~special);
-#if E3_ITEM_QUEUE
       // enqueue the ITEM if any of its strips needs the bitmaps (one ballot; the strips are flattened when the queue is drained)
       {
         const unsigned bal = __ballot_sync(0xffffffffu, want != 0);
@@ -334,24 +295,6 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
           qb_n += __popc(bal);
         }
       }
-#else
-      // enqueue the strips that need the bitmaps: exclusive scan of the per-lane counts
-      if (__any_sync(0xffffffffu, want != 0)) {
-        const int cnt = __popc(want);
-        int sc = cnt;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-          const int t = __shfl_up_sync(0xffffffffu, sc, o);
-          if (lane >= o) sc += t;
-        }
-        int pb = qb_n + sc - cnt;
-        qb_n += __shfl_sync(0xffffffffu, sc, 31);
-        const uint32_t ent0 = (uint32_t)e | ((uint32_t)ts0 << 5);
-#pragma unroll
-        for (int g = 0; g < E3_G; ++g)
-          if (want & (1u << (4 * g))) wm.qb[pb++] = ent0 + ((uint32_t)g << 5);
-      }
-#endif
       if (__any_sync(0xffffffffu, special != 0)) {                 // rare: strips through gray pixels
 #pragma unroll
         for (int g = 0; g < E3_G; ++g) {
@@ -361,19 +304,13 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
         }
       }
     };
-#if E3_TWO_PHASE
     // Round 0: every lane takes the FIRST item of its own edge (no owner search).  Edges found blocked there -- an
-    // all-blocking block within their first 128 pixels -- are finished: what lies behind the first obstacle cannot
-    // change the result (the reference returns at it), so their remaining items are never looked at.
-    const bool may_overflow = true;
+    // all-blocking block within their first 112 pixels -- are finished: what lies behind the first obstacle cannot
+    // change the result (the reference returns at it), so their remaining items are never looked at.  The queues are not
+    // drained between the two phases: that lets more edges finish early but costs more than it saves (0.905 against 0.760 ms).
     __syncwarp();
     process_item(lane, 0, my_items > 0);
     __syncwarp();
-#if E3_TWO_PHASE == 2
-    // resolving the first items' bitmaps now lets more edges finish early, but the extra, half-empty drain costs more than
-    // it saves: measured 0.905 ms against 0.760 ms
-    if (__any_sync(0xffffffffu, my_items > 1) && (qb_n | qg_n)) drain();
-#endif
     int rem = (my_items <= 1 || wm.obst[lane] != 0) ? 0 : my_items - 1;
     int incl = rem;
 #pragma unroll
@@ -383,7 +320,7 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
     }
     const int total = __shfl_sync(0xffffffffu, incl, 31);
     for (int w0 = 0; w0 < total; w0 += 32) {
-      if (may_overflow && (qb_n > E3_QB_LIMIT || qg_n > E3_QG - 32 * E3_G)) drain();
+      if (qb_n > E3_QB_LIMIT || qg_n > E3_QG - 32 * E3_G) drain();
       const int w = w0 + lane;
       int e = 0;                                                    // owner: the first lane whose inclusive sum exceeds w
 #pragma unroll
@@ -395,29 +332,6 @@ edge_validity_v3_kernel(MapDev m, const double2* __restrict__ from, const double
       process_item(e, 1 + w - excl, w < total);
       __syncwarp();
     }
-#else
-    // every lane owns at least one (possibly empty) item so that the inclusive prefix sums are strictly increasing and the
-    // owner of a flattened position can be ranked with a bitmask
-    int incl = max(1, my_items);
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-      const int t = __shfl_up_sync(0xffffffffu, incl, o);
-      if (lane >= o) incl += t;
-    }
-    const int total = __shfl_sync(0xffffffffu, incl, 31);
-    const bool may_overflow = total * E3_G > min(E3_QB, E3_QG);     // warp-uniform
-    __syncwarp();
-    for (int w0 = 0; w0 < total; w0 += 32) {
-      if (may_overflow && (qb_n > E3_QB_LIMIT || qg_n > E3_QG - 32 * E3_G)) drain();
-      const int d = incl - w0;                                    // edge `lane` ends before window position d
-      const int e_base = __popc(__ballot_sync(0xffffffffu, d <= 0));
-      const unsigned marks = __reduce_or_sync(0xffffffffu, (d >= 1 && d <= 32) ? (1u << (d - 1)) : 0u);
-      const int e = min(31, e_base + __popc(marks & lt_mask));
-      const int p_prev = __shfl_sync(0xffffffffu, incl, (e + 31) & 31);
-      process_item(e, w0 + lane - (e ? p_prev : 0), w0 + lane < total);
-      __syncwarp();
-    }
-#endif
     // ---- pass 2: bitmaps / pixels of the strips that are still undecided
     if (qb_n | qg_n) drain();
     __syncwarp();

@@ -2,42 +2,16 @@
 #pragma once
 #include "map_dev.cuh"
 
-#ifndef E3_SHR_FMA
-#define E3_SHR_FMA 0       // measured: moving the shifts to IMAD.HI loses 2-4 % (the FMA-heavy pipe is as narrow as the ALU pipe)
-#endif
-#ifndef E3_ADDR_MODE
-#define E3_ADDR_MODE 0      // bit0 / bit1: first / second class lookup of a strip uses word loads + rotate
-#endif
-#ifndef E3_FINE_MODE
-#define E3_FINE_MODE 0       // 1: per-pixel IMAD.HI instead of the 64-bit running sum (slower, same reason)
-#endif
-#ifndef E3_START_PIXEL
-#define E3_START_PIXEL 0     // byte look-up of the start pixel in mixed blocks: measured 0.729 ms against 0.710 ms without (scattered load in the set-up)
-#endif
-#ifndef E3_TWO_PHASE
-#define E3_TWO_PHASE 1     // first item of every edge by its own lane, remaining items only for edges not yet blocked
-#endif
 #define E3_LOG_BS 4
 #define E3_BS 16
-#ifndef E3_G
-#define E3_G 7              // consecutive strips of one edge per lane and round (<= 8: one class nibble each); measured with the
+#define E3_G 7              // consecutive strips of one edge per item (<= 8: one class nibble each); measured with the
                             // two-phase pass 1 on c5: G = 4 / 5 / 6 / 7 / 8 -> 0.768 / 0.754 / 0.721 / 0.710 / 0.760 ms
-#endif
-#define E3_QB 512           // bitmap-queue entries per warp (a round adds at most 32 * E3_G)
+#define E3_QB 512           // bitmap-queue words per warp: items, then the strip scratch they are flattened into
 #define E3_QG 256           // byte-queue entries per warp
-#ifndef E3_ITEM_QUEUE
-#define E3_ITEM_QUEUE 1     // the bitmap queue holds items (edge, first strip, strip mask) and is flattened when drained
-#endif
 #define E3_QI ((E3_QB - 32 * 8) / 2)          // item entries (2 words each) in front of the strip scratch (32 items x 8 strips)
-#if E3_ITEM_QUEUE
 #define E3_QB_LIMIT (E3_QI - 32)              // items; a round adds at most 32
-#else
-#define E3_QB_LIMIT (E3_QB - 32 * E3_G)       // strips; a round adds at most 32 * E3_G
-#endif
 #define E3_BIAS 65536ull
-#ifndef E3_MAX_WARPS
 #define E3_MAX_WARPS 32
-#endif
 
 #define K_FREE 0u
 #define K_MIXED 1u          // blocking and free pixels, nothing else: the bitmap decides
@@ -47,20 +21,10 @@
 // Fixed-point slope S ~ dy * 2^32 / dx for 0 <= dy <= dx < 2^15.  hi32(k * S + 2^16) == floor(k * dy / dx) for every
 // 0 <= k <= dx as long as |dy * 2^32 / dx - S| < 1.9 (DESIGN.md 3.1), so S need not be the exact floor: one correctly
 // rounded reciprocal, one multiply and a saturating conversion (dy == dx -> 2^32 - 1) on the FP64 pipe replace two 32-bit
-// integer divisions (~40 ALU/FMA instructions, the pipes that bound the kernel).  E3_SLOPE_DIV = 1 keeps the divisions.
-// tests/test_oracle_golden.py::test_fixed_point_minor_offset_is_exact replays both variants in IEEE arithmetic.
-#ifndef E3_SLOPE_DIV
-#define E3_SLOPE_DIV 0
-#endif
+// integer divisions (~40 ALU/FMA instructions, the pipes that bound the kernel).
+// tests/test_oracle_golden.py::test_fixed_point_minor_offset_is_exact replays this and the exact division in IEEE arithmetic.
 __device__ __forceinline__ uint32_t slope_fixed_point(int dy, int dx) {
-#if E3_SLOPE_DIV
-  if (dy == dx) return 0xFFFFFFFFu;
-  const uint32_t d = (uint32_t)dx, num = (uint32_t)dy << 16;
-  const uint32_t q1 = num / d, r1 = num - q1 * d;
-  return (q1 << 16) + ((r1 << 16) / d);
-#else
   return __double2uint_rz(__dmul_rn(__dmul_rn((double)dy, 4294967296.0), __drcp_rn((double)dx)));
-#endif
 }
 
 // n' of pixel k = hi32(k * S + (n0m << 32 | 2^16))
@@ -69,18 +33,9 @@ __device__ __forceinline__ int32_t minor_m(uint32_t k, uint32_t S, int32_t n0m) 
 }
 
 
-// x >> s for a compile-time s, on the ALU pipe (SHF) or the FMA pipe (IMAD.HI): the kernel is bound by integer issue on
-// these two pipes, so the split between them is tuned (E3_* switches, measured on B200; DESIGN.md 3.1)
-template <bool FMA>
-__device__ __forceinline__ uint32_t shr_c(uint32_t x, int s) { return FMA ? __umulhi(x, 1u << (32 - s)) : x >> s; }
-
-// 2-bit class of block idx from the plane in shared memory (16 per 32-bit word)
-template <bool WORD>
+// 2-bit class of block idx from the plane in shared memory (16 per 32-bit word) by a byte load; word loads with a rotate
+// were measured slower (DESIGN.md 3.1)
 __device__ __forceinline__ uint32_t plane_class(const unsigned char* plane, uint32_t idx) {
-  if (WORD) {
-    const uint32_t w = ((const uint32_t*)plane)[__umulhi(idx, 1u << 28)];
-    return __funnelshift_r(w, w, idx * 2u) & 3u;           // rotate by 2 * idx mod 32
-  }
   return ((uint32_t)plane[idx >> 2] >> ((idx * 2u) & 6u)) & 3u;
 }
 

@@ -459,7 +459,6 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
   if (!radii_cached) {
     ctx->radii_n = 0;
     int nt = (int)std::min<int64_t>(std::max(2u, std::thread::hardware_concurrency()) / 2, 8);   // leave cores to the driver's copies
-    if (const char* v = getenv("PORRT_PRM_RADII_THREADS")) { const int k = atoi(v); if (k >= 1 && k <= 64) nt = k; }
     if (world > 1) nt = std::max(1, nt / world + 1);                                                // the box's cores are shared by all ranks
     if (m < 20000) nt = 1;
     for (int t = 0; t < nt; ++t)

@@ -10,12 +10,10 @@
 //   DOOR : 255 free | 0 obstacle | 1..253 zone id + 1 | 254 gray pixel without zone id (reference panics)
 //   SHELF: the raw gray value (class = 255 free, 127..254 low obstacle, 0..126 high obstacle)
 //
-// Kernel shape (edge validity): a warp takes 32 edges, every lane sets up one of them (pixel endpoints, octant,
-// exact-division magic), then the warp walks the 32 edges one after the other with its lanes striding the
-// Bresenham parameter k (pixel k of the line in closed form, A5), four 32-pixel chunks in flight per lane,
-// and reduces each chunk with __ballot_sync / __reduce_min_sync / __reduce_max_sync.
-#include <cstdlib>
-
+// This file holds the map upload (fused grid, zone positions, world validities, and the class data of both edge kernels),
+// the state-validity and visibility kernels, the large-map edge kernel (class bytes in global memory, for maps whose class
+// plane does not fit in shared memory; the product's edge kernel is edge3.cu), the dispatch between the two edge kernels,
+// and the chunked host-buffer pipeline behind every host-array edge entry point.
 #include "common.cuh"
 #include "map_dev.cuh"
 
@@ -97,8 +95,7 @@ __device__ __forceinline__ int32_t rec_minor(const EdgeRec& r, int32_t k) {
 #define V2_QCAP 512  // queue entries per warp
 #define V2_MINB 4
 
-// V2_G: consecutive strips of one edge handled by a lane per round (amortises the owner search)
-template <int KIND, int LOG_BS, int V2_G, bool INDEXED>
+template <int KIND, bool INDEXED>
 __global__ void __launch_bounds__(EDGE_BLOCK, V2_MINB) edge_validity_v2_kernel(MapDev m, const double2* __restrict__ from,
                                                                       const double2* __restrict__ to, int64_t n,
                                                                       int32_t* __restrict__ out_vid,
@@ -107,7 +104,9 @@ __global__ void __launch_bounds__(EDGE_BLOCK, V2_MINB) edge_validity_v2_kernel(M
                                                                       const uint64_t* __restrict__ validities,
                                                                       const int32_t* __restrict__ from_idx,
                                                                       const int32_t* __restrict__ to_idx) {
+  constexpr int LOG_BS = 4;   // the class bytes are built for 16 x 16 blocks
   constexpr int BS = 1 << LOG_BS;
+  constexpr int V2_G = 4;     // consecutive strips of one edge handled by a lane per round (amortises the owner search)
   constexpr int WARPS = EDGE_BLOCK / 32;
   __shared__ EdgeRec s_rec[WARPS][32];
   __shared__ uint32_t s_flags[WARPS][32];     // F_* per edge
@@ -115,7 +114,6 @@ __global__ void __launch_bounds__(EDGE_BLOCK, V2_MINB) edge_validity_v2_kernel(M
   __shared__ uint32_t s_queue[WARPS][V2_QCAP];
   __shared__ int32_t s_qcount[WARPS];
   const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  static_assert(LOG_BS == 4, "the class bytes are built for 16 x 16 blocks");
   const uint8_t* __restrict__ coarse = m.coarse;
   const int cw = m.coarse_cw;
   const int64_t warp = ((int64_t)blockIdx.x * EDGE_BLOCK + threadIdx.x) >> 5;
@@ -529,7 +527,7 @@ int32_t map_edge_launch(porrt_ctx* ctx, const double* from_dev, const double* to
   const uint64_t* val = ctx->d_validities.as<uint64_t>();
   const int grid = edge_grid(ctx, n);
   const bool shelf = ctx->map.kind == PORRT_DOMAIN_SHELF;
-#define LAUNCH_LARGE(K, I) edge_validity_v2_kernel<K, 4, 4, I><<<grid, EDGE_BLOCK, 0, st>>>(ctx->map, from, to, n, out.vid, out.vid8, out.mask, val, from_idx, to_idx)
+#define LAUNCH_LARGE(K, I) edge_validity_v2_kernel<K, I><<<grid, EDGE_BLOCK, 0, st>>>(ctx->map, from, to, n, out.vid, out.vid8, out.mask, val, from_idx, to_idx)
   if (from_idx) { if (shelf) LAUNCH_LARGE(PORRT_DOMAIN_SHELF, true); else LAUNCH_LARGE(PORRT_DOMAIN_DOOR, true); }
   else { if (shelf) LAUNCH_LARGE(PORRT_DOMAIN_SHELF, false); else LAUNCH_LARGE(PORRT_DOMAIN_DOOR, false); }
 #undef LAUNCH_LARGE
@@ -554,6 +552,7 @@ PORRT_API int32_t porrt_ctx_set_option(porrt_ctx* ctx, int32_t option, int64_t v
   switch (option) {
     case PORRT_OPT_FORCE_LARGE_MAP_PATH: ctx->force_large_map_path = value != 0; return PORRT_OK;
     case PORRT_OPT_FORCE_GLOBAL_SWEEPS: ctx->force_global_sweeps = value != 0; return PORRT_OK;
+    case PORRT_OPT_FORCE_THREAD_PER_QUERY_NN: ctx->force_thread_per_query_nn = value != 0; return PORRT_OK;
     default: return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_ctx_set_option: unknown option");
   }
 }
@@ -624,7 +623,6 @@ static int32_t edge_pipeline(porrt_ctx* ctx, const EdgeJob& job, int64_t n) {
   int64_t CH = n / 8;
   const int64_t ch_lo = ((int64_t)1 << 18) * scale, ch_hi = ((int64_t)1 << 21) * scale;
   CH = CH < ch_lo ? ch_lo : (CH > ch_hi ? ch_hi : CH);
-  if (const char* v = getenv("PORRT_EDGE_CHUNK_LOG2")) { const int l = atoi(v); if (l >= 10 && l <= 26) CH = (int64_t)1 << l; }
   const int64_t ch = n < CH ? n : CH;
   bool pinned = is_pinned_host(job.in[0]) && (job.n_in < 2 || is_pinned_host(job.in[1])) &&
                 is_pinned_host(job.out_vid8 ? (const void*)job.out_vid8 : (const void*)job.out_vid) &&

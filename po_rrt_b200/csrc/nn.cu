@@ -663,54 +663,11 @@ __global__ void copy_u32_i32_kernel(const uint32_t* __restrict__ in, int64_t n, 
   if (i < n) out[i] = (int32_t)in[i];
 }
 
-// Fast path: one warp sorts one segment in shared memory (bitonic network on (key, id) pairs, <= SEG_SORT_CAP entries).
-// Keys are distinct inside a segment (ids are distinct and ranks are a permutation), so no stability concern arises.
-#define SEG_SORT_CAP 256
-#define SEG_SORT_WARPS 4
-__global__ void __launch_bounds__(SEG_SORT_WARPS * 32) seg_sort_small_kernel(const int64_t* __restrict__ offsets, int64_t m, int32_t* __restrict__ ids,
-                                                                             const int32_t* __restrict__ key_of_id, int32_t* __restrict__ n_big,
-                                                                             int min_len /* shorter segments are already sorted */) {
-  __shared__ uint64_t s_kv[SEG_SORT_WARPS][SEG_SORT_CAP];
-  const int lane = threadIdx.x & 31, wib = threadIdx.x >> 5;
-  const int64_t seg = (int64_t)blockIdx.x * SEG_SORT_WARPS + wib;
-  if (seg >= m) return;
-  const int64_t s = offsets[seg];
-  const int len = (int)min((int64_t)0x7fffffff, offsets[seg + 1] - s);
-  if (len < min_len) return;
-  if (len > SEG_SORT_CAP) { if (lane == 0) atomicAdd(n_big, 1); return; }
-  int np2 = 2;
-  while (np2 < len) np2 <<= 1;
-  uint64_t* kv = s_kv[wib];
-  for (int i = lane; i < np2; i += 32) {
-    uint64_t v = ~0ull;
-    if (i < len) {
-      const int32_t id = ids[s + i];
-      const uint32_t key = key_of_id ? (uint32_t)key_of_id[id] : (uint32_t)id;
-      v = ((uint64_t)key << 32) | (uint32_t)id;
-    }
-    kv[i] = v;
-  }
-  __syncwarp();
-  for (int k = 2; k <= np2; k <<= 1)
-    for (int j = k >> 1; j > 0; j >>= 1) {
-      for (int t = lane; t < (np2 >> 1); t += 32) {
-        const int i = ((t & ~(j - 1)) << 1) | (t & (j - 1));  // index with bit j cleared
-        const int p = i | j;
-        const uint64_t a = kv[i], b = kv[p];
-        const bool up = (i & k) == 0;
-        if ((a > b) == up) { kv[i] = b; kv[p] = a; }
-      }
-      __syncwarp();
-    }
-  for (int i = lane; i < len; i += 32) ids[s + i] = (int32_t)(uint32_t)kv[i];
-}
-
 // Register path for the common case (<= 256 entries; a radius query at the c5 shape returns ~43): one warp per segment, R
 // 32-bit values per lane (element i = r * 32 + lane), bitonic network by __shfl_xor (partner in another lane) or a register
 // swap (partner in the same lane); no shared memory, no barriers.  Sorting values are the ids themselves, or -- BY_KEY --
 // the keys key_of_id[id], which must then be a permutation of 0..key_limit-1 (kd pre-order ranks are): the sorted keys are
-// mapped back through id_of_key.  Longer segments are counted in n_big (global radix sort); the shared-memory network above
-// remains as the A/B variant (PORRT_SEGSORT_NO_REGS).
+// mapped back through id_of_key.  Longer segments go to seg_sort_mid_kernel or are counted for the global radix sort.
 template <int R>
 __device__ __forceinline__ void warp_bitonic_u32(uint32_t (&v)[R], int lane, int np2) {
 #pragma unroll
@@ -846,41 +803,33 @@ int32_t segments_sort_by_key_dev(porrt_ctx* ctx, const int64_t* offsets_dev, int
   cudaStream_t st = ctx->stream;
   if (m <= 0 || (seg_list_dev && n_listed <= 0)) return PORRT_OK;
   const int64_t m_run = seg_list_dev ? n_listed : m;
-  static const bool no_regs = getenv("PORRT_SEGSORT_NO_REGS") != nullptr;   // A/B switch: shared-memory network for everything
   CUDA_TRY(ctx, ctx->scratch[4].ensure(16 + (size_t)m * 4 + (key_of_id_dev ? (size_t)key_limit * 4 : 0)));
   int32_t* d_big = ctx->scratch[4].as<int32_t>();   // [0] n_mid (257..4096, listed), [1] n_big (longer)
   int32_t* d_mid_list = d_big + 4;
   int32_t* d_inv = d_mid_list + m;
   CUDA_TRY(ctx, cudaMemsetAsync(d_big, 0, 8, st));
-  int32_t n_mid = 0, n_big = 0;
-  int64_t total = 0;
-  if (!no_regs) {
-    if (key_of_id_dev) {
-      invert_perm_kernel<<<div_up(key_limit, 256), 256, 0, st>>>(key_of_id_dev, key_limit, d_inv);
-      LAUNCH_CHECK(ctx);
-      seg_sort_reg_kernel<true><<<div_up(m_run, SEG_REG_WARPS), SEG_REG_WARPS * 32, 0, st>>>(offsets_dev, m_run, ids_dev, key_of_id_dev, d_inv, d_big, d_mid_list, seg_list_dev);
-    } else {
-      seg_sort_reg_kernel<false><<<div_up(m_run, SEG_REG_WARPS), SEG_REG_WARPS * 32, 0, st>>>(offsets_dev, m_run, ids_dev, nullptr, nullptr, d_big, d_mid_list, seg_list_dev);
-    }
+  if (key_of_id_dev) {
+    invert_perm_kernel<<<div_up(key_limit, 256), 256, 0, st>>>(key_of_id_dev, key_limit, d_inv);
     LAUNCH_CHECK(ctx);
-    int32_t cnt[2] = {0, 0};
-    { const int32_t rcf = read_flags_dev(ctx, d_big, 2, cnt, st); if (rcf) return rcf; }
-    n_mid = cnt[0]; n_big = cnt[1];
-    if (n_mid > 0 && n_big == 0) {
-      if (key_of_id_dev) seg_sort_mid_kernel<true><<<n_mid, 256, 0, st>>>(offsets_dev, d_mid_list, ids_dev, key_of_id_dev, d_inv);
-      else seg_sort_mid_kernel<false><<<n_mid, 256, 0, st>>>(offsets_dev, d_mid_list, ids_dev, nullptr, nullptr);
-      LAUNCH_CHECK(ctx);
-    }
-    if (n_big == 0) return PORRT_OK;
+    seg_sort_reg_kernel<true><<<div_up(m_run, SEG_REG_WARPS), SEG_REG_WARPS * 32, 0, st>>>(offsets_dev, m_run, ids_dev, key_of_id_dev, d_inv, d_big, d_mid_list, seg_list_dev);
   } else {
-    seg_sort_small_kernel<<<div_up(m, SEG_SORT_WARPS), SEG_SORT_WARPS * 32, 0, st>>>(offsets_dev, m, ids_dev, key_of_id_dev, d_big + 1, 2);
-    LAUNCH_CHECK(ctx);
-    CUDA_TRY(ctx, cudaMemcpyAsync(&n_big, d_big + 1, 4, cudaMemcpyDeviceToHost, st));
+    seg_sort_reg_kernel<false><<<div_up(m_run, SEG_REG_WARPS), SEG_REG_WARPS * 32, 0, st>>>(offsets_dev, m_run, ids_dev, nullptr, nullptr, d_big, d_mid_list, seg_list_dev);
   }
+  LAUNCH_CHECK(ctx);
+  int32_t cnt[2] = {0, 0};
+  { const int32_t rcf = read_flags_dev(ctx, d_big, 2, cnt, st); if (rcf) return rcf; }
+  const int32_t n_mid = cnt[0], n_big = cnt[1];
+  if (n_mid > 0 && n_big == 0) {
+    if (key_of_id_dev) seg_sort_mid_kernel<true><<<n_mid, 256, 0, st>>>(offsets_dev, d_mid_list, ids_dev, key_of_id_dev, d_inv);
+    else seg_sort_mid_kernel<false><<<n_mid, 256, 0, st>>>(offsets_dev, d_mid_list, ids_dev, nullptr, nullptr);
+    LAUNCH_CHECK(ctx);
+  }
+  if (n_big == 0) return PORRT_OK;
+  int64_t total = 0;
   CUDA_TRY(ctx, cudaMemcpyAsync(&total, offsets_dev + m, 8, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
-  if (n_big == 0 || total <= 1) return PORRT_OK;
-  // some segment exceeds the shared-memory network: one global stable LSD radix sort on (segment, key) orders them all
+  if (total <= 1) return PORRT_OK;
+  // some segment is longer than SEG_MID_CAP: one global stable LSD radix sort on (segment, key) orders them all
   const int key_bits = bits_for((uint64_t)(key_limit > 1 ? key_limit - 1 : 1));
   const int seg_bits = bits_for((uint64_t)(m > 1 ? m - 1 : 1));
   // (scratch 5 / 6 here, 8..10 inside radix_sort_pairs: callers keep their segment data elsewhere)

@@ -149,26 +149,21 @@ __device__ __forceinline__ void tile_stage(const GridDev& g, const Tile& T, doub
 //   C  warp per 32 queries: one atomicAdd reserves the warp's slots of a staging buffer, then the lanes write each query's ids
 //      side by side (128-byte lines instead of 32 partial sectors per store).
 // A second, pure copy kernel moves the lists to their CSR places once the global scan of the counts is known.
-// The kernel is persistent (as many CTAs as fit an SM, each striding over the tiles).  The tile staging can be double-buffered
-// (NR_BUFS = 2: while the CTA works on tile i the bulk-async copies of tile i + 1 are in flight into the other buffer, two
-// mbarriers, byte-count completion) -- measured against ONE buffer with two more resident CTAs per SM, the latter wins (see NR_BUFS).
+// The kernel is persistent (as many CTAs as fit an SM, each striding over the tiles) and stages each tile into ONE buffer: 37 KiB,
+// 6 CTAs per SM whose other warps cover the copy, 0.545 ms for the whole query at V = Q = 1e6.  Double-buffered (the next tile's
+// bulk copies in flight on a second mbarrier) it needs 55 KiB, fits 4 CTAs per SM and takes 0.58 ms; one buffer with 5 CTAs per
+// SM 0.57-0.60 ms (interleaved A/B on one box).  More resident warps beat the explicit prefetch here.
 // Queries whose list would not fit (> NR_LCAP hits), cells with more than NR_CCAP candidates, tiles too dense to stage and warps
 // that find the staging buffer full are appended to the fallback list and answered by nn.cu's thread-per-query kernels -- same
 // bits, only slower.
 #define NR_THREADS 128
-#ifndef NR_CAP
-#define NR_CAP 704           // staged vertices per tile and buffer: 11 KiB + 3 KiB ids (c5 shape: ~440 per tile)
+#define NR_CAP 704           // staged vertices per tile: 11 KiB + 3 KiB ids (c5 shape: ~440 per tile)
 #define NR_CCAP 176          // merged candidates per query cell (3 x 3 cells; c5 shape: 131 +- 11)
 #define NR_LCAP 80           // hits per query kept in the thread's row
 #define NR_LSTRIDE 84        // bytes per row (list positions fit a byte): 21 words, odd -> the lanes' rows fall into different banks
 #define NR_CTAS_PER_SM 6
-// staging buffers per CTA.  2 = the next tile's bulk copies fly while this one is worked on (two mbarriers): 55 KiB, 4 CTAs per SM,
-// 0.58 ms for the whole query at V = Q = 1e6.  1 = one buffer, 37 KiB, 6 CTAs per SM whose other warps cover the copy: 0.545 ms
-// (interleaved A/B on one box; 5 CTAs with one buffer: 0.57-0.60).  More resident warps beat the explicit prefetch here.
-#define NR_BUFS 1
-#endif
 #define NR_RUNS 9
-#define NR_SMEM (NR_BUFS * (NR_CAP * 16 + (NR_CAP + 24) * 4 + NT_W * NR_CCAP * 2) + NT_W * NR_CCAP * 6 + NR_THREADS * NR_LSTRIDE)
+#define NR_SMEM (NR_CAP * 16 + (NR_CAP + 24) * 4 + NT_W * NR_CCAP * 2 + NT_W * NR_CCAP * 6 + NR_THREADS * NR_LSTRIDE)
 
 __device__ __forceinline__ void nt_mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(nt_smem_u32(bar)) : "memory");
@@ -277,25 +272,22 @@ __global__ void __launch_bounds__(NR_THREADS) nt_radius_collect_kernel(
     int n_tiles, int32_t* __restrict__ counts, int64_t* __restrict__ stg_off, int32_t* __restrict__ staging,
     unsigned long long* __restrict__ stg_cursor, int64_t stg_cap, int32_t* __restrict__ fb_list, int32_t* __restrict__ fb_n) {
   extern __shared__ __align__(128) unsigned char nr_smem[];
-  double2* const s_xy0 = (double2*)nr_smem;                    // two staging buffers: coordinates | ids | merge scripts
-  double2* const s_xy1 = NR_BUFS == 2 ? s_xy0 + NR_CAP : s_xy0;
-  int32_t* const s_id0 = (int32_t*)(s_xy1 + NR_CAP);
-  int32_t* const s_id1 = NR_BUFS == 2 ? s_id0 + NR_CAP + 24 : s_id0;
-  uint16_t* const s_sc0 = (uint16_t*)(s_id1 + NR_CAP + 24);
-  uint16_t* const s_sc1 = NR_BUFS == 2 ? s_sc0 + NT_W * NR_CCAP : s_sc0;
-  int32_t* s_cid = (int32_t*)(s_sc1 + NT_W * NR_CCAP);         // [NT_W][NR_CCAP] merged candidate ids ...
+  double2* const s_xy = (double2*)nr_smem;                     // the staging buffer: coordinates | ids | merge scripts
+  int32_t* const s_id = (int32_t*)(s_xy + NR_CAP);
+  uint16_t* const s_sc = (uint16_t*)(s_id + NR_CAP + 24);
+  int32_t* s_cid = (int32_t*)(s_sc + NT_W * NR_CCAP);          // [NT_W][NR_CCAP] merged candidate ids ...
   uint16_t* s_cxy = (uint16_t*)(s_cid + NT_W * NR_CCAP);       // [NT_W][NR_CCAP] ... and where their coordinates are staged
   uint8_t* s_lst = (uint8_t*)(s_cxy + NT_W * NR_CCAP);         // [NR_THREADS][NR_LSTRIDE] list positions of a query's hits
-  __shared__ uint64_t s_bar[2];
+  __shared__ uint64_t s_bar;
   __shared__ NrRun s_run[NT_W][NR_RUNS];
   __shared__ int32_t s_ccnt[NT_W];                             // merged candidates of a query cell; -1: no script (fallback)
   __shared__ int32_t s_coff[NT_W + 1];                         // where the cells' scripts start in the staged script range
   const int tid = threadIdx.x, lane = tid & 31;
-  if (tid == 0) { nt_mbar_init(&s_bar[0]); nt_mbar_init(&s_bar[1]); }
+  if (tid == 0) nt_mbar_init(&s_bar);
   __syncthreads();
   uint8_t* lst = s_lst + tid * NR_LSTRIDE;
-  // thread 0: one phase of `bar` per tile -- the bulk copies of the tile's three vertex ranges and of its cells' scripts
-  auto stage = [&](const Tile& T, double2* d_xy, int32_t* d_id, uint16_t* d_sc, uint64_t* bar) {
+  // thread 0: one phase of s_bar per tile -- the bulk copies of the tile's three vertex ranges and of its cells' scripts
+  auto stage = [&](const Tile& T) {
     uint32_t bytes = 0, sc_bytes = 0;
     const int64_t ca = (int64_t)T.cy * g.cells_x + T.cxa, cb = (int64_t)T.cy * g.cells_x + T.cxb;
     if (T.staged && T.nq > 0) {
@@ -303,37 +295,21 @@ __global__ void __launch_bounds__(NR_THREADS) nt_radius_collect_kernel(
         if (T.len[r] > 0) bytes += (uint32_t)T.len[r] * 16u + (uint32_t)((((int)(T.k0[r] & 3) + T.len[r] + 3) & ~3) * 4);
       sc_bytes = (uint32_t)(nbr_start[cb + 1] - nbr_start[ca]) * 2u;
     }
-    if (bytes == 0) { nt_mbar_arrive(bar); return; }
-    nt_mbar_expect(bar, bytes + sc_bytes);
+    if (bytes == 0) { nt_mbar_arrive(&s_bar); return; }
+    nt_mbar_expect(&s_bar, bytes + sc_bytes);
     for (int r = 0; r < 3; ++r)
       if (T.len[r] > 0) {
-        nt_bulk_g2s(d_xy + T.xoff[r], g.vxy + T.k0[r], (uint32_t)T.len[r] * 16u, bar);
+        nt_bulk_g2s(s_xy + T.xoff[r], g.vxy + T.k0[r], (uint32_t)T.len[r] * 16u, &s_bar);
         const int ph = (int)(T.k0[r] & 3);
-        nt_bulk_g2s(d_id + T.ioff[r] - ph, g.vid + (T.k0[r] - ph), (uint32_t)(((ph + T.len[r] + 3) & ~3) * 4), bar);
+        nt_bulk_g2s(s_id + T.ioff[r] - ph, g.vid + (T.k0[r] - ph), (uint32_t)(((ph + T.len[r] + 3) & ~3) * 4), &s_bar);
       }
-    if (sc_bytes) nt_bulk_g2s(d_sc, script + nbr_start[ca], sc_bytes, bar);
+    if (sc_bytes) nt_bulk_g2s(s_sc, script + nbr_start[ca], sc_bytes, &s_bar);
   };
   int it = 0;
-  if (NR_BUFS == 2 && tid == 0 && (int)blockIdx.x < n_tiles) {
-    const Tile T0 = tile_setup_at(g, qstart, tiles_per_row, NR_CAP, blockIdx.x);
-    stage(T0, s_xy0, s_id0, s_sc0, &s_bar[0]);
-  }
   for (int tile = blockIdx.x; tile < n_tiles; tile += gridDim.x, ++it) {
-    const int buf = NR_BUFS == 2 ? (it & 1) : 0;
     const Tile T = tile_setup_at(g, qstart, tiles_per_row, NR_CAP, tile);
-    if (NR_BUFS == 2) {
-      if (tid == 0 && tile + (int)gridDim.x < n_tiles) {   // prefetch the next tile into the other buffer (free since the last barrier)
-        const Tile Tn = tile_setup_at(g, qstart, tiles_per_row, NR_CAP, tile + gridDim.x);
-        stage(Tn, buf ? s_xy0 : s_xy1, buf ? s_id0 : s_id1, buf ? s_sc0 : s_sc1, &s_bar[buf ^ 1]);
-      }
-      nt_mbar_wait(&s_bar[buf], (uint32_t)((it >> 1) & 1));
-    } else {                                               // one buffer: the other resident CTAs cover the copy
-      if (tid == 0) stage(T, s_xy0, s_id0, s_sc0, &s_bar[0]);
-      nt_mbar_wait(&s_bar[0], (uint32_t)(it & 1));
-    }
-    const double2* xy = buf ? s_xy1 : s_xy0;
-    const int32_t* sid = buf ? s_id1 : s_id0;
-    const uint16_t* ssc = buf ? s_sc1 : s_sc0;
+    if (tid == 0) stage(T);
+    nt_mbar_wait(&s_bar, (uint32_t)(it & 1));
     const int n_qc = (T.nq > 0 && T.staged) ? T.cxb - T.cxa + 1 : 0;
     // ---- S: the nine runs of every query cell, then its merged candidate list by the cell's script
     if (tid < n_qc * NR_RUNS) {
@@ -363,12 +339,12 @@ __global__ void __launch_bounds__(NR_THREADS) nt_radius_collect_kernel(
     __syncthreads();
     for (int qc = 0; qc < n_qc; ++qc) {
       const int n_c = s_ccnt[qc];
-      const uint16_t* sc = ssc + s_coff[qc];
+      const uint16_t* sc = s_sc + s_coff[qc];
       for (int e = tid; e < n_c; e += NR_THREADS) {
         const uint32_t code = sc[e];
         const NrRun R = s_run[qc][code >> 12];
         const int pos = (int)(code & 0xfffu);
-        s_cid[qc * NR_CCAP + e] = sid[R.id0 + pos];
+        s_cid[qc * NR_CCAP + e] = s_id[R.id0 + pos];
         s_cxy[qc * NR_CCAP + e] = (uint16_t)(R.xy0 + pos);
       }
     }
@@ -399,16 +375,16 @@ __global__ void __launch_bounds__(NR_THREADS) nt_radius_collect_kernel(
           int j = 0;
           if (!reach) {
             for (; j + 4 <= n_c; j += 4) {
-              const double d0 = dist2(xy[cxy[j]], p.x, p.y), d1 = dist2(xy[cxy[j + 1]], p.x, p.y);
-              const double d2 = dist2(xy[cxy[j + 2]], p.x, p.y), d3 = dist2(xy[cxy[j + 3]], p.x, p.y);
+              const double d0 = dist2(s_xy[cxy[j]], p.x, p.y), d1 = dist2(s_xy[cxy[j + 1]], p.x, p.y);
+              const double d2 = dist2(s_xy[cxy[j + 2]], p.x, p.y), d3 = dist2(s_xy[cxy[j + 3]], p.x, p.y);
               const uint32_t i0 = (uint32_t)cid[j], i1 = (uint32_t)cid[j + 1], i2 = (uint32_t)cid[j + 2], i3 = (uint32_t)cid[j + 3];
               take(j, d0 <= Tr && i0 < limit); take(j + 1, d1 <= Tr && i1 < limit);
               take(j + 2, d2 <= Tr && i2 < limit); take(j + 3, d3 <= Tr && i3 < limit);
             }
-            for (; j < n_c; ++j) take(j, dist2(xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit);
+            for (; j < n_c; ++j) take(j, dist2(s_xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit);
           } else {
             for (; j < n_c; ++j)
-              take(j, dist2(xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit && reach_bit(reach, g.reach_words, cid[j], wq));
+              take(j, dist2(s_xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit && reach_bit(reach, g.reach_words, cid[j], wq));
           }
           if (cnt > NR_LCAP) fallback = true;
         }
@@ -670,7 +646,7 @@ static int32_t nt_bin(porrt_ctx* ctx, const GridDev& g, const double* q_dev, con
 
 bool nn_tile_usable(const porrt_ctx* ctx, int64_t m) {
   // worth the binning passes only for real batches; the grid must be addressable with 32-bit cell ids and tile counts
-  return m >= 2048 && (int64_t)ctx->cells_x * ctx->cells_y < (1ll << 30) && getenv("PORRT_NN_NO_TILES") == nullptr;
+  return m >= 2048 && (int64_t)ctx->cells_x * ctx->cells_y < (1ll << 30) && !ctx->force_thread_per_query_nn;
 }
 
 // the merge scripts of the current vertex set (see nbr_script_kernel); built on the first large radius batch after

@@ -1,5 +1,5 @@
 #!/bin/bash
-# build_variant.sh NAME "-DNR_CAP=544 ..." -> build/libporrt_NAME.so (A/B builds of the kernels; select with PORRT_B200_LIB)
+# build_variant.sh NAME "EXTRA_NVCC_FLAGS" -> build/libporrt_NAME.so (A/B builds of the kernels; select with PORRT_B200_LIB)
 set -e
 cd "$(dirname "$0")/../po_rrt_b200/csrc"
 mkdir -p ../../build/$1

@@ -1,5 +1,6 @@
 """CPU-side checks of the drop-in boundary: the C-ABI library loads and exports every symbol include/porrt_b200.h
 declares (no compute calls -- there is no GPU here), and the product fails loudly without a device."""
+import glob
 import os
 import re
 import subprocess
@@ -112,3 +113,35 @@ def test_rust_build_script_lists_the_makefile_sources():
         src = open(os.path.join(ROOT, "integration", "rust", "src", f)).read()
         for name in sorted(set(re.findall(r"\b(porrt_[a-z0-9_]+)\s*\(", src))):
             assert ("pub fn %s(" % name) in ffi, (f, name)
+
+
+# DESIGN.md 0: no run-time backend switch and no environment variable that selects an implementation.  The CUDA sources read
+# PORRT_DEBUG (diagnostic prints) and PORRT_NCCL_LIB (where NCCL is loaded from, include/porrt_b200.h) and nothing else, and no
+# `#ifndef` leaves a constant open to a -D override; paths that tests must reach on inputs where the library would not choose them
+# are context options (PORRT_OPT_FORCE_*).
+def _csrc_without_comments():
+    paths = sorted(glob.glob(os.path.join(ROOT, "po_rrt_b200", "csrc", "*.cu*")))
+    assert paths
+    for p in paths:
+        src = re.sub(r"/\*.*?\*/", "", open(p).read(), flags=re.S)
+        yield os.path.basename(p), re.sub(r"//[^\n]*", "", src)
+
+
+def test_library_reads_only_documented_environment_variables():
+    allowed = {"PORRT_DEBUG", "PORRT_NCCL_LIB"}
+    found = [(name, m.group(1).strip()) for name, src in _csrc_without_comments() for m in re.finditer(r"\bgetenv\s*\(([^)]*)\)", src)]
+    assert found
+    bad = [(name, arg) for name, arg in found if not arg.startswith('"') or arg.strip('"') not in allowed]
+    assert not bad, "environment variables read by the library beyond %s: %s" % (sorted(allowed), bad)
+
+
+def test_library_has_no_ifndef_knobs():
+    # an include guard is `#ifndef X` directly followed by a bare `#define X`; anything else is a compile-time knob
+    bad = []
+    for name, src in _csrc_without_comments():
+        lines = [l.strip() for l in src.splitlines() if l.strip()]
+        for i, l in enumerate(lines):
+            m = re.match(r"#\s*ifndef\s+(\w+)$", l)
+            if m and not (i + 1 < len(lines) and re.fullmatch(r"#\s*define\s+%s" % m.group(1), lines[i + 1])):
+                bad.append((name, m.group(1)))
+    assert not bad, "#ifndef knobs in the library sources: %s" % bad

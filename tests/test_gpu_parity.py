@@ -441,7 +441,7 @@ def _prm_compare(ctx, occ, zones, kind, n_iter, max_step, search_radius, start=(
     return prm, oprm
 
 
-def test_nn_tiles_equal_thread_per_query(ctx, monkeypatch):
+def test_nn_tiles_equal_thread_per_query(ctx):
     """nn_tile.cu (TMA-staged tiles) against nn.cu's thread-per-query kernels on the same batches: mixed radii (some wider
     than a cell -> index-list fallback), prefix limits, reachability filters, NaN / far-away queries, clustered vertices
     (tiles that exceed the staging buffer), k = 1 / 5 / 16 / 32"""
@@ -468,9 +468,11 @@ def test_nn_tiles_equal_thread_per_query(ctx, monkeypatch):
         return out
 
     got = run()
-    monkeypatch.setenv("PORRT_NN_NO_TILES", "1")
-    want = run()
-    monkeypatch.delenv("PORRT_NN_NO_TILES")
+    ctx.set_option(P.OPT_FORCE_THREAD_PER_QUERY_NN, 1)
+    try:
+        want = run()
+    finally:
+        ctx.set_option(P.OPT_FORCE_THREAD_PER_QUERY_NN, 0)
     for key in want:
         for a, b in zip(got[key], want[key]):
             np.testing.assert_array_equal(a, b, err_msg=key)
@@ -1352,11 +1354,11 @@ def otree_prefix_radius(pts, q, r):
     return np.asarray(offs, np.int64), np.asarray(ids, np.int32), None
 
 
-def test_c_abi_harness():
+def test_c_abi_harness(tmp_path):
     """the C ABI called from plain C (tests/c_abi_harness.c, gcc -std=c99), not through ctypes"""
     import subprocess
     root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    exe = os.path.join(root, "tests", "_c_abi_harness")
+    exe = str(tmp_path / "c_abi_harness")
     libdir = os.path.join(root, "po_rrt_b200")
     subprocess.run(["gcc", "-std=c99", "-O1", "-Wall", "-Wextra", "-pedantic", "-I", os.path.join(root, "include"),
                     os.path.join(root, "tests", "c_abi_harness.c"), "-o", exe, "-L", libdir, "-lporrt_b200", "-lm",

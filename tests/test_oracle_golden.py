@@ -397,7 +397,7 @@ def test_bresenham_doc_example_and_closed_form():
 
 
 def test_fixed_point_minor_offset_is_exact():
-    """edge3.cu / edge4.cu: floor(k*dy/dx) == hi32(k*S + 2^16) for every 0 <= dy <= dx < 2^15 and 0 <= k <= dx (DESIGN.md 3.1),
+    """edge3.cu: floor(k*dy/dx) == hi32(k*S + 2^16) for every 0 <= dy <= dx < 2^15 and 0 <= k <= dx (DESIGN.md 3.1),
     both for the exact S = min(floor(dy*2^32/dx), 2^32-1) and for the S the kernels compute on the FP64 pipe,
     trunc_sat(dy * 2^32 * rn(1/dx)) -- replayed here in IEEE double arithmetic (numpy division and multiplication are correctly
     rounded like __drcp_rn / __dmul_rn).  Exhaustive for dx <= 160, all dy / sampled k for large dx."""

@@ -311,11 +311,11 @@ def test_plan_in_more_dimensions(dim):
 
 
 @pytest.mark.gpu
-def test_c_client():
+def test_c_client(tmp_path):
     """tests/pto_c_client.c: the planner API driven from plain C (gcc -std=c99) with the world model in C callbacks, three-dimensional
     states, malloc()ed observer arrays the planner frees -- the policy branches on the observed door as it must"""
     _lib()
-    exe = os.path.join(ROOT, "tests", "_pto_c_client")
+    exe = str(tmp_path / "pto_c_client")
     libdir = os.path.join(ROOT, "po_rrt_b200")
     subprocess.run(["gcc", "-std=c99", "-O1", "-Wall", "-Wextra", "-pedantic", "-I", os.path.join(ROOT, "include"),
                     os.path.join(ROOT, "tests", "pto_c_client.c"), "-o", exe, "-L", libdir, "-lpo_rrt_c", "-lm", "-Wl,-rpath," + libdir], check=True)
