@@ -391,6 +391,26 @@ int32_t porrt_reach_final_nodes_for_world(porrt_reach* r, int32_t world, int64_t
 int32_t porrt_reach_finals(porrt_reach* r, int64_t* out_ids, uint64_t* out_masks, int64_t cap, int64_t* out_n);          /* :82-84 */
 int32_t porrt_reach_is_final_set_complete(porrt_reach* r, int32_t* out_complete);                                       /* :86-95 */
 
+/* ------------------------------------------------------------------ PTO roadmap growth on the device (pto_grow.cu, DESIGN.md 3.8)
+ * PTO::grow_graph (pto.rs:55-139) on the uploaded map (Map or MapShelfDomain, N = 2), as ONE call.  The two sampler streams are
+ * Pcg64::seed_from_u64(sampler_seed), like PTO::new (seed 0 in the reference); continuous samples in [low, up).  Goals are a
+ * SquareGoal (common.rs:304-350): goals_xy[2 * n_goals], goal_masks[n_goals * mask_words], max_dist.  Loop condition as the
+ * reference: i < n_iter_min || (!is_final_set_complete && i < n_iter_max).
+ * The roadmap stays on the device; porrt_pto_fetch copies it out.  out_sizes[4] = iterations, nodes, directed edges, final nodes.
+ * *out_complete = is_final_set_complete() at the end (the reference's plan() fails when 0, pto_c.rs:214).
+ * PORRT_ERR_PANIC where the reference panics, with *out_panic_code (nullable) = PORRT_INVALID for expect("Start from a valid
+ * state!") or the PORRT_PANIC_* code of the first state / edge check that panics, and out_sizes[0] = that iteration.
+ * out_counters (nullable [4]): windows, iterations re-speculated, conflicts by nearest neighbour, conflicts by radius / kd slot. */
+int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const double low[2], const double up[2], uint64_t sampler_seed,
+                       const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
+                       double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
+                       int64_t* out_sizes, int32_t* out_complete, int32_t* out_panic_code, int64_t* out_counters);
+/* the roadmap of the last porrt_pto_grow on this ctx, every pointer nullable: xy[2V], node_vid[V], children CSR in the reference's
+ * insertion order (row_ptr[V+1], col[E], edge_vid[E]; parents(k) == children(k) as sequences, pto.rs:111-120), reach[V * mask_words]
+ * (Reachability::reachability), final ids + finality masks in add_final_node order (pto.rs:122-124) */
+int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
+                        int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks);
+
 /* ------------------------------------------------------------------ multi-GPU (SURVEY.md 8(e))
  * The reference is single-threaded and has no distributed code; what shards are its independent units (edge checks,
  * radius / NN queries, the worlds of plan_qmdp).  One process and one ctx per GPU; map and vertex set replicated.

@@ -7,7 +7,7 @@ use std::process::Command;
 
 const CU_SOURCES: &[&str] = &[
     "ctx.cu", "map.cu", "edge3.cu", "nn.cu", "nn_tile.cu", "graph.cu", "colsolve.cu", "sssp_frontier.cu", "belief_tables.cu", "belief_explicit.cu",
-    "mmprm.cu", "refine.cu", "comm.cu", "host_side.cu", "formats.cu", "diag.cu",
+    "mmprm.cu", "refine.cu", "comm.cu", "host_side.cu", "formats.cu", "diag.cu", "pto_grow.cu",
 ];
 const HEADERS: &[&str] = &[
     "common.cuh", "colsolve.cuh", "belief_tables.cuh", "sssp_frontier.cuh", "map_dev.cuh", "edge_common.cuh", "nn_dev.cuh", "pcg64.h",

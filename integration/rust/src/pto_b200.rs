@@ -5,18 +5,80 @@
 //! belief graph stays IMPLICIT on the device (belief node id = node * B + belief, node types and observation edges from
 //! per-visible-zone-set tables, DESIGN.md 3.3): reachable beliefs + one visibility test per NODE + `porrt_belief_vi`, then the
 //! policy walk `porrt_extract_policy` (belief_graph.rs:184-267).  Expected costs are bit-identical to conditional_dijkstra's.
-//! Roadmap growth (`PTO::grow_graph`, pto.rs:55-139) stays sequential and unchanged; through `B200Domain`'s per-query methods it
-//! runs on the same library (batches of one).
+//! Roadmap growth (`PTO::grow_graph`, pto.rs:55-139) has its swap too: `grow_graph_b200` runs the whole loop in ONE
+//! `porrt_pto_grow` (speculative windows with an exact in-order commit, DESIGN.md 3.8) and copies the roadmap, the reachability
+//! masks and the final nodes back into the planner's own structures, bit for bit what `grow_graph` builds.
 #![cfg(feature = "b200")]
 
 use super::PTO;
-use crate::b200::{words_from_mask, B200Domain};
+use crate::b200::{mask_from_words, words_from_mask, B200Domain};
 use crate::b200_ffi::*;
 use crate::common::*;
 use crate::pto_graph::PTOFuncs;
 use crate::qmdp_policy_extractor::b200::export_csr;
 
 impl<'a> PTO<'a, B200Domain<'a>, 2> {
+    /// PTO::grow_graph (pto.rs:55-139) on the device.  The samplers are PTO::new's (seed 0); the goal is a SquareGoal given as its
+    /// (state, world mask) pairs.  Panics where the reference panics, returns Err where it does (pto.rs:131-138).
+    pub fn grow_graph_b200(&mut self, start: &[f64; 2], goals: &[([f64; 2], WorldMask)], goal_max_dist: f64, max_step: f64,
+                           search_radius: f64, n_iter_min: usize, n_iter_max: usize) -> Result<(), &'static str> {
+        let ctx = self.fns.ctx;
+        let mw = self.fns.mask_words();
+        let goals_xy: Vec<f64> = goals.iter().flat_map(|(s, _)| s.iter().copied()).collect();
+        let goal_masks: Vec<u64> = goals.iter().flat_map(|(_, m)| words_from_mask(m, mw)).collect();
+        let (low, up) = (self.continuous_sampler.low, self.continuous_sampler.up);
+        let (mut sizes, mut counters) = ([0i64; 4], [0i64; 4]);
+        let (mut complete, mut panic_code) = (0i32, 0i32);
+        let rc = unsafe {
+            porrt_pto_grow(ctx.raw(), start.as_ptr(), low.as_ptr(), up.as_ptr(), 0, goals_xy.as_ptr(), goal_masks.as_ptr(),
+                           goals.len() as i32, goal_max_dist, max_step, search_radius, n_iter_min as i64, n_iter_max as i64,
+                           sizes.as_mut_ptr(), &mut complete, &mut panic_code, counters.as_mut_ptr())
+        };
+        ctx.check(rc); // PORRT_ERR_PANIC -> the reference's panic, with the library's message
+        let (v, e, n_finals) = (sizes[1] as usize, sizes[2] as usize, sizes[3] as usize);
+        let mut xy = vec![0f64; 2 * v];
+        let mut node_vid = vec![0i32; v];
+        let mut row_ptr = vec![0i64; v + 1];
+        let (mut col, mut edge_vid) = (vec![0i32; e], vec![0i32; e]);
+        let mut reach = vec![0u64; v * mw];
+        let (mut fin_ids, mut fin_masks) = (vec![0i64; n_finals], vec![0u64; n_finals * mw]);
+        ctx.check(unsafe {
+            porrt_pto_fetch(ctx.raw(), xy.as_mut_ptr(), node_vid.as_mut_ptr(), row_ptr.as_mut_ptr(), col.as_mut_ptr(), edge_vid.as_mut_ptr(),
+                            reach.as_mut_ptr(), fin_ids.as_mut_ptr(), fin_masks.as_mut_ptr())
+        });
+        let n_worlds = self.n_worlds;
+        for k in 0..v {
+            self.graph.add_node([xy[2 * k], xy[2 * k + 1]], node_vid[k] as usize);
+            self.kdtree.add([xy[2 * k], xy[2 * k + 1]], k);
+        }
+        for u in 0..v {
+            let (a, b) = (row_ptr[u] as usize, row_ptr[u + 1] as usize);
+            let row: Vec<PTOEdge> = (a..b).map(|k| PTOEdge { id: col[k] as usize, validity_id: edge_vid[k] as usize }).collect();
+            self.graph.nodes[u].parents = row.clone(); // parents(k) == children(k) as sequences (pto.rs:111-120)
+            self.graph.nodes[u].children = row;
+        }
+        // Reachability (pto_reachability.rs) through its own API: the add_edge calls of pto.rs:111-120 replayed in insertion order --
+        // the early part of row k (columns < k, kd order) is what node k added -- give the device's masks back bit for bit
+        let validities = self.fns.world_validities();
+        self.conservative_reachability.set_root(validities[node_vid[0] as usize].clone());
+        for k in 1..v {
+            self.conservative_reachability.add_node(validities[node_vid[k] as usize].clone());
+            let early: Vec<&PTOEdge> = self.graph.nodes[k].children.iter().filter(|c| c.id < k).collect();
+            for c in &early {
+                self.conservative_reachability.add_edge(c.id, k, &validities[c.validity_id]);
+            }
+            for c in &early {
+                self.conservative_reachability.add_edge(k, c.id, &validities[c.validity_id]);
+            }
+        }
+        debug_assert!((0..v).all(|k| *self.conservative_reachability.reachability(k) == mask_from_words(&reach[k * mw..(k + 1) * mw], n_worlds)));
+        for k in 0..n_finals {
+            self.conservative_reachability.add_final_node(fin_ids[k] as usize, &mask_from_words(&fin_masks[k * mw..(k + 1) * mw], n_worlds));
+        }
+        self.n_it = sizes[0] as usize;
+        if complete != 0 { Ok(()) } else { Err("final nodes are not reached for each world") }
+    }
+
     pub fn plan_belief_space_b200(&mut self, start_belief_state: &BeliefState) -> Policy<2> {
         assert_belief_state_validity(start_belief_state);
         let ctx = self.fns.ctx;

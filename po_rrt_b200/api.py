@@ -854,6 +854,60 @@ class Reachability:
         return bool(out.value)
 
 
+class PTO:
+    """src/pto.rs PTO::grow_graph on the device (porrt_pto_grow): `fns` is an uploaded Map / MapShelfDomain, the two sampler streams
+    are seeded with `seed` like PTO::new.  The roadmap stays on the device until graph_arrays() / reach_masks() / finals() ask."""
+
+    def __init__(self, fns, low, up, seed=0):
+        self.fns, self.ctx = fns, fns.ctx
+        self.low, self.up, self.seed = _f64(low), _f64(up), int(seed)
+        self.n_it, self.sizes, self.counters = 0, (0, 0, 0, 0), (0, 0, 0, 0)
+
+    def grow_graph(self, start, goal, max_step, search_radius, n_iter_min, n_iter_max):
+        """-> 0 when every world reaches a final node, 1 otherwise (pto.rs:131-138); PorrtError where the reference panics
+        (e.code == 5, e.panic_code = the state / edge check's code, PORRT_INVALID for an invalid start)"""
+        self.fns._need()
+        c = self.ctx
+        start = _f64(start)
+        sizes, counters = np.zeros(4, np.int64), np.zeros(4, np.int64)
+        complete, panic = C.c_int32(), C.c_int32()
+        rc = c.lib.porrt_pto_grow(c.h, _p(start), _p(self.low), _p(self.up), self.seed, _p(goal.goals), _p(goal.masks), len(goal.goals),
+                                  goal.max_dist, float(max_step), float(search_radius), int(n_iter_min), int(n_iter_max), _p(sizes),
+                                  C.byref(complete), C.byref(panic), _p(counters))
+        self.n_it, self.sizes, self.counters = int(sizes[0]), tuple(int(x) for x in sizes), tuple(int(x) for x in counters)
+        if rc:
+            err = PorrtError(rc, (c.lib.porrt_last_error(c.h) or b"").decode())
+            err.panic_code = panic.value
+            raise err
+        return 0 if complete.value else 1
+
+    def graph_arrays(self):
+        """-> xy[V,2], node_vid[V], row_ptr[V+1], col[E], edge_vid[E]: the children adjacency in insertion order"""
+        _, V, E, _ = self.sizes
+        xy, nv = np.empty((V, 2)), np.empty(V, np.int32)
+        rp, col, ev = np.empty(V + 1, np.int64), np.empty(E, np.int32), np.empty(E, np.int32)
+        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, _p(xy), _p(nv), _p(rp), _p(col), _p(ev), None, None, None))
+        return xy, nv, rp, col, ev
+
+    def reach_masks(self):
+        """Reachability::reachability of every node as [V, n_worlds] 0/1"""
+        V = self.sizes[1]
+        nw = self.fns.n_worlds()
+        words = np.empty((V, self.fns.mask_words), np.uint64)
+        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, None, None, None, None, None, _p(words), None, None))
+        bits = np.zeros((V, nw), np.uint8)
+        for w in range(nw):
+            bits[:, w] = (words[:, w // 64] >> np.uint64(w % 64)) & np.uint64(1)
+        return bits
+
+    def finals(self):
+        """final node ids and their finality masks ([n, mask_words] u64), in add_final_node order"""
+        F = self.sizes[3]
+        ids, masks = np.empty(F, np.int64), np.empty((F, self.fns.mask_words), np.uint64)
+        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, None, None, None, None, None, None, _p(ids), _p(masks)))
+        return ids, masks
+
+
 def react_qmdp(ctx, row_ptr, col, xy, cost_to_goals, start_node, belief, common_horizon):
     """QMdpPolicyExtractor::react_qmdp (qmdp_policy_extractor.rs:38-123) over plan_qmdp's cost table -> (paths as lists of
     node ids, one per world; length of the common prefix).  ctx may be None (host walk)."""

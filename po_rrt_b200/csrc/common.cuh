@@ -162,6 +162,9 @@ struct porrt_ctx {
     std::vector<int64_t> row_ptr; std::vector<int32_t> col, belief_id; std::vector<uint8_t> type;
   } mm;
 
+  // ---- last PTO growth (pto_grow.cu): the roadmap stays on the device until porrt_pto_fetch
+  struct PtoGrow* pto = nullptr;
+
   // ---- multi-GPU (comm.cu): NCCL communicator bound at run time; world 1 = no communicator
   void* comm = nullptr;
   int comm_rank = 0, comm_world = 1;
@@ -261,6 +264,12 @@ int32_t segments_sort_by_key_dev(porrt_ctx* ctx, const int64_t* offsets_dev, int
                                  const int32_t* key_of_id_dev, int64_t key_limit, const int32_t* seg_list_dev = nullptr, int64_t n_listed = 0);
 int32_t radix_sort_pairs(porrt_ctx* ctx, uint64_t* keys, uint32_t* vals, int64_t n, int key_bits);
 int bits_for(uint64_t max_value);
+// graph.cu: children CSR from per-node early lists (PRM build tail; PTO growth with edge validity ids)
+int32_t late_list_csr_dev(porrt_ctx* ctx, const int64_t* seg_off, int64_t n, const int32_t* compact, const int32_t* early_cnt,
+                          const int32_t* early_vid, int32_t* late_cnt, int32_t* cursor, int64_t* late_off, int32_t* late_vals,
+                          int64_t* row_ptr, int32_t* col, int32_t* vid);
+// pto_grow.cu
+void pto_grow_release(porrt_ctx* ctx);
 int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, double max_step, double search_radius,
                        const double* ms_arr, const double* sr_arr, int64_t* out_row_ptr, int32_t* out_col, int64_t cap,
                        int64_t* out_n_edges, double* out_phase_ms, const int64_t* group_ptr = nullptr, int32_t n_groups = 0);

@@ -55,6 +55,7 @@ PORRT_API int32_t porrt_ctx_destroy(porrt_ctx* ctx) {
   for (DevBuf& b : ctx->nn_tmp) b.release();
   ctx->nn_stage.release(); ctx->nn_stage2.release(); ctx->comm_tmp.release(); ctx->d_nbr_start.release(); ctx->d_nbr_script.release();
   for (DevBuf& b : ctx->scratch) b.release();
+  pto_grow_release(ctx);
   ctx->kd_buf.release(); ctx->d_prm_row.release(); ctx->d_prm_col.release(); ctx->d_bel_succ.release(); ctx->bel.dev.release();
   if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
   for (PinBuf& b : ctx->pin) b.release();

@@ -373,17 +373,57 @@ __global__ void prm_rowptr_kernel(const int64_t* __restrict__ early_off, const i
   if (i <= m) row_ptr[i] = early_off[i] + late_off[i];
 }
 
+// early_vid / vid (nullable together): the validity id of every edge rides along (PTO growth, pto_grow.cu).  A late entry k of row
+// seg is the edge seg <-> k that node k logged in its own early list; its id is looked up there (early lists are short).
 __global__ void prm_fill_kernel(const int64_t* __restrict__ offsets, int64_t m, const int32_t* __restrict__ compact,
                                 const int32_t* __restrict__ early_cnt, const int64_t* __restrict__ late_off,
-                                const int32_t* __restrict__ late_vals, const int64_t* __restrict__ row_ptr, int32_t* __restrict__ col) {
+                                const int32_t* __restrict__ late_vals, const int64_t* __restrict__ row_ptr, int32_t* __restrict__ col,
+                                const int32_t* __restrict__ early_vid, int32_t* __restrict__ vid) {
   const int lane = threadIdx.x & 31;
   const int64_t seg = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
   if (seg >= m) return;
   const int64_t s = offsets[seg], r = row_ptr[seg];
   const int32_t c = early_cnt[seg];
-  for (int32_t k = lane; k < c; k += 32) col[r + k] = compact[s + k];
+  for (int32_t k = lane; k < c; k += 32) {
+    col[r + k] = compact[s + k];
+    if (vid) vid[r + k] = early_vid[s + k];
+  }
   const int64_t ls = late_off[seg], le = late_off[seg + 1];
-  for (int64_t k = ls + lane; k < le; k += 32) col[r + c + (k - ls)] = late_vals[k];
+  for (int64_t k = ls + lane; k < le; k += 32) {
+    const int32_t later = late_vals[k];
+    col[r + c + (k - ls)] = later;
+    if (vid) {
+      const int64_t ks = offsets[later];
+      int32_t v = -1;
+      for (int32_t q = 0; q < early_cnt[later]; ++q)
+        if (compact[ks + q] == (int32_t)seg) { v = early_vid[ks + q]; break; }
+      vid[r + c + (k - ls)] = v;
+    }
+  }
+}
+
+// The children CSR of a roadmap whose edges were logged per new node (row k = its early list, then the later nodes that listed k,
+// ascending): the tail of the PRM build below as one call.  seg_off[n + 1] (seg_off[n] = early entries), early_cnt[n]; work
+// buffers: late_cnt / cursor [n] int32, late_off [n + 1] int64, late_vals [seg_off[n]] int32.  Enqueued on ctx->stream.
+int32_t late_list_csr_dev(porrt_ctx* ctx, const int64_t* seg_off, int64_t n, const int32_t* compact, const int32_t* early_cnt,
+                          const int32_t* early_vid, int32_t* late_cnt, int32_t* cursor, int64_t* late_off, int32_t* late_vals,
+                          int64_t* row_ptr, int32_t* col, int32_t* vid) {
+  cudaStream_t st = ctx->stream;
+  CUDA_TRY(ctx, cudaMemsetAsync(late_cnt, 0, (size_t)n * 4, st));
+  CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, (size_t)n * 4, st));
+  prm_late_count_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(seg_off, n, compact, early_cnt, late_cnt);
+  LAUNCH_CHECK(ctx);
+  int32_t rc = scan_exclusive_i64(ctx, late_cnt, n, late_off);
+  if (rc) return rc;
+  prm_rowptr_kernel<<<div_up(n + 1, 256), 256, 0, st>>>(seg_off, late_off, n, row_ptr);
+  LAUNCH_CHECK(ctx);
+  prm_late_scatter_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(seg_off, n, compact, early_cnt, late_off, cursor, late_vals);
+  LAUNCH_CHECK(ctx);
+  rc = segments_sort_by_key_dev(ctx, late_off, n, late_vals, nullptr, n);   // later nodes ascending
+  if (rc) return rc;
+  prm_fill_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(seg_off, n, compact, early_cnt, late_off, late_vals, row_ptr, col, early_vid, vid);
+  LAUNCH_CHECK(ctx);
+  return PORRT_OK;
 }
 
 // ms_arr / sr_arr (nullable): per-sample (max_step, search_radius) of the add_sample call that created node k -- the multi-modal
@@ -697,7 +737,7 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
       if (r1 > r0) {
         rc = segments_sort_by_key_dev(ctx, d_late_off + r0, r1 - r0, d_vals, nullptr, n);   // later nodes ascending
         if (rc) return rc;
-        prm_fill_kernel<<<div_up((r1 - r0) * 32, 256), 256, 0, st>>>(d_seg_off + r0, r1 - r0, d_compact, d_early_cnt + r0, d_late_off + r0, d_vals, d_row_ptr + r0, d_col);
+        prm_fill_kernel<<<div_up((r1 - r0) * 32, 256), 256, 0, st>>>(d_seg_off + r0, r1 - r0, d_compact, d_early_cnt + r0, d_late_off + r0, d_vals, d_row_ptr + r0, d_col, nullptr, nullptr);
         LAUNCH_CHECK(ctx);
       }
       cudaEvent_t ev = evs[b];
@@ -716,7 +756,7 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
     LAUNCH_CHECK(ctx);
     rc = segments_sort_by_key_dev(ctx, d_late_off, n, d_vals, nullptr, n);   // later nodes ascending
     if (rc) return rc;
-    prm_fill_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(d_seg_off, n, d_compact, d_early_cnt, d_late_off, d_vals, d_row_ptr, d_col);
+    prm_fill_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(d_seg_off, n, d_compact, d_early_cnt, d_late_off, d_vals, d_row_ptr, d_col, nullptr, nullptr);
     LAUNCH_CHECK(ctx);
     CUDA_TRY(ctx, cudaMemcpyAsync(out_row_ptr, d_row_ptr, (size_t)(n + 1) * 8, cudaMemcpyDeviceToHost, st));
     if (out_col && cap >= n_edges) {
