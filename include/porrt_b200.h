@@ -407,9 +407,29 @@ int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const double low[2
                        int64_t* out_sizes, int32_t* out_complete, int32_t* out_panic_code, int64_t* out_counters);
 /* the roadmap of the last porrt_pto_grow on this ctx, every pointer nullable: xy[2V], node_vid[V], children CSR in the reference's
  * insertion order (row_ptr[V+1], col[E], edge_vid[E]; parents(k) == children(k) as sequences, pto.rs:111-120), reach[V * mask_words]
- * (Reachability::reachability), final ids + finality masks in add_final_node order (pto.rs:122-124) */
+ * (Reachability::reachability), final ids + finality masks in add_final_node order (pto.rs:122-124).
+ * After a porrt_pto_grow_batch this is roadmap 0 of that batch (porrt_pto_fetch_roadmap(ctx, 0, ...)). */
 int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
                         int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks);
+/* porrt_pto_grow for n_roadmaps independent roadmaps in ONE call: roadmap r samples with Pcg64::seed_from_u64(sampler_seeds[r]);
+ * map, start, bounds, goals and parameters are shared.  Each roadmap equals porrt_pto_grow with its seed, counters included.
+ * out_sizes[4 * n] and out_counters (nullable, [4 * n]) hold porrt_pto_grow's four values per roadmap.  out_status[r] = 0 when
+ * roadmap r's final set is complete, 1 when it is not, PORRT_ERR_PANIC when its growth panics: then out_panic_code[r] (nullable
+ * [n]) and out_sizes[4 r] are the code and the iteration porrt_pto_grow reports.  A panic stops only its own roadmap; the call
+ * still returns PORRT_OK.  The whole call fails like porrt_pto_grow on bad arguments, no map, overlapping goal masks and
+ * low >= up.  n_roadmaps must lie in 1 .. PORRT_PTO_MAX_ROADMAPS (a launch grid's y dimension) and the device's free memory must
+ * hold them at their starting size (about 31 MB each at 4096 + iterations, DESIGN.md 3.8), else PORRT_ERR_INVALID_ARG; running
+ * out of memory while the roadmaps grow is PORRT_ERR_CUDA.  The batch replaces the ctx's last growth: porrt_pto_fetch_roadmap
+ * reads roadmap r, porrt_pto_fetch reads roadmap 0. */
+#define PORRT_PTO_MAX_ROADMAPS 65535
+int32_t porrt_pto_grow_batch(porrt_ctx* ctx, int32_t n_roadmaps, const uint64_t* sampler_seeds, const double start[2], const double low[2],
+                             const double up[2], const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
+                             double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes,
+                             int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters);
+/* porrt_pto_fetch for roadmap r of the last porrt_pto_grow_batch (a porrt_pto_grow is a batch of one).  PORRT_ERR_INVALID_ARG
+ * when nothing has been grown, r is out of range, or roadmap r panicked. */
+int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
+                                int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks);
 
 /* ------------------------------------------------------------------ multi-GPU (SURVEY.md 8(e))
  * The reference is single-threaded and has no distributed code; what shards are its independent units (edge checks,

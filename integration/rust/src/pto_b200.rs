@@ -7,7 +7,8 @@
 //! policy walk `porrt_extract_policy` (belief_graph.rs:184-267).  Expected costs are bit-identical to conditional_dijkstra's.
 //! Roadmap growth (`PTO::grow_graph`, pto.rs:55-139) has its swap too: `grow_graph_b200` runs the whole loop in ONE
 //! `porrt_pto_grow` (speculative windows with an exact in-order commit, DESIGN.md 3.8) and copies the roadmap, the reachability
-//! masks and the final nodes back into the planner's own structures, bit for bit what `grow_graph` builds.
+//! masks and the final nodes back into the planner's own structures, bit for bit what `grow_graph` builds; `grow_graphs_b200`
+//! grows one planner per seed in ONE `porrt_pto_grow_batch` (the roadmaps share each window's launches, DESIGN.md 3.8).
 #![cfg(feature = "b200")]
 
 use super::PTO;
@@ -35,6 +36,49 @@ impl<'a> PTO<'a, B200Domain<'a>, 2> {
                            sizes.as_mut_ptr(), &mut complete, &mut panic_code, counters.as_mut_ptr())
         };
         ctx.check(rc); // PORRT_ERR_PANIC -> the reference's panic, with the library's message
+        self.copy_back_b200(0, &sizes);
+        if complete != 0 { Ok(()) } else { Err("final nodes are not reached for each world") }
+    }
+
+    /// PTO::grow_graph for one planner per seed in `seeds`, all grown in ONE `porrt_pto_grow_batch` call on this planner's map:
+    /// planner r is `PTO::new(self.fns)` with both samplers seeded `seeds[r]`, filled with the roadmap, reachability and final
+    /// nodes `grow_graph` builds with that seed.  Start, goal and parameters as `grow_graph_b200`.  A panic in one roadmap panics
+    /// here with its code once the batch has been grown; Err where `grow_graph` returns Err (pto.rs:131-138).
+    pub fn grow_graphs_b200(&self, seeds: &[u64], start: &[f64; 2], goals: &[([f64; 2], WorldMask)], goal_max_dist: f64,
+                            max_step: f64, search_radius: f64, n_iter_min: usize, n_iter_max: usize)
+                            -> Vec<(Self, Result<(), &'static str>)> {
+        let ctx = self.fns.ctx;
+        let mw = self.fns.mask_words();
+        let n = seeds.len();
+        let goals_xy: Vec<f64> = goals.iter().flat_map(|(s, _)| s.iter().copied()).collect();
+        let goal_masks: Vec<u64> = goals.iter().flat_map(|(_, m)| words_from_mask(m, mw)).collect();
+        let (low, up) = (self.continuous_sampler.low, self.continuous_sampler.up);
+        let (mut sizes, mut counters) = (vec![0i64; 4 * n], vec![0i64; 4 * n]);
+        let (mut status, mut panic_code) = (vec![0i32; n], vec![0i32; n]);
+        ctx.check(unsafe {
+            porrt_pto_grow_batch(ctx.raw(), n as i32, seeds.as_ptr(), start.as_ptr(), low.as_ptr(), up.as_ptr(), goals_xy.as_ptr(),
+                                 goal_masks.as_ptr(), goals.len() as i32, goal_max_dist, max_step, search_radius, n_iter_min as i64,
+                                 n_iter_max as i64, sizes.as_mut_ptr(), status.as_mut_ptr(), panic_code.as_mut_ptr(),
+                                 counters.as_mut_ptr())
+        });
+        for r in 0..n {
+            assert!(status[r] != 5, "roadmap of seed {} panics at iteration {} (code {})", seeds[r], sizes[4 * r], panic_code[r]);
+        }
+        (0..n)
+            .map(|r| {
+                let mut pto = PTO::new(self.fns);
+                let s = [sizes[4 * r], sizes[4 * r + 1], sizes[4 * r + 2], sizes[4 * r + 3]];
+                pto.copy_back_b200(r as i32, &s);
+                (pto, if status[r] == 0 { Ok(()) } else { Err("final nodes are not reached for each world") })
+            })
+            .collect()
+    }
+
+    /// roadmap r of the ctx's last growth (`porrt_pto_fetch_roadmap`, sizes = iterations, nodes, directed edges, final nodes) into
+    /// this planner's graph, kd-tree, reachability and n_it, bit for bit what `grow_graph` builds
+    fn copy_back_b200(&mut self, r: i32, sizes: &[i64; 4]) {
+        let ctx = self.fns.ctx;
+        let mw = self.fns.mask_words();
         let (v, e, n_finals) = (sizes[1] as usize, sizes[2] as usize, sizes[3] as usize);
         let mut xy = vec![0f64; 2 * v];
         let mut node_vid = vec![0i32; v];
@@ -43,8 +87,8 @@ impl<'a> PTO<'a, B200Domain<'a>, 2> {
         let mut reach = vec![0u64; v * mw];
         let (mut fin_ids, mut fin_masks) = (vec![0i64; n_finals], vec![0u64; n_finals * mw]);
         ctx.check(unsafe {
-            porrt_pto_fetch(ctx.raw(), xy.as_mut_ptr(), node_vid.as_mut_ptr(), row_ptr.as_mut_ptr(), col.as_mut_ptr(), edge_vid.as_mut_ptr(),
-                            reach.as_mut_ptr(), fin_ids.as_mut_ptr(), fin_masks.as_mut_ptr())
+            porrt_pto_fetch_roadmap(ctx.raw(), r, xy.as_mut_ptr(), node_vid.as_mut_ptr(), row_ptr.as_mut_ptr(), col.as_mut_ptr(),
+                                    edge_vid.as_mut_ptr(), reach.as_mut_ptr(), fin_ids.as_mut_ptr(), fin_masks.as_mut_ptr())
         });
         let n_worlds = self.n_worlds;
         for k in 0..v {
@@ -76,7 +120,6 @@ impl<'a> PTO<'a, B200Domain<'a>, 2> {
             self.conservative_reachability.add_final_node(fin_ids[k] as usize, &mask_from_words(&fin_masks[k * mw..(k + 1) * mw], n_worlds));
         }
         self.n_it = sizes[0] as usize;
-        if complete != 0 { Ok(()) } else { Err("final nodes are not reached for each world") }
     }
 
     pub fn plan_belief_space_b200(&mut self, start_belief_state: &BeliefState) -> Policy<2> {

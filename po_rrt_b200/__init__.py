@@ -5,9 +5,9 @@ this package is the thin host-side mirror of the reference's interface used by t
 There is no CPU fallback: importing works anywhere, creating a Context needs the built library and a B200.
 """
 from .api import (DOOR, SHELF, INVALID, PANIC_OOB, PANIC_ZONE_UNWRAP, PANIC_MULTI_ZONE, NODE_ACTION, NODE_OBSERVATION,
-                  NODE_UNKNOWN, OPT_FORCE_LARGE_MAP_PATH, OPT_FORCE_GLOBAL_SWEEPS, OPT_FORCE_THREAD_PER_QUERY_NN, BeliefGraph, Context, KdTree, Map, MapShelfDomain, PRM, PTO, PorrtError, Reachability, Sampler, SquareGoal, dijkstra_worlds, dijkstra_worlds_resident_prm, heuristic_radius, mmprm_plan,
+                  NODE_UNKNOWN, OPT_FORCE_LARGE_MAP_PATH, OPT_FORCE_GLOBAL_SWEEPS, OPT_FORCE_THREAD_PER_QUERY_NN, BeliefGraph, Context, KdTree, Map, MapShelfDomain, PRM, PTO, PTOBatch, PorrtError, Reachability, Sampler, SquareGoal, dijkstra_worlds, dijkstra_worlds_resident_prm, heuristic_radius, mmprm_plan,
                   plan_belief_space, refine_policy_shortcut, refine_policy_reparent, policy_decompose, policy_expected_cost, react_qmdp, steer, words_from_bits)
 from . import synth
 
-__all__ = ["BeliefGraph", "Context", "Map", "MapShelfDomain", "KdTree", "PRM", "PTO", "PorrtError", "dijkstra_worlds", "mmprm_plan", "plan_belief_space",
+__all__ = ["BeliefGraph", "Context", "Map", "MapShelfDomain", "KdTree", "PRM", "PTO", "PTOBatch", "PorrtError", "dijkstra_worlds", "mmprm_plan", "plan_belief_space",
            "words_from_bits", "synth", "Reachability", "Sampler", "SquareGoal", "heuristic_radius", "react_qmdp", "steer"]

@@ -97,6 +97,8 @@ SIGNATURES = {
     "porrt_reachable_belief_states": (i32, [vp, vp, vp, i32, pp(i32)]),
     "porrt_pto_grow": (i32, [vp, vp, vp, vp, C.c_uint64, vp, vp, i32, f64, f64, f64, i64, i64, vp, pp(i32), pp(i32), vp]),
     "porrt_pto_fetch": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "porrt_pto_grow_batch": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, i32, f64, f64, f64, i64, i64, vp, vp, vp, vp]),
+    "porrt_pto_fetch_roadmap": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
     "porrt_comm_unique_id": (i32, [vp]),
     "porrt_comm_init": (i32, [vp, vp, i32, i32]),
     "porrt_comm_destroy": (i32, [vp]),

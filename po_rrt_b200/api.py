@@ -23,6 +23,7 @@ ERR_CAPACITY = 4
 OPT_FORCE_LARGE_MAP_PATH = 1
 OPT_FORCE_GLOBAL_SWEEPS = 2
 OPT_FORCE_THREAD_PER_QUERY_NN = 3
+PTO_MAX_ROADMAPS = 65535   # PORRT_PTO_MAX_ROADMAPS
 
 
 class PorrtError(RuntimeError):
@@ -881,31 +882,99 @@ class PTO:
             raise err
         return 0 if complete.value else 1
 
+    def _fetch(self, *outs):
+        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, *outs))
+
     def graph_arrays(self):
         """-> xy[V,2], node_vid[V], row_ptr[V+1], col[E], edge_vid[E]: the children adjacency in insertion order"""
-        _, V, E, _ = self.sizes
-        xy, nv = np.empty((V, 2)), np.empty(V, np.int32)
-        rp, col, ev = np.empty(V + 1, np.int64), np.empty(E, np.int32), np.empty(E, np.int32)
-        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, _p(xy), _p(nv), _p(rp), _p(col), _p(ev), None, None, None))
-        return xy, nv, rp, col, ev
+        return _roadmap_graph_arrays(self._fetch, self.sizes)
 
     def reach_masks(self):
         """Reachability::reachability of every node as [V, n_worlds] 0/1"""
-        V = self.sizes[1]
-        nw = self.fns.n_worlds()
-        words = np.empty((V, self.fns.mask_words), np.uint64)
-        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, None, None, None, None, None, _p(words), None, None))
-        bits = np.zeros((V, nw), np.uint8)
-        for w in range(nw):
-            bits[:, w] = (words[:, w // 64] >> np.uint64(w % 64)) & np.uint64(1)
-        return bits
+        return _roadmap_reach_masks(self._fetch, self.sizes, self.fns)
 
     def finals(self):
         """final node ids and their finality masks ([n, mask_words] u64), in add_final_node order"""
-        F = self.sizes[3]
-        ids, masks = np.empty(F, np.int64), np.empty((F, self.fns.mask_words), np.uint64)
-        self.ctx.check(self.ctx.lib.porrt_pto_fetch(self.ctx.h, None, None, None, None, None, None, _p(ids), _p(masks)))
-        return ids, masks
+        return _roadmap_finals(self._fetch, self.sizes, self.fns)
+
+
+class PTOBatch:
+    """PTO::grow_graph for one roadmap per seed in `seeds`, all in one device call (porrt_pto_grow_batch); map, start, goal and
+    parameters are shared.  Roadmap r is what PTO(fns, low, up, seeds[r]) grows, counters included.  After grow_graph the
+    attributes n_it[R], sizes[R, 4], counters[R, 4] and panic_code[R] hold one row per roadmap; graph_arrays(r), reach_masks(r)
+    and finals(r) read roadmap r.  The batch replaces the context's last growth (PTO objects on the same context then read
+    roadmap 0)."""
+
+    def __init__(self, fns, low, up, seeds):
+        self.fns, self.ctx = fns, fns.ctx
+        self.low, self.up = _f64(low), _f64(up)
+        self.seeds = np.ascontiguousarray(np.asarray(seeds, dtype=np.uint64).reshape(-1))
+        R = len(self.seeds)
+        self.n_it, self.panic_code = np.zeros(R, np.int64), np.zeros(R, np.int32)
+        self.sizes, self.counters = np.zeros((R, 4), np.int64), np.zeros((R, 4), np.int64)
+
+    def __len__(self):
+        return len(self.seeds)
+
+    def grow_graph(self, start, goal, max_step, search_radius, n_iter_min, n_iter_max):
+        """-> status[R]: 0 when every world of roadmap r reaches a final node, 1 otherwise, PorrtError.code 5 (PORRT_ERR_PANIC)
+        where roadmap r's growth panics (its code in panic_code[r], its iteration in n_it[r]).  Raises PorrtError when the call as
+        a whole fails (bad arguments, no map, overlapping goal masks, low >= up, too many roadmaps)."""
+        self.fns._need()
+        c = self.ctx
+        R = len(self.seeds)
+        status = np.zeros(R, np.int32)
+        rc = c.lib.porrt_pto_grow_batch(c.h, R, _p(self.seeds), _p(_f64(start)), _p(self.low), _p(self.up), _p(goal.goals), _p(goal.masks),
+                                        len(goal.goals), goal.max_dist, float(max_step), float(search_radius), int(n_iter_min),
+                                        int(n_iter_max), _p(self.sizes), _p(status), _p(self.panic_code), _p(self.counters))
+        self.n_it = self.sizes[:, 0].copy()
+        c.check(rc)
+        return status
+
+    def _fetcher(self, r):
+        def fetch(*outs):
+            self.ctx.check(self.ctx.lib.porrt_pto_fetch_roadmap(self.ctx.h, int(r), *outs))
+        return fetch
+
+    def graph_arrays(self, r):
+        """PTO.graph_arrays of roadmap r"""
+        return _roadmap_graph_arrays(self._fetcher(r), self.sizes[r])
+
+    def reach_masks(self, r):
+        """PTO.reach_masks of roadmap r"""
+        return _roadmap_reach_masks(self._fetcher(r), self.sizes[r], self.fns)
+
+    def finals(self, r):
+        """PTO.finals of roadmap r"""
+        return _roadmap_finals(self._fetcher(r), self.sizes[r], self.fns)
+
+
+# the arrays of a device-grown roadmap; fetch(xy, node_vid, row_ptr, col, edge_vid, reach, final_ids, final_masks) is
+# porrt_pto_fetch or porrt_pto_fetch_roadmap, sizes = (iterations, V, E, finals)
+def _roadmap_graph_arrays(fetch, sizes):
+    _, V, E, _ = (int(x) for x in sizes)
+    xy, nv = np.empty((V, 2)), np.empty(V, np.int32)
+    rp, col, ev = np.empty(V + 1, np.int64), np.empty(E, np.int32), np.empty(E, np.int32)
+    fetch(_p(xy), _p(nv), _p(rp), _p(col), _p(ev), None, None, None)
+    return xy, nv, rp, col, ev
+
+
+def _roadmap_reach_masks(fetch, sizes, fns):
+    V = int(sizes[1])
+    nw = fns.n_worlds()
+    words = np.empty((V, fns.mask_words), np.uint64)
+    fetch(None, None, None, None, None, _p(words), None, None)
+    bits = np.zeros((V, nw), np.uint8)
+    for w in range(nw):
+        bits[:, w] = (words[:, w // 64] >> np.uint64(w % 64)) & np.uint64(1)
+    return bits
+
+
+def _roadmap_finals(fetch, sizes, fns):
+    F = int(sizes[3])
+    ids, masks = np.empty(F, np.int64), np.empty((F, fns.mask_words), np.uint64)
+    fetch(None, None, None, None, None, None, _p(ids), _p(masks))
+    return ids, masks
 
 
 def react_qmdp(ctx, row_ptr, col, xy, cost_to_goals, start_node, belief, common_horizon):

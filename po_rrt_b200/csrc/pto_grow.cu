@@ -17,9 +17,17 @@
 // kd pre-order (the order KdTree::nearest_neighbors returns hits in) is decided by each node's root-to-node branch bits: the first
 // 64 are kept as a key (MSB first), deeper ties -- chains of exact duplicates, e.g. repeated goal samples -- are resolved by
 // walking parent links, so the key length is not capped.
+//
+// porrt_pto_grow_batch grows R roadmaps that differ only in their sampler seed through the same kernels: each keeps its own state
+// (PtoRoad, control block r), the kernels find roadmap r's pointers in device arrays of descriptors, a speculate launch covers
+// every window slot of every roadmap and a commit launch is one CTA per roadmap.  porrt_pto_grow is the batch of one.
 #include <algorithm>
 #include <cmath>
 #include <climits>
+#include <cstring>
+#include <memory>
+#include <string>
+#include <vector>
 
 #include "common.cuh"
 #include "map_dev.cuh"
@@ -36,36 +44,54 @@
 enum { C_V = 0, C_IT, C_W, C_DONE, C_PANIC, C_DRAWN, C_STALL, C_NFIN, C_E, C_WINDOWS, C_RESPEC, C_CONF_NN, C_CONF_RAD, C_NODE_CAP,
        C_EDGE_CAP, C_N };
 
-struct PtoGrow {
+struct PtoRoad {   // one roadmap of a batch: its state, its samples, its speculation scratch and its result
   // roadmap [node_cap]
   DevBuf xy, node_vid, reach, child, parent, depth, key, final_idx, gain, epoch, edge_off, ecnt;
   DevBuf fin_ids, fin_goal, fin_acc;          // finals in add order, the goal each one hit, accumulated finality [words]
   DevBuf log_nbr, log_vid;                    // edge log (neighbour, validity id) grouped by new node, commit order
-  DevBuf samples, worlds, radius;             // iteration i (1-based) at [i - 1]; heuristic_radius(n) at [n]
-  DevBuf goals, goal_masks, ctl;
+  DevBuf samples, worlds;                     // iteration i (1-based) at [i - 1]
   DevBuf spec;                                // per-slot speculation results + hit lists [PG_WMAX * node_cap]
-  DevBuf csr_row, csr_col, csr_vid, work;     // the assembled roadmap + assembly work space
-  int64_t node_cap = 0, edge_cap = 0, drawn_cap = 0, radius_n = 0;
-  int words = 1;
-  // the last result (porrt_pto_fetch)
+  DevBuf csr_row, csr_col, csr_vid;           // the assembled roadmap
+  int64_t node_cap = 0, edge_cap = 0;
+  // the last result (porrt_pto_fetch_roadmap)
   bool have = false;
   int64_t V = 0, E = 0, n_finals = 0;
+  DevBuf* bufs[23] = {&xy, &node_vid, &reach, &child, &parent, &depth, &key, &final_idx, &gain, &epoch, &edge_off, &ecnt, &fin_ids,
+                      &fin_goal, &fin_acc, &log_nbr, &log_vid, &samples, &worlds, &spec, &csr_row, &csr_col, &csr_vid};
+  PtoRoad() = default;
+  PtoRoad(const PtoRoad&) = delete;           // bufs points into this object
+  size_t bytes() const { size_t s = 0; for (DevBuf* b : bufs) s += b->cap; return s; }
+  void release() { for (DevBuf* b : bufs) b->release(); }
+};
+
+struct PtoGrow {
+  std::vector<std::unique_ptr<PtoRoad>> roads;   // the roadmaps of the last batch; a single growth is the batch of one
+  DevBuf radius;                                 // heuristic_radius(n) at [n]
+  DevBuf goals, goal_masks;
+  DevBuf ctl;                                    // control blocks, roadmap r at [r * C_N]
+  DevBuf pg_desc, spec_desc, caps;               // PgDev / SpecDev of every roadmap; node cap, edge cap, samples drawn of each
+  DevBuf work;                                   // CSR assembly work space, one roadmap at a time
+  PinBuf ctl_host;                               // every control block, as the last look saw it
+  std::vector<char> desc_host;                   // what pg_desc + spec_desc hold
+  int64_t radius_n = 0;
+  int words = 1;
+  int32_t n_have = 0;                            // roadmaps of the last batch; 0: nothing grown
   std::vector<uint64_t> goal_masks_host;
 };
 
 void pto_grow_release(porrt_ctx* ctx) {
   PtoGrow* g = ctx->pto;
   if (!g) return;
-  DevBuf* all[] = {&g->xy, &g->node_vid, &g->reach, &g->child, &g->parent, &g->depth, &g->key, &g->final_idx, &g->gain, &g->epoch,
-                   &g->edge_off, &g->ecnt, &g->fin_ids, &g->fin_goal, &g->fin_acc, &g->log_nbr, &g->log_vid, &g->samples, &g->worlds,
-                   &g->radius, &g->goals, &g->goal_masks, &g->ctl, &g->spec, &g->csr_row, &g->csr_col, &g->csr_vid, &g->work};
+  for (auto& r : g->roads) r->release();
+  DevBuf* all[] = {&g->radius, &g->goals, &g->goal_masks, &g->ctl, &g->pg_desc, &g->spec_desc, &g->caps, &g->work};
   for (DevBuf* b : all) b->release();
+  g->ctl_host.release();
   delete g;
   ctx->pto = nullptr;
 }
 
 // ------------------------------------------------------------------------------------------------ device
-struct PgDev {     // roadmap pointers (by value into every kernel)
+struct PgDev {     // one roadmap's pointers; the kernels read roadmap r's from a device array of them
   double2* xy; int32_t* node_vid; uint64_t* reach; int32_t* child; int32_t* parent; int32_t* depth; uint64_t* key;
   int32_t* final_idx; uint64_t* gain; int32_t* epoch; int64_t* edge_off; int32_t* ecnt;
   int32_t* fin_ids; int32_t* fin_goal; uint64_t* fin_acc; int32_t* log_nbr; int32_t* log_vid;
@@ -142,9 +168,11 @@ __device__ __forceinline__ double pg_block_min(double v, double* sh) {
   return r;
 }
 
-// ---- speculate: one CTA per iteration of the window, reading only the committed state S0
+// ---- speculate: one CTA per iteration of the window (blockIdx.x) and roadmap (blockIdx.y), reading only the committed state S0
 template <int KIND>
-__global__ void __launch_bounds__(PG_SPEC_THREADS) pto_speculate_kernel(MapDev m, PgDev g, SpecDev s) {
+__global__ void __launch_bounds__(PG_SPEC_THREADS) pto_speculate_kernel(MapDev m, const PgDev* __restrict__ gs, const SpecDev* __restrict__ ss) {
+  const PgDev& g = gs[blockIdx.y];
+  const SpecDev& s = ss[blockIdx.y];
   __shared__ double sh_d[PG_SPEC_THREADS / 32];
   __shared__ int32_t sh_i[4];
   const int32_t* ctl = g.ctl;
@@ -249,8 +277,10 @@ __device__ __forceinline__ int pg_block_scan(bool f, int* pos, int* sh) {
   return total;
 }
 
-// ---- commit: one CTA walks the window in order, each iteration in the order of pto.rs:79-135
-__global__ void __launch_bounds__(PG_COMMIT_THREADS) pto_commit_kernel(PgDev g, SpecDev s) {
+// ---- commit: one CTA per roadmap walks its window in order, each iteration in the order of pto.rs:79-135
+__global__ void __launch_bounds__(PG_COMMIT_THREADS) pto_commit_kernel(const PgDev* __restrict__ gs, const SpecDev* __restrict__ ss) {
+  const PgDev& g = gs[blockIdx.x];
+  const SpecDev& s = ss[blockIdx.x];
   __shared__ int32_t touched[PG_TOUCH_CAP];
   __shared__ int sh_scan[PG_COMMIT_THREADS / 32];
   __shared__ int32_t n_touched, overflow, conflict_nn, conflict_rad, panic_idx, sh_goal;
@@ -418,8 +448,9 @@ __global__ void __launch_bounds__(PG_COMMIT_THREADS) pto_commit_kernel(PgDev g, 
   }
 }
 
-// start: node 0 (KdTree root, Reachability::set_root) or the panic of expect("Start from a valid state!")
-__global__ void pto_init_kernel(MapDev m, PgDev g, double2 start) {
+// start: node 0 (KdTree root, Reachability::set_root) or the panic of expect("Start from a valid state!"); one CTA per roadmap
+__global__ void pto_init_kernel(MapDev m, const PgDev* __restrict__ gs, double2 start) {
+  const PgDev& g = gs[blockIdx.x];
   const int tid = threadIdx.x;
   int32_t* ctl = g.ctl;
   const int32_t sv = state_validity_of(m, start.x, start.y);
@@ -437,10 +468,17 @@ __global__ void pto_init_kernel(MapDev m, PgDev g, double2 start) {
   }
 }
 
-__global__ void pto_set_kernel(int32_t* ctl, int idx, int32_t v) { ctl[idx] = v; }
-__global__ void pto_fill_i32_kernel(int32_t* p, int64_t n, int32_t v) {
-  const int64_t k = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (k < n) p[k] = v;
+// what the host grew or drew since the last look: caps[3 r ..] = node cap, edge cap, samples drawn of roadmap r
+__global__ void pto_caps_kernel(int32_t* ctl, const int32_t* __restrict__ caps, int n) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  ctl[(size_t)r * C_N + C_NODE_CAP] = caps[3 * r];
+  ctl[(size_t)r * C_N + C_EDGE_CAP] = caps[3 * r + 1];
+  ctl[(size_t)r * C_N + C_DRAWN] = caps[3 * r + 2];
+}
+// every control block into pinned host memory in one look (no DMA engine, like read_flags_dev)
+__global__ void pto_ctl_to_host_kernel(const int32_t* __restrict__ d, int n, volatile int32_t* h) {
+  for (int k = blockIdx.x * blockDim.x + threadIdx.x; k < n; k += gridDim.x * blockDim.x) h[k] = d[k];
 }
 __global__ void pto_set_i64_kernel(int64_t* p, const int32_t* ctl, int idx) { *p = ctl[idx]; }
 
@@ -451,25 +489,26 @@ static double host_heuristic_radius(int64_t n_nodes, double max_step, double sea
   return s < max_step ? s : max_step;
 }
 
-static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, double max_step, double goal_max_dist, int n_goals, int64_t nmin, int64_t nmax) {
-  PgDev d;
-  d.xy = g->xy.as<double2>(); d.node_vid = g->node_vid.as<int32_t>(); d.reach = g->reach.as<uint64_t>(); d.child = g->child.as<int32_t>();
-  d.parent = g->parent.as<int32_t>(); d.depth = g->depth.as<int32_t>(); d.key = g->key.as<uint64_t>(); d.final_idx = g->final_idx.as<int32_t>();
-  d.gain = g->gain.as<uint64_t>(); d.epoch = g->epoch.as<int32_t>(); d.edge_off = g->edge_off.as<int64_t>(); d.ecnt = g->ecnt.as<int32_t>();
-  d.fin_ids = g->fin_ids.as<int32_t>(); d.fin_goal = g->fin_goal.as<int32_t>(); d.fin_acc = g->fin_acc.as<uint64_t>();
-  d.log_nbr = g->log_nbr.as<int32_t>(); d.log_vid = g->log_vid.as<int32_t>();
-  d.samples = g->samples.as<double2>(); d.worlds = g->worlds.as<int32_t>(); d.radius = g->radius.as<double>();
+static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double max_step, double goal_max_dist, int n_goals,
+                    int64_t nmin, int64_t nmax) {
+  PgDev d = {};
+  d.xy = r->xy.as<double2>(); d.node_vid = r->node_vid.as<int32_t>(); d.reach = r->reach.as<uint64_t>(); d.child = r->child.as<int32_t>();
+  d.parent = r->parent.as<int32_t>(); d.depth = r->depth.as<int32_t>(); d.key = r->key.as<uint64_t>(); d.final_idx = r->final_idx.as<int32_t>();
+  d.gain = r->gain.as<uint64_t>(); d.epoch = r->epoch.as<int32_t>(); d.edge_off = r->edge_off.as<int64_t>(); d.ecnt = r->ecnt.as<int32_t>();
+  d.fin_ids = r->fin_ids.as<int32_t>(); d.fin_goal = r->fin_goal.as<int32_t>(); d.fin_acc = r->fin_acc.as<uint64_t>();
+  d.log_nbr = r->log_nbr.as<int32_t>(); d.log_vid = r->log_vid.as<int32_t>();
+  d.samples = r->samples.as<double2>(); d.worlds = r->worlds.as<int32_t>(); d.radius = g->radius.as<double>();
   d.goals = g->goals.as<double2>(); d.goal_masks = g->goal_masks.as<uint64_t>(); d.validities = ctx->d_validities.as<uint64_t>();
-  d.ctl = g->ctl.as<int32_t>();
+  d.ctl = ctl;
   d.words = g->words; d.n_worlds = ctx->n_worlds; d.n_goals = n_goals; d.goal_max_dist = goal_max_dist; d.max_step = max_step;
   d.n_iter_min = nmin; d.n_iter_max = nmax;
   return d;
 }
 
-static SpecDev spec_dev(PtoGrow* g) {
-  SpecDev s;
-  const int64_t W = PG_WMAX, h = g->node_cap;
-  char* p = g->spec.as<char>();
+static SpecDev spec_dev(PtoRoad* r) {
+  SpecDev s = {};
+  const int64_t W = PG_WMAX, h = r->node_cap;
+  char* p = r->spec.as<char>();
   auto take = [&](size_t bytes) { char* q = p; p += (bytes + 15) & ~(size_t)15; return q; };
   s.nn = (int32_t*)take(W * 4); s.nn_d = (double*)take(W * 8); s.q = (double2*)take(W * 16); s.svid = (int32_t*)take(W * 4);
   s.nn_vid = (int32_t*)take(W * 4); s.n_hits = (int32_t*)take(W * 4); s.slot = (int32_t*)take(W * 4);
@@ -479,13 +518,14 @@ static SpecDev spec_dev(PtoGrow* g) {
   return s;
 }
 static size_t spec_bytes(int64_t h) { return (size_t)PG_WMAX * (4 + 8 + 16 + 4 * 4 + (size_t)h * 36) + 16 * 16; }
+static size_t node_bytes(int words) { return 72 + 16 * (size_t)words; }   // every per-node array below, per node
 
 // every per-node array holds node_cap entries, kept across growth (DevBuf::grow_keep)
-static int32_t pg_grow_nodes(porrt_ctx* ctx, PtoGrow* g, int64_t want, int64_t V_now) {
+static int32_t pg_grow_nodes(porrt_ctx* ctx, PtoRoad* g, int words, int64_t want, int64_t V_now) {
   if (want <= g->node_cap) return PORRT_OK;
   const int64_t cap = std::max<int64_t>(want, 2 * g->node_cap);
   cudaStream_t st = ctx->stream;
-  const size_t w8 = (size_t)g->words * 8;
+  const size_t w8 = (size_t)words * 8;
   struct { DevBuf* b; size_t per; } arr[] = {{&g->xy, 16}, {&g->node_vid, 4}, {&g->reach, w8}, {&g->child, 8}, {&g->parent, 4},
       {&g->depth, 4}, {&g->key, 8}, {&g->final_idx, 4}, {&g->gain, w8}, {&g->epoch, 4}, {&g->edge_off, 8}, {&g->ecnt, 4},
       {&g->fin_ids, 4}, {&g->fin_goal, 4}};
@@ -496,8 +536,8 @@ static int32_t pg_grow_nodes(porrt_ctx* ctx, PtoGrow* g, int64_t want, int64_t V
 }
 
 // heuristic_radius(n) for every n a window can reach (host libm, DESIGN.md 4)
-static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, double max_step, double search_radius) {
-  const int64_t rn = g->node_cap + PG_WMAX + 2;
+static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, int64_t node_cap, double max_step, double search_radius) {
+  const int64_t rn = node_cap + PG_WMAX + 2;
   if (rn <= g->radius_n) return PORRT_OK;
   std::vector<double> r((size_t)rn);
   for (int64_t n = 0; n < rn; ++n) r[(size_t)n] = n == 0 ? 0.0 : host_heuristic_radius(n, max_step, search_radius);
@@ -508,22 +548,36 @@ static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, double max_step, doub
   return PORRT_OK;
 }
 
-PORRT_API int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const double low[2], const double up[2], uint64_t sampler_seed,
-                                 const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
-                                 double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
-                                 int64_t* out_sizes, int32_t* out_complete, int32_t* out_panic_code, int64_t* out_counters) {
+// one host sample stream per roadmap: pto.rs:141-149, the continuous and the discrete sampler seeded alike
+struct PgStream {
+  Pcg64 cont, disc;
+  int64_t drawn;
+  std::vector<double> smp;      // the last draw, until its copy has run (the next look synchronises first)
+  std::vector<int32_t> wld;
+};
+
+// PTO::grow_graph for n roadmaps that differ only in their sampler seed.  Every roadmap runs the host decisions and the windows the
+// single growth would run: each look grows its buffers and draws its samples by the same rules, then PG_BATCH windows of every
+// roadmap that is still running go out in one speculate and one commit launch per window.
+static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const uint64_t* seeds, const double start[2], const double low[2],
+                             const double up[2], const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
+                             double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes,
+                             int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters) {
   CTX_CHECK(ctx);
   if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
   if (!start || !low || !up || (n_goals > 0 && (!goals_xy || !goal_masks)) || n_goals < 0 || n_iter_min < 0 || n_iter_max < 0 ||
-      !out_sizes || !out_complete)
-    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_grow: bad arguments");
+      !out_sizes || !out_status || !seeds)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": bad arguments");
+  if (n < 1 || n > PORRT_PTO_MAX_ROADMAPS)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": n_roadmaps must be in 1 .. " + std::to_string(PORRT_PTO_MAX_ROADMAPS));
   if (!ctx->pto) ctx->pto = new PtoGrow();
   PtoGrow* g = ctx->pto;
-  g->have = false;
-  for (int k = 0; k < 4; ++k) out_sizes[k] = 0;
-  *out_complete = 0;
-  if (out_panic_code) *out_panic_code = 0;
-  if (out_counters) for (int k = 0; k < 4; ++k) out_counters[k] = 0;
+  g->n_have = 0;
+  for (auto& r : g->roads) r->have = false;
+  for (int64_t k = 0; k < 4 * (int64_t)n; ++k) out_sizes[k] = 0;
+  for (int32_t r = 0; r < n; ++r) out_status[r] = 0;
+  if (out_panic_code) for (int32_t r = 0; r < n; ++r) out_panic_code[r] = 0;
+  if (out_counters) for (int64_t k = 0; k < 4 * (int64_t)n; ++k) out_counters[k] = 0;
   const int words = ctx->mask_words, n_worlds = ctx->n_worlds;
   // SquareGoal::new (common.rs:304-350): world_to_goal, asserting that no world has two goals (:320)
   std::vector<double> world_goal((size_t)n_worlds * 2, 0.0);
@@ -534,145 +588,266 @@ PORRT_API int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const do
       return porrt_fail(ctx, PORRT_ERR_PANIC, "ContinuousSampler: low < up required (rand asserts it)");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  g->words = words;
-  g->goal_masks_host.assign(goal_masks ? goal_masks : nullptr, goal_masks ? goal_masks + (size_t)n_goals * words : nullptr);
   // the loop runs at least n_iter_min and at most max(n_iter_min, n_iter_max) iterations
   const int64_t bound = std::min<int64_t>(std::max(n_iter_min, n_iter_max), INT32_MAX - 2 * PG_WMAX);
+  const bool runs = 0 < n_iter_min || 0 < n_iter_max;   // the loop condition before the first iteration (no finals yet)
+  const int64_t cap0 = std::min<int64_t>(bound, 4096) + PG_BATCH * PG_WMAX + 1;
+  const int64_t draw0 = runs ? std::min(n_iter_min + 4096, bound) : 0;
+  {  // every roadmap must fit at its starting size: what the buffers below take, growth factors included
+    const double per = 1.5 * (double)(cap0 + 1) * node_bytes(words) + 1.25 * spec_bytes(cap0) + 2 * 1.25 * 64.0 * cap0 +
+                       1.5 * 20.0 * draw0 + 1e5;
+    size_t free_b = 0, total_b = 0;
+    CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
+    double held = 0;
+    for (auto& r : g->roads) held += (double)r->bytes();
+    if ((double)n * per > (double)free_b + held)
+      return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": " + std::to_string(n) + " roadmaps need about " +
+                        std::to_string((int64_t)(n * per / 1e6)) + " MB to start, the device has " +
+                        std::to_string((int64_t)((free_b + held) / 1e6)) + " MB");
+  }
+  for (size_t r = (size_t)n; r < g->roads.size(); ++r) g->roads[r]->release();
+  g->roads.resize((size_t)n);
+  for (auto& r : g->roads) if (!r) r.reset(new PtoRoad());
+  g->words = words;
+  g->goal_masks_host.assign(goal_masks ? goal_masks : nullptr, goal_masks ? goal_masks + (size_t)n_goals * words : nullptr);
   // buffers: nodes grow with the roadmap, samples are drawn ahead of the windows
-  g->node_cap = 0; g->radius_n = 0;
-  int32_t rc = pg_grow_nodes(ctx, g, std::min<int64_t>(bound, 4096) + PG_BATCH * PG_WMAX + 1, 0);
-  if (rc) return rc;
-  rc = pg_radius_table(ctx, g, max_step, search_radius);
-  if (rc) return rc;
-  g->edge_cap = std::max<int64_t>(g->edge_cap, 16 * g->node_cap);
-  CUDA_TRY(ctx, g->log_nbr.ensure((size_t)g->edge_cap * 4));
-  CUDA_TRY(ctx, g->log_vid.ensure((size_t)g->edge_cap * 4));
-  CUDA_TRY(ctx, g->fin_acc.ensure((size_t)words * 8));
+  g->radius_n = 0;
+  int32_t rc;
+  for (auto& rp : g->roads) {
+    PtoRoad* r = rp.get();
+    r->node_cap = 0;
+    if ((rc = pg_grow_nodes(ctx, r, words, cap0, 0))) return rc;
+    r->edge_cap = std::max<int64_t>(r->edge_cap, 16 * r->node_cap);
+    CUDA_TRY(ctx, r->log_nbr.ensure((size_t)r->edge_cap * 4));
+    CUDA_TRY(ctx, r->log_vid.ensure((size_t)r->edge_cap * 4));
+    CUDA_TRY(ctx, r->fin_acc.ensure((size_t)words * 8));
+  }
+  if ((rc = pg_radius_table(ctx, g, cap0, max_step, search_radius))) return rc;
   CUDA_TRY(ctx, g->goals.ensure((size_t)std::max(n_goals, 1) * 16));
   CUDA_TRY(ctx, g->goal_masks.ensure((size_t)std::max(n_goals, 1) * words * 8));
-  CUDA_TRY(ctx, g->ctl.ensure(C_N * 4 + 64));
+  CUDA_TRY(ctx, g->ctl.ensure((size_t)n * C_N * 4 + 64));
+  CUDA_TRY(ctx, g->ctl_host.ensure((size_t)n * C_N * 4));
+  CUDA_TRY(ctx, g->caps.ensure((size_t)n * 3 * 4));
+  CUDA_TRY(ctx, g->pg_desc.ensure((size_t)n * sizeof(PgDev)));
+  CUDA_TRY(ctx, g->spec_desc.ensure((size_t)n * sizeof(SpecDev)));
   if (n_goals > 0) {
     CUDA_TRY(ctx, cudaMemcpyAsync(g->goals.p, goals_xy, (size_t)n_goals * 16, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(g->goal_masks.p, goal_masks, (size_t)n_goals * words * 8, cudaMemcpyHostToDevice, st));
   }
+  int32_t* ctl = g->ctl.as<int32_t>();
+  // the descriptors, re-uploaded whenever a buffer moved
+  std::vector<char> desc((size_t)n * (sizeof(PgDev) + sizeof(SpecDev)));
+  g->desc_host.clear();
+  auto upload_desc = [&]() -> int32_t {
+    PgDev* pd = (PgDev*)desc.data();
+    SpecDev* sd = (SpecDev*)(desc.data() + (size_t)n * sizeof(PgDev));
+    for (int32_t r = 0; r < n; ++r) {
+      pd[r] = pg_dev(ctx, g, g->roads[r].get(), ctl + (size_t)r * C_N, max_step, goal_max_dist, n_goals, n_iter_min, n_iter_max);
+      sd[r] = spec_dev(g->roads[r].get());
+    }
+    if (desc == g->desc_host) return PORRT_OK;
+    CUDA_TRY(ctx, cudaMemcpyAsync(g->pg_desc.p, pd, (size_t)n * sizeof(PgDev), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(g->spec_desc.p, sd, (size_t)n * sizeof(SpecDev), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));   // desc is rewritten at the next look
+    g->desc_host = desc;
+    return PORRT_OK;
+  };
+  // node cap, edge cap and samples drawn of every roadmap into its control block, when one of them changed
+  std::vector<int32_t> caps((size_t)n * 3, 0), caps_dev((size_t)n * 3, -1);
+  auto upload_caps = [&]() -> int32_t {
+    for (int32_t r = 0; r < n; ++r) {
+      caps[3 * (size_t)r] = (int32_t)std::min<int64_t>(g->roads[r]->node_cap, INT32_MAX);
+      caps[3 * (size_t)r + 1] = (int32_t)std::min<int64_t>(g->roads[r]->edge_cap, INT32_MAX);
+    }
+    if (caps == caps_dev) return PORRT_OK;
+    CUDA_TRY(ctx, cudaMemcpyAsync(g->caps.p, caps.data(), caps.size() * 4, cudaMemcpyHostToDevice, st));
+    pto_caps_kernel<<<div_up(n, 128), 128, 0, st>>>(ctl, g->caps.as<int32_t>(), n);
+    LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));   // caps is rewritten at the next look
+    caps_dev = caps;
+    return PORRT_OK;
+  };
+  std::vector<PgStream> hs;
+  hs.reserve((size_t)n);
+  for (int32_t r = 0; r < n; ++r) hs.push_back(PgStream{Pcg64::seed_from_u64(seeds[r]), Pcg64::seed_from_u64(seeds[r]), 0, {}, {}});
   // pto.rs:141-149: one discrete draw per iteration, a continuous draw only when i % 100 != 0 (then goal_example(world))
-  Pcg64 cont = Pcg64::seed_from_u64(sampler_seed), disc = Pcg64::seed_from_u64(sampler_seed);
-  std::vector<double> smp;
-  std::vector<int32_t> wld;
-  int64_t drawn = 0;
-  auto draw = [&](int64_t upto) -> int32_t {
+  auto draw = [&](int32_t r, int64_t upto) -> int32_t {
+    PgStream& h = hs[(size_t)r];
+    PtoRoad* d = g->roads[r].get();
     upto = std::min(upto, bound);
-    if (upto <= drawn) return PORRT_OK;
-    const int64_t n = upto - drawn;
-    smp.resize((size_t)n * 2); wld.resize((size_t)n);
-    for (int64_t k = 0; k < n; ++k) {
-      const int64_t i = drawn + k + 1;
-      const int32_t w = (int32_t)disc.below((uint64_t)n_worlds);
-      wld[(size_t)k] = w;
-      if (i % 100 == 0) { smp[2 * k] = world_goal[2 * (size_t)w]; smp[2 * k + 1] = world_goal[2 * (size_t)w + 1]; }
-      else { smp[2 * k] = cont.range_f64(low[0], up[0]); smp[2 * k + 1] = cont.range_f64(low[1], up[1]); }
+    if (upto <= h.drawn) return PORRT_OK;
+    const int64_t m = upto - h.drawn;
+    h.smp.resize((size_t)m * 2); h.wld.resize((size_t)m);
+    for (int64_t k = 0; k < m; ++k) {
+      const int64_t i = h.drawn + k + 1;
+      const int32_t w = (int32_t)h.disc.below((uint64_t)n_worlds);
+      h.wld[(size_t)k] = w;
+      if (i % 100 == 0) { h.smp[2 * k] = world_goal[2 * (size_t)w]; h.smp[2 * k + 1] = world_goal[2 * (size_t)w + 1]; }
+      else { h.smp[2 * k] = h.cont.range_f64(low[0], up[0]); h.smp[2 * k + 1] = h.cont.range_f64(low[1], up[1]); }
     }
-    CUDA_TRY(ctx, g->samples.grow_keep((size_t)upto * 16, (size_t)drawn * 16, st));
-    CUDA_TRY(ctx, g->worlds.grow_keep((size_t)upto * 4, (size_t)drawn * 4, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(g->samples.as<double>() + 2 * drawn, smp.data(), (size_t)n * 16, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(g->worlds.as<int32_t>() + drawn, wld.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));   // the host vectors are reused by the next draw
-    drawn = upto;
-    pto_set_kernel<<<1, 1, 0, st>>>(g->ctl.as<int32_t>(), C_DRAWN, (int32_t)drawn);
-    LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, d->samples.grow_keep((size_t)upto * 16, (size_t)h.drawn * 16, st));
+    CUDA_TRY(ctx, d->worlds.grow_keep((size_t)upto * 4, (size_t)h.drawn * 4, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d->samples.as<double>() + 2 * h.drawn, h.smp.data(), (size_t)m * 16, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d->worlds.as<int32_t>() + h.drawn, h.wld.data(), (size_t)m * 4, cudaMemcpyHostToDevice, st));
+    h.drawn = upto;
+    caps[3 * (size_t)r + 2] = (int32_t)upto;
     return PORRT_OK;
   };
-  auto set_caps = [&]() -> int32_t {
-    pto_set_kernel<<<1, 1, 0, st>>>(g->ctl.as<int32_t>(), C_NODE_CAP, (int32_t)std::min<int64_t>(g->node_cap, INT32_MAX));
+  auto look = [&](int32_t* f) -> int32_t {   // every control block
+    volatile int32_t* h = g->ctl_host.as<int32_t>();
+    const int m = n * C_N;
+    pto_ctl_to_host_kernel<<<std::min(div_up(m, 256), 64), 256, 0, st>>>(ctl, m, h);
     LAUNCH_CHECK(ctx);
-    pto_set_kernel<<<1, 1, 0, st>>>(g->ctl.as<int32_t>(), C_EDGE_CAP, (int32_t)std::min<int64_t>(g->edge_cap, INT32_MAX));
-    LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    for (int k = 0; k < m; ++k) f[k] = h[k];
     return PORRT_OK;
   };
-  PgDev d = pg_dev(ctx, g, max_step, goal_max_dist, n_goals, n_iter_min, n_iter_max);
-  pto_init_kernel<<<1, 64, 0, st>>>(ctx->map, d, make_double2(start[0], start[1]));
+  if ((rc = upload_desc())) return rc;
+  pto_init_kernel<<<n, 64, 0, st>>>(ctx->map, g->pg_desc.as<PgDev>(), make_double2(start[0], start[1]));
   LAUNCH_CHECK(ctx);
-  if ((rc = set_caps())) return rc;
-  const bool runs = 0 < n_iter_min || 0 < n_iter_max;   // the loop condition before the first iteration (no finals yet)
-  if (runs && (rc = draw(n_iter_min + 4096))) return rc;
-  int32_t f[C_N];
+  if (runs) for (int32_t r = 0; r < n; ++r) if ((rc = draw(r, n_iter_min + 4096))) return rc;
+  if ((rc = upload_caps())) return rc;
+  std::vector<int32_t> fv((size_t)n * C_N);
+  int32_t* f = fv.data();
   for (;;) {
-    if ((rc = read_flags_dev(ctx, g->ctl.as<int32_t>(), C_N, f, st))) return rc;
-    if (f[C_DONE] || !runs) break;
-    const int64_t V = f[C_V], it = f[C_IT];
-    if (it >= bound) break;
-    // room for the next batch of windows: nodes (every commit adds at most one), edges (the commit stalls when they run out)
-    if (V + PG_BATCH * PG_WMAX + 1 > g->node_cap) {
-      if ((rc = pg_grow_nodes(ctx, g, V + PG_BATCH * PG_WMAX + 1, V))) return rc;
-      if ((rc = pg_radius_table(ctx, g, max_step, search_radius))) return rc;
-      if ((rc = set_caps())) return rc;
+    if ((rc = look(f))) return rc;
+    if (!runs) break;
+    bool running = false;
+    int64_t node_cap = 0;
+    for (int32_t r = 0; r < n; ++r) {
+      const int32_t* fr = f + (size_t)r * C_N;
+      PtoRoad* d = g->roads[r].get();
+      if (!fr[C_DONE] && fr[C_IT] < bound) {
+        running = true;
+        const int64_t V = fr[C_V], it = fr[C_IT];
+        // room for the next batch of windows: nodes (every commit adds at most one), edges (the commit stalls when they run out)
+        if (V + PG_BATCH * PG_WMAX + 1 > d->node_cap && (rc = pg_grow_nodes(ctx, d, words, V + PG_BATCH * PG_WMAX + 1, V))) return rc;
+        if (fr[C_STALL] || (int64_t)fr[C_E] + 64 * PG_BATCH * PG_WMAX > d->edge_cap) {
+          const int64_t want = std::max<int64_t>(2 * d->edge_cap, (int64_t)fr[C_E] + V + 1 + 64 * PG_BATCH * PG_WMAX);
+          CUDA_TRY(ctx, d->log_nbr.grow_keep((size_t)want * 4, (size_t)fr[C_E] * 4, st));
+          CUDA_TRY(ctx, d->log_vid.grow_keep((size_t)want * 4, (size_t)fr[C_E] * 4, st));
+          d->edge_cap = want;
+        }
+        const int64_t drawn = hs[(size_t)r].drawn;
+        if (drawn < bound && drawn - it < 2 * PG_BATCH * PG_WMAX && (rc = draw(r, drawn + std::max<int64_t>(4096, drawn / 2)))) return rc;
+      }
+      node_cap = std::max(node_cap, d->node_cap);
     }
-    if (f[C_STALL] || (int64_t)f[C_E] + 64 * PG_BATCH * PG_WMAX > g->edge_cap) {
-      const int64_t want = std::max<int64_t>(2 * g->edge_cap, (int64_t)f[C_E] + V + 1 + 64 * PG_BATCH * PG_WMAX);
-      CUDA_TRY(ctx, g->log_nbr.grow_keep((size_t)want * 4, (size_t)f[C_E] * 4, st));
-      CUDA_TRY(ctx, g->log_vid.grow_keep((size_t)want * 4, (size_t)f[C_E] * 4, st));
-      g->edge_cap = want;
-      if ((rc = set_caps())) return rc;
-    }
-    if (drawn < bound && drawn - it < 2 * PG_BATCH * PG_WMAX && (rc = draw(drawn + std::max<int64_t>(4096, drawn / 2)))) return rc;
-    d = pg_dev(ctx, g, max_step, goal_max_dist, n_goals, n_iter_min, n_iter_max);
-    const SpecDev s = spec_dev(g);
+    if (!running) break;
+    if ((rc = pg_radius_table(ctx, g, node_cap, max_step, search_radius))) return rc;
+    if ((rc = upload_caps())) return rc;
+    if ((rc = upload_desc())) return rc;
+    const PgDev* pd = g->pg_desc.as<PgDev>();
+    const SpecDev* sd = g->spec_desc.as<SpecDev>();
     for (int k = 0; k < PG_BATCH; ++k) {
-      if (ctx->map.kind == PORRT_DOMAIN_SHELF) pto_speculate_kernel<PORRT_DOMAIN_SHELF><<<PG_WMAX, PG_SPEC_THREADS, 0, st>>>(ctx->map, d, s);
-      else pto_speculate_kernel<PORRT_DOMAIN_DOOR><<<PG_WMAX, PG_SPEC_THREADS, 0, st>>>(ctx->map, d, s);
+      if (ctx->map.kind == PORRT_DOMAIN_SHELF) pto_speculate_kernel<PORRT_DOMAIN_SHELF><<<dim3(PG_WMAX, n), PG_SPEC_THREADS, 0, st>>>(ctx->map, pd, sd);
+      else pto_speculate_kernel<PORRT_DOMAIN_DOOR><<<dim3(PG_WMAX, n), PG_SPEC_THREADS, 0, st>>>(ctx->map, pd, sd);
       LAUNCH_CHECK(ctx);
-      pto_commit_kernel<<<1, PG_COMMIT_THREADS, 0, st>>>(d, s);
+      pto_commit_kernel<<<n, PG_COMMIT_THREADS, 0, st>>>(pd, sd);
       LAUNCH_CHECK(ctx);
     }
   }
-  const int64_t V = f[C_V], E = f[C_E];
-  out_sizes[0] = f[C_IT];
-  if (out_counters) { out_counters[0] = f[C_WINDOWS]; out_counters[1] = f[C_RESPEC]; out_counters[2] = f[C_CONF_NN]; out_counters[3] = f[C_CONF_RAD]; }
-  if (f[C_DONE] == 2) {
-    if (out_panic_code) *out_panic_code = f[C_PANIC];
-    const bool at_start = f[C_WINDOWS] == 0;   // the init kernel found the start invalid: no window ever ran
-    out_sizes[0] = at_start ? 0 : f[C_IT] + 1;  // the iteration whose check panicked
-    return porrt_fail(ctx, PORRT_ERR_PANIC, at_start ? "Start from a valid state! (pto.rs:57, state validity code " + std::to_string(f[C_PANIC]) + ")"
-                                                     : "porrt_pto_grow: a state / edge check hit a reference panic (code " + std::to_string(f[C_PANIC]) + ")");
+  // per roadmap: outputs, then the children CSR from the edge log (graph.cu's late-list kernels, carrying the validity ids)
+  size_t work = 64;
+  for (int32_t r = 0; r < n; ++r) {
+    const int32_t* fr = f + (size_t)r * C_N;
+    int64_t* sz = out_sizes + 4 * (size_t)r;
+    sz[0] = fr[C_IT];
+    if (out_counters) {
+      int64_t* c = out_counters + 4 * (size_t)r;
+      c[0] = fr[C_WINDOWS]; c[1] = fr[C_RESPEC]; c[2] = fr[C_CONF_NN]; c[3] = fr[C_CONF_RAD];
+    }
+    if (fr[C_DONE] == 2) {
+      out_status[r] = PORRT_ERR_PANIC;
+      if (out_panic_code) out_panic_code[r] = fr[C_PANIC];
+      sz[0] = fr[C_WINDOWS] == 0 ? 0 : fr[C_IT] + 1;   // the iteration whose check panicked; 0: the init kernel found the start invalid
+      continue;
+    }
+    const int64_t V = fr[C_V], E = fr[C_E];
+    work = std::max(work, (size_t)V * 8 + (size_t)(V + 1) * 8 + (size_t)std::max<int64_t>(E, 1) * 4 + 64);
   }
-  // the children CSR from the edge log (graph.cu's late-list kernels, carrying the validity ids)
-  CUDA_TRY(ctx, g->csr_row.ensure((size_t)(V + 1) * 8));
-  CUDA_TRY(ctx, g->csr_col.ensure((size_t)std::max<int64_t>(2 * E, 1) * 4));
-  CUDA_TRY(ctx, g->csr_vid.ensure((size_t)std::max<int64_t>(2 * E, 1) * 4));
-  CUDA_TRY(ctx, g->work.ensure((size_t)V * 8 + (size_t)(V + 1) * 8 + (size_t)std::max<int64_t>(E, 1) * 4 + 64));
-  int32_t* late_cnt = g->work.as<int32_t>();
-  int32_t* cursor = late_cnt + V;
-  int64_t* late_off = (int64_t*)(cursor + V);
-  int32_t* late_vals = (int32_t*)(late_off + V + 1);
-  pto_set_i64_kernel<<<1, 1, 0, st>>>(g->edge_off.as<int64_t>() + V, g->ctl.as<int32_t>(), C_E);
-  LAUNCH_CHECK(ctx);
-  rc = late_list_csr_dev(ctx, g->edge_off.as<int64_t>(), V, g->log_nbr.as<int32_t>(), g->ecnt.as<int32_t>(), g->log_vid.as<int32_t>(),
-                         late_cnt, cursor, late_off, late_vals, g->csr_row.as<int64_t>(), g->csr_col.as<int32_t>(), g->csr_vid.as<int32_t>());
-  if (rc) return rc;
-  std::vector<uint64_t> fin((size_t)words);
-  CUDA_TRY(ctx, cudaMemcpyAsync(fin.data(), g->fin_acc.p, (size_t)words * 8, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, g->work.ensure(work));
+  std::vector<uint64_t> fin((size_t)n * words);
+  for (int32_t r = 0; r < n; ++r) {
+    const int32_t* fr = f + (size_t)r * C_N;
+    if (out_status[r] == PORRT_ERR_PANIC) continue;
+    PtoRoad* d = g->roads[r].get();
+    const int64_t V = fr[C_V], E = fr[C_E];
+    CUDA_TRY(ctx, d->csr_row.ensure((size_t)(V + 1) * 8));
+    CUDA_TRY(ctx, d->csr_col.ensure((size_t)std::max<int64_t>(2 * E, 1) * 4));
+    CUDA_TRY(ctx, d->csr_vid.ensure((size_t)std::max<int64_t>(2 * E, 1) * 4));
+    int32_t* late_cnt = g->work.as<int32_t>();
+    int32_t* cursor = late_cnt + V;
+    int64_t* late_off = (int64_t*)(cursor + V);
+    int32_t* late_vals = (int32_t*)(late_off + V + 1);
+    pto_set_i64_kernel<<<1, 1, 0, st>>>(d->edge_off.as<int64_t>() + V, ctl + (size_t)r * C_N, C_E);
+    LAUNCH_CHECK(ctx);
+    rc = late_list_csr_dev(ctx, d->edge_off.as<int64_t>(), V, d->log_nbr.as<int32_t>(), d->ecnt.as<int32_t>(), d->log_vid.as<int32_t>(),
+                           late_cnt, cursor, late_off, late_vals, d->csr_row.as<int64_t>(), d->csr_col.as<int32_t>(), d->csr_vid.as<int32_t>());
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(fin.data() + (size_t)r * words, d->fin_acc.p, (size_t)words * 8, cudaMemcpyDeviceToHost, st));
+  }
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
-  bool complete = f[C_NFIN] > 0;
-  for (int w = 0; w < words; ++w) {
-    const int rem = n_worlds - 64 * w;
-    const uint64_t want = rem >= 64 ? ~0ull : ((1ull << rem) - 1ull);
-    if ((fin[(size_t)w] & want) != want) complete = false;
+  for (int32_t r = 0; r < n; ++r) {
+    if (out_status[r] == PORRT_ERR_PANIC) continue;
+    const int32_t* fr = f + (size_t)r * C_N;
+    PtoRoad* d = g->roads[r].get();
+    bool complete = fr[C_NFIN] > 0;
+    for (int w = 0; w < words; ++w) {
+      const int rem = n_worlds - 64 * w;
+      const uint64_t want = rem >= 64 ? ~0ull : ((1ull << rem) - 1ull);
+      if ((fin[(size_t)r * words + w] & want) != want) complete = false;
+    }
+    d->have = true; d->V = fr[C_V]; d->E = 2 * (int64_t)fr[C_E]; d->n_finals = fr[C_NFIN];
+    int64_t* sz = out_sizes + 4 * (size_t)r;
+    sz[1] = d->V; sz[2] = d->E; sz[3] = d->n_finals;
+    out_status[r] = complete ? 0 : 1;
   }
-  g->have = true; g->V = V; g->E = 2 * E; g->n_finals = f[C_NFIN];
-  out_sizes[1] = V; out_sizes[2] = 2 * E; out_sizes[3] = f[C_NFIN];
-  *out_complete = complete ? 1 : 0;
+  g->n_have = n;
   return PORRT_OK;
 }
 
-PORRT_API int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
-                                  int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks) {
+PORRT_API int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const double low[2], const double up[2], uint64_t sampler_seed,
+                                 const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
+                                 double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
+                                 int64_t* out_sizes, int32_t* out_complete, int32_t* out_panic_code, int64_t* out_counters) {
   CTX_CHECK(ctx);
-  PtoGrow* g = ctx->pto;
-  if (!g || !g->have) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_fetch: no roadmap grown on this ctx");
+  if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
+  if (!out_complete) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_grow: bad arguments");
+  int32_t status = 0, panic = 0;
+  const int32_t rc = pto_grow_impl(ctx, "porrt_pto_grow", 1, &sampler_seed, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
+                                   max_step, search_radius, n_iter_min, n_iter_max, out_sizes, &status, &panic, out_counters);
+  *out_complete = rc == PORRT_OK && status == 0 ? 1 : 0;
+  if (rc) return rc;
+  if (out_panic_code) *out_panic_code = panic;
+  if (status != PORRT_ERR_PANIC) return PORRT_OK;
+  return porrt_fail(ctx, PORRT_ERR_PANIC, out_sizes[0] == 0 ? "Start from a valid state! (pto.rs:57, state validity code " + std::to_string(panic) + ")"
+                                                            : "porrt_pto_grow: a state / edge check hit a reference panic (code " + std::to_string(panic) + ")");
+}
+
+PORRT_API int32_t porrt_pto_grow_batch(porrt_ctx* ctx, int32_t n_roadmaps, const uint64_t* sampler_seeds, const double start[2],
+                                       const double low[2], const double up[2], const double* goals_xy, const uint64_t* goal_masks,
+                                       int32_t n_goals, double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min,
+                                       int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code,
+                                       int64_t* out_counters) {
+  return pto_grow_impl(ctx, "porrt_pto_grow_batch", n_roadmaps, sampler_seeds, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
+                       max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
+}
+
+PORRT_API int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr,
+                                          int32_t* out_col, int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids,
+                                          uint64_t* out_final_masks) {
+  CTX_CHECK(ctx);
+  PtoGrow* pg = ctx->pto;
+  if (!pg || pg->n_have == 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_fetch: no roadmap grown on this ctx");
+  if (r < 0 || r >= pg->n_have)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_fetch_roadmap: roadmap " + std::to_string(r) + " of " + std::to_string(pg->n_have));
+  const PtoRoad* g = pg->roads[r].get();
+  if (!g->have) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_fetch: roadmap " + std::to_string(r) + " panicked");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const int64_t V = g->V, E = g->E, F = g->n_finals;
-  const size_t words = (size_t)g->words;
+  const size_t words = (size_t)pg->words;
   if (out_xy) CUDA_TRY(ctx, cudaMemcpyAsync(out_xy, g->xy.p, (size_t)V * 16, cudaMemcpyDeviceToHost, st));
   if (out_node_vid) CUDA_TRY(ctx, cudaMemcpyAsync(out_node_vid, g->node_vid.p, (size_t)V * 4, cudaMemcpyDeviceToHost, st));
   if (out_row_ptr) CUDA_TRY(ctx, cudaMemcpyAsync(out_row_ptr, g->csr_row.p, (size_t)(V + 1) * 8, cudaMemcpyDeviceToHost, st));
@@ -687,7 +862,12 @@ PORRT_API int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_n
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
   for (int64_t k = 0; k < F; ++k) {
     if (out_final_ids) out_final_ids[k] = ids[(size_t)k];
-    if (out_final_masks) memcpy(out_final_masks + (size_t)k * words, g->goal_masks_host.data() + (size_t)goal[(size_t)k] * words, words * 8);
+    if (out_final_masks) memcpy(out_final_masks + (size_t)k * words, pg->goal_masks_host.data() + (size_t)goal[(size_t)k] * words, words * 8);
   }
   return PORRT_OK;
+}
+
+PORRT_API int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
+                                  int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks) {
+  return porrt_pto_fetch_roadmap(ctx, 0, out_xy, out_node_vid, out_row_ptr, out_col, out_edge_vid, out_reach, out_final_ids, out_final_masks);
 }
