@@ -14,8 +14,6 @@
 // Panics of the reference become PORRT_ERR_PANIC: a parent of a reached node with Unknown type (:139-141) or an Observation
 // node with a child of p <= 0 (:130) -- such nodes are never updated (the reference stops at their first evaluation), and the
 // call fails iff one of them has a child with a finite distance, which is exactly when the reference would have evaluated it.
-#include <map>
-
 #include <math_constants.h>
 
 #include "common.cuh"
@@ -216,55 +214,18 @@ PORRT_API int32_t porrt_extract_policy_graph_nd(porrt_ctx* ctx, int32_t dim, int
   if (V <= 0) return porrt_fail(ctx, PORRT_ERR_PANIC, "no belief state graph! (belief_graph.rs:186)");
   if (!dist || !graph_args_ok(V, row_ptr, col, xy, node_type, belief_id, beliefs, B, n_worlds, dim))
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "extract_policy_graph: bad arguments");
-  const int nw = n_worlds;
-  auto norm2 = [&](int64_t a, int64_t c) {
-    double d2 = 0.0;
-    for (int k = 0; k < dim; ++k) { const double dx = xy[dim * c + k] - xy[dim * a + k]; d2 += dx * dx; }
-    return std::sqrt(d2);
-  };
-  auto tp = [&](int64_t parent, int64_t child) {
-    const double* bp = beliefs + (size_t)belief_id[parent] * nw;
-    const double* bc = beliefs + (size_t)belief_id[child] * nw;
-    double s = 0.0;
-    for (int i = 0; i < nw; ++i) s = s + (bc[i] > 0.0 ? bp[i] : 0.0);
-    return s;
-  };
-  struct PN { int32_t node, parent; uint8_t leaf; };
-  std::vector<PN> pol;
-  std::vector<std::pair<int64_t, int64_t>> lifo;   // (policy node, belief node)
-  pol.push_back({0, -1, 0});
-  lifo.push_back({0, 0});
-  struct Child { int64_t id; double cost_to_child, expected_from_child; };
-  while (!lifo.empty()) {
-    const auto top = lifo.back();
-    lifo.pop_back();
-    const int64_t bn = top.second;
-    std::map<int32_t, std::vector<Child>> by_belief;   // BTreeMap keyed by child.belief_id (:228-241)
-    for (int64_t e = row_ptr[bn]; e < row_ptr[bn + 1]; ++e) {
-      const int64_t c = col[e];
-      by_belief[belief_id[c]].push_back({c, norm2(bn, c), dist[c]});
-    }
-    for (auto& kv : by_belief) {
-      int64_t best_id = kv.second[0].id;
-      const double p = tp(bn, best_id);
-      if (!(p > 0.0)) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p > 0.0) (belief_graph.rs:250)");
-      double best_cost = std::numeric_limits<double>::infinity();
-      for (const Child& c : kv.second) {
-        const double cost = p * (c.cost_to_child + c.expected_from_child);
-        if (cost < best_cost) { best_cost = cost; best_id = c.id; }
-      }
-      if (!(p * dist[best_id] <= dist[bn])) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p * cost[best] <= cost[node]) (belief_graph.rs:261)");
-      const bool leaf = dist[best_id] == 0.0;
-      const int64_t pid = (int64_t)pol.size();
-      pol.push_back({(int32_t)best_id, (int32_t)top.first, (uint8_t)leaf});
-      if (!leaf) lifo.push_back({pid, best_id});
-      if ((int64_t)pol.size() > 64 * V + 1024) return porrt_fail(ctx, PORRT_ERR_PANIC, "extract_policy_graph: policy does not terminate");
-    }
-  }
+  std::vector<PolicyNode> pol;
+  const int32_t rc = get_best_expected_children(
+      ctx, "extract_policy_graph", V, beliefs, n_worlds,
+      [&](int64_t id, auto&& fn) { for (int64_t e = row_ptr[id]; e < row_ptr[id + 1]; ++e) fn((int64_t)col[e]); },
+      [&](int64_t id) { return belief_id[id]; },
+      [&](int64_t a, int64_t c) { return norm2(xy + dim * a, xy + dim * c, dim); },
+      [&](int64_t id) { return dist[id]; }, pol);
+  if (rc) return rc;
   if (out_n) *out_n = (int64_t)pol.size();
   if (out_expected_cost) *out_expected_cost = dist[0];
   if ((int64_t)pol.size() > cap || !out_belief_node || !out_parent || !out_is_leaf)
     return porrt_fail(ctx, PORRT_ERR_CAPACITY, "extract_policy_graph: cap too small");
-  for (size_t k = 0; k < pol.size(); ++k) { out_belief_node[k] = pol[k].node; out_parent[k] = pol[k].parent; out_is_leaf[k] = pol[k].leaf; }
+  for (size_t k = 0; k < pol.size(); ++k) { out_belief_node[k] = (int32_t)pol[k].id; out_parent[k] = pol[k].parent; out_is_leaf[k] = pol[k].leaf; }
   return PORRT_OK;
 }

@@ -1,10 +1,14 @@
-// common.cuh -- context, error handling and device-buffer plumbing shared by the libporrt_b200 translation units.
+// common.cuh -- context, error handling, device-buffer plumbing and the reference's host formulas shared by the libporrt_b200
+// translation units.
 #pragma once
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <cmath>
 #include <cstdio>
 #include <cstring>
+#include <limits>
+#include <map>
 #include <string>
 #include <vector>
 
@@ -127,13 +131,13 @@ struct porrt_ctx {
   int32_t nn_fb_n = 0;   // queries of the last tile pass left to the thread-per-query kernels
   int32_t reach_words = 1;  // u64 words per vertex of the reachability filter of the running NN call
 
-  // ---- last belief VI result (graph.cu), kept for porrt_extract_policy
+  // ---- last belief VI result (graph.cu), kept for porrt_extract_policy, porrt_belief_result and the refiners (refine.cu)
   struct BeliefState_ {
     int64_t V = 0; int32_t B = 0, n_worlds = 0;
     std::vector<int64_t> row_ptr; std::vector<int32_t> col, edge_vid; std::vector<double> xy;
+    std::vector<int32_t> node_vid;                // [V] validity id of each roadmap node
     std::vector<double> beliefs;
     const double* dist = nullptr; const uint8_t* type = nullptr;   // live in ctx->pin[3] (pinned: the V*B table comes back by DMA)
-    std::vector<uint8_t> exists;                  // [V*B]
     std::vector<int32_t> node_obs_set;            // [V] index into obs tables
     std::vector<int64_t> succ_ptr;                // [(n_sets*B)+1]
     std::vector<int32_t> succ_belief;             // successor belief ids
@@ -147,8 +151,43 @@ struct porrt_ctx {
     std::vector<int32_t> colpos;
     std::vector<std::vector<double>> col_dist;    // [B] lazily fetched columns (empty = not fetched)
     std::vector<std::vector<uint8_t>> col_type;
+    bool fetch_failed = false;                    // a column fetch failed since the caller last cleared this
+
+    // Value and node type of belief node id = node * B + belief: from the host table, or from the belief's column, fetched from
+    // the device on first use (a policy touches a few dozen of the B columns, 8 * V bytes each).  A failed fetch reads as 0.
+    double value(porrt_ctx* ctx, int64_t id) {
+      if (on_host) return dist[(size_t)id];
+      const int b = (int)(id % B);
+      return column(ctx, b) ? col_dist[(size_t)b][(size_t)(id / B)] : 0.0;
+    }
+    uint8_t node_type(porrt_ctx* ctx, int64_t id) {
+      if (on_host) return type[(size_t)id];
+      const int b = (int)(id % B);
+      return column(ctx, b) ? col_type[(size_t)b][(size_t)(id / B)] : (uint8_t)0;
+    }
+    // fn(child id) for the children of belief node id in the reference's stored order (pto.rs:206-255): an Observation node's
+    // successor beliefs compatible with its node's validity, or an Action node's edges whose end and edge validity its belief allows
+    template <class F> void for_children(porrt_ctx* ctx, int64_t id, F&& fn) {
+      const int64_t n = id / B;
+      const int b = (int)(id % B);
+      const uint8_t ty = node_type(ctx, id);
+      if (ty == PORRT_NODE_OBSERVATION) {
+        const int64_t sp = (int64_t)node_obs_set[(size_t)n] * B + b;
+        for (int64_t k = succ_ptr[(size_t)sp]; k < succ_ptr[(size_t)sp + 1]; ++k) {
+          const int32_t cb = succ_belief[(size_t)k];
+          if (compat[(size_t)cb * n_validities + node_vid[(size_t)n]]) fn(n * B + cb);
+        }
+      } else if (ty == PORRT_NODE_ACTION) {
+        for (int64_t e = row_ptr[(size_t)n]; e < row_ptr[(size_t)n + 1]; ++e) {
+          const int32_t c = col[(size_t)e];
+          if (compat[(size_t)b * n_validities + node_vid[(size_t)c]] && compat[(size_t)b * n_validities + edge_vid[(size_t)e]]) fn((int64_t)c * B + b);
+        }
+      }
+    }
+    // whether column b is on the host, fetching it if need be (graph.cu); a failed fetch leaves it unfetched and sets fetch_failed
+    bool column(porrt_ctx* ctx, int b) { return !col_dist[(size_t)b].empty() || fetch_column(ctx, b); }
+    bool fetch_column(porrt_ctx* ctx, int b);
   } bel;
-  std::vector<int32_t> bel_node_vid;
   DevBuf d_bel_succ;                   // observation successor tables of the running / last porrt_belief_vi (belief_tables.cu)
   // last PRM result, kept on the device (valid until the next call on this ctx)
   int64_t prm_n = 0, prm_edges = 0;
@@ -218,6 +257,66 @@ static inline void tfinish(porrt_ctx* ctx) {  // call after the stream has been 
 }
 
 static inline int div_up(int64_t a, int64_t b) { return (int)((a + b - 1) / b); }
+
+// ---- host formulas of the reference (the kernels have their own __d*_rn forms).  The host objects are built with
+// -ffp-contract=off, so these round like the reference's f64 code.
+// norm2 (common.rs:203-213): the squares of b - a summed from 0.0 in dimension order
+static inline double norm2(const double* a, const double* b, int dim) {
+  double d2 = 0.0;
+  for (int k = 0; k < dim; ++k) { const double dx = b[k] - a[k]; d2 += dx * dx; }
+  return std::sqrt(d2);
+}
+// transition_probability (common.rs:188-190): the parent's mass on the worlds the child belief holds possible
+static inline double transition_probability(const double* parent, const double* child, int n_worlds) {
+  double s = 0.0;
+  for (int i = 0; i < n_worlds; ++i) s = s + (child[i] > 0.0 ? parent[i] : 0.0);
+  return s;
+}
+// heuristic_radius (common.rs:357-369): libm ln / pow like Rust's f64::ln / powf
+static inline double heuristic_radius(int64_t n_nodes, double max_step, double search_radius, int dim) {
+  const double n = (double)n_nodes;
+  const double s = search_radius * std::pow(std::log(n) / n, 1.0 / (double)dim);
+  return s < max_step ? s : max_step;
+}
+
+// extract_policy / get_best_expected_children (belief_graph.rs:184-267) on the host, over any belief graph of n_nodes belief
+// nodes rooted at id 0: for_children(id, fn) calls fn(child id) in stored order, belief_of(id) is the id's row of
+// beliefs[. * n_worlds], cost(parent id, child id) the edge cost, dist(id) the expected cost to the goals.  pol: (belief node
+// id, parent, leaf) per policy node in creation order.  The reference's asserts are PORRT_ERR_PANIC; `name` names the caller in
+// the message of a walk that does not terminate.
+struct PolicyNode { int64_t id; int32_t parent; uint8_t leaf; };
+template <class ForChildren, class BeliefOf, class Cost, class Dist>
+int32_t get_best_expected_children(porrt_ctx* ctx, const char* name, int64_t n_nodes, const double* beliefs, int n_worlds,
+                                   ForChildren&& for_children, BeliefOf&& belief_of, Cost&& cost, Dist&& dist, std::vector<PolicyNode>& pol) {
+  struct Child { int64_t id; double cost_to_child, expected_from_child; };
+  std::vector<std::pair<int64_t, int64_t>> lifo;   // (policy node, belief node)
+  pol.assign(1, PolicyNode{0, -1, 0});
+  lifo.push_back({0, 0});
+  while (!lifo.empty()) {
+    const auto top = lifo.back();
+    lifo.pop_back();
+    const int64_t bn = top.second;
+    std::map<int32_t, std::vector<Child>> by_belief;   // BTreeMap keyed by child.belief_id (:228-241)
+    for_children(bn, [&](int64_t c) { by_belief[belief_of(c)].push_back({c, cost(bn, c), dist(c)}); });
+    for (auto& kv : by_belief) {
+      int64_t best_id = kv.second[0].id;
+      const double p = transition_probability(beliefs + (size_t)belief_of(bn) * n_worlds, beliefs + (size_t)belief_of(best_id) * n_worlds, n_worlds);
+      if (!(p > 0.0)) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p > 0.0) (belief_graph.rs:250)");
+      double best_cost = std::numeric_limits<double>::infinity();
+      for (const Child& c : kv.second) {
+        const double cst = p * (c.cost_to_child + c.expected_from_child);
+        if (cst < best_cost) { best_cost = cst; best_id = c.id; }
+      }
+      if (!(p * dist(best_id) <= dist(bn))) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p * cost[best] <= cost[node]) (belief_graph.rs:261)");
+      const bool leaf = dist(best_id) == 0.0;
+      const int64_t pid = (int64_t)pol.size();
+      pol.push_back({best_id, (int32_t)top.first, (uint8_t)leaf});
+      if (!leaf) lifo.push_back({pid, best_id});
+      if ((int64_t)pol.size() > 64 * n_nodes + 1024) return porrt_fail(ctx, PORRT_ERR_PANIC, std::string(name) + ": policy does not terminate");
+    }
+  }
+  return PORRT_OK;
+}
 
 // comm.cu
 void comm_shard_range(int64_t n, int rank, int world, int64_t* lo, int64_t* hi);

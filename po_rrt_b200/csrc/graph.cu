@@ -282,13 +282,6 @@ PORRT_API int32_t porrt_kd_preorder_rank(porrt_ctx* ctx, const double* xy, int64
   return PORRT_OK;
 }
 
-// heuristic_radius (common.rs:357-369): host libm ln/pow like Rust's f64::ln/powf; never evaluated on the device.
-static double heuristic_radius(size_t n_nodes, double max_step, double search_radius, size_t dim) {
-  double n = (double)n_nodes;
-  double s = search_radius * std::pow(std::log(n) / n, 1.0 / (double)dim);
-  return s < max_step ? s : max_step;
-}
-
 // ================================================================================================ PRM build
 __global__ void iota_u32_kernel(uint32_t* __restrict__ out, int64_t n) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -506,7 +499,7 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
         const int64_t per = (m + nt - 1) / nt, k0 = lo + t * per, k1 = std::min<int64_t>(hi, k0 + per);   // contiguous: no shared cache lines
         for (int64_t k = k0; k < k1; ++k) {
           const int64_t kl = gb ? k - (int64_t)gb[k] : k;   // index inside the node's own roadmap
-          radius[k] = kl == 0 ? -1.0 : heuristic_radius((size_t)kl + 1, ms_arr ? ms_arr[k] : max_step, sr_arr ? sr_arr[k] : search_radius, 2);
+          radius[k] = kl == 0 ? -1.0 : heuristic_radius(kl + 1, ms_arr ? ms_arr[k] : max_step, sr_arr ? sr_arr[k] : search_radius, 2);
         }
       });
   }
@@ -559,7 +552,7 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
   start_kd();
 
   // 1. bin vertices; cell = the smallest radius in use (the last one) so late queries touch 3x3 cells
-  double r_last = n > 1 ? heuristic_radius((size_t)n, max_step, search_radius, 2) : -1.0;
+  double r_last = n > 1 ? heuristic_radius(n, max_step, search_radius, 2) : -1.0;
   if (ms_arr || sr_arr) {   // per-sample parameters: the smallest positive radius in use (needs the radii: no overlap here)
     for (auto& x : th) if (x.joinable()) x.join();
     r_last = -1.0;
@@ -1000,13 +993,8 @@ PORRT_API int32_t porrt_sssp_worlds_prm(porrt_ctx* ctx, const int64_t* finals_pt
 }
 
 // ================================================================================================ belief-space VI
-// host-side belief algebra (common.rs:188-190,256-264,352-355; map_io.rs:244-278; map_shelves_io.rs:206-239)
+// host-side belief algebra (common.rs:256-264,352-355; map_io.rs:244-278; map_shelves_io.rs:206-239)
 typedef std::vector<double> Belief;
-static double transition_probability(const double* parent, const double* child, int n) {
-  double s = 0.0;
-  for (int i = 0; i < n; ++i) s = s + (child[i] > 0.0 ? parent[i] : 0.0);
-  return s;
-}
 static uint64_t belief_hash(const double* bs, int n) {
   uint64_t h = 0, p10 = 1;
   for (int i = 0; i < n; ++i) {
@@ -1535,7 +1523,7 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
   R.colpos = colpos;
   R.col_dist.assign((size_t)B, std::vector<double>()); R.col_type.assign((size_t)B, std::vector<uint8_t>());
   R.dist = nullptr; R.type = nullptr;
-  ctx->bel_node_vid.assign(node_vid, node_vid + V);
+  R.node_vid.assign(node_vid, node_vid + V);
   if (out_dist || out_type) {
     int32_t rc = belief_download_full(ctx, nullptr, out_dist, out_type);
     if (rc) return rc;
@@ -1565,96 +1553,46 @@ PORRT_API int32_t porrt_belief_result(porrt_ctx* ctx, const double** out_dist, c
   return PORRT_OK;
 }
 
+bool porrt_ctx::BeliefState_::fetch_column(porrt_ctx* ctx, int b) {
+  std::vector<double>& d = col_dist[(size_t)b];
+  std::vector<uint8_t>& t = col_type[(size_t)b];
+  d.resize((size_t)V); t.resize((size_t)V);
+  const size_t at = (size_t)colpos[(size_t)b] * V;
+  if (cudaSetDevice(ctx->device) == cudaSuccess &&
+      cudaMemcpyAsync(d.data(), d_dist_cm + at, (size_t)V * 8, cudaMemcpyDeviceToHost, ctx->stream) == cudaSuccess &&
+      cudaMemcpyAsync(t.data(), d_type_cm + at, (size_t)V, cudaMemcpyDeviceToHost, ctx->stream) == cudaSuccess &&
+      cudaStreamSynchronize(ctx->stream) == cudaSuccess)
+    return true;
+  d.clear(); t.clear();
+  fetch_failed = true;
+  return false;
+}
+
 // ================================================================================================ policy extraction
 PORRT_API int32_t porrt_extract_policy(porrt_ctx* ctx, int32_t* out_node, int32_t* out_belief, int32_t* out_parent,
                                        uint8_t* out_is_leaf, int64_t cap, int64_t* out_n, double* out_expected_cost) {
   CTX_CHECK(ctx);
   auto& R = ctx->bel;
   if (R.V <= 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "extract_policy: run porrt_belief_vi first");
-  const int B = R.B, nw = R.n_worlds, nv = R.n_validities;
-  const std::vector<int32_t>& nvid = ctx->bel_node_vid;
-  // values / types of belief node id = node * B + belief.  When the table is still on the device only, the walk fetches the
-  // columns (beliefs) it visits -- a policy touches a few dozen of the B columns, 8 * V bytes each
-  bool fetch_failed = false;
-  auto column = [&](int b) {
-    if (R.col_dist[(size_t)b].empty()) {
-      R.col_dist[(size_t)b].resize((size_t)R.V); R.col_type[(size_t)b].resize((size_t)R.V);
-      cudaSetDevice(ctx->device);
-      if (cudaMemcpyAsync(R.col_dist[(size_t)b].data(), R.d_dist_cm + (size_t)R.colpos[(size_t)b] * R.V, (size_t)R.V * 8, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
-          cudaMemcpyAsync(R.col_type[(size_t)b].data(), R.d_type_cm + (size_t)R.colpos[(size_t)b] * R.V, (size_t)R.V, cudaMemcpyDeviceToHost, ctx->stream) != cudaSuccess ||
-          cudaStreamSynchronize(ctx->stream) != cudaSuccess)
-        fetch_failed = true;
-    }
-  };
-  auto dist_at = [&](int64_t id) -> double {
-    if (R.on_host) return R.dist[(size_t)id];
-    const int b = (int)(id % B);
-    column(b);
-    return R.col_dist[(size_t)b][(size_t)(id / B)];
-  };
-  auto type_at = [&](int64_t id) -> uint8_t {
-    if (R.on_host) return R.type[(size_t)id];
-    const int b = (int)(id % B);
-    column(b);
-    return R.col_type[(size_t)b][(size_t)(id / B)];
-  };
-  auto state = [&](int64_t n) { return &R.xy[2 * n]; };
-  auto norm2 = [&](const double* a, const double* b) {
-    double d2 = 0.0;
-    for (int k = 0; k < 2; ++k) { double dx = b[k] - a[k]; d2 += dx * dx; }
-    return std::sqrt(d2);
-  };
-  struct PN { int32_t node, belief, parent; uint8_t leaf; };
-  std::vector<PN> pol;
-  std::vector<std::pair<int64_t, int64_t>> lifo;  // (policy node, belief node id)
-  pol.push_back({0, 0, -1, 0});
-  lifo.push_back({0, 0});
-  struct Child { int64_t id; double cost_to_child, expected_from_child; };
-  while (!lifo.empty()) {
-    auto top = lifo.back();
-    lifo.pop_back();
-    const int64_t bn = top.second, n = bn / B;
-    const int b = (int)(bn % B);
-    // children of the belief node in stored order (observation edges first if Observation, else action edges)
-    std::map<int32_t, std::vector<Child>> by_belief;  // BTreeMap keyed by child.belief_id (belief_graph.rs:228-241)
-    const uint8_t ty = type_at(bn);
-    if (ty == PORRT_NODE_OBSERVATION) {
-      const int64_t sp = (int64_t)R.node_obs_set[n] * B + b;
-      for (int64_t k = R.succ_ptr[sp]; k < R.succ_ptr[sp + 1]; ++k) {
-        const int32_t cb = R.succ_belief[k];
-        if (!R.compat[(size_t)cb * nv + nvid[n]]) continue;
-        const int64_t cid = n * B + cb;
-        by_belief[cb].push_back({cid, norm2(state(n), state(n)), dist_at(cid)});
-      }
-    } else if (ty == PORRT_NODE_ACTION) {
-      for (int64_t e = R.row_ptr[n]; e < R.row_ptr[n + 1]; ++e) {
-        const int32_t c = R.col[e];
-        if (!R.compat[(size_t)b * nv + nvid[c]] || !R.compat[(size_t)b * nv + R.edge_vid[e]]) continue;
-        const int64_t cid = (int64_t)c * B + b;
-        by_belief[b].push_back({cid, norm2(state(n), state(c)), dist_at(cid)});
-      }
-    }
-    for (auto& kv : by_belief) {
-      int64_t best_id = kv.second[0].id;
-      const double p = transition_probability(&R.beliefs[(size_t)b * nw], &R.beliefs[(size_t)(best_id % B) * nw], nw);
-      if (!(p > 0.0)) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p > 0.0) (belief_graph.rs:250)");
-      double best_cost = std::numeric_limits<double>::infinity();
-      for (const Child& c : kv.second) {
-        const double cost = p * (c.cost_to_child + c.expected_from_child);
-        if (cost < best_cost) { best_cost = cost; best_id = c.id; }
-      }
-      if (fetch_failed) return porrt_fail(ctx, PORRT_ERR_CUDA, "extract_policy: fetching a value column failed");
-      if (!(p * dist_at(best_id) <= dist_at(bn))) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p * cost[best] <= cost[node]) (belief_graph.rs:261)");
-      const bool leaf = dist_at(best_id) == 0.0;
-      const int64_t pid = (int64_t)pol.size();
-      pol.push_back({(int32_t)(best_id / B), (int32_t)(best_id % B), (int32_t)top.first, (uint8_t)leaf});
-      if (!leaf) lifo.push_back({pid, best_id});
-      if ((int64_t)pol.size() > 64 * R.V * (int64_t)B + 1024) return porrt_fail(ctx, PORRT_ERR_PANIC, "extract_policy: policy does not terminate");
-    }
-  }
+  const int B = R.B;
+  // the walk over the implicit V x B belief graph; an Observation child keeps its parent's state, so its cost is norm2(state n, state n)
+  R.fetch_failed = false;
+  std::vector<PolicyNode> pol;
+  const int32_t rc = get_best_expected_children(
+      ctx, "extract_policy", R.V * (int64_t)B, R.beliefs.data(), R.n_worlds,
+      [&](int64_t id, auto&& fn) { R.for_children(ctx, id, fn); },
+      [&](int64_t id) { return (int32_t)(id % B); },
+      [&](int64_t a, int64_t c) { return norm2(&R.xy[2 * (size_t)(a / B)], &R.xy[2 * (size_t)(c / B)], 2); },
+      [&](int64_t id) { return R.value(ctx, id); }, pol);
+  const double expected_cost = R.value(ctx, 0);
+  // a failed fetch read as 0: it outranks any assert the walk tested on such a value
+  if (R.fetch_failed) return porrt_fail(ctx, PORRT_ERR_CUDA, "extract_policy: fetching a value column failed");
+  if (rc) return rc;
   if (out_n) *out_n = (int64_t)pol.size();
-  if (out_expected_cost) *out_expected_cost = dist_at(0);
+  if (out_expected_cost) *out_expected_cost = expected_cost;
   if ((int64_t)pol.size() > cap || !out_node || !out_belief || !out_parent || !out_is_leaf) return porrt_fail(ctx, PORRT_ERR_CAPACITY, "extract_policy: cap too small");
-  for (size_t k = 0; k < pol.size(); ++k) { out_node[k] = pol[k].node; out_belief[k] = pol[k].belief; out_parent[k] = pol[k].parent; out_is_leaf[k] = pol[k].leaf; }
+  for (size_t k = 0; k < pol.size(); ++k) {
+    out_node[k] = (int32_t)(pol[k].id / B); out_belief[k] = (int32_t)(pol[k].id % B); out_parent[k] = pol[k].parent; out_is_leaf[k] = pol[k].leaf;
+  }
   return PORRT_OK;
 }

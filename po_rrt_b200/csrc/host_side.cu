@@ -16,9 +16,7 @@
 // ------------------------------------------------------------------------------------------------ B4 / B5
 PORRT_API int32_t porrt_heuristic_radius(int64_t n_nodes, double max_step, double search_radius, int32_t dim, double* out_radius) {
   if (!out_radius || dim <= 0 || n_nodes < 0) return PORRT_ERR_INVALID_ARG;
-  const double n = (double)n_nodes;
-  const double s = search_radius * std::pow(std::log(n) / n, 1.0 / (double)dim);   // f64::ln, f64::powf
-  *out_radius = s < max_step ? s : max_step;
+  *out_radius = heuristic_radius(n_nodes, max_step, search_radius, dim);
   return PORRT_OK;
 }
 
@@ -234,11 +232,6 @@ PORRT_API int32_t porrt_qmdp_react(porrt_ctx* ctx, int64_t V, const int64_t* row
   for (int64_t e = 0; e < row_ptr[V]; ++e)
     if (col[e] < 0 || col[e] >= V) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_qmdp_react: malformed CSR");
   const int64_t guard_max = 10 * V + 10;
-  auto norm2 = [&](int64_t a, int64_t b) {
-    double d2 = 0.0;
-    for (int c = 0; c < 2; ++c) { const double dx = xy[2 * b + c] - xy[2 * a + c]; d2 += dx * dx; }
-    return std::sqrt(d2);
-  };
   // get_common_path (:65-87)
   std::vector<int32_t> common;
   int64_t id = start_node;
@@ -254,7 +247,7 @@ PORRT_API int32_t porrt_qmdp_react(porrt_ctx* ctx, int64_t V, const int64_t* row
       for (int w = 0; w < n_worlds; ++w) exp_cost += cost_to_goals[(size_t)w * V + c] * belief[w];
       if (exp_cost < best_c) { best = c; best_c = exp_cost; }
     }
-    acc += norm2(id, best);
+    acc += norm2(xy + 2 * id, xy + 2 * best, 2);
     id = best;
     smallest = best_c;
     if (++guard > guard_max) return porrt_fail(ctx, PORRT_ERR_PANIC, "porrt_qmdp_react: the common path never ends (the reference would loop forever)");

@@ -483,12 +483,6 @@ __global__ void pto_ctl_to_host_kernel(const int32_t* __restrict__ d, int n, vol
 __global__ void pto_set_i64_kernel(int64_t* p, const int32_t* ctl, int idx) { *p = ctl[idx]; }
 
 // ------------------------------------------------------------------------------------------------ host
-static double host_heuristic_radius(int64_t n_nodes, double max_step, double search_radius) {   // common.rs:357-369, host libm
-  const double n = (double)n_nodes;
-  const double s = search_radius * std::pow(std::log(n) / n, 1.0 / 2.0);
-  return s < max_step ? s : max_step;
-}
-
 static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double max_step, double goal_max_dist, int n_goals,
                     int64_t nmin, int64_t nmax) {
   PgDev d = {};
@@ -540,7 +534,7 @@ static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, int64_t node_cap, dou
   const int64_t rn = node_cap + PG_WMAX + 2;
   if (rn <= g->radius_n) return PORRT_OK;
   std::vector<double> r((size_t)rn);
-  for (int64_t n = 0; n < rn; ++n) r[(size_t)n] = n == 0 ? 0.0 : host_heuristic_radius(n, max_step, search_radius);
+  for (int64_t n = 0; n < rn; ++n) r[(size_t)n] = n == 0 ? 0.0 : heuristic_radius(n, max_step, search_radius, 2);
   CUDA_TRY(ctx, g->radius.ensure((size_t)rn * 8));
   CUDA_TRY(ctx, cudaMemcpyAsync(g->radius.p, r.data(), (size_t)rn * 8, cudaMemcpyHostToDevice, ctx->stream));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));

@@ -281,20 +281,14 @@ static bool policy_parents_ok(const int32_t* parent, int64_t n) {
 // Policy::compute_expected_costs_to_goals (common.rs:131-153) over flat arrays: a policy as (state, belief, parent) per node in
 // creation order; children are folded in increasing index, a child's own sum is complete before its parent adds it.
 static double policy_expected_cost_flat(const double* beliefs, int nw, const double* out_xy, const int32_t* out_belief, const int32_t* out_parent, int64_t n_out) {
-  auto transition_probability = [&](int pb, int cb) {
-    double s = 0.0;
-    for (int i = 0; i < nw; ++i) s = s + (beliefs[(size_t)cb * nw + i] > 0.0 ? beliefs[(size_t)pb * nw + i] : 0.0);
-    return s;
-  };
   std::vector<double> prob((size_t)n_out, 0.0), pq((size_t)n_out, 0.0), edge_term((size_t)n_out, 0.0), below((size_t)n_out, 0.0);
   prob[0] = 1.0;
   for (int64_t k = 1; k < n_out; ++k) {
     const int32_t par = out_parent[k];
     if (par < 0) continue;   // a piece that recompose left unconnected: not under the root
-    const double q = transition_probability(out_belief[par], out_belief[k]);
-    const double dx = out_xy[2 * k] - out_xy[2 * (size_t)par], dy = out_xy[2 * k + 1] - out_xy[2 * (size_t)par + 1];
-    const double cost = std::sqrt(dx * dx + dy * dy);   // norm2(parent, child), common.rs:203-213
-    pq[(size_t)k] = prob[(size_t)par] * q;              // p * q
+    const double q = transition_probability(beliefs + (size_t)out_belief[par] * nw, beliefs + (size_t)out_belief[k] * nw, nw);
+    const double cost = norm2(&out_xy[2 * (size_t)par], &out_xy[2 * k], 2);
+    pq[(size_t)k] = prob[(size_t)par] * q;             // p * q
     prob[(size_t)k] = pq[(size_t)k];
     edge_term[(size_t)k] = pq[(size_t)k] * cost;        // (p * q) * cost
   }
@@ -474,10 +468,7 @@ struct PieceTree {
     while (!st.empty()) {
       F& f = st.back();
       const double* fs = &xy[2 * (size_t)f.node];
-      if (f.stage == 0) {
-        const double dx = s[0] - fs[0], dy = s[1] - fs[1];     // norm2(from.state, a.state)
-        if (std::sqrt(dx * dx + dy * dy) <= r) out.push_back(f.node);
-      }
+      if (f.stage == 0 && norm2(s, fs, 2) <= r) out.push_back(f.node);   // norm2(from.state, a.state)
       if (f.stage >= 2) { st.pop_back(); continue; }
       const int stage = f.stage++, axis = f.axis;
       int32_t child = -1;
@@ -500,44 +491,12 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
   if (n_pol <= 0 || !pol_node || !pol_belief || !pol_parent || !(radius >= 0.0) || !out_n)
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "refine_policy_reparent: bad arguments");
   const int B = R.B, nw = R.n_worlds, nv = R.n_validities;
-  const std::vector<int32_t>& nvid = ctx->bel_node_vid;
   for (int64_t k = 0; k < n_pol; ++k)
     if (pol_node[k] < 0 || pol_node[k] >= R.V || pol_belief[k] < 0 || pol_belief[k] >= B || pol_parent[k] >= k || (k > 0 && pol_parent[k] < 0) || (k == 0 && pol_parent[k] != -1))
       return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "refine_policy_reparent: not a policy in creation order");
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
-  // node types of the belief graph: from the host table, or column by column from the device (as the policy walk does)
-  bool fetch_failed = false;
-  auto type_at = [&](int64_t id) -> uint8_t {
-    if (R.on_host) return R.type[(size_t)id];
-    const int b = (int)(id % B);
-    if (R.col_dist[(size_t)b].empty()) {
-      R.col_dist[(size_t)b].resize((size_t)R.V); R.col_type[(size_t)b].resize((size_t)R.V);
-      if (cudaMemcpyAsync(R.col_dist[(size_t)b].data(), R.d_dist_cm + (size_t)R.colpos[(size_t)b] * R.V, (size_t)R.V * 8, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-          cudaMemcpyAsync(R.col_type[(size_t)b].data(), R.d_type_cm + (size_t)R.colpos[(size_t)b] * R.V, (size_t)R.V, cudaMemcpyDeviceToHost, st) != cudaSuccess ||
-          cudaStreamSynchronize(st) != cudaSuccess)
-        fetch_failed = true;
-    }
-    return R.col_type[(size_t)b][(size_t)(id / B)];
-  };
-  // children of a belief node in the reference's stored order (pto.rs:206-255): observation edges, or action edges
-  auto for_children = [&](int64_t bn, auto&& fn) {
-    const int64_t n = bn / B;
-    const int b = (int)(bn % B);
-    const uint8_t ty = type_at(bn);
-    if (ty == PORRT_NODE_OBSERVATION) {
-      const int64_t sp = (int64_t)R.node_obs_set[(size_t)n] * B + b;
-      for (int64_t k = R.succ_ptr[(size_t)sp]; k < R.succ_ptr[(size_t)sp + 1]; ++k) {
-        const int32_t cb = R.succ_belief[(size_t)k];
-        if (R.compat[(size_t)cb * nv + nvid[(size_t)n]]) fn(n * B + cb);
-      }
-    } else if (ty == PORRT_NODE_ACTION) {
-      for (int64_t e = R.row_ptr[(size_t)n]; e < R.row_ptr[(size_t)n + 1]; ++e) {
-        const int32_t c = R.col[(size_t)e];
-        if (R.compat[(size_t)b * nv + nvid[(size_t)c]] && R.compat[(size_t)b * nv + R.edge_vid[(size_t)e]]) fn((int64_t)c * B + b);
-      }
-    }
-  };
+  R.fetch_failed = false;
   // ---- Policy::decompose (common.rs:85-129)
   std::vector<std::vector<int64_t>> pieces;
   std::vector<std::vector<int32_t>> successors;
@@ -551,7 +510,6 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
   const bool dbg = getenv("PORRT_DEBUG") != nullptr;
   auto now_ms = [] { return std::chrono::duration<double, std::milli>(std::chrono::steady_clock::now().time_since_epoch()).count(); };
   double tph[6] = {now_ms(), 0, 0, 0, 0, 0};
-  auto norm2 = [](const double* a, const double* b) { const double dx = b[0] - a[0], dy = b[1] - a[1]; return std::sqrt(dx * dx + dy * dy); };
   std::vector<PieceTree> trees(pieces.size());
   int64_t tree_nodes = 0;
   std::vector<uint32_t> stamp((size_t)R.V * B, 0);   // visited set of build_tree: stamp == piece + 1
@@ -569,7 +527,7 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
       const int64_t pn = pieces[p][k];
       const int64_t bg = (int64_t)pol_node[pn] * B + pol_belief[pn];
       const double* s = &R.xy[2 * (size_t)pol_node[pn]];
-      T.add(s, (int32_t)k - 1, k ? norm2(&R.xy[2 * (size_t)pol_node[pieces[p][k - 1]]], s) : 0.0, bg);
+      T.add(s, (int32_t)k - 1, k ? norm2(&R.xy[2 * (size_t)pol_node[pieces[p][k - 1]]], s, 2) : 0.0, bg);
       visited.insert(bg);
     }
     T.belief = pol_belief[pieces[p][0]];
@@ -587,16 +545,16 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
         // leaves behind is visited or beyond the seed's radius for every later one too), so the others are skipped unexpanded
         if (expanded[(size_t)from_bg] == expand_tag) continue;
         expanded[(size_t)from_bg] = expand_tag;
-        for_children(from_bg, [&](int64_t child) {
+        R.for_children(ctx, from_bg, [&](int64_t child) {
           const double* cs = &R.xy[2 * (size_t)(child / B)];
           if (visited.count(child)) return;
-          const double d = norm2(sx, cs);
+          const double d = norm2(sx, cs, 2);
           if (!(d <= radius)) return;
           const int32_t me = T.add(cs, tree_id, d, child);
           visited.insert(child);
-          for_children(child, [&](int64_t cc) { if (!visited.count(cc)) q.push_back({me, cc}); });
+          R.for_children(ctx, child, [&](int64_t cc) { if (!visited.count(cc)) q.push_back({me, cc}); });
         });
-        if (fetch_failed) return porrt_fail(ctx, PORRT_ERR_CUDA, "refine_policy_reparent: fetching a value column failed");
+        if (R.fetch_failed) return porrt_fail(ctx, PORRT_ERR_CUDA, "refine_policy_reparent: fetching a value column failed");
         if ((int64_t)T.size() > (int64_t)R.V * B) return porrt_fail(ctx, PORRT_ERR_PANIC, "refine_policy_reparent: tree larger than the belief graph");
       }
     }
@@ -711,7 +669,7 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
         for (int64_t k = nb_ptr[(size_t)(base + u)]; k < nb_ptr[(size_t)(base + u) + 1]; ++k)
           if (valid[(size_t)k]) nd.push_back({nb_ids[(size_t)k], T.dist_from_root(nb_ids[(size_t)k])});   // all read before this pop reparents anybody
         for (const auto& kv : nd) {
-          const double cost = norm2(&T.xy[2 * (size_t)u], &T.xy[2 * (size_t)kv.first]);
+          const double cost = norm2(&T.xy[2 * (size_t)u], &T.xy[2 * (size_t)kv.first], 2);
           if (du + cost < kv.second) {
             T.parent[(size_t)kv.first] = u; T.parent_cost[(size_t)kv.first] = cost;
             q.push(kv.first, du + cost);
