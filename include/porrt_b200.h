@@ -418,7 +418,7 @@ int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, i
  * [n]) and out_sizes[4 r] are the code and the iteration porrt_pto_grow reports.  A panic stops only its own roadmap; the call
  * still returns PORRT_OK.  The whole call fails like porrt_pto_grow on bad arguments, no map, overlapping goal masks and
  * low >= up.  n_roadmaps must lie in 1 .. PORRT_PTO_MAX_ROADMAPS (a launch grid's y dimension) and the device's free memory must
- * hold them at their starting size (about 31 MB each at 4096 + iterations, DESIGN.md 3.8), else PORRT_ERR_INVALID_ARG; running
+ * hold them at their starting size (about 28 MB each at 4096 + iterations, DESIGN.md 3.8), else PORRT_ERR_INVALID_ARG; running
  * out of memory while the roadmaps grow is PORRT_ERR_CUDA.  The batch replaces the ctx's last growth: porrt_pto_fetch_roadmap
  * reads roadmap r, porrt_pto_fetch reads roadmap 0. */
 #define PORRT_PTO_MAX_ROADMAPS 65535

@@ -133,23 +133,17 @@ PORRT_API int32_t porrt_conditional_dijkstra_nd(porrt_ctx* ctx, int32_t dim, int
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const int64_t E = row_ptr[V];
-  DevBuf& g = ctx->scratch[3];
-  const size_t need = (size_t)(V + 1) * 8 + (size_t)E * 20 + (size_t)V * ((size_t)dim * 8 + 16 + 8 + 4 + 2) + (size_t)B * n_worlds * 8 + (size_t)n_finals * 4 + 1024;
-  CUDA_TRY(ctx, g.ensure(need));
-  char* b = g.as<char>();
-  auto take = [&](size_t bytes) { char* p = b; b += (bytes + 15) & ~(size_t)15; return p; };
-  int64_t* d_row = (int64_t*)take((size_t)(V + 1) * 8);
-  double* d_xy = (double*)take((size_t)V * dim * 8);
-  double* d_cost = (double*)take((size_t)E * 8);
-  double* d_prob = (double*)take((size_t)E * 8);
-  double* d_dist = (double*)take((size_t)V * 8);
-  double* d_beliefs = (double*)take((size_t)B * n_worlds * 8);
-  int32_t* d_col = (int32_t*)take((size_t)E * 4);
-  int32_t* d_bid = (int32_t*)take((size_t)V * 4);
-  int32_t* d_finals = (int32_t*)take((size_t)n_finals * 4 + 4);
-  int32_t* d_flags = (int32_t*)take(16);   // [0] changed, [1] panic node
-  uint8_t* d_type = (uint8_t*)take((size_t)V);
-  uint8_t* d_frozen = (uint8_t*)take((size_t)V);
+  int64_t* d_row;
+  double *d_xy, *d_cost, *d_prob, *d_dist, *d_beliefs;
+  int32_t *d_col, *d_bid, *d_finals, *d_flags;   // d_flags: [0] changed, [1] panic node
+  uint8_t *d_type, *d_frozen;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_row = c.take<int64_t>(V + 1);
+    d_xy = c.take<double>((size_t)V * dim); d_cost = c.take<double>(E); d_prob = c.take<double>(E); d_dist = c.take<double>(V);
+    d_beliefs = c.take<double>((size_t)B * n_worlds);
+    d_col = c.take<int32_t>(E); d_bid = c.take<int32_t>(V); d_finals = c.take<int32_t>(n_finals + 1); d_flags = c.take<int32_t>(4);
+    d_type = c.take<uint8_t>(V); d_frozen = c.take<uint8_t>(V);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_row, row_ptr, (size_t)(V + 1) * 8, cudaMemcpyHostToDevice, st));
   if (E) CUDA_TRY(ctx, cudaMemcpyAsync(d_col, col, (size_t)E * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_xy, xy, (size_t)V * dim * 8, cudaMemcpyHostToDevice, st));

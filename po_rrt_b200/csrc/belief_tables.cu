@@ -147,29 +147,19 @@ int32_t belief_succ_tables(porrt_ctx* ctx, const double* beliefs_host, int32_t B
   std::vector<int32_t> sid((size_t)B);
   for (int b = 0; b < B; ++b) { sh[(size_t)b] = sorted[(size_t)b].first; sid[(size_t)b] = sorted[(size_t)b].second; }
 
-  // ---- inputs + work space (scratch[4]); outputs (ctx->d_bel_succ) are sized after the scan
-  DevBuf& wsb = ctx->scratch[4];
+  // ---- inputs + work space (ws_query); outputs (ctx->d_bel_succ) are sized after the scan
   const size_t zw = ctx->zone_world_masks.size();
-  const size_t in_bytes = (size_t)B * nw * 8 + (size_t)n_sets * 8 + (size_t)(n_sets + 1) * 8 + zw * 8 + (size_t)B * 28 + 16 * 16;
-  const size_t ws_bytes = (size_t)n_slots * ((size_t)nw * 8 + 4 + 8 + 4 + 8) + 64 + 16 * 16;
-  CUDA_TRY(ctx, wsb.ensure(in_bytes + ws_bytes));
-  char* p = wsb.as<char>();
-  auto take = [&](size_t bytes) { char* q = p; p += (bytes + 15) & ~(size_t)15; return q; };
-  double* d_beliefs = (double*)take((size_t)B * nw * 8);
-  uint64_t* d_sets = (uint64_t*)take((size_t)n_sets * 8);
-  int64_t* d_set_off = (int64_t*)take((size_t)(n_sets + 1) * 8);
-  uint64_t* d_zw = (uint64_t*)take(zw * 8 + 8);
-  uint64_t* d_sh = (uint64_t*)take((size_t)B * 8);
-  uint64_t* d_bhash = (uint64_t*)take((size_t)B * 8);
-  int32_t* d_sid = (int32_t*)take((size_t)B * 4);
-  int32_t* d_level = (int32_t*)take((size_t)B * 4);
-  int32_t* d_colpos = (int32_t*)take((size_t)B * 4);
-  int32_t* d_err = (int32_t*)take(16);
-  double* d_work = (double*)take((size_t)n_slots * nw * 8);
-  double* d_slot_p = (double*)take((size_t)n_slots * 8);
-  int64_t* d_pos = (int64_t*)take((size_t)(n_slots + 1) * 8);
-  int32_t* d_slot_id = (int32_t*)take((size_t)n_slots * 4);
-  int32_t* d_flag = (int32_t*)take((size_t)n_slots * 4);
+  double *d_beliefs, *d_work, *d_slot_p;
+  uint64_t *d_sets, *d_zw, *d_sh, *d_bhash;
+  int64_t *d_set_off, *d_pos;
+  int32_t *d_sid, *d_level, *d_colpos, *d_err, *d_slot_id, *d_flag;
+  CUDA_TRY(ctx, carve(ctx->ws_query, [&](Carve& c) {
+    d_beliefs = c.take<double>((size_t)B * nw); d_sets = c.take<uint64_t>(n_sets); d_set_off = c.take<int64_t>(n_sets + 1);
+    d_zw = c.take<uint64_t>(zw + 1); d_sh = c.take<uint64_t>(B); d_bhash = c.take<uint64_t>(B);
+    d_sid = c.take<int32_t>(B); d_level = c.take<int32_t>(B); d_colpos = c.take<int32_t>(B); d_err = c.take<int32_t>(4);
+    d_work = c.take<double>((size_t)n_slots * nw); d_slot_p = c.take<double>(n_slots); d_pos = c.take<int64_t>(n_slots + 1);
+    d_slot_id = c.take<int32_t>(n_slots); d_flag = c.take<int32_t>(n_slots);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_beliefs, beliefs_host, (size_t)B * nw * 8, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_sets, sets.data(), (size_t)n_sets * 8, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_set_off, set_off.data(), (size_t)(n_sets + 1) * 8, cudaMemcpyHostToDevice, st));
@@ -199,14 +189,11 @@ int32_t belief_succ_tables(porrt_ctx* ctx, const double* beliefs_host, int32_t B
   if (err & 1) return porrt_fail(ctx, PORRT_ERR_PANIC, "no id corresponding to this belief state! (belief_graph.rs:69)");
   if (err & 2) return porrt_fail(ctx, PORRT_ERR_PANIC, "assert!(p > 0.0) (belief_graph.rs:130)");
   const int64_t n_sb = (int64_t)n_sets * B;
-  DevBuf& ob = ctx->d_bel_succ;   // dedicated: the tables are read until the last level is done (sssp_frontier.cu owns scratch[5..7])
-  CUDA_TRY(ctx, ob.ensure((size_t)(n_sb + 1) * 8 + (size_t)n_succ * 16 + 4 * 16 + 16));
-  char* o = ob.as<char>();
-  auto take_o = [&](size_t bytes) { char* q = o; o += (bytes + 15) & ~(size_t)15; return q; };
-  out->succ_ptr = (int64_t*)take_o((size_t)(n_sb + 1) * 8);
-  out->succ_p = (double*)take_o((size_t)n_succ * 8 + 8);
-  out->succ_b = (int32_t*)take_o((size_t)n_succ * 4 + 4);
-  out->succ_col = (int32_t*)take_o((size_t)n_succ * 4 + 4);
+  // dedicated: the tables are read until the last level is done, while the frontier path works in sort_keys .. ws_state
+  CUDA_TRY(ctx, carve(ctx->d_bel_succ, [&](Carve& c) {
+    out->succ_ptr = c.take<int64_t>(n_sb + 1); out->succ_p = c.take<double>(n_succ + 1);
+    out->succ_b = c.take<int32_t>(n_succ + 1); out->succ_col = c.take<int32_t>(n_succ + 1);
+  }));
   out->n_succ = n_succ;
   out->levels_ok = !(err & 4);
   out->beliefs = d_beliefs;

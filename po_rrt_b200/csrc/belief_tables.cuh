@@ -7,7 +7,7 @@
 
 struct porrt_ctx;
 
-struct BeliefSuccDev {        // device pointers (ctx->d_bel_succ / scratch[4]), valid until the next belief_vi call
+struct BeliefSuccDev {        // device pointers (ctx->d_bel_succ / ws_query), valid until the next belief_vi call
   int64_t* succ_ptr;          // [n_sets * B + 1]
   int32_t* succ_b;            // successor belief ids, emission order of observe()
   int32_t* succ_col;          // the same as columns of colsolve.cu (colpos[succ_b])

@@ -64,6 +64,27 @@ struct PinBuf {  // grow-only pinned host staging
   template <class T> T* as() const { return (T*)p; }
 };
 
+// The layout of one block of work space, written once as a function layout(Carve&) that takes its pieces in order.  carve() runs it
+// twice: a size pass without a base (offsets as integers), then, after ensure(size), the pass that assigns the real pointers.
+// Bases from cudaMalloc / cudaHostAlloc are 256-byte aligned, so a piece's alignment holds for its address too.
+struct Carve {
+  uintptr_t base = 0, off = 0;   // base 0: the size pass (every take returns nullptr)
+  template <class T> T* take(size_t count, size_t align = 16) {
+    off = (off + align - 1) & ~(uintptr_t)(align - 1);
+    T* p = base ? (T*)(base + off) : nullptr;
+    off += count * sizeof(T);
+    return p;
+  }
+};
+template <class Layout> size_t carve_size(Layout&& layout) { Carve c; layout(c); return c.off; }
+template <class Buf, class Layout> cudaError_t carve(Buf& buf, Layout&& layout) {
+  const cudaError_t e = buf.ensure(carve_size(layout));
+  if (e != cudaSuccess) return e;
+  Carve c{(uintptr_t)buf.p};
+  layout(c);
+  return cudaSuccess;
+}
+
 // Device-side description of an uploaded map (passed by value to kernels).
 struct MapDev {
   const uint8_t* grid;  // fused code grid, tiled (see map.cu: tile_addr)
@@ -122,7 +143,7 @@ struct porrt_ctx {
   double cell = 0, inv_cell = 0, org_x = 0, org_y = 0;
   int32_t cells_x = 0, cells_y = 0;
   DevBuf d_vxy_sorted, d_vid_sorted, d_cell_start, d_vxy, d_vcell;
-  DevBuf nn_tmp[3];      // nn_tile.cu: query bins
+  DevBuf nn_bins;        // nn_tile.cu: query bins (nt_layout), or the merge scripts' sizes while they are built
   DevBuf d_nbr_start, d_nbr_script;   // nn_tile.cu: per-cell merge scripts of the 3 x 3 neighbourhood (built lazily per vertex set)
   bool nbr_ready = false;
   DevBuf nn_stage;       // nn_tile.cu: tile-ordered staging of the radius lists + per-query staging offsets
@@ -137,7 +158,7 @@ struct porrt_ctx {
     std::vector<int64_t> row_ptr; std::vector<int32_t> col, edge_vid; std::vector<double> xy;
     std::vector<int32_t> node_vid;                // [V] validity id of each roadmap node
     std::vector<double> beliefs;
-    const double* dist = nullptr; const uint8_t* type = nullptr;   // live in ctx->pin[3] (pinned: the V*B table comes back by DMA)
+    const double* dist = nullptr; const uint8_t* type = nullptr;   // live in ctx->pin_bel (pinned: the V*B table comes back by DMA)
     std::vector<int32_t> node_obs_set;            // [V] index into obs tables
     std::vector<int64_t> succ_ptr;                // [(n_sets*B)+1]
     std::vector<int32_t> succ_belief;             // successor belief ids
@@ -193,7 +214,7 @@ struct porrt_ctx {
   int64_t prm_n = 0, prm_edges = 0;
   const int64_t* prm_row_ptr = nullptr;
   const int32_t* prm_col = nullptr;
-  const void* radii_ptr = nullptr; int64_t radii_lo = 0, radii_n = 0; double radii_ms = 0, radii_sr = 0;   // what pin[1] holds: heuristic_radius(k + 1) for k in [radii_lo, radii_n)
+  const void* radii_ptr = nullptr; int64_t radii_lo = 0, radii_n = 0; double radii_ms = 0, radii_sr = 0;   // what pin_radii holds: heuristic_radius(k + 1) for k in [radii_lo, radii_n)
   DevBuf d_prm_row, d_prm_col;         // dedicated: the retained CSR must survive later calls that reuse the shared scratch
 
   // ---- last multi-modal PRM result (mmprm.cu): the explicit belief graph, kept for porrt_mmprm_fetch_graph
@@ -208,12 +229,33 @@ struct porrt_ctx {
   void* comm = nullptr;
   int comm_rank = 0, comm_world = 1;
 
-  // ---- scratch
-  DevBuf kd_buf;                       // kd pre-order rank work space (its own: the rank runs concurrently with the binning sort)
+  // ---- work space.  The rule: a function carves only from buffers that no function above it on the call stack holds pointers
+  // into.  Call trees that never nest share the large buffers: a DevBuf never shrinks, so a buffer per user would keep the sum of
+  // their peaks.  Users of each buffer:
+  DevBuf kd_buf;      // kd_preorder_rank_dev (its own: the PRM build runs the rank on a helper thread next to the binning sort)
   cudaStream_t aux_stream = nullptr;   // second compute stream (created on first use): kd rank next to radius / edge batches
-  DevBuf scratch[12];
-  PinBuf pin[6];
-  PinBuf pin_flags;      // a few counters the kernels write straight into host memory (no DMA engine: see read_flags_dev, nn.cu)
+  DevBuf ws_main;     // the entry points' inputs and work blocks: porrt_radius_query, knn_host, porrt_state_validity, porrt_visibility,
+                      // porrt_transition_valid, the shortcut and Reparent refiners, porrt_sssp_worlds(_prm), porrt_belief_vi,
+                      // porrt_conditional_dijkstra_graph, the PRM build's per-node arrays; edge_pipeline's chunk slots
+  DevBuf ws_owner;    // map upload: the occupancy image; PRM build: the owner of each candidate, then the packed neighbour lists
+  DevBuf ws_vid;      // map upload: the zone image; PRM build: the candidates' validity ids, then the late lists and cursors
+  DevBuf ws_table;    // map upload: zone statistics; the radius id lists of porrt_radius_query and the PRM build
+                      // (nn_radius_count_fill_dev's ids_buf); sssp_core's value table and finals; belief_download_full's
+                      // [node][belief] table
+  DevBuf ws_query;    // nn_radius_count_fill_dev: staging offsets, counts and the wide-query list; nn_vertices_set_dev's bounding
+                      // box; edge_pipeline's id check flag; belief_succ_tables' inputs and work space; porrt_measure_l2_gather's sink
+  DevBuf ws_seg;      // segments_sort_by_key_dev: its counters, mid-length segment list and inverse key permutation
+  DevBuf sort_keys, sort_vals;   // nn_vertices_set_dev's and segments_sort_by_key_dev's (radix path) pairs to sort; sf_build_graph's
+                                 // Morton order (keys) and transposed graph (vals); porrt_edge_validity_csr_i8's row_ptr (keys)
+  DevBuf ws_state;    // nn_vertices_set_dev: cell counts; sf_relax: the frontier state (sf_state_layout), with sssp_frontier_run's value table behind it
+  DevBuf radix_keys, radix_vals, radix_hist;   // radix_sort_pairs: the second key / value array, the histograms and tile bases;
+                      // porrt_kd_preorder_rank's coordinates and ranks (radix_vals); the PRM build's shard summaries (radix_hist)
+  DevBuf scan_sums;   // scan_exclusive_i64: block sums
+  PinBuf pin_edge;    // edge_pipeline: pinned twins of the chunk slots for pageable callers
+  PinBuf pin_radii;   // the PRM build's heuristic_radius table (kept across calls: radii_ptr)
+  PinBuf pin_bel;     // belief_download_full: the host V x B table of the last porrt_belief_vi (bel.dist / bel.type)
+  PinBuf pin_row, pin_col;   // porrt_mmprm_plan: the grouped PRM's CSR
+  PinBuf pin_flags;   // a few counters the kernels write straight into host memory (no DMA engine: see read_flags_dev, nn.cu)
 };
 
 #define CTX_CHECK(ctx) do { if (!(ctx)) return PORRT_ERR_INVALID_ARG; } while (0)
@@ -223,12 +265,13 @@ static inline int32_t porrt_fail(porrt_ctx* ctx, int32_t code, const std::string
   return code;
 }
 
+// (the expression's text is cut at 200 characters: a carve() call spells out its whole layout)
 #define CUDA_TRY(ctx, expr)                                                                        \
   do {                                                                                             \
     cudaError_t _e = (expr);                                                                       \
     if (_e != cudaSuccess) {                                                                       \
       char _b[512];                                                                                \
-      snprintf(_b, sizeof(_b), "%s:%d %s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(_e)); \
+      snprintf(_b, sizeof(_b), "%s:%d %.200s -> %s", __FILE__, __LINE__, #expr, cudaGetErrorString(_e)); \
       return porrt_fail(ctx, PORRT_ERR_CUDA, _b);                                                  \
     }                                                                                              \
   } while (0)

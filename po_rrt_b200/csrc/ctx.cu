@@ -52,14 +52,15 @@ PORRT_API int32_t porrt_ctx_destroy(porrt_ctx* ctx) {
   ctx->d_plane.release(); ctx->d_bits.release();
   ctx->d_vxy_sorted.release(); ctx->d_vid_sorted.release(); ctx->d_cell_start.release();
   ctx->d_vxy.release(); ctx->d_vcell.release();
-  for (DevBuf& b : ctx->nn_tmp) b.release();
+  ctx->nn_bins.release();
   ctx->nn_stage.release(); ctx->nn_stage2.release(); ctx->comm_tmp.release(); ctx->d_nbr_start.release(); ctx->d_nbr_script.release();
-  for (DevBuf& b : ctx->scratch) b.release();
+  for (DevBuf* b : {&ctx->ws_main, &ctx->ws_owner, &ctx->ws_vid, &ctx->ws_table, &ctx->ws_query, &ctx->ws_seg, &ctx->sort_keys,
+                    &ctx->sort_vals, &ctx->ws_state, &ctx->radix_keys, &ctx->radix_vals, &ctx->radix_hist, &ctx->scan_sums})
+    b->release();
   pto_grow_release(ctx);
   ctx->kd_buf.release(); ctx->d_prm_row.release(); ctx->d_prm_col.release(); ctx->d_bel_succ.release(); ctx->bel.dev.release();
   if (ctx->aux_stream) cudaStreamDestroy(ctx->aux_stream);
-  for (PinBuf& b : ctx->pin) b.release();
-  ctx->pin_flags.release();
+  for (PinBuf* b : {&ctx->pin_edge, &ctx->pin_radii, &ctx->pin_bel, &ctx->pin_row, &ctx->pin_col, &ctx->pin_flags}) b->release();
   for (int s = 0; s < MAX_SLOTS; ++s) {
     if (ctx->ev_in[s]) cudaEventDestroy(ctx->ev_in[s]);
     if (ctx->ev_k[s]) cudaEventDestroy(ctx->ev_k[s]);

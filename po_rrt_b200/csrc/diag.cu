@@ -34,7 +34,7 @@ PORRT_API int32_t porrt_measure_l2_gather(porrt_ctx* ctx, int64_t buffer_bytes, 
   CUDA_TRY(ctx, buf.ensure((size_t)bytes + 64));
   cudaStream_t st = ctx->stream;
   CUDA_TRY(ctx, cudaMemsetAsync(buf.p, 1, (size_t)bytes, st));
-  CUDA_TRY(ctx, ctx->scratch[4].ensure(16));
+  CUDA_TRY(ctx, ctx->ws_query.ensure(16));
   const uint32_t mask = (uint32_t)(bytes / 32 - 1);
   const int rounds = 256, blocks = ctx->sm_count * 32;
   cudaEvent_t e0, e1;
@@ -43,7 +43,7 @@ PORRT_API int32_t porrt_measure_l2_gather(porrt_ctx* ctx, int64_t buffer_bytes, 
   double best = 0.0;
   for (int it = 0; it < 6; ++it) {
     cudaEventRecord(e0, st);
-    l2_gather_kernel<<<blocks, 256, 0, st>>>(buf.as<uint32_t>(), mask, rounds, 12345u + it, ctx->scratch[4].as<uint32_t>());
+    l2_gather_kernel<<<blocks, 256, 0, st>>>(buf.as<uint32_t>(), mask, rounds, 12345u + it, ctx->ws_query.as<uint32_t>());
     ctx->launches += 1;
     cudaEventRecord(e1, st);
     if (cudaEventSynchronize(e1) != cudaSuccess) break;

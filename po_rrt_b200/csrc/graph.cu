@@ -180,18 +180,17 @@ int32_t kd_preorder_rank_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, in
 #define KD_TRY(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) return fail(#expr, _e); } while (0)
 #define KD_LAUNCHED() do { ++launches; KD_TRY(cudaGetLastError()); } while (0)
   if (n <= 0) return PORRT_OK;
-  KD_TRY(ctx->kd_buf.ensure((size_t)n * 4 * 8 + (size_t)n + 128));
-  char* b = ctx->kd_buf.as<char>();
-  int32_t* cur = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* child = (int32_t*)b; b += (size_t)n * 8;
-  int32_t* size = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* parent = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* node_depth = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* exits = (int32_t*)b; b += (size_t)n * 4;     // two-phase start only
-  int32_t* up = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* remaining = (int32_t*)b; b += 16;
+  int32_t *cur, *child, *size, *parent, *node_depth, *exits, *up, *remaining;
+  uint8_t* side;
+  KD_TRY(carve(ctx->kd_buf, [&](Carve& c) {
+    cur = c.take<int32_t>(n); child = c.take<int32_t>(2 * n); size = c.take<int32_t>(n); parent = c.take<int32_t>(n);
+    node_depth = c.take<int32_t>(n);
+    exits = c.take<int32_t>(n);     // two-phase start only
+    up = c.take<int32_t>(n);
+    remaining = c.take<int32_t>(2);
+    side = c.take<uint8_t>(n);
+  }));
   int32_t* max_depth = remaining + 1;
-  uint8_t* side = (uint8_t*)b;
   const int blocks = div_up(n, 256);
   kd_init_kernel<<<blocks, 256, 0, st>>>(n, cur, child, size, node_depth, out_rank_dev, root_of_dev);
   KD_LAUNCHED();
@@ -270,9 +269,9 @@ PORRT_API int32_t porrt_kd_preorder_rank(porrt_ctx* ctx, const double* xy, int64
   if (n < 0 || (n > 0 && !out_rank)) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "kd_preorder_rank: bad arguments");
   if (n == 0) return PORRT_OK;
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  CUDA_TRY(ctx, ctx->scratch[9].ensure((size_t)n * 20));
-  double* d_xy = ctx->scratch[9].as<double>();
-  int32_t* d_rank = (int32_t*)(ctx->scratch[9].as<char>() + (size_t)n * 16);
+  double* d_xy;
+  int32_t* d_rank;
+  CUDA_TRY(ctx, carve(ctx->radix_vals, [&](Carve& c) { d_xy = c.take<double>(2 * n); d_rank = c.take<int32_t>(n); }));
   if (xy) CUDA_TRY(ctx, cudaMemcpyAsync(d_xy, xy, (size_t)n * 16, cudaMemcpyHostToDevice, ctx->stream));
   else d_xy = ctx->d_vxy.as<double>();
   int32_t rc = kd_preorder_rank_dev(ctx, d_xy, n, d_rank, nullptr);
@@ -452,8 +451,8 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
   // radii: node k (k >= 1) queries with heuristic_radius(k + 1) -- n_nodes AFTER adding the new node (prm.rs:61-65).
   // libm on host threads, started now and joined after the device has binned the vertices and ranked the kd-tree
   // (neither needs the radii): ~3.6 ms at n = 1e6 that used to sit in front of the device work.
-  CUDA_TRY(ctx, ctx->pin[1].ensure((size_t)n * 8));   // pinned: the upload after the join is one async DMA
-  double* radius = ctx->pin[1].as<double>();
+  CUDA_TRY(ctx, ctx->pin_radii.ensure((size_t)n * 8));   // pinned: the upload after the join is one async DMA
+  double* radius = ctx->pin_radii.as<double>();
   // multi-GPU (comm.cu): this rank answers the queries of new nodes [lo, hi) only -- and needs only their radii
   const int world = ctx->comm_world;
   int64_t lo = 0, hi = n;
@@ -507,26 +506,23 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
 
   // device inputs
   CUDA_TRY(ctx, ctx->d_vxy.ensure((size_t)n * 16));
-  DevBuf& aux = ctx->scratch[3];
-  // carved below: 1 + 3 arrays of 8 bytes, 4 (+ 1 for grouped builds) of 4 bytes per node, + the "+1" entries and the flag
-  CUDA_TRY(ctx, aux.ensure((size_t)n * (8 + 3 * 8 + 4 * 4 + (gb ? 4 : 0)) + 3 * 8 + 16 + 256));
-  CUDA_TRY(ctx, ctx->d_prm_row.ensure((size_t)(n + 1) * 8));   // the result lives in its own buffers: it is retained (porrt_prm_fetch,
-  char* b = aux.as<char>();                                     // porrt_graph_from_prm) while later calls reuse the shared scratch
-  double* d_radius = (double*)b; b += (size_t)n * 8;
-  int64_t* d_off = (int64_t*)b; b += (size_t)(n + 1) * 8;
-  int64_t* d_early_off = (int64_t*)b; b += (size_t)(n + 1) * 8;
-  int64_t* d_late_off = (int64_t*)b; b += (size_t)(n + 1) * 8;
-  int64_t* d_row_ptr = ctx->d_prm_row.as<int64_t>();
-  uint32_t* d_prefix = (uint32_t*)b; b += (size_t)n * 4;
-  int32_t* d_rank = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* d_early_cnt = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* d_late_cnt = (int32_t*)b; b += (size_t)n * 4;
-  int32_t* d_flag = (int32_t*)b; b += 16;
+  double* d_radius;
+  int64_t *d_off, *d_early_off, *d_late_off;
+  uint32_t* d_prefix;
+  int32_t *d_rank, *d_early_cnt, *d_late_cnt, *d_flag;
   uint32_t* d_group_base = nullptr;
-  if (gb) {
-    d_group_base = (uint32_t*)b; b += (size_t)n * 4;
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_group_base, gb, (size_t)n * 4, cudaMemcpyHostToDevice, st));
-  }
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_radius = c.take<double>(n);
+    d_off = c.take<int64_t>(n + 1); d_early_off = c.take<int64_t>(n + 1); d_late_off = c.take<int64_t>(n + 1);
+    d_prefix = c.take<uint32_t>(n);
+    d_rank = c.take<int32_t>(n); d_early_cnt = c.take<int32_t>(n); d_late_cnt = c.take<int32_t>(n);
+    d_flag = c.take<int32_t>(4);
+    if (gb) d_group_base = c.take<uint32_t>(n);
+  }));
+  // the result lives in its own buffers: it is retained (porrt_prm_fetch, porrt_graph_from_prm) while later calls reuse the work space
+  CUDA_TRY(ctx, ctx->d_prm_row.ensure((size_t)(n + 1) * 8));
+  int64_t* d_row_ptr = ctx->d_prm_row.as<int64_t>();
+  if (gb) CUDA_TRY(ctx, cudaMemcpyAsync(d_group_base, gb, (size_t)n * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_vxy.p, samples_xy, (size_t)n * 16, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemsetAsync(d_late_cnt, 0, (size_t)n * 4, st));
   CUDA_TRY(ctx, cudaMemsetAsync(d_flag, 0, 4, st));
@@ -576,20 +572,20 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
   // (bins and kd ranks above are replicated on every rank; from here on the rank works on its shard [lo, hi))
   // 3. prefix-restricted radius queries: neighbours(k) = { j < k : norm2(x_j, x_k) <= r_k }
   int64_t total = 0;
-  rc = nn_radius_count_fill_dev(ctx, ctx->d_vxy.as<double>() + 2 * lo, d_radius + lo, m, d_prefix + lo, nullptr, nullptr, d_off, &ctx->scratch[2], &total,
+  rc = nn_radius_count_fill_dev(ctx, ctx->d_vxy.as<double>() + 2 * lo, d_radius + lo, m, d_prefix + lo, nullptr, nullptr, d_off, &ctx->ws_table, &total,
                                 d_group_base ? d_group_base + lo : nullptr, false, false);
   if (rc) return rc;
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
   t1 = now_ms(); ph[2] = t1 - t0; t0 = t1;
 
-  int32_t* d_ids = ctx->scratch[2].as<int32_t>();
+  int32_t* d_ids = ctx->ws_table.as<int32_t>();
 
   // 4. edge checks neighbour -> new node (prm.rs:91-96); the order inside a list does not matter to them
   const int64_t tot1 = std::max<int64_t>(total, 1);
-  CUDA_TRY(ctx, ctx->scratch[0].ensure((size_t)tot1 * 4));  // owner (= new node id)
-  CUDA_TRY(ctx, ctx->scratch[1].ensure((size_t)tot1 * 4));  // validity ids
-  int32_t* d_owner = ctx->scratch[0].as<int32_t>();
-  int32_t* d_vid = ctx->scratch[1].as<int32_t>();
+  CUDA_TRY(ctx, ctx->ws_owner.ensure((size_t)tot1 * 4));  // owner (= new node id)
+  CUDA_TRY(ctx, ctx->ws_vid.ensure((size_t)tot1 * 4));    // validity ids
+  int32_t* d_owner = ctx->ws_owner.as<int32_t>();
+  int32_t* d_vid = ctx->ws_vid.as<int32_t>();
   if (total > 0) {
     seg_owner_kernel<<<div_up(m * 32, 256), 256, 0, st>>>(d_off, m, (int32_t)lo, d_owner);
     LAUNCH_CHECK(ctx);
@@ -616,8 +612,8 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     if (flag >= -1) {
       // valid neighbours packed densely, then every list put into kd pre-order (2/3 of the candidates are left to sort)
-      CUDA_TRY(ctx, ctx->scratch[0].ensure((size_t)std::max<int64_t>(n_half, 1) * 4));   // the owner list is dead by now
-      int32_t* d_dense = ctx->scratch[0].as<int32_t>();
+      CUDA_TRY(ctx, ctx->ws_owner.ensure((size_t)std::max<int64_t>(n_half, 1) * 4));   // the owner list is dead by now
+      int32_t* d_dense = ctx->ws_owner.as<int32_t>();
       prm_pack_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(d_off, d_early_off, n, d_ids, d_early_cnt, d_dense);
       LAUNCH_CHECK(ctx);
       const double tw = now_ms();
@@ -643,8 +639,8 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
     int64_t* d_local_off = d_late_off;   // free until the transpose below
     rc = scan_exclusive_i64(ctx, d_early_cnt + lo, m, d_local_off);
     if (rc) return rc;
-    CUDA_TRY(ctx, ctx->scratch[10].ensure((size_t)world * 16 + 64));
-    int64_t* d_summary = ctx->scratch[10].as<int64_t>();
+    CUDA_TRY(ctx, ctx->radix_hist.ensure((size_t)world * 16 + 64));
+    int64_t* d_summary = ctx->radix_hist.as<int64_t>();
     prm_shard_summary_kernel<<<1, 1, 0, st>>>(d_local_off + m, d_flag, d_summary + 2 * ctx->comm_rank);
     LAUNCH_CHECK(ctx);
     std::vector<int64_t> off16(world + 1);
@@ -665,8 +661,8 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
     }
     n_half = ids_off[world] / 4;
     if (flag >= -1) {
-      CUDA_TRY(ctx, ctx->scratch[0].ensure((size_t)std::max<int64_t>(n_half, 1) * 4));   // the owner list is dead by now
-      int32_t* d_dense = ctx->scratch[0].as<int32_t>();
+      CUDA_TRY(ctx, ctx->ws_owner.ensure((size_t)std::max<int64_t>(n_half, 1) * 4));   // the owner list is dead by now
+      int32_t* d_dense = ctx->ws_owner.as<int32_t>();
       if (m > 0) {
         prm_pack_kernel<<<div_up(m * 32, 256), 256, 0, st>>>(d_off, d_local_off, m, d_ids, d_early_cnt + lo, d_dense + ids_off[ctx->comm_rank] / 4);
         LAUNCH_CHECK(ctx);
@@ -692,12 +688,10 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
   const int64_t n_edges = 2 * n_half;
   *out_n_edges = n_edges;
   const int64_t half1 = std::max<int64_t>(n_half, 1);
-  // the validity ids (scratch 1) are dead after the compaction: late lists + cursors go there (the segment sort's radix
-  // fallback owns scratch 5 / 6 and 8..10)
-  CUDA_TRY(ctx, ctx->scratch[1].ensure((size_t)half1 * 4 + (size_t)n * 4));
+  // the validity ids are dead after the compaction: late lists + cursors go there
+  int32_t *d_vals, *d_cursor;
+  CUDA_TRY(ctx, carve(ctx->ws_vid, [&](Carve& c) { d_vals = c.take<int32_t>(half1); d_cursor = c.take<int32_t>(n); }));
   CUDA_TRY(ctx, ctx->d_prm_col.ensure((size_t)std::max<int64_t>(n_edges, 1) * 4));
-  int32_t* d_vals = ctx->scratch[1].as<int32_t>();
-  int32_t* d_cursor = d_vals + half1;
   int32_t* d_col = ctx->d_prm_col.as<int32_t>();
   CUDA_TRY(ctx, cudaMemsetAsync(d_cursor, 0, (size_t)n * 4, st));
   prm_late_count_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(d_seg_off, n, d_compact, d_early_cnt, d_late_cnt);
@@ -823,7 +817,7 @@ __global__ void scatter_zero_kernel(double* __restrict__ d, const int64_t* __res
 // plan_qmdp on a graph that already lives on the device (all d_* are device pointers; h_val = host copy of the validity table).
 // Roadmaps whose value column fits in shared memory go to the on-chip column solver (colsolve.cu, one column per world), larger
 // ones to the frontier relaxation over global memory (sssp_frontier.cu).  out_dist (host, [Wall][V]) may be null: the table then
-// stays on the device only (timing, device-resident pipelines).  Work space: scratch[2]; porrt_ctx_last_phase_ms afterwards:
+// stays on the device only (timing, device-resident pipelines).  Work space: ws_table; porrt_ctx_last_phase_ms afterwards:
 // [0] device ms of the backups, [1] edge records / (parent, world) pairs worked through.
 static int32_t sssp_core(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_col, const double* d_xy, int64_t V, int64_t E,
                          const int32_t* d_nvid, const uint64_t* d_val, const uint64_t* h_val, int32_t n_validities, int32_t mask_words,
@@ -850,26 +844,30 @@ static int32_t sssp_core(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_
       }
     }
   const int64_t n_fin = cols ? (int64_t)zero_idx.size() : (int64_t)fin_nw.size() / 2;
-  DevBuf& g = ctx->scratch[2];
-  const size_t need = (size_t)V * Wall * 8 + (size_t)n_fin * 8 + 64 +
-                      (cols ? (size_t)(V + 1) * 8 + (size_t)E * 20 + (size_t)Wall * 32 : 0) + 12 * 16 + 256;
-  CUDA_TRY(ctx, g.ensure(need));
-  char* b = g.as<char>();
-  auto take = [&](size_t bytes) { char* p = b; b += (bytes + 15) & ~(size_t)15; return p; };
-  double* d_out = (double*)take((size_t)V * Wall * 8);   // [Wall][V]: this rank fills rows wlo..whi, the gather the rest
-  int32_t* d_flag = (int32_t*)take(16);
+  double* d_out;   // [Wall][V]: this rank fills rows wlo..whi, the gather the rest
+  int32_t* d_flag;
+  int64_t* d_zero = nullptr;                           // column solver
+  double *d_cost = nullptr, *d_cost_t = nullptr;
+  uint32_t *d_ce = nullptr, *d_rs = nullptr, *d_cursor = nullptr;
+  uint64_t* d_cmask = nullptr;
+  int32_t* d_fin = nullptr;                            // frontier
+  CUDA_TRY(ctx, carve(ctx->ws_table, [&](Carve& c) {
+    d_out = c.take<double>((size_t)V * Wall);
+    d_flag = c.take<int32_t>(4);
+    if (W > 0 && cols) {
+      d_zero = c.take<int64_t>(n_fin + 1);
+      d_cost = c.take<double>(E); d_cost_t = c.take<double>(E);
+      d_ce = c.take<uint32_t>(E); d_rs = c.take<uint32_t>(V + 1); d_cursor = c.take<uint32_t>(V + 1);
+      d_cmask = c.take<uint64_t>((size_t)Wall * 4);
+    } else if (W > 0) {
+      d_fin = c.take<int32_t>(2 * n_fin + 2);
+    }
+  }));
   int sweeps = 0;
   double offers = 0.0;
   tstart(ctx);
   if (W > 0 && cols) {
     // one column per world, solved on chip; d_out is the column-major table itself
-    int64_t* d_zero = (int64_t*)take((size_t)n_fin * 8 + 8);
-    double* d_cost = (double*)take((size_t)E * 8);
-    double* d_cost_t = (double*)take((size_t)E * 8);
-    uint32_t* d_ce = (uint32_t*)take((size_t)E * 4);
-    uint32_t* d_rs = (uint32_t*)take((size_t)(V + 1) * 4);
-    uint32_t* d_cursor = (uint32_t*)take((size_t)(V + 1) * 4);
-    uint64_t* d_cmask = (uint64_t*)take((size_t)Wall * 32);
     std::vector<uint64_t> cmask((size_t)Wall * 4, world_view ? 0 : ~(uint64_t)0);
     if (world_view)
       for (int w = 0; w < Wall; ++w)
@@ -900,7 +898,6 @@ static int32_t sssp_core(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     offers = (double)off;
   } else if (W > 0) {
-    int32_t* d_fin = (int32_t*)take((size_t)n_fin * 8 + 8);
     // (node, world) pairs interleaved on the host -> two arrays on the device
     std::vector<int32_t> split((size_t)n_fin * 2);
     for (int64_t k = 0; k < n_fin; ++k) { split[(size_t)k] = fin_nw[(size_t)2 * k]; split[(size_t)(n_fin + k)] = fin_nw[(size_t)2 * k + 1]; }
@@ -942,16 +939,15 @@ PORRT_API int32_t porrt_sssp_worlds(porrt_ctx* ctx, int64_t V, const int64_t* ro
   if (world_view)
     for (int64_t u = 0; u < V; ++u)
       if (node_vid[u] < 0 || node_vid[u] >= n_validities) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "sssp_worlds: node validity id out of range");
-  DevBuf& g = ctx->scratch[3];
   const size_t nvw = world_view ? (size_t)n_validities * mask_words : 0;
-  CUDA_TRY(ctx, g.ensure((size_t)(V + 1) * 8 + (size_t)E * 4 + (size_t)V * 20 + nvw * 8 + 8 * 16));
-  char* b = g.as<char>();
-  auto take = [&](size_t bytes) { char* p = b; b += (bytes + 15) & ~(size_t)15; return p; };
-  int64_t* d_row = (int64_t*)take((size_t)(V + 1) * 8);
-  double* d_xy = (double*)take((size_t)V * 16);
-  int32_t* d_col = (int32_t*)take((size_t)E * 4);
-  int32_t* d_nvid = (int32_t*)take((size_t)V * 4);
-  uint64_t* d_val = (uint64_t*)take(nvw * 8);
+  int64_t* d_row;
+  double* d_xy;
+  int32_t *d_col, *d_nvid;
+  uint64_t* d_val;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_row = c.take<int64_t>(V + 1); d_xy = c.take<double>(2 * V); d_col = c.take<int32_t>(E); d_nvid = c.take<int32_t>(V);
+    d_val = c.take<uint64_t>(nvw);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_row, row_ptr, (size_t)(V + 1) * 8, cudaMemcpyHostToDevice, st));
   if (E) CUDA_TRY(ctx, cudaMemcpyAsync(d_col, col, (size_t)E * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_xy, xy, (size_t)V * 16, cudaMemcpyHostToDevice, st));
@@ -976,11 +972,10 @@ PORRT_API int32_t porrt_sssp_worlds_prm(porrt_ctx* ctx, const int64_t* finals_pt
   const int64_t V = ctx->prm_n, E = ctx->prm_edges;
   const int nv = ctx->n_validities;
   // node validity ids on the device; obstacles (-1) get an extra all-zero validity row appended to the table
-  DevBuf& g = ctx->scratch[3];
   const size_t nvw = (size_t)(nv + 1) * ctx->mask_words;
-  CUDA_TRY(ctx, g.ensure((size_t)V * 4 + nvw * 8 + 64));
-  int32_t* d_nvid = g.as<int32_t>();
-  uint64_t* d_val = (uint64_t*)(g.as<char>() + (((size_t)V * 4 + 15) & ~(size_t)15));
+  int32_t* d_nvid;
+  uint64_t* d_val;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) { d_nvid = c.take<int32_t>(V); d_val = c.take<uint64_t>(nvw); }));
   std::vector<uint64_t> val(ctx->validities);
   val.resize(nvw, 0);
   CUDA_TRY(ctx, cudaMemcpyAsync(d_val, val.data(), nvw * 8, cudaMemcpyHostToDevice, ctx->stream));
@@ -1216,15 +1211,15 @@ static int32_t belief_download_full(porrt_ctx* ctx, const double* d_dist_nb, dou
   const int B = R.B;
   const size_t nb = (size_t)V * B;
   if (!d_dist_nb) {
-    CUDA_TRY(ctx, ctx->scratch[3].ensure(nb * 8));
-    double* d = ctx->scratch[3].as<double>();
+    CUDA_TRY(ctx, ctx->ws_table.ensure(nb * 8));
+    double* d = ctx->ws_table.as<double>();
     belief_untranspose_kernel<<<dim3(div_up(V, 32), div_up(B, 32)), 256, 0, st>>>(R.d_dist_cm, V, R.d_colpos, V, B, d);
     LAUNCH_CHECK(ctx);
     d_dist_nb = d;
   }
-  CUDA_TRY(ctx, ctx->pin[3].ensure(nb * 9 + 64));
-  double* h_dist = ctx->pin[3].as<double>();
-  uint8_t* h_type = (uint8_t*)(h_dist + nb);
+  double* h_dist;
+  uint8_t* h_type;
+  CUDA_TRY(ctx, carve(ctx->pin_bel, [&](Carve& c) { h_dist = c.take<double>(nb); h_type = c.take<uint8_t>(nb); }));
   const int n_pieces = nb > (1u << 20) ? 8 : 1;
   for (int k = 0; k < n_pieces; ++k) {
     const size_t lo = nb * (size_t)k / (size_t)n_pieces, hi = nb * (size_t)(k + 1) / (size_t)n_pieces;
@@ -1369,39 +1364,38 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
   // final belief nodes as indices into the [column][node] table the backups run on
   for (int64_t& z : zero_idx) { const int64_t f = z / B; const int b2 = (int)(z % B); z = (int64_t)colpos[(size_t)b2] * V + f; }
 
-  DevBuf& g = ctx->scratch[3];
-  const size_t need = (size_t)(V + 1) * 16 + (size_t)E * 28 + (size_t)V * 16 + 2 * compat.size() + (size_t)V * 17 +
-                      (size_t)Bp * 40 + (cols ? 0 : (size_t)V * Bp * 8) + zero_idx.size() * 8 + 24 * 16 + 512;
-  CUDA_TRY(ctx, g.ensure(need));
-  char* b = g.as<char>();
-  auto take = [&](size_t bytes) { char* p = b; b += (bytes + 15) & ~(size_t)15; return p; };
-  int64_t* d_row = (int64_t*)take((size_t)(V + 1) * 8);
-  double* d_cost = (double*)take((size_t)E * 8);
-  double* d_xy = (double*)take((size_t)V * 16);
-  double* d_table_m = cols ? nullptr : (double*)take((size_t)V * Bp * 8);   // frontier path: the table in Morton numbering, [column][pos]
+  int64_t* d_row;
+  double *d_cost, *d_xy, *d_cost_t;
+  double* d_table_m = nullptr;   // frontier path: the table in Morton numbering, [column][pos]
+  uint64_t* d_cmask;
+  int32_t *d_col, *d_evid, *d_nvid, *d_nset, *d_col_belief, *d_changed;
+  uint32_t *d_ce, *d_rs, *d_cursor;
+  uint8_t* d_compat;
+  int64_t* d_zero;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_row = c.take<int64_t>(V + 1);
+    d_cost = c.take<double>(E);
+    d_xy = c.take<double>(2 * V);
+    if (!cols) d_table_m = c.take<double>((size_t)V * Bp);
+    d_cmask = c.take<uint64_t>((size_t)Bp * 4);
+    d_col = c.take<int32_t>(E); d_evid = c.take<int32_t>(E);
+    d_ce = c.take<uint32_t>(E); d_rs = c.take<uint32_t>(V + 1); d_cursor = c.take<uint32_t>(V + 1);
+    d_cost_t = c.take<double>(E);
+    d_nvid = c.take<int32_t>(V); d_nset = c.take<int32_t>(V); d_col_belief = c.take<int32_t>(Bp);
+    d_changed = c.take<int32_t>(4);
+    d_compat = c.take<uint8_t>(compat.size());
+    d_zero = c.take<int64_t>(zero_idx.size() + 1);
+  }));
   // the column solver's table ([column][node]), the node types and the column map outlive the call (lazy result, policy walk)
   auto& R = ctx->bel;
   R.V = 0; R.on_host = false;
-  CUDA_TRY(ctx, R.dev.ensure((size_t)V * Bp * 9 + (size_t)V * B + (size_t)B * 4 + 4 * 16));
-  char* rb = R.dev.as<char>();
-  auto take_r = [&](size_t bytes) { char* p = rb; rb += (bytes + 15) & ~(size_t)15; return p; };
-  double* d_dist_cm = (double*)take_r((size_t)V * Bp * 8);
-  uint8_t* d_type = (uint8_t*)take_r((size_t)V * B);
-  uint8_t* d_type_cm = (uint8_t*)take_r((size_t)V * Bp);
-  int32_t* d_colpos = (int32_t*)take_r((size_t)B * 4);
-  uint64_t* d_cmask = (uint64_t*)take((size_t)Bp * 32);
-  int32_t* d_col = (int32_t*)take((size_t)E * 4);
-  int32_t* d_evid = (int32_t*)take((size_t)E * 4);
-  uint32_t* d_ce = (uint32_t*)take((size_t)E * 4);
-  uint32_t* d_rs = (uint32_t*)take((size_t)(V + 1) * 4);
-  uint32_t* d_cursor = (uint32_t*)take((size_t)(V + 1) * 4);
-  double* d_cost_t = (double*)take((size_t)E * 8);
-  int32_t* d_nvid = (int32_t*)take((size_t)V * 4);
-  int32_t* d_nset = (int32_t*)take((size_t)V * 4);
-  int32_t* d_col_belief = (int32_t*)take((size_t)Bp * 4);
-  int32_t* d_changed = (int32_t*)take(16);
-  uint8_t* d_compat = (uint8_t*)take(compat.size());
-  int64_t* d_zero = (int64_t*)take(zero_idx.size() * 8 + 8);
+  double* d_dist_cm;
+  uint8_t *d_type, *d_type_cm;
+  int32_t* d_colpos;
+  CUDA_TRY(ctx, carve(R.dev, [&](Carve& c) {
+    d_dist_cm = c.take<double>((size_t)V * Bp); d_type = c.take<uint8_t>((size_t)V * B); d_type_cm = c.take<uint8_t>((size_t)V * Bp);
+    d_colpos = c.take<int32_t>(B);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_row, row_ptr, (size_t)(V + 1) * 8, cudaMemcpyHostToDevice, st));
   if (E) {
     CUDA_TRY(ctx, cudaMemcpyAsync(d_col, col, (size_t)E * 4, cudaMemcpyHostToDevice, st));

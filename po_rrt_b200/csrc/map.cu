@@ -396,22 +396,22 @@ PORRT_API int32_t porrt_map_upload(porrt_ctx* ctx, const uint8_t* occ, const uin
   ctx->has_map = false;
   cudaStream_t st = ctx->stream;
   const size_t px = (size_t)H * W;
-  CUDA_TRY(ctx, ctx->scratch[0].ensure(px));
-  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->scratch[0].p, occ, px, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, ctx->ws_owner.ensure(px));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws_owner.p, occ, px, cudaMemcpyHostToDevice, st));
   const uint8_t* d_zone = nullptr;
   int n_zones = 0, n_worlds = 0;
   std::vector<double> zone_pos;
   const double ppm = (double)W / (up[0] - low[0]);  // map_io.rs:91
   if (zone) {
-    CUDA_TRY(ctx, ctx->scratch[1].ensure(px));
-    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->scratch[1].p, zone, px, cudaMemcpyHostToDevice, st));
-    d_zone = ctx->scratch[1].as<uint8_t>();
-    CUDA_TRY(ctx, ctx->scratch[2].ensure(768 * 4));
-    CUDA_TRY(ctx, cudaMemsetAsync(ctx->scratch[2].p, 0, 768 * 4, st));
-    zone_stats_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(d_zone, H, W, ctx->scratch[2].as<uint32_t>());
+    CUDA_TRY(ctx, ctx->ws_vid.ensure(px));
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws_vid.p, zone, px, cudaMemcpyHostToDevice, st));
+    d_zone = ctx->ws_vid.as<uint8_t>();
+    CUDA_TRY(ctx, ctx->ws_table.ensure(768 * 4));
+    CUDA_TRY(ctx, cudaMemsetAsync(ctx->ws_table.p, 0, 768 * 4, st));
+    zone_stats_kernel<<<ctx->sm_count * 4, 256, 0, st>>>(d_zone, H, W, ctx->ws_table.as<uint32_t>());
     LAUNCH_CHECK(ctx);
     uint32_t stats[768];
-    CUDA_TRY(ctx, cudaMemcpyAsync(stats, ctx->scratch[2].p, sizeof(stats), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(stats, ctx->ws_table.p, sizeof(stats), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     int max_id = 0;  // init_zone_ids (map_io.rs:130-145): n_zones = max id + 1, 1 even without any zone pixel
     for (int z = 0; z < 255; ++z)
@@ -456,7 +456,7 @@ PORRT_API int32_t porrt_map_upload(porrt_ctx* ctx, const uint8_t* occ, const uin
   const int tiles_x = (W + 15) / 16, tiles_y = (H + 7) / 8;
   const size_t grid_bytes = (size_t)tiles_x * tiles_y * 128;
   CUDA_TRY(ctx, ctx->d_grid.ensure(grid_bytes));
-  fuse_tile_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->scratch[0].as<uint8_t>(), d_zone, H, W, tiles_x, tiles_y, kind,
+  fuse_tile_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(ctx->ws_owner.as<uint8_t>(), d_zone, H, W, tiles_x, tiles_y, kind,
                                                       ctx->d_grid.as<uint8_t>());
   LAUNCH_CHECK(ctx);
   {  // class bytes of the 16 x 16 blocks (large-map path)
@@ -594,8 +594,8 @@ __global__ void csr_rows_kernel(const int64_t* __restrict__ row_ptr, int64_t V, 
 // ------------------------------------------------------------------------------------------------ host-buffer pipeline
 // Every host-buffer edge entry point is one chunked pipeline: H2D(c+1) | kernel(c) | D2H(c-1) on three streams over MAX_SLOTS
 // device slots.  Caller buffers that are pinned (cudaHostAlloc / torch pin_memory) are DMA'd directly, pageable ones are
-// staged through the ctx's pinned buffer.  A slot is carved with a 256-byte-aligned bump allocator (the kernels read endpoints
-// as 16-byte vectors and write 8-byte masks; chunk sizes are arbitrary).
+// staged through the ctx's pinned buffer.  Slot pieces are 256-byte aligned (the kernels read endpoints as 16-byte vectors and write
+// 8-byte masks; chunk sizes are arbitrary).
 struct EdgeJob {
   enum Mode { COORDS, INDEXED, CSR } mode = COORDS;
   const void* in[2] = {nullptr, nullptr};   // per-edge host input arrays: COORDS from/to xy (16 B), INDEXED from/to ids (4 B), CSR col (4 B)
@@ -609,8 +609,6 @@ struct EdgeJob {
   int csr_row_is_to = 1;                    // CSR: 1 = edge col[e] -> row (prm.rs:93, neighbour -> new node), 0 = row -> col[e]
   const char* name = "porrt_edge_validity";
 };
-
-static inline size_t align256(size_t x) { return (x + 255) & ~(size_t)255; }
 
 static int32_t edge_pipeline(porrt_ctx* ctx, const EdgeJob& job, int64_t n) {
   const int words = ctx->mask_words;
@@ -628,22 +626,26 @@ static int32_t edge_pipeline(porrt_ctx* ctx, const EdgeJob& job, int64_t n) {
                 is_pinned_host(job.out_vid8 ? (const void*)job.out_vid8 : (const void*)job.out_vid) &&
                 (!job.out_mask || is_pinned_host(job.out_mask));
   const int slots = MAX_SLOTS;
-  // slot layout (offsets valid for the device slot and, for pageable callers, its pinned twin)
-  size_t off_in[2] = {0, 0}, off_rows = 0, off_vid = 0, off_mask = 0, slot_bytes = 0;
-  for (int k = 0; k < job.n_in; ++k) { off_in[k] = slot_bytes; slot_bytes = align256(slot_bytes + (size_t)ch * job.in_elem[k]); }
-  if (job.mode == EdgeJob::CSR) { off_rows = slot_bytes; slot_bytes = align256(slot_bytes + (size_t)ch * 4); }
-  off_vid = slot_bytes; slot_bytes = align256(slot_bytes + (size_t)ch * vid_elem);
-  if (job.out_mask) { off_mask = slot_bytes; slot_bytes = align256(slot_bytes + (size_t)ch * 8 * words); }
-  CUDA_TRY(ctx, ctx->scratch[3].ensure(slot_bytes * slots));
-  if (!pinned) CUDA_TRY(ctx, ctx->pin[0].ensure(slot_bytes * slots));
+  // the slots, laid out alike in the device buffer and, for pageable callers, its pinned twin
+  struct Slot { char* in[2]; int32_t* rows; char* vid; char* mask; } dev[MAX_SLOTS] = {}, host[MAX_SLOTS] = {};
+  auto slot_layout = [&](Carve& c, Slot* sl) {
+    for (int s = 0; s < slots; ++s) {
+      for (int k = 0; k < job.n_in; ++k) sl[s].in[k] = c.take<char>((size_t)ch * job.in_elem[k], 256);
+      if (job.mode == EdgeJob::CSR) sl[s].rows = c.take<int32_t>(ch, 256);
+      sl[s].vid = c.take<char>((size_t)ch * vid_elem, 256);
+      if (job.out_mask) sl[s].mask = c.take<char>((size_t)ch * 8 * words, 256);
+    }
+  };
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) { slot_layout(c, dev); }));
+  if (!pinned) CUDA_TRY(ctx, carve(ctx->pin_edge, [&](Carve& c) { slot_layout(c, host); }));
   cudaStream_t st = ctx->stream;
   const int64_t n_chunks = (n + ch - 1) / ch;
   const double* d_xy = ctx->d_vxy.as<double>();
   const int64_t V = ctx->n_vertices;
   int32_t* d_bad = nullptr;
   if (job.mode != EdgeJob::COORDS) {
-    CUDA_TRY(ctx, ctx->scratch[4].ensure(16));
-    d_bad = ctx->scratch[4].as<int32_t>();
+    CUDA_TRY(ctx, ctx->ws_query.ensure(16));
+    d_bad = ctx->ws_query.as<int32_t>();
     CUDA_TRY(ctx, cudaMemsetAsync(d_bad, 0, 4, st));
   }
   // the copy streams must not run ahead of work already queued on the compute stream
@@ -653,15 +655,14 @@ static int32_t edge_pipeline(porrt_ctx* ctx, const EdgeJob& job, int64_t n) {
   auto unstage = [&](int64_t c) {   // pageable outputs: copy chunk c out of its pinned slot
     const int s = (int)(c % slots);
     const int64_t off = c * ch, cnt = (n - off) < ch ? (n - off) : ch;
-    const char* hb = ctx->pin[0].as<char>() + slot_bytes * s;
-    memcpy(h_vid_base + (size_t)off * vid_elem, hb + off_vid, (size_t)cnt * vid_elem);
-    if (job.out_mask) memcpy(job.out_mask + off * words, hb + off_mask, (size_t)cnt * 8 * words);
+    memcpy(h_vid_base + (size_t)off * vid_elem, host[s].vid, (size_t)cnt * vid_elem);
+    if (job.out_mask) memcpy(job.out_mask + off * words, host[s].mask, (size_t)cnt * 8 * words);
   };
   for (int64_t c = 0; c < n_chunks; ++c) {
     const int s = (int)(c % slots);
     const int64_t off = c * ch, cnt = (n - off) < ch ? (n - off) : ch;
-    char* dbase = ctx->scratch[3].as<char>() + slot_bytes * s;
-    char* hb = pinned ? nullptr : ctx->pin[0].as<char>() + slot_bytes * s;
+    const Slot& d = dev[s];
+    const Slot& h = host[s];
     if (c >= slots) {
       // slot reuse: its previous D2H must be complete (also frees the pinned staging of that slot)
       CUDA_TRY(ctx, cudaEventSynchronize(ctx->ev_out[s]));
@@ -669,28 +670,27 @@ static int32_t edge_pipeline(porrt_ctx* ctx, const EdgeJob& job, int64_t n) {
     }
     for (int k = 0; k < job.n_in; ++k) {
       const char* src = (const char*)job.in[k] + (size_t)off * job.in_elem[k];
-      if (!pinned) { memcpy(hb + off_in[k], src, (size_t)cnt * job.in_elem[k]); src = hb + off_in[k]; }
-      CUDA_TRY(ctx, cudaMemcpyAsync(dbase + off_in[k], src, (size_t)cnt * job.in_elem[k], cudaMemcpyHostToDevice, ctx->copy_in));
+      if (!pinned) { memcpy(h.in[k], src, (size_t)cnt * job.in_elem[k]); src = h.in[k]; }
+      CUDA_TRY(ctx, cudaMemcpyAsync(d.in[k], src, (size_t)cnt * job.in_elem[k], cudaMemcpyHostToDevice, ctx->copy_in));
     }
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_in[s], ctx->copy_in));
     CUDA_TRY(ctx, cudaStreamWaitEvent(st, ctx->ev_in[s], 0));
     EdgeOut o;
-    if (job.out_vid8) o.vid8 = (int8_t*)(dbase + off_vid); else o.vid = (int32_t*)(dbase + off_vid);
-    if (job.out_mask) o.mask = (uint64_t*)(dbase + off_mask);
+    if (job.out_vid8) o.vid8 = (int8_t*)d.vid; else o.vid = (int32_t*)d.vid;
+    if (job.out_mask) o.mask = (uint64_t*)d.mask;
     int32_t rc;
     if (job.mode == EdgeJob::COORDS) {
-      rc = map_edge_launch(ctx, (const double*)(dbase + off_in[0]), (const double*)(dbase + off_in[1]), nullptr, nullptr, cnt, o, st);
+      rc = map_edge_launch(ctx, (const double*)d.in[0], (const double*)d.in[1], nullptr, nullptr, cnt, o, st);
     } else {
-      int32_t* d_a = (int32_t*)(dbase + off_in[0]);
-      int32_t* d_b = job.mode == EdgeJob::INDEXED ? (int32_t*)(dbase + off_in[1]) : nullptr;
+      int32_t* d_a = (int32_t*)d.in[0];
+      int32_t* d_b = job.mode == EdgeJob::INDEXED ? (int32_t*)d.in[1] : nullptr;
       idx_check_kernel<<<div_up(cnt, 256), 256, 0, st>>>(d_a, d_b, cnt, (int32_t)V, d_bad);
       LAUNCH_CHECK(ctx);
       if (job.mode == EdgeJob::CSR) {
-        int32_t* d_rows = (int32_t*)(dbase + off_rows);
-        csr_rows_kernel<<<div_up(cnt, 256), 256, 0, st>>>(job.row_ptr_dev, job.csr_rows, off, cnt, d_rows);
+        csr_rows_kernel<<<div_up(cnt, 256), 256, 0, st>>>(job.row_ptr_dev, job.csr_rows, off, cnt, d.rows);
         LAUNCH_CHECK(ctx);
-        rc = job.csr_row_is_to ? map_edge_launch(ctx, d_xy, d_xy, d_a, d_rows, cnt, o, st)
-                               : map_edge_launch(ctx, d_xy, d_xy, d_rows, d_a, cnt, o, st);
+        rc = job.csr_row_is_to ? map_edge_launch(ctx, d_xy, d_xy, d_a, d.rows, cnt, o, st)
+                               : map_edge_launch(ctx, d_xy, d_xy, d.rows, d_a, cnt, o, st);
       } else {
         rc = map_edge_launch(ctx, d_xy, d_xy, d_a, d_b, cnt, o, st);
       }
@@ -698,11 +698,11 @@ static int32_t edge_pipeline(porrt_ctx* ctx, const EdgeJob& job, int64_t n) {
     if (rc) return rc;
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_k[s], st));
     CUDA_TRY(ctx, cudaStreamWaitEvent(ctx->copy_out, ctx->ev_k[s], 0));
-    char* h_vid = pinned ? h_vid_base + (size_t)off * vid_elem : hb + off_vid;
-    CUDA_TRY(ctx, cudaMemcpyAsync(h_vid, dbase + off_vid, (size_t)cnt * vid_elem, cudaMemcpyDeviceToHost, ctx->copy_out));
+    char* h_vid = pinned ? h_vid_base + (size_t)off * vid_elem : h.vid;
+    CUDA_TRY(ctx, cudaMemcpyAsync(h_vid, d.vid, (size_t)cnt * vid_elem, cudaMemcpyDeviceToHost, ctx->copy_out));
     if (job.out_mask) {
-      char* h_mask = pinned ? (char*)(job.out_mask + off * words) : hb + off_mask;
-      CUDA_TRY(ctx, cudaMemcpyAsync(h_mask, dbase + off_mask, (size_t)cnt * 8 * words, cudaMemcpyDeviceToHost, ctx->copy_out));
+      char* h_mask = pinned ? (char*)(job.out_mask + off * words) : h.mask;
+      CUDA_TRY(ctx, cudaMemcpyAsync(h_mask, d.mask, (size_t)cnt * 8 * words, cudaMemcpyDeviceToHost, ctx->copy_out));
     }
     CUDA_TRY(ctx, cudaEventRecord(ctx->ev_out[s], ctx->copy_out));
   }
@@ -784,10 +784,10 @@ PORRT_API int32_t porrt_edge_validity_csr_i8(porrt_ctx* ctx, const int64_t* row_
   if (n_rows > ctx->n_vertices || row_ptr[0] != 0 || n < 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_edge_validity_csr_i8: rows exceed the vertex set / row_ptr[0] != 0");
   if (n == 0) return PORRT_OK;
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  CUDA_TRY(ctx, ctx->scratch[5].ensure((size_t)(n_rows + 1) * 8));
-  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->scratch[5].p, row_ptr, (size_t)(n_rows + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
+  CUDA_TRY(ctx, ctx->sort_keys.ensure((size_t)(n_rows + 1) * 8));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ctx->sort_keys.p, row_ptr, (size_t)(n_rows + 1) * 8, cudaMemcpyHostToDevice, ctx->stream));
   EdgeJob j; j.mode = EdgeJob::CSR; j.in[0] = col; j.in_elem[0] = 4; j.n_in = 1; j.out_vid8 = out_vid8;
-  j.row_ptr_dev = ctx->scratch[5].as<int64_t>(); j.csr_rows = n_rows; j.csr_row_is_to = row_is_to ? 1 : 0;
+  j.row_ptr_dev = ctx->sort_keys.as<int64_t>(); j.csr_rows = n_rows; j.csr_row_is_to = row_is_to ? 1 : 0;
   j.name = "porrt_edge_validity_csr_i8";
   return edge_pipeline(ctx, j, n);
 }
@@ -809,9 +809,9 @@ PORRT_API int32_t porrt_state_validity(porrt_ctx* ctx, const double* xy, int64_t
   if (n < 0 || (n > 0 && (!xy || !out_vid))) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_state_validity: bad arguments");
   if (n == 0) return PORRT_OK;
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  CUDA_TRY(ctx, ctx->scratch[3].ensure((size_t)n * 20));
-  double* d_xy = ctx->scratch[3].as<double>();
-  int32_t* d_out = (int32_t*)(ctx->scratch[3].as<char>() + (size_t)n * 16);
+  double* d_xy;
+  int32_t* d_out;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) { d_xy = c.take<double>(2 * n); d_out = c.take<int32_t>(n); }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_xy, xy, (size_t)n * 16, cudaMemcpyHostToDevice, ctx->stream));
   int32_t rc = porrt_state_validity_dev(ctx, d_xy, n, d_out);
   if (rc) return rc;
@@ -841,10 +841,10 @@ PORRT_API int32_t porrt_visibility(porrt_ctx* ctx, const double* xy, int64_t n, 
   if (n < 0 || (n > 0 && (!xy || !out_mask || !out_status))) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_visibility: bad arguments");
   if (n == 0) return PORRT_OK;
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
-  CUDA_TRY(ctx, ctx->scratch[3].ensure((size_t)n * 28));
-  double* d_xy = ctx->scratch[3].as<double>();
-  uint64_t* d_mask = (uint64_t*)(ctx->scratch[3].as<char>() + (size_t)n * 16);
-  int32_t* d_status = (int32_t*)(ctx->scratch[3].as<char>() + (size_t)n * 24);
+  double* d_xy;
+  uint64_t* d_mask;
+  int32_t* d_status;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) { d_xy = c.take<double>(2 * n); d_mask = c.take<uint64_t>(n); d_status = c.take<int32_t>(n); }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_xy, xy, (size_t)n * 16, cudaMemcpyHostToDevice, ctx->stream));
   int32_t rc = porrt_visibility_dev(ctx, d_xy, n, d_mask, d_status);
   if (rc) return rc;

@@ -41,8 +41,8 @@ PORRT_API int32_t porrt_mmprm_plan(porrt_ctx* ctx, int32_t n_modes, const int64_
   // 1. the PRMs of all modes in ONE grouped build (prm_build_impl, graph.cu): one binning, one radius batch, one edge batch, one
   //    CSR over global node ids; a node only sees earlier nodes of its own mode.  (Per-mode calls cost ~1 ms of launch latency
   //    each: 66 ms for 63 modes against ~4 ms for the grouped build.)
-  CUDA_TRY(ctx, ctx->pin[4].ensure((size_t)(T + 1) * 8));   // pinned staging: the CSR comes back by DMA, not through pageable copies
-  int64_t* rp = ctx->pin[4].as<int64_t>();
+  CUDA_TRY(ctx, ctx->pin_row.ensure((size_t)(T + 1) * 8));   // pinned staging: the CSR comes back by DMA, not through pageable copies
+  int64_t* rp = ctx->pin_row.as<int64_t>();
   const int32_t* cl = nullptr;
   int64_t ne = 0;
   {
@@ -51,12 +51,12 @@ PORRT_API int32_t porrt_mmprm_plan(porrt_ctx* ctx, int32_t n_modes, const int64_
     if (rc != PORRT_OK && rc != PORRT_ERR_CAPACITY) return rc;
     for (int k = 0; k < 7; ++k) ctx->last_ms[k] = prm_ph[k];   // porrt_ctx_last_phase_ms: [radii, bin, radius, kd_rank, order, edges, csr]
     ctx->n_last = 7;
-    CUDA_TRY(ctx, ctx->pin[5].ensure((size_t)std::max<int64_t>(ne, 1) * 4));
+    CUDA_TRY(ctx, ctx->pin_col.ensure((size_t)std::max<int64_t>(ne, 1) * 4));
     if (ne > 0) {
-      rc = porrt_prm_fetch(ctx, nullptr, ctx->pin[5].as<int32_t>(), ne);
+      rc = porrt_prm_fetch(ctx, nullptr, ctx->pin_col.as<int32_t>(), ne);
       if (rc) return rc;
     }
-    cl = ctx->pin[5].as<int32_t>();
+    cl = ctx->pin_col.as<int32_t>();
   }
   t1 = mm_now_ms(); ph[0] = t1 - t0; t0 = t1;
 

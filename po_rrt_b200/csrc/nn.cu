@@ -108,8 +108,8 @@ int32_t scan_exclusive_i64(porrt_ctx* ctx, const int32_t* counts_dev, int64_t n,
   cudaStream_t st = ctx->stream;
   if (n == 0) { CUDA_TRY(ctx, cudaMemsetAsync(out_dev, 0, 8, st)); return PORRT_OK; }
   const int64_t nb = (n + SCAN_TILE - 1) / SCAN_TILE;
-  CUDA_TRY(ctx, ctx->scratch[11].ensure((size_t)nb * 8 + 8));
-  int64_t* sums = ctx->scratch[11].as<int64_t>();
+  CUDA_TRY(ctx, ctx->scan_sums.ensure((size_t)nb * 8 + 8));
+  int64_t* sums = ctx->scan_sums.as<int64_t>();
   scan_block_kernel<<<(int)nb, SCAN_BLOCK, 0, st>>>(counts_dev, n, out_dev, sums);
   LAUNCH_CHECK(ctx);
   scan_sums_kernel<<<1, 1024, 0, st>>>(sums, nb, out_dev + n);
@@ -172,18 +172,18 @@ __global__ void __launch_bounds__(RS_WARPS * 32) rs_scatter_kernel(const uint64_
   }
 }
 
-// sorts in place (result ends in keys/vals); tmp buffers from ctx scratch 8..10
+// sorts in place (result ends in keys/vals); work space radix_keys, radix_vals, radix_hist
 int32_t radix_sort_pairs(porrt_ctx* ctx, uint64_t* keys, uint32_t* vals, int64_t n, int key_bits) {
   if (n <= 1) return PORRT_OK;
   cudaStream_t st = ctx->stream;
   const int64_t n_tiles = (n + RS_TILE - 1) / RS_TILE;
-  CUDA_TRY(ctx, ctx->scratch[8].ensure((size_t)n * 8));
-  CUDA_TRY(ctx, ctx->scratch[9].ensure((size_t)n * 4));
-  CUDA_TRY(ctx, ctx->scratch[10].ensure((size_t)n_tiles * 256 * 12 + 16));
-  uint64_t* k2 = ctx->scratch[8].as<uint64_t>();
-  uint32_t* v2 = ctx->scratch[9].as<uint32_t>();
-  int64_t* bases = ctx->scratch[10].as<int64_t>();
-  int32_t* hist = (int32_t*)(ctx->scratch[10].as<char>() + ((size_t)n_tiles * 256 + 1) * 8);
+  CUDA_TRY(ctx, ctx->radix_keys.ensure((size_t)n * 8));
+  CUDA_TRY(ctx, ctx->radix_vals.ensure((size_t)n * 4));
+  int64_t* bases;
+  int32_t* hist;
+  CUDA_TRY(ctx, carve(ctx->radix_hist, [&](Carve& c) { bases = c.take<int64_t>((size_t)n_tiles * 256 + 1); hist = c.take<int32_t>((size_t)n_tiles * 256); }));
+  uint64_t* k2 = ctx->radix_keys.as<uint64_t>();
+  uint32_t* v2 = ctx->radix_vals.as<uint32_t>();
   uint64_t *ki = keys, *ko = k2;
   uint32_t *vi = vals, *vo = v2;
   const int blocks = (int)((n_tiles + RS_WARPS - 1) / RS_WARPS);
@@ -270,13 +270,13 @@ int32_t nn_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, dou
   double blo[2], bhi[2];
   if (lo && hi) { blo[0] = lo[0]; blo[1] = lo[1]; bhi[0] = hi[0]; bhi[1] = hi[1]; }
   else {
-    CUDA_TRY(ctx, ctx->scratch[4].ensure(32));
+    CUDA_TRY(ctx, ctx->ws_query.ensure(32));
     unsigned long long init[4] = {~0ull, ~0ull, 0ull, 0ull};
-    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->scratch[4].p, init, 32, cudaMemcpyHostToDevice, st));
-    bbox_kernel<<<ctx->sm_count * 4, 256, 0, st>>>((const double2*)xy_dev, n, ctx->scratch[4].as<double>());
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws_query.p, init, 32, cudaMemcpyHostToDevice, st));
+    bbox_kernel<<<ctx->sm_count * 4, 256, 0, st>>>((const double2*)xy_dev, n, ctx->ws_query.as<double>());
     LAUNCH_CHECK(ctx);
     unsigned long long enc[4];
-    CUDA_TRY(ctx, cudaMemcpyAsync(enc, ctx->scratch[4].p, 32, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(enc, ctx->ws_query.p, 32, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     double dec[4];
     for (int k = 0; k < 4; ++k) {
@@ -299,21 +299,21 @@ int32_t nn_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, dou
   }
   ctx->cell = cell; ctx->inv_cell = 1.0 / cell; ctx->org_x = blo[0]; ctx->org_y = blo[1];
   const int64_t n_cells = (int64_t)ctx->cells_x * ctx->cells_y;
-  CUDA_TRY(ctx, ctx->scratch[5].ensure((size_t)n * 8));       // keys
-  CUDA_TRY(ctx, ctx->scratch[6].ensure((size_t)n * 4));       // vals
-  CUDA_TRY(ctx, ctx->scratch[7].ensure((size_t)n_cells * 4)); // counts
+  CUDA_TRY(ctx, ctx->sort_keys.ensure((size_t)n * 8));
+  CUDA_TRY(ctx, ctx->sort_vals.ensure((size_t)n * 4));
+  CUDA_TRY(ctx, ctx->ws_state.ensure((size_t)n_cells * 4));   // cell counts
   CUDA_TRY(ctx, ctx->d_cell_start.ensure((size_t)(n_cells + 1) * 8));
   CUDA_TRY(ctx, ctx->d_vxy_sorted.ensure((size_t)n * 16));
   CUDA_TRY(ctx, ctx->d_vid_sorted.ensure((size_t)n * 4));
-  CUDA_TRY(ctx, cudaMemsetAsync(ctx->scratch[7].p, 0, (size_t)n_cells * 4, st));
+  CUDA_TRY(ctx, cudaMemsetAsync(ctx->ws_state.p, 0, (size_t)n_cells * 4, st));
   cell_key_kernel<<<div_up(n, 256), 256, 0, st>>>((const double2*)xy_dev, n, ctx->org_x, ctx->org_y, ctx->inv_cell, ctx->cells_x, ctx->cells_y,
-                                                  ctx->scratch[5].as<uint64_t>(), ctx->scratch[6].as<uint32_t>(), ctx->scratch[7].as<int32_t>());
+                                                  ctx->sort_keys.as<uint64_t>(), ctx->sort_vals.as<uint32_t>(), ctx->ws_state.as<int32_t>());
   LAUNCH_CHECK(ctx);
-  int32_t rc = scan_exclusive_i64(ctx, ctx->scratch[7].as<int32_t>(), n_cells, ctx->d_cell_start.as<int64_t>());
+  int32_t rc = scan_exclusive_i64(ctx, ctx->ws_state.as<int32_t>(), n_cells, ctx->d_cell_start.as<int64_t>());
   if (rc) return rc;
-  rc = radix_sort_pairs(ctx, ctx->scratch[5].as<uint64_t>(), ctx->scratch[6].as<uint32_t>(), n, bits_for((uint64_t)n_cells - 1));
+  rc = radix_sort_pairs(ctx, ctx->sort_keys.as<uint64_t>(), ctx->sort_vals.as<uint32_t>(), n, bits_for((uint64_t)n_cells - 1));
   if (rc) return rc;
-  gather_vertices_kernel<<<div_up(n, 256), 256, 0, st>>>((const double2*)xy_dev, ctx->scratch[6].as<uint32_t>(), n,
+  gather_vertices_kernel<<<div_up(n, 256), 256, 0, st>>>((const double2*)xy_dev, ctx->sort_vals.as<uint32_t>(), n,
                                                          ctx->d_vxy_sorted.as<double2>(), ctx->d_vid_sorted.as<int32_t>());
   LAUNCH_CHECK(ctx);
   ctx->n_vertices = n;
@@ -544,9 +544,17 @@ int32_t nn_radius_count_fill_dev(porrt_ctx* ctx, const double* q_dev, const doub
     return PORRT_OK;
   }
   GridDev g = grid_dev(ctx);
-  CUDA_TRY(ctx, ctx->scratch[4].ensure((size_t)m * 12 + 64));
-  int64_t* stg_off = ctx->scratch[4].as<int64_t>();
-  int32_t* counts = (int32_t*)(stg_off + m);
+  // prefix-restricted queries over many cells get a warp each (radius_wide_kernel); the list is built once for both passes
+  const bool wide = prefix_dev != nullptr && m >= 1024;
+  int64_t* stg_off;
+  int32_t* counts;
+  int32_t* n_wide = nullptr;   // [0] the length of the wide-query list that follows 16 ints on
+  CUDA_TRY(ctx, carve(ctx->ws_query, [&](Carve& c) {
+    stg_off = c.take<int64_t>(m);
+    counts = c.take<int32_t>(m);
+    if (wide) n_wide = c.take<int32_t>(16 + m);
+  }));
+  int32_t* wide_list = wide ? n_wide + 16 : nullptr;
   // grouped vertex sets (prefix_lo): the other groups' vertices share the cells, staging them all would only cost; the
   // thread-per-query kernel skips to its own group inside each cell list
   // allow_tiles = false (the PRM build): the radii there are LARGER than the cell (cell = the last, smallest radius), so the tiles could
@@ -555,16 +563,7 @@ int32_t nn_radius_count_fill_dev(porrt_ctx* ctx, const double* q_dev, const doub
   const int32_t* fb_list = nullptr;
   const int32_t* staging = nullptr;
   int32_t fb_n = 0;
-  // prefix-restricted queries over many cells get a warp each (radius_wide_kernel); the list is built once for both passes
-  const bool wide = prefix_dev != nullptr && m >= 1024;
-  int32_t* wide_list = nullptr;
-  int32_t* n_wide = nullptr;
-  if (wide) {
-    CUDA_TRY(ctx, ctx->scratch[9].ensure((size_t)m * 4 + 64));
-    n_wide = ctx->scratch[9].as<int32_t>();
-    wide_list = n_wide + 16;
-    CUDA_TRY(ctx, cudaMemsetAsync(n_wide, 0, 4, st));
-  }
+  if (wide) CUDA_TRY(ctx, cudaMemsetAsync(n_wide, 0, 4, st));
   const int wide_grid = ctx->sm_count * 8;
   int64_t staged_total = -1;   // >= 0: the tiles served every query and this is the number of hits
   if (tiles) {
@@ -581,12 +580,12 @@ int32_t nn_radius_count_fill_dev(porrt_ctx* ctx, const double* q_dev, const doub
   const bool one_pass = n_rest > 0 && n_rest <= ((int64_t)8 << 20);
   int32_t* stage2 = nullptr; int64_t* stg_off2 = nullptr; int32_t* over_list = nullptr; int32_t* over_n = nullptr;
   if (one_pass) {
-    const size_t off_bytes = ((size_t)m * 8 + 255) & ~(size_t)255, list_bytes = ((size_t)n_rest * 4 + 256 + 255) & ~(size_t)255;
-    CUDA_TRY(ctx, ctx->nn_stage2.ensure(off_bytes + list_bytes + (size_t)n_rest * RADIUS_STAGE_CAP * 4));
-    stg_off2 = ctx->nn_stage2.as<int64_t>();
-    over_n = (int32_t*)(ctx->nn_stage2.as<char>() + off_bytes);
+    CUDA_TRY(ctx, carve(ctx->nn_stage2, [&](Carve& c) {
+      stg_off2 = c.take<int64_t>(m, 256);
+      over_n = c.take<int32_t>(16 + n_rest, 256);   // the count, then the list 16 ints on
+      stage2 = c.take<int32_t>((size_t)n_rest * RADIUS_STAGE_CAP, 256);
+    }));
     over_list = over_n + 16;
-    stage2 = (int32_t*)(ctx->nn_stage2.as<char>() + off_bytes + list_bytes);
     CUDA_TRY(ctx, cudaMemsetAsync(stg_off2, 0xff, (size_t)m * 8, st));   // -1: not in a slot
     CUDA_TRY(ctx, cudaMemsetAsync(over_n, 0, 4, st));
   }
@@ -803,10 +802,14 @@ int32_t segments_sort_by_key_dev(porrt_ctx* ctx, const int64_t* offsets_dev, int
   cudaStream_t st = ctx->stream;
   if (m <= 0 || (seg_list_dev && n_listed <= 0)) return PORRT_OK;
   const int64_t m_run = seg_list_dev ? n_listed : m;
-  CUDA_TRY(ctx, ctx->scratch[4].ensure(16 + (size_t)m * 4 + (key_of_id_dev ? (size_t)key_limit * 4 : 0)));
-  int32_t* d_big = ctx->scratch[4].as<int32_t>();   // [0] n_mid (257..4096, listed), [1] n_big (longer)
-  int32_t* d_mid_list = d_big + 4;
-  int32_t* d_inv = d_mid_list + m;
+  int32_t* d_big;   // [0] n_mid (257..4096, listed), [1] n_big (longer)
+  int32_t* d_mid_list;
+  int32_t* d_inv = nullptr;
+  CUDA_TRY(ctx, carve(ctx->ws_seg, [&](Carve& c) {
+    d_big = c.take<int32_t>(4);
+    d_mid_list = c.take<int32_t>(m);
+    if (key_of_id_dev) d_inv = c.take<int32_t>(key_limit);
+  }));
   CUDA_TRY(ctx, cudaMemsetAsync(d_big, 0, 8, st));
   if (key_of_id_dev) {
     invert_perm_kernel<<<div_up(key_limit, 256), 256, 0, st>>>(key_of_id_dev, key_limit, d_inv);
@@ -832,11 +835,10 @@ int32_t segments_sort_by_key_dev(porrt_ctx* ctx, const int64_t* offsets_dev, int
   // some segment is longer than SEG_MID_CAP: one global stable LSD radix sort on (segment, key) orders them all
   const int key_bits = bits_for((uint64_t)(key_limit > 1 ? key_limit - 1 : 1));
   const int seg_bits = bits_for((uint64_t)(m > 1 ? m - 1 : 1));
-  // (scratch 5 / 6 here, 8..10 inside radix_sort_pairs: callers keep their segment data elsewhere)
-  CUDA_TRY(ctx, ctx->scratch[5].ensure((size_t)total * 8));
-  CUDA_TRY(ctx, ctx->scratch[6].ensure((size_t)total * 4));
-  uint64_t* keys = ctx->scratch[5].as<uint64_t>();
-  uint32_t* vals = ctx->scratch[6].as<uint32_t>();
+  CUDA_TRY(ctx, ctx->sort_keys.ensure((size_t)total * 8));
+  CUDA_TRY(ctx, ctx->sort_vals.ensure((size_t)total * 4));
+  uint64_t* keys = ctx->sort_keys.as<uint64_t>();
+  uint32_t* vals = ctx->sort_vals.as<uint32_t>();
   seg_key_kernel<<<div_up(m * 32, 256), 256, 0, st>>>(offsets_dev, m, ids_dev, key_of_id_dev, key_bits, keys, vals);
   LAUNCH_CHECK(ctx);
   int32_t rc = radix_sort_pairs(ctx, keys, vals, total, key_bits + seg_bits);
@@ -861,18 +863,18 @@ PORRT_API int32_t porrt_radius_query(porrt_ctx* ctx, const double* q_xy, const d
   cudaStream_t st = ctx->stream;
   if (m == 0) { if (out_offsets) out_offsets[0] = 0; if (out_total) *out_total = 0; return PORRT_OK; }
   const int64_t V = ctx->n_vertices;
-  // device inputs: q | radius | prefix | world | reach | offsets
-  size_t need = (size_t)m * (16 + 8 + 4 + 4 + 8) + 64 + reach_bytes;
-  CUDA_TRY(ctx, ctx->scratch[3].ensure(need));
-  char* b = ctx->scratch[3].as<char>();
-  double* d_q = (double*)b; b += (size_t)m * 16;
-  double* d_r = (double*)b; b += (size_t)m * 8;
-  int64_t* d_off = (int64_t*)b; b += (size_t)(m + 1) * 8;
+  double *d_q, *d_r;
+  int64_t* d_off;
   uint64_t* d_reach = nullptr;
-  if (reach_mask) { d_reach = (uint64_t*)b; b += reach_bytes; }
   uint32_t* d_prefix = nullptr; uint32_t* d_world = nullptr;
-  if (prefix_limit) { d_prefix = (uint32_t*)b; b += (size_t)m * 4; }
-  if (world) { d_world = (uint32_t*)b; b += (size_t)m * 4; }
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_q = c.take<double>((size_t)m * 2);
+    d_r = c.take<double>(m);
+    d_off = c.take<int64_t>(m + 1);
+    if (reach_mask) d_reach = c.take<uint64_t>(reach_bytes / 8);
+    if (prefix_limit) d_prefix = c.take<uint32_t>(m);
+    if (world) d_world = c.take<uint32_t>(m);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_q, q_xy, (size_t)m * 16, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_r, radius, (size_t)m * 8, cudaMemcpyHostToDevice, st));
   if (d_prefix) CUDA_TRY(ctx, cudaMemcpyAsync(d_prefix, prefix_limit, (size_t)m * 4, cudaMemcpyHostToDevice, st));
@@ -880,7 +882,7 @@ PORRT_API int32_t porrt_radius_query(porrt_ctx* ctx, const double* q_xy, const d
   if (d_reach) CUDA_TRY(ctx, cudaMemcpyAsync(d_reach, reach_mask, reach_bytes, cudaMemcpyHostToDevice, st));
   int64_t total = 0;
   tstart(ctx);  // phases: [count+scan+fill, order restore, D2H]
-  int32_t rc = nn_radius_count_fill_dev(ctx, d_q, d_r, m, d_prefix, d_reach, d_world, d_off, &ctx->scratch[2], &total, nullptr, true);
+  int32_t rc = nn_radius_count_fill_dev(ctx, d_q, d_r, m, d_prefix, d_reach, d_world, d_off, &ctx->ws_table, &total, nullptr, true);
   if (rc) return rc;
   tmark(ctx);
   if (out_total) *out_total = total;
@@ -891,7 +893,7 @@ PORRT_API int32_t porrt_radius_query(porrt_ctx* ctx, const double* q_xy, const d
   }
   tmark(ctx);   // (the id order comes out of the search itself now; the phase is kept so that the list keeps its three entries)
   CUDA_TRY(ctx, cudaMemcpyAsync(out_offsets, d_off, (size_t)(m + 1) * 8, cudaMemcpyDeviceToHost, st));
-  if (total > 0) CUDA_TRY(ctx, cudaMemcpyAsync(out_ids, ctx->scratch[2].p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
+  if (total > 0) CUDA_TRY(ctx, cudaMemcpyAsync(out_ids, ctx->ws_table.p, (size_t)total * 4, cudaMemcpyDeviceToHost, st));
   tmark(ctx);
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
   tfinish(ctx);
@@ -1075,17 +1077,18 @@ static int32_t knn_host(porrt_ctx* ctx, const double* q_xy, int64_t m, int k, co
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const int64_t V = ctx->n_vertices;
-  size_t need = (size_t)m * (16 + 4 + 4) + (size_t)m * k * 12 + reach_bytes + 64;
-  CUDA_TRY(ctx, ctx->scratch[3].ensure(need));
-  char* b = ctx->scratch[3].as<char>();
-  double* d_q = (double*)b; b += (size_t)m * 16;
-  double* d_dist = (double*)b; b += (size_t)m * k * 8;
+  double *d_q, *d_dist;
   uint64_t* d_reach = nullptr;
-  if (reach_mask) { d_reach = (uint64_t*)b; b += reach_bytes; }
-  int32_t* d_ids = (int32_t*)b; b += (size_t)m * k * 4;
-  int32_t* d_ties = (int32_t*)b; b += (size_t)m * 4;
+  int32_t *d_ids, *d_ties;
   uint32_t* d_world = nullptr;
-  if (world) { d_world = (uint32_t*)b; b += (size_t)m * 4; }
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_q = c.take<double>((size_t)m * 2);
+    d_dist = c.take<double>((size_t)m * k);
+    if (reach_mask) d_reach = c.take<uint64_t>(reach_bytes / 8);
+    d_ids = c.take<int32_t>((size_t)m * k);
+    d_ties = c.take<int32_t>(m);
+    if (world) d_world = c.take<uint32_t>(m);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_q, q_xy, (size_t)m * 16, cudaMemcpyHostToDevice, st));
   if (d_world) CUDA_TRY(ctx, cudaMemcpyAsync(d_world, world, (size_t)m * 4, cudaMemcpyHostToDevice, st));
   if (d_reach) CUDA_TRY(ctx, cudaMemcpyAsync(d_reach, reach_mask, reach_bytes, cudaMemcpyHostToDevice, st));

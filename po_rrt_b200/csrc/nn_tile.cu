@@ -369,7 +369,7 @@ __global__ void __launch_bounds__(NR_THREADS) nt_radius_collect_kernel(
           const int n_c = s_ccnt[qc];
           // ids ascend along the list, so do the hits.  Branch-free body, four candidates in flight: the loop is bound by the
           // latency of its dependent shared-memory loads (index -> coordinates), not by issue
-          auto take = [&](int j, bool hit) {
+          auto keep = [&](int j, bool hit) {
             if (hit) { lst[min(cnt, NR_LCAP - 1)] = (uint8_t)j; ++cnt; }      // (overflow is caught by cnt > NR_LCAP below)
           };
           int j = 0;
@@ -378,13 +378,13 @@ __global__ void __launch_bounds__(NR_THREADS) nt_radius_collect_kernel(
               const double d0 = dist2(s_xy[cxy[j]], p.x, p.y), d1 = dist2(s_xy[cxy[j + 1]], p.x, p.y);
               const double d2 = dist2(s_xy[cxy[j + 2]], p.x, p.y), d3 = dist2(s_xy[cxy[j + 3]], p.x, p.y);
               const uint32_t i0 = (uint32_t)cid[j], i1 = (uint32_t)cid[j + 1], i2 = (uint32_t)cid[j + 2], i3 = (uint32_t)cid[j + 3];
-              take(j, d0 <= Tr && i0 < limit); take(j + 1, d1 <= Tr && i1 < limit);
-              take(j + 2, d2 <= Tr && i2 < limit); take(j + 3, d3 <= Tr && i3 < limit);
+              keep(j, d0 <= Tr && i0 < limit); keep(j + 1, d1 <= Tr && i1 < limit);
+              keep(j + 2, d2 <= Tr && i2 < limit); keep(j + 3, d3 <= Tr && i3 < limit);
             }
-            for (; j < n_c; ++j) take(j, dist2(s_xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit);
+            for (; j < n_c; ++j) keep(j, dist2(s_xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit);
           } else {
             for (; j < n_c; ++j)
-              take(j, dist2(s_xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit && reach_bit(reach, g.reach_words, cid[j], wq));
+              keep(j, dist2(s_xy[cxy[j]], p.x, p.y) <= Tr && (uint32_t)cid[j] < limit && reach_bit(reach, g.reach_words, cid[j], wq));
           }
           if (cnt > NR_LCAP) fallback = true;
         }
@@ -617,12 +617,11 @@ struct NtBins {
 
 static int32_t nt_layout(porrt_ctx* ctx, const GridDev& g, int64_t m, NtBins* B) {
   const int64_t n_cells = (int64_t)g.cells_x * g.cells_y;
-  CUDA_TRY(ctx, ctx->nn_tmp[0].ensure((size_t)m * 12 + 64));                 // qcell | qorder | fb_list
-  CUDA_TRY(ctx, ctx->nn_tmp[1].ensure((size_t)n_cells * 8 + 64));            // qcount | cursor | fb_n
-  CUDA_TRY(ctx, ctx->nn_tmp[2].ensure((size_t)(n_cells + 1) * 8));           // qstart
-  B->qcell = ctx->nn_tmp[0].as<int32_t>(); B->qorder = B->qcell + m; B->fb_list = B->qorder + m;
-  B->qcount = ctx->nn_tmp[1].as<int32_t>(); B->cursor = B->qcount + n_cells; B->fb_n = B->cursor + n_cells;
-  B->qstart = ctx->nn_tmp[2].as<int64_t>();
+  CUDA_TRY(ctx, carve(ctx->nn_bins, [&](Carve& c) {
+    B->qcell = c.take<int32_t>(m); B->qorder = c.take<int32_t>(m); B->fb_list = c.take<int32_t>(m);
+    B->qcount = c.take<int32_t>(n_cells); B->cursor = c.take<int32_t>(n_cells); B->fb_n = c.take<int32_t>(1);
+    B->qstart = c.take<int64_t>(n_cells + 1);
+  }));
   B->tiles_per_row = (g.cells_x + NT_W - 1) / NT_W;
   B->n_tiles = B->tiles_per_row * g.cells_y;
   return PORRT_OK;
@@ -634,7 +633,7 @@ static int32_t nt_bin(porrt_ctx* ctx, const GridDev& g, const double* q_dev, con
   const int64_t n_cells = (int64_t)g.cells_x * g.cells_y;
   int32_t rc0 = nt_layout(ctx, g, m, B);
   if (rc0) return rc0;
-  CUDA_TRY(ctx, cudaMemsetAsync(B->qcount, 0, (size_t)n_cells * 8 + 4, st));
+  CUDA_TRY(ctx, cudaMemsetAsync(B->qcount, 0, (char*)(B->fb_n + 1) - (char*)B->qcount, st));   // qcount, cursor and fb_n
   nt_bin_kernel<KNN><<<div_up(m, 256), 256, 0, st>>>(g, (const double2*)q_dev, radius_dev, m, B->qcell, B->qcount, B->fb_list, B->fb_n);
   LAUNCH_CHECK(ctx);
   int32_t rc = scan_exclusive_i64(ctx, B->qcount, n_cells, B->qstart);
@@ -656,8 +655,8 @@ static int32_t nn_tile_build_scripts(porrt_ctx* ctx, const GridDev& g) {
   cudaStream_t st = ctx->stream;
   const int64_t n_cells = (int64_t)g.cells_x * g.cells_y;
   CUDA_TRY(ctx, ctx->d_nbr_start.ensure((size_t)(n_cells + 1) * 8));
-  CUDA_TRY(ctx, ctx->nn_tmp[1].ensure((size_t)n_cells * 8 + 64));
-  int32_t* sizes = ctx->nn_tmp[1].as<int32_t>();
+  CUDA_TRY(ctx, ctx->nn_bins.ensure((size_t)n_cells * 4));
+  int32_t* sizes = ctx->nn_bins.as<int32_t>();
   nbr_size_kernel<<<div_up(n_cells, 256), 256, 0, st>>>(g, sizes);
   LAUNCH_CHECK(ctx);
   int32_t rc = scan_exclusive_i64(ctx, sizes, n_cells, ctx->d_nbr_start.as<int64_t>());
@@ -687,9 +686,9 @@ int32_t nn_tile_radius_collect(porrt_ctx* ctx, const GridDev& g, const double* q
   if (rc) return rc;
   // staging: room for 64 hits per query on average; warps that find it full fall back
   const int64_t stg_cap = m * 64 + 4096;
-  CUDA_TRY(ctx, ctx->nn_stage.ensure((size_t)stg_cap * 4 + 64));
-  int32_t* staging = ctx->nn_stage.as<int32_t>();
-  unsigned long long* cursor = (unsigned long long*)(staging + stg_cap + (stg_cap & 1));
+  int32_t* staging;
+  unsigned long long* cursor;
+  CUDA_TRY(ctx, carve(ctx->nn_stage, [&](Carve& c) { staging = c.take<int32_t>(stg_cap); cursor = c.take<unsigned long long>(1); }));
   CUDA_TRY(ctx, cudaMemsetAsync(cursor, 0, 8, st));
   CUDA_TRY(ctx, cudaMemsetAsync(stg_off_dev, 0xff, (size_t)m * 8, st));
   static bool attr_set[16] = {};

@@ -499,19 +499,18 @@ static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double
   return d;
 }
 
-static SpecDev spec_dev(PtoRoad* r) {
-  SpecDev s = {};
-  const int64_t W = PG_WMAX, h = r->node_cap;
-  char* p = r->spec.as<char>();
-  auto take = [&](size_t bytes) { char* q = p; p += (bytes + 15) & ~(size_t)15; return q; };
-  s.nn = (int32_t*)take(W * 4); s.nn_d = (double*)take(W * 8); s.q = (double2*)take(W * 16); s.svid = (int32_t*)take(W * 4);
-  s.nn_vid = (int32_t*)take(W * 4); s.n_hits = (int32_t*)take(W * 4); s.slot = (int32_t*)take(W * 4);
-  s.hit_id = (int32_t*)take(W * h * 4); s.hit_d = (double*)take(W * h * 8); s.hit_vid = (int32_t*)take(W * h * 4);
-  s.tmp_id = (int32_t*)take(W * h * 4); s.tmp_d = (double*)take(W * h * 8); s.rank = (int32_t*)take(W * h * 4);
+// the speculation block of a roadmap with h hits per slot: 44 bytes per slot, 32 per hit.  The kernels index slot b < C_W <= PG_WMAX
+// and hit k < V0 <= node_cap = hcap.
+static void spec_layout(Carve& c, SpecDev& s, int64_t h) {
+  const size_t W = PG_WMAX, Wh = W * (size_t)h;
+  s.nn = c.take<int32_t>(W); s.nn_d = c.take<double>(W); s.q = c.take<double2>(W); s.svid = c.take<int32_t>(W);
+  s.nn_vid = c.take<int32_t>(W); s.n_hits = c.take<int32_t>(W); s.slot = c.take<int32_t>(W);
+  s.hit_id = c.take<int32_t>(Wh); s.hit_d = c.take<double>(Wh); s.hit_vid = c.take<int32_t>(Wh);
+  s.tmp_id = c.take<int32_t>(Wh); s.tmp_d = c.take<double>(Wh); s.rank = c.take<int32_t>(Wh);
   s.hcap = h;
-  return s;
 }
-static size_t spec_bytes(int64_t h) { return (size_t)PG_WMAX * (4 + 8 + 16 + 4 * 4 + (size_t)h * 36) + 16 * 16; }
+static size_t spec_bytes(int64_t h) { SpecDev s; return carve_size([&](Carve& c) { spec_layout(c, s, h); }); }
+static SpecDev spec_dev(PtoRoad* r) { SpecDev s = {}; Carve c{(uintptr_t)r->spec.p}; spec_layout(c, s, r->node_cap); return s; }
 static size_t node_bytes(int words) { return 72 + 16 * (size_t)words; }   // every per-node array below, per node
 
 // every per-node array holds node_cap entries, kept across growth (DevBuf::grow_keep)
@@ -742,6 +741,13 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
     }
   }
   // per roadmap: outputs, then the children CSR from the edge log (graph.cu's late-list kernels, carrying the validity ids)
+  // CSR assembly work space of a roadmap of V nodes and E edges (late_list_csr_dev), one roadmap at a time
+  int32_t *late_cnt, *cursor, *late_vals;
+  int64_t* late_off;
+  auto csr_work = [&](Carve& c, int64_t V, int64_t E) {
+    late_cnt = c.take<int32_t>(V); cursor = c.take<int32_t>(V); late_off = c.take<int64_t>(V + 1);
+    late_vals = c.take<int32_t>(std::max<int64_t>(E, 1));
+  };
   size_t work = 64;
   for (int32_t r = 0; r < n; ++r) {
     const int32_t* fr = f + (size_t)r * C_N;
@@ -758,7 +764,7 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
       continue;
     }
     const int64_t V = fr[C_V], E = fr[C_E];
-    work = std::max(work, (size_t)V * 8 + (size_t)(V + 1) * 8 + (size_t)std::max<int64_t>(E, 1) * 4 + 64);
+    work = std::max(work, carve_size([&](Carve& c) { csr_work(c, V, E); }));
   }
   CUDA_TRY(ctx, g->work.ensure(work));
   std::vector<uint64_t> fin((size_t)n * words);
@@ -770,10 +776,8 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
     CUDA_TRY(ctx, d->csr_row.ensure((size_t)(V + 1) * 8));
     CUDA_TRY(ctx, d->csr_col.ensure((size_t)std::max<int64_t>(2 * E, 1) * 4));
     CUDA_TRY(ctx, d->csr_vid.ensure((size_t)std::max<int64_t>(2 * E, 1) * 4));
-    int32_t* late_cnt = g->work.as<int32_t>();
-    int32_t* cursor = late_cnt + V;
-    int64_t* late_off = (int64_t*)(cursor + V);
-    int32_t* late_vals = (int32_t*)(late_off + V + 1);
+    Carve c{(uintptr_t)g->work.p};
+    csr_work(c, V, E);
     pto_set_i64_kernel<<<1, 1, 0, st>>>(d->edge_off.as<int64_t>() + V, ctl + (size_t)r * C_N, C_E);
     LAUNCH_CHECK(ctx);
     rc = late_list_csr_dev(ctx, d->edge_off.as<int64_t>(), V, d->log_nbr.as<int32_t>(), d->ecnt.as<int32_t>(), d->log_vid.as<int32_t>(),

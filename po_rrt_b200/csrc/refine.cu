@@ -69,14 +69,13 @@ PORRT_API int32_t porrt_transition_valid(porrt_ctx* ctx, const double* from_xy, 
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   cudaStream_t st = ctx->stream;
   const size_t nv = (size_t)ctx->n_validities;
-  CUDA_TRY(ctx, ctx->scratch[3].ensure((size_t)n * (32 + 12 + 4 + 1) + nv + 64));
-  char* b = ctx->scratch[3].as<char>();
-  double* d_from = (double*)b; b += (size_t)n * 16;
-  double* d_to = (double*)b; b += (size_t)n * 16;
-  int32_t* d_tmp = (int32_t*)b; b += (size_t)n * 12;
-  int32_t* d_status = (int32_t*)b; b += (size_t)n * 4;
-  uint8_t* d_valid = (uint8_t*)b; b += (size_t)n;
-  uint8_t* d_compat = (uint8_t*)b;
+  double *d_from, *d_to;
+  int32_t *d_tmp, *d_status;
+  uint8_t *d_valid, *d_compat;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_from = c.take<double>(2 * n); d_to = c.take<double>(2 * n); d_tmp = c.take<int32_t>(3 * n); d_status = c.take<int32_t>(n);
+    d_valid = c.take<uint8_t>(n); d_compat = c.take<uint8_t>(nv);
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_from, from_xy, (size_t)n * 16, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_to, to_xy, (size_t)n * 16, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_compat, compat_row, nv, cudaMemcpyHostToDevice, st));
@@ -200,17 +199,16 @@ PORRT_API int32_t porrt_partial_shortcut_batch(porrt_ctx* ctx, double* states_xy
   if (list.empty()) return PORRT_OK;
   const int64_t n_states = piece_ptr[n_pieces];
   const size_t n_active = list.size();
-  DevBuf& g = ctx->scratch[3];
-  CUDA_TRY(ctx, g.ensure((size_t)n_states * 16 + (size_t)(n_pieces + 1) * 4 + n_active * 4 + trials.size() * 4 + (size_t)n_pieces * (nv + 8) + 8 * 16));
-  char* b = g.as<char>();
-  auto take = [&](size_t bytes) { char* q = b; b += (bytes + 15) & ~(size_t)15; return q; };
-  double2* d_states = (double2*)take((size_t)n_states * 16);
-  int32_t* d_ptr = (int32_t*)take((size_t)(n_pieces + 1) * 4);
-  int32_t* d_list = (int32_t*)take(n_active * 4);
-  uint32_t* d_trials = (uint32_t*)take(trials.size() * 4);
-  uint8_t* d_compat = (uint8_t*)take((size_t)n_pieces * nv);
-  int32_t* d_commits = (int32_t*)take((size_t)n_pieces * 4);
-  int32_t* d_status = (int32_t*)take((size_t)n_pieces * 4);
+  double2* d_states;
+  int32_t *d_ptr, *d_list, *d_commits, *d_status;
+  uint32_t* d_trials;
+  uint8_t* d_compat;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_states = c.take<double2>(n_states); d_ptr = c.take<int32_t>(n_pieces + 1); d_list = c.take<int32_t>(n_active);
+    d_trials = c.take<uint32_t>(trials.size()); d_compat = c.take<uint8_t>((size_t)n_pieces * nv);
+    d_commits = c.take<int32_t>(n_pieces);
+    d_status = c.take<int32_t>(n_pieces + 4);   // + 16 bytes: the memset below clears commits and status in one call
+  }));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_states, states_xy, (size_t)n_states * 16, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_ptr, piece_ptr, (size_t)(n_pieces + 1) * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_list, list.data(), n_active * 4, cudaMemcpyHostToDevice, st));
@@ -621,22 +619,16 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
   if (n_pairs > 0) {
     // the device expands (node, neighbour) index pairs into endpoint coordinates itself: 4 bytes per pair cross the bus, not 36
     const size_t n = (size_t)n_pairs, nn = (size_t)n_nodes_all, nrows = (size_t)B * nv;
-    auto al = [](size_t x) { return (x + 255) & ~(size_t)255; };
-    CUDA_TRY(ctx, ctx->scratch[3].ensure(al(n * 16) * 2 + al(n * 12) + al(n * 4) * 3 + al(n) + al(nn * 16) + al((nn + 1) * 8) + al(nn * 4) * 2 + al(nrows) + 256));
-    char* b = ctx->scratch[3].as<char>();
-    auto take = [&](size_t bytes) { char* q = b; b += al(bytes); return q; };
-    double* d_from = (double*)take(n * 16);
-    double* d_to = (double*)take(n * 16);
-    int32_t* d_tmp = (int32_t*)take(n * 12);
-    int32_t* d_status = (int32_t*)take(n * 4);
-    int32_t* d_row = (int32_t*)take(n * 4);
-    int32_t* d_nb = (int32_t*)take(n * 4);
-    uint8_t* d_valid = (uint8_t*)take(n);
-    double* d_nxy = (double*)take(nn * 16);
-    int64_t* d_nptr = (int64_t*)take((nn + 1) * 8);
-    int32_t* d_nbase = (int32_t*)take(nn * 4);
-    int32_t* d_nrow = (int32_t*)take(nn * 4);
-    uint8_t* d_compat = (uint8_t*)take(nrows);
+    double *d_from, *d_to, *d_nxy;
+    int32_t *d_tmp, *d_status, *d_row, *d_nb, *d_nbase, *d_nrow;
+    uint8_t *d_valid, *d_compat;
+    int64_t* d_nptr;
+    CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+      d_from = c.take<double>(2 * n, 256); d_to = c.take<double>(2 * n, 256); d_tmp = c.take<int32_t>(3 * n, 256);
+      d_status = c.take<int32_t>(n, 256); d_row = c.take<int32_t>(n, 256); d_nb = c.take<int32_t>(n, 256); d_valid = c.take<uint8_t>(n, 256);
+      d_nxy = c.take<double>(2 * nn, 256); d_nptr = c.take<int64_t>(nn + 1, 256); d_nbase = c.take<int32_t>(nn, 256);
+      d_nrow = c.take<int32_t>(nn, 256); d_compat = c.take<uint8_t>(nrows, 256);
+    }));
     CUDA_TRY(ctx, cudaMemcpyAsync(d_nb, nb_ids.data(), n * 4, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(d_nxy, node_xy.data(), nn * 16, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(d_nptr, nb_ptr.data(), (nn + 1) * 8, cudaMemcpyHostToDevice, st));

@@ -291,16 +291,17 @@ __global__ void sf_zero_finals_kernel(const int32_t* __restrict__ fin_node, cons
 }
 }  // namespace
 
-// Morton numbering + transposed adjacency of a roadmap on the device (work space: scratch[5], scratch[6]; radix sort: scratch[8..10]).
+// Morton numbering (work space: sort_keys) + transposed adjacency (sort_vals) of a roadmap on the device.
 int32_t sf_build_graph(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_col, const int32_t* d_evid, const double* d_xy, int64_t V,
                        int64_t E, SfGraph* out, cudaStream_t st) {
   if (V > 0x7fffffff) return porrt_fail(ctx, PORRT_ERR_UNSUPPORTED, "value backups: more than 2^31 nodes");
-  DevBuf& ob = ctx->scratch[5];
-  CUDA_TRY(ctx, ob.ensure((size_t)V * 16 + 64 + 4 * 16));
-  uint64_t* d_keys = ob.as<uint64_t>();
-  uint32_t* d_order = (uint32_t*)(ob.as<char>() + (((size_t)V * 8 + 15) & ~(size_t)15));
-  int32_t* d_perm = (int32_t*)((char*)d_order + (((size_t)V * 4 + 15) & ~(size_t)15));
-  unsigned long long* d_box = (unsigned long long*)((char*)d_perm + (((size_t)V * 4 + 15) & ~(size_t)15));
+  uint64_t* d_keys;
+  uint32_t* d_order;
+  int32_t* d_perm;
+  unsigned long long* d_box;
+  CUDA_TRY(ctx, carve(ctx->sort_keys, [&](Carve& c) {
+    d_keys = c.take<uint64_t>(V); d_order = c.take<uint32_t>(V); d_perm = c.take<int32_t>(V); d_box = c.take<unsigned long long>(4);
+  }));
   const unsigned long long init[4] = {~0ull, ~0ull, 0ull, 0ull};
   CUDA_TRY(ctx, cudaMemcpyAsync(d_box, init, 32, cudaMemcpyHostToDevice, st));
   sf_bbox_kernel<<<ctx->sm_count * 4, 256, 0, st>>>((const double2*)d_xy, V, d_box);
@@ -311,16 +312,14 @@ int32_t sf_build_graph(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_co
   if (rc) return rc;
   sf_perm_kernel<<<div_up(V, 256), 256, 0, st>>>(d_order, V, d_perm);
   LAUNCH_CHECK(ctx);
-  DevBuf& tb = ctx->scratch[6];
-  CUDA_TRY(ctx, tb.ensure((size_t)(V + 1) * 8 + (size_t)E * 14 + (size_t)V * 4 + 6 * 16 + 64));
-  char* p = tb.as<char>();
-  auto take = [&](size_t bytes) { char* q = p; p += (bytes + 15) & ~(size_t)15; return q; };
-  int64_t* d_row_t = (int64_t*)take((size_t)(V + 1) * 8);
-  double* d_cost_t = (double*)take((size_t)E * 8);
-  int32_t* d_col_t = (int32_t*)take((size_t)E * 4 + 4);
-  uint16_t* d_evid_t = (uint16_t*)take((size_t)E * 2 + 4);
-  int32_t* d_cnt = (int32_t*)take((size_t)V * 4);
-  double* d_sum = (double*)take(16);
+  int64_t* d_row_t;
+  double *d_cost_t, *d_sum;
+  int32_t *d_col_t, *d_cnt;
+  uint16_t* d_evid_t;
+  CUDA_TRY(ctx, carve(ctx->sort_vals, [&](Carve& c) {
+    d_row_t = c.take<int64_t>(V + 1); d_cost_t = c.take<double>(E); d_col_t = c.take<int32_t>(E + 1); d_evid_t = c.take<uint16_t>(E + 2);
+    d_cnt = c.take<int32_t>(V); d_sum = c.take<double>(2);
+  }));
   CUDA_TRY(ctx, cudaMemsetAsync(d_cnt, 0, (size_t)V * 4, st));
   if (E > 0) {
     sf_count_kernel<<<div_up(E, 256), 256, 0, st>>>(d_col, d_perm, E, d_cnt);
@@ -348,33 +347,35 @@ int32_t sf_build_graph(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_co
   return PORRT_OK;
 }
 
+// The frontier state of sf_relax over V nodes and W columns in ws_state; with `table`, a [W][V] value table behind it.  Every user of
+// ws_state carves through this layout, so sf_relax never moves a table its caller placed there.
+static void sf_state_layout(Carve& c, SfArgs& a, int64_t V, int32_t W, double** table) {
+  const int words = (W + 63) / 64;
+  a.pair_cap = (int32_t)std::min<int64_t>(V * (int64_t)W, std::max<int64_t>(4 << 20, 4 * V));
+  a.dirty[0] = c.take<unsigned long long>((size_t)V * words); a.dirty[1] = c.take<unsigned long long>((size_t)V * words);
+  a.inq[0] = c.take<int32_t>(V); a.inq[1] = c.take<int32_t>(V);
+  a.list[0] = c.take<int32_t>(V); a.list[1] = c.take<int32_t>(V);
+  a.counter = c.take<int32_t>(4);
+  a.offers = c.take<unsigned long long>(2);
+  a.thr = c.take<double>(4);
+  a.min_far = c.take<unsigned long long>(4);
+  a.pair_count = c.take<int32_t>(4);
+  a.pairs = c.take<int2>(a.pair_cap);
+  if (table) *table = c.take<double>((size_t)V * W);
+}
+
 // Relaxes W value columns to their fixed point.  dist[w * V + pos] (Morton numbering) holds the initial values on entry -- +inf, the
 // sources' values, the sign bit on every entry that must not be relaxed -- and the result on exit (signs kept).  cmask (nullable):
-// [W][4] validity ids an edge must carry to be admissible in column w (needs g.evid_t).  Work space: scratch[7].
+// [W][4] validity ids an edge must carry to be admissible in column w (needs g.evid_t).  Work space: ws_state.
 int32_t sf_relax(porrt_ctx* ctx, const SfGraph& g, double* dist, int32_t W, const uint64_t* cmask, int32_t* out_rounds, double* out_offers,
                  cudaStream_t st) {
   const int64_t V = g.V;
   const int words = (W + 63) / 64;
   if (W <= 0) { if (out_rounds) *out_rounds = 0; if (out_offers) *out_offers = 0.0; return PORRT_OK; }
-  const int64_t pair_cap = std::min<int64_t>(V * (int64_t)W, std::max<int64_t>(4 << 20, 4 * V));
-  DevBuf& sb = ctx->scratch[7];
-  CUDA_TRY(ctx, sb.ensure(2 * (size_t)V * words * 8 + 4 * (size_t)V * 4 + 192 + 14 * 16 + (size_t)pair_cap * 8));
-  char* p = sb.as<char>();
-  auto take = [&](size_t bytes) { char* q = p; p += (bytes + 15) & ~(size_t)15; return q; };
   SfArgs a = {};
+  CUDA_TRY(ctx, carve(ctx->ws_state, [&](Carve& c) { sf_state_layout(c, a, V, W, nullptr); }));
   a.row_t = g.row_t; a.col_t = g.col_t; a.cost_t = g.cost_t; a.evid_t = g.evid_t; a.cmask = cmask; a.V = V; a.W = W; a.words = words;
   a.dist = dist; a.delta = g.delta;
-  a.dirty[0] = (unsigned long long*)take((size_t)V * words * 8);
-  a.dirty[1] = (unsigned long long*)take((size_t)V * words * 8);
-  a.inq[0] = (int32_t*)take((size_t)V * 4); a.inq[1] = (int32_t*)take((size_t)V * 4);
-  a.list[0] = (int32_t*)take((size_t)V * 4); a.list[1] = (int32_t*)take((size_t)V * 4);
-  a.counter = (int32_t*)take(16);
-  a.offers = (unsigned long long*)take(16);
-  a.thr = (double*)take(32);
-  a.min_far = (unsigned long long*)take(32);
-  a.pair_count = (int32_t*)take(16);
-  a.pair_cap = (int32_t)pair_cap;
-  a.pairs = (int2*)take((size_t)pair_cap * 8);
   CUDA_TRY(ctx, cudaMemsetAsync(a.dirty[0], 0, 2 * (((size_t)V * words * 8 + 15) & ~(size_t)15), st));
   CUDA_TRY(ctx, cudaMemsetAsync(a.inq[0], 0, 2 * (((size_t)V * 4 + 15) & ~(size_t)15), st));
   CUDA_TRY(ctx, cudaMemsetAsync(a.counter, 0, 32 + 32, st));   // counters, offers, thresholds (0.0)
@@ -411,7 +412,8 @@ int32_t sf_relax(porrt_ctx* ctx, const SfGraph& g, double* dist, int32_t W, cons
 }
 
 // plan_qmdp's world columns.  All pointers are device pointers.  fin_node / fin_world: the finals of the worlds [wlo, wlo + W) as
-// (node, local world) pairs.  out_wv receives rows [0, W) of the [world][node] table.  Work space: scratch[5..10].
+// (node, local world) pairs.  out_wv receives rows [0, W) of the [world][node] table.  Work space: ws_state (the value table behind
+// sf_relax's state) and sf_build_graph's.
 int32_t sssp_frontier_run(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_col, const double* d_xy, int64_t V, int64_t E,
                           const int32_t* d_node_vid, const uint64_t* d_validities, int32_t mask_words, int32_t wlo, int32_t W,
                           const int32_t* d_fin_node, const int32_t* d_fin_world, int64_t n_fin, double* d_out_wv, int32_t* out_rounds,
@@ -419,12 +421,9 @@ int32_t sssp_frontier_run(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d
   SfGraph g;
   int32_t rc = sf_build_graph(ctx, d_row, d_col, nullptr, d_xy, V, E, &g, st);
   if (rc) return rc;
-  // the value table lives behind the frontier state of sf_relax in scratch[7]: sized here so that sf_relax's ensure() does not move it
-  const int words = (W + 63) / 64;
-  const int64_t pair_cap = std::min<int64_t>(V * (int64_t)W, std::max<int64_t>(4 << 20, 4 * V));
-  const size_t state_bytes = 2 * (size_t)V * words * 8 + 4 * (size_t)V * 4 + 192 + 14 * 16 + (size_t)pair_cap * 8;
-  CUDA_TRY(ctx, ctx->scratch[7].ensure(state_bytes + (size_t)V * W * 8 + 64));
-  double* dist = (double*)(ctx->scratch[7].as<char>() + ((state_bytes + 63) & ~(size_t)63));
+  double* dist;
+  SfArgs unused = {};
+  CUDA_TRY(ctx, carve(ctx->ws_state, [&](Carve& c) { sf_state_layout(c, unused, V, W, &dist); }));
   sf_init_kernel<<<div_up(V * (int64_t)W, 256), 256, 0, st>>>(d_node_vid, d_validities, mask_words, g.order, V, W, wlo, dist);
   LAUNCH_CHECK(ctx);
   if (n_fin > 0) {

@@ -135,6 +135,15 @@ def test_library_reads_only_documented_environment_variables():
     assert not bad, "environment variables read by the library beyond %s: %s" % (sorted(allowed), bad)
 
 
+def test_work_space_is_carved_from_named_buffers():
+    # every block of work space is laid out once (Carve, common.cuh) in a buffer with a name and listed users, not by a bump lambda
+    # of its own or in a numbered slot whose owner nothing records
+    bad = []
+    for name, src in _csrc_without_comments():
+        bad += [(name, m.group(0)) for m in re.finditer(r"\b(?:scratch|pin)\s*\[\s*\d+\s*\]|\bauto\s+take\w*\s*=\s*\[", src)]
+    assert not bad, "numbered work-space slots or hand-written take lambdas: %s" % bad
+
+
 def test_library_has_no_ifndef_knobs():
     # an include guard is `#ifndef X` directly followed by a bare `#define X`; anything else is a compile-time knob
     bad = []
