@@ -13,8 +13,8 @@
 // A column of V doubles fits in shared memory (227 KB: up to 6 columns of a 4.7 k-node roadmap), so one CTA solves C columns
 // completely on chip with a label-correcting worklist: a node whose value improved pushes it to its parents (12-byte records of
 // the transposed adjacency, read from L2) with shared-memory atomicMin, rounds until no node is dirty.  No kernel launch, no
-// global barrier and no HBM/L2 gather of dist per sweep, and work only where values move -- the thread-per-(node, column)
-// Jacobi sweeps of graph.cu re-evaluate the whole table 40-80 times.
+// global barrier and no HBM/L2 gather of dist per sweep, and work only where values move -- round 1's thread-per-(node, column)
+// Jacobi sweeps re-evaluated the whole table 40-80 times.  graph.cu's value-column driver runs it one level at a time.
 // Measured on the config-4 shape (4685 nodes x 4095 beliefs, 12 levels): Jacobi sweeps 43 ms -> pull sweeps on chip 20 ms
 // (54 sweeps, issue/latency bound; sweeping the nodes sorted along x / y did not cut the sweeps: a CTA has 256 nodes in flight,
 // wider than a hop) -> push worklist 10.6 ms -> dirty nodes collected into a CTA-wide queue per round 5.3 ms.

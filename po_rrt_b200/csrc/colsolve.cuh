@@ -25,7 +25,7 @@ struct ColSolveArgs {
   // belief mode only
   const uint8_t* type_cm;      // [n_columns][V] PORRT_NODE_* (255 = the belief node does not exist)
   const int32_t* node_set;     // [V] index of the node's visible-zone set
-  const int32_t* col_belief;   // [n_columns] belief id of a column
+  const int32_t* col_belief;   // [positions] the column at a position (belief id), -1 = padding
   const int64_t* succ_ptr;     // [n_sets * B + 1]
   const int32_t* succ_col;     // successor COLUMNS (positions, not belief ids)
   const double* succ_p;

@@ -132,7 +132,7 @@ struct porrt_ctx {
   std::vector<uint64_t> zone_world_masks;  // DOOR: zones_to_worlds [n_zones * mask_words]
   DevBuf d_grid, d_coarse, d_validities, d_zone_pos, d_plane, d_bits;
   bool force_large_map_path = false;   // PORRT_OPT_FORCE_LARGE_MAP_PATH (tests): run map.cu's kernel although edge3.cu's would fit
-  bool force_global_sweeps = false;    // PORRT_OPT_FORCE_GLOBAL_SWEEPS (tests): value backups by graph.cu's sweeps although colsolve.cu would fit
+  bool force_global_sweeps = false;    // PORRT_OPT_FORCE_GLOBAL_SWEEPS (tests): value backups by the frontier relaxation (sssp_frontier.cu) although colsolve.cu would fit
   bool force_thread_per_query_nn = false;  // PORRT_OPT_FORCE_THREAD_PER_QUERY_NN (tests): nn.cu's kernels although nn_tile.cu's would serve
   // host copies of the raw images are NOT kept: the product never walks pixels on the CPU.
 
@@ -235,19 +235,22 @@ struct porrt_ctx {
   DevBuf kd_buf;      // kd_preorder_rank_dev (its own: the PRM build runs the rank on a helper thread next to the binning sort)
   cudaStream_t aux_stream = nullptr;   // second compute stream (created on first use): kd rank next to radius / edge batches
   DevBuf ws_main;     // the entry points' inputs and work blocks: porrt_radius_query, knn_host, porrt_state_validity, porrt_visibility,
-                      // porrt_transition_valid, the shortcut and Reparent refiners, porrt_sssp_worlds(_prm), porrt_belief_vi,
+                      // porrt_transition_valid, the shortcut and Reparent refiners, porrt_sssp_worlds(_prm) and porrt_belief_vi (held
+                      // while graph.cu's value-column driver runs, which carves from ws_state),
                       // porrt_conditional_dijkstra_graph, the PRM build's per-node arrays; edge_pipeline's chunk slots
   DevBuf ws_owner;    // map upload: the occupancy image; PRM build: the owner of each candidate, then the packed neighbour lists
   DevBuf ws_vid;      // map upload: the zone image; PRM build: the candidates' validity ids, then the late lists and cursors
   DevBuf ws_table;    // map upload: zone statistics; the radius id lists of porrt_radius_query and the PRM build
-                      // (nn_radius_count_fill_dev's ids_buf); sssp_core's value table and finals; belief_download_full's
-                      // [node][belief] table
+                      // (nn_radius_count_fill_dev's ids_buf); sssp_core's world table, world masks and column map;
+                      // belief_download_full's [node][belief] table
   DevBuf ws_query;    // nn_radius_count_fill_dev: staging offsets, counts and the wide-query list; nn_vertices_set_dev's bounding
                       // box; edge_pipeline's id check flag; belief_succ_tables' inputs and work space; porrt_measure_l2_gather's sink
   DevBuf ws_seg;      // segments_sort_by_key_dev: its counters, mid-length segment list and inverse key permutation
   DevBuf sort_keys, sort_vals;   // nn_vertices_set_dev's and segments_sort_by_key_dev's (radix path) pairs to sort; sf_build_graph's
                                  // Morton order (keys) and transposed graph (vals); porrt_edge_validity_csr_i8's row_ptr (keys)
-  DevBuf ws_state;    // nn_vertices_set_dev: cell counts; sf_relax: the frontier state (sf_state_layout), with sssp_frontier_run's value table behind it
+  DevBuf ws_state;    // nn_vertices_set_dev: cell counts; sf_relax: the frontier state (sf_state_layout); the value-column driver
+                      // (graph.cu): its block behind that state (sf_state_reserve): the Morton-numbered table, the finals, the
+                      // column solver's counters and transposed graph
   DevBuf radix_keys, radix_vals, radix_hist;   // radix_sort_pairs: the second key / value array, the histograms and tile bases;
                       // porrt_kd_preorder_rank's coordinates and ranks (radix_vals); the PRM build's shard summaries (radix_hist)
   DevBuf scan_sums;   // scan_exclusive_i64: block sums

@@ -806,116 +806,277 @@ __global__ void edge_cost_kernel(const int64_t* __restrict__ row_ptr, const int3
   }
 }
 
+// ================================================================================================ value columns
+// Both value tables -- plan_qmdp's dist[.][world] and porrt_belief_vi's dist[.][belief] -- are sets of columns, each a shortest-path
+// problem on the same roadmap (DESIGN 3.3).  One driver solves them: value_columns_prepare chooses the schedule (the on-chip column
+// solver, colsolve.cu, or the frontier relaxation, sssp_frontier.cu) and writes the initial table; value_columns_solve runs the
+// levels in order.  Only the column kind (COLSOLVE_WORLD / COLSOLVE_BELIEF) tells the two tables apart.
+
+// Columns sit at positions level by level; a level's columns do not depend on each other (world columns: one level; belief columns:
+// the support size, see porrt_belief_vi).  With `shards` > 1 every level is cut into `shards` shards of EQUAL width -- the last
+// positions of a shard may be unused padding -- so that the exchange after a level is one plain ncclAllGather; rank r owns the
+// positions [lo + r * per, lo + r * per + count_r), count_r from comm_shard_range.
+struct ColumnLayout {
+  struct Level { int lo, per, n_real; };
+  std::vector<Level> levels;
+  std::vector<int32_t> colpos;   // [columns] position of a column
+  std::vector<int32_t> poscol;   // [positions] column at a position, -1 = padding
+  int shards;
+};
+static ColumnLayout column_layout(const std::vector<int32_t>& level_key, int shards) {
+  const int n = (int)level_key.size();
+  std::vector<int32_t> by_level((size_t)n);
+  for (int c = 0; c < n; ++c) by_level[(size_t)c] = c;
+  std::stable_sort(by_level.begin(), by_level.end(), [&](int32_t x, int32_t y) { return level_key[(size_t)x] < level_key[(size_t)y]; });
+  ColumnLayout L;
+  L.colpos.resize((size_t)n);
+  L.shards = shards;
+  for (int c = 0; c < n;) {
+    int e = c;
+    while (e < n && level_key[(size_t)by_level[(size_t)e]] == level_key[(size_t)by_level[(size_t)c]]) ++e;
+    const int n_real = e - c, per = (n_real + shards - 1) / shards, lo = (int)L.poscol.size();
+    L.poscol.resize((size_t)lo + (size_t)per * shards, -1);
+    for (int r = 0; r < shards; ++r) {
+      int64_t a, b;
+      comm_shard_range(n_real, r, shards, &a, &b);
+      for (int64_t j = a; j < b; ++j) {
+        const int pos = lo + r * per + (int)(j - a);
+        L.poscol[(size_t)pos] = by_level[(size_t)(c + j)];
+        L.colpos[(size_t)by_level[(size_t)(c + j)]] = pos;
+      }
+    }
+    L.levels.push_back({lo, per, n_real});
+    c = e;
+  }
+  return L;
+}
+
+// The columns and what the driver leaves between its two steps (device pointers unless said otherwise).
+struct ValueColumns {
+  int kind;                                    // COLSOLVE_WORLD / COLSOLVE_BELIEF
+  const int64_t* row; const int32_t* col; const double* xy; int64_t V, E;
+  const int32_t* evid;                         // edge validity ids (belief columns), or null
+  int32_t n_validities;                        // (colsolve_fits)
+  const ColumnLayout* layout;                  // host
+  // cs.dist_cm: the caller's [position][node] table (ld = V), the result; cs.col_belief: the column at a position (layout->poscol);
+  // cs.cmask: [position][4] the validity ids below 256 a column admits (world: node ids; belief: edge ids); cs.nvid (world columns:
+  // may be null = every node valid) and the belief tables as colsolve_level reads them
+  ColSolveArgs cs;
+  const uint64_t* validities; int32_t mask_words;   // world columns on the frontier: the worlds of a node validity id (any number of ids)
+  // set by value_columns_prepare
+  bool on_chip;
+  SfGraph g;
+  double* morton;                              // frontier: the table in Morton numbering, behind sf_relax's state in ws_state
+  const int2* fin; int64_t n_fin;              // the finals as (position, node)
+};
+
 __global__ void fill_inf_kernel(double* __restrict__ d, int64_t n) {
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) d[i] = INFINITY;
 }
-__global__ void scatter_zero_kernel(double* __restrict__ d, const int64_t* __restrict__ idx, int64_t n) {
+// finals at positions [lo, hi): 0, the sign kept (a fixed entry stays fixed); perm: the node numbering of the table, null = the
+// caller's (several finals may name the same entry: same value)
+__global__ void scatter_zero_kernel(double* __restrict__ table, const int2* __restrict__ fin, int64_t n, const int32_t* __restrict__ perm,
+                                    int64_t V, int lo, int hi) {
   const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i < n) d[idx[i]] = 0.0;
+  if (i >= n || fin[i].x < lo || fin[i].x >= hi) return;
+  double* d = table + (int64_t)fin[i].x * V + (perm ? perm[fin[i].y] : fin[i].y);
+  *d = (__double_as_longlong(*d) < 0) ? -0.0 : 0.0;
+}
+// Frontier: the initial values of the positions [lo, hi) of one level in the Morton-numbered table, written without reading the
+// entry: +inf, with the sign bit where it must not be relaxed -- in a world column a node invalid in the world (PTOGraphWorldView::
+// parents filters by the parent node); in a belief column everything but the Action nodes, whose Observation nodes hold
+// sum_k p_k * (0.0 + dist[n][succ_k])  (belief_graph.rs:125-135) from the finished levels.  Padding stays +inf.  The finals come after.
+__global__ void level_init_kernel(ColSolveArgs a, int kind, int lo, int hi, const uint32_t* __restrict__ order,
+                                  const uint64_t* __restrict__ validities, int mask_words, double* __restrict__ table) {
+  const int64_t V = a.V;
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= (int64_t)(hi - lo) * V) return;
+  const int c = lo + (int)(t / V);
+  const int64_t pos = t - (int64_t)(c - lo) * V;
+  const int32_t col = a.col_belief[c];
+  const int64_t n = order[pos];
+  double v = INFINITY;
+  bool fixed = false;
+  if (col >= 0 && kind == COLSOLVE_WORLD) {
+    fixed = a.nvid && !((validities[(int64_t)a.nvid[n] * mask_words + (col >> 6)] >> (col & 63)) & 1);
+  } else if (col >= 0) {
+    const uint8_t ty = a.type_cm[(int64_t)c * V + n];
+    fixed = ty != PORRT_NODE_ACTION;
+    if (ty == PORRT_NODE_OBSERVATION) {
+      const int32_t nv = a.nvid[n];
+      const int64_t sp = (int64_t)a.node_set[n] * a.B + col;
+      double alt = 0.0;
+      for (int64_t k = a.succ_ptr[sp]; k < a.succ_ptr[sp + 1]; ++k) {
+        const int32_t cc = a.succ_col[k];
+        if (!((a.cmask[(int64_t)cc * 4 + (nv >> 6)] >> (nv & 63)) & 1)) continue;   // successor belief node does not exist here
+        alt = __dadd_rn(alt, __dmul_rn(a.succ_p[k], __dadd_rn(0.0, fabs(table[(int64_t)cc * V + pos]))));
+      }
+      if (alt < v) v = alt;
+    }
+  }
+  table[(int64_t)c * V + pos] = fixed ? -v : v;
+}
+// Morton-numbered table (signs) -> out[position][node]
+__global__ void unpermute_kernel(const double* __restrict__ table, const int32_t* __restrict__ perm, int64_t V, int64_t n_pos, double* __restrict__ out) {
+  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (t >= n_pos * V) return;
+  const int64_t c = t / V, n = t - c * V;
+  out[t] = fabs(table[c * V + perm[n]]);
 }
 
-// plan_qmdp on a graph that already lives on the device (all d_* are device pointers; h_val = host copy of the validity table).
-// Roadmaps whose value column fits in shared memory go to the on-chip column solver (colsolve.cu, one column per world), larger
-// ones to the frontier relaxation over global memory (sssp_frontier.cu).  out_dist (host, [Wall][V]) may be null: the table then
-// stays on the device only (timing, device-resident pipelines).  Work space: ws_table; porrt_ctx_last_phase_ms afterwards:
-// [0] device ms of the backups, [1] edge records / (parent, world) pairs worked through.
+// Chooses the schedule, builds its graph and writes the initial table: +inf, 0 at the finals (the frontier writes its levels when
+// they start, value_columns_solve).  fin: the finals as (position, node).  Work space: ws_state (and sf_build_graph's).
+static int32_t value_columns_prepare(porrt_ctx* ctx, ValueColumns& vc, const std::vector<int2>& fin, cudaStream_t st) {
+  const int64_t V = vc.V, E = vc.E, n_pos = (int64_t)vc.layout->poscol.size();
+  vc.on_chip = colsolve_fits(V, E, vc.n_validities) && !ctx->force_global_sweeps;
+  vc.n_fin = (int64_t)fin.size();
+  int per_max = 0;
+  for (const ColumnLayout::Level& L : vc.layout->levels) per_max = std::max(per_max, L.per);
+  if (!vc.on_chip) {   // Morton numbering + transposed adjacency, with the edge validity ids if the columns have any
+    int32_t rc = sf_build_graph(ctx, vc.row, vc.col, vc.evid, vc.xy, V, E, &vc.g, st);
+    if (rc) return rc;
+  }
+  int2* d_fin;
+  double *d_cost = nullptr, *d_cost_t = nullptr;
+  uint32_t *d_ce = nullptr, *d_rs = nullptr, *d_cursor = nullptr;
+  CUDA_TRY(ctx, carve(ctx->ws_state, [&](Carve& c) {
+    if (!vc.on_chip) { sf_state_reserve(c, V, per_max); vc.morton = c.take<double>((size_t)V * n_pos); }
+    d_fin = c.take<int2>(vc.n_fin);
+    vc.cs.sweeps_out = c.take<int32_t>(4);
+    if (vc.on_chip) {
+      d_cost = c.take<double>(E); d_cost_t = c.take<double>(E);
+      d_ce = c.take<uint32_t>(E); d_rs = c.take<uint32_t>(V + 1); d_cursor = c.take<uint32_t>(V + 1);
+    }
+  }));
+  vc.fin = d_fin;
+  vc.cs.offers_out = (unsigned long long*)(vc.cs.sweeps_out + 2);
+  if (vc.n_fin) CUDA_TRY(ctx, cudaMemcpyAsync(d_fin, fin.data(), (size_t)vc.n_fin * sizeof(int2), cudaMemcpyHostToDevice, st));
+  if (!vc.on_chip) return PORRT_OK;
+  edge_cost_kernel<<<div_up(V * 32, 256), 256, 0, st>>>(vc.row, vc.col, (const double2*)vc.xy, V, d_cost);
+  LAUNCH_CHECK(ctx);
+  int32_t rc = colsolve_pack(ctx, vc.row, vc.col, vc.evid, d_cost, V, E, d_rs, d_ce, d_cost_t, d_cursor, st);
+  if (rc) return rc;
+  vc.cs.row_start = d_rs; vc.cs.cost = d_cost_t; vc.cs.ce = d_ce;
+  fill_inf_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(vc.cs.dist_cm, V * n_pos);
+  LAUNCH_CHECK(ctx);
+  if (vc.n_fin) {
+    scatter_zero_kernel<<<div_up(vc.n_fin, 256), 256, 0, st>>>(vc.cs.dist_cm, d_fin, vc.n_fin, nullptr, V, 0, (int)n_pos);
+    LAUNCH_CHECK(ctx);
+  }
+  CUDA_TRY(ctx, cudaMemsetAsync(vc.cs.sweeps_out, 0, 16, st));
+  return PORRT_OK;
+}
+
+// Runs the levels in order, this rank's shard of each, and all-gathers every level before the next one reads it; leaves the table as
+// [position][node] in vc.cs.dist_cm and marks the end of the backups (tmark).  out_sweeps: the most sweeps / rounds of a level;
+// out_offers: the edge records / (parent, column) pairs worked through, summed.
+static int32_t value_columns_solve(porrt_ctx* ctx, ValueColumns& vc, int32_t* out_sweeps, double* out_offers, cudaStream_t st) {
+  const ColumnLayout& lay = *vc.layout;
+  const int64_t V = vc.V, n_pos = (int64_t)lay.poscol.size();
+  const int rank = lay.shards > 1 ? ctx->comm_rank : 0;
+  double* table = vc.on_chip ? vc.cs.dist_cm : vc.morton;
+  int32_t sweeps = 0;
+  double offers = 0.0;
+  for (const ColumnLayout::Level& L : lay.levels) {
+    int64_t a, b;
+    comm_shard_range(L.n_real, rank, lay.shards, &a, &b);
+    const int mine = L.lo + rank * L.per, n_mine = (int)(b - a);
+    int32_t rc;
+    if (vc.on_chip) {
+      rc = colsolve_level(ctx, vc.cs, vc.kind, mine, mine + n_mine, st);
+    } else {
+      level_init_kernel<<<div_up((int64_t)L.per * V, 256), 256, 0, st>>>(vc.cs, vc.kind, mine, mine + L.per, vc.g.order, vc.validities,
+                                                                          vc.mask_words, table);
+      LAUNCH_CHECK(ctx);
+      if (vc.n_fin) {
+        scatter_zero_kernel<<<div_up(vc.n_fin, 256), 256, 0, st>>>(table, vc.fin, vc.n_fin, vc.g.perm, V, mine, mine + L.per);
+        LAUNCH_CHECK(ctx);
+      }
+      int32_t rounds = 0;
+      double off = 0.0;
+      rc = sf_relax(ctx, vc.g, table + (int64_t)mine * V, n_mine, vc.g.evid_t ? vc.cs.cmask + (int64_t)mine * 4 : nullptr, &rounds, &off, st);
+      sweeps = std::max(sweeps, rounds);
+      offers += off;
+    }
+    if (rc) return rc;
+    if (lay.shards > 1) {
+      std::vector<int64_t> off((size_t)lay.shards + 1);
+      for (int r = 0; r <= lay.shards; ++r) off[(size_t)r] = (int64_t)(L.lo + r * L.per) * V * 8;
+      rc = comm_all_gatherv_dev(ctx, nullptr, table, off.data(), st);
+      if (rc) return rc;
+    }
+  }
+  if (!vc.on_chip) {
+    unpermute_kernel<<<div_up(n_pos * V, 256), 256, 0, st>>>(vc.morton, vc.g.perm, V, n_pos, vc.cs.dist_cm);
+    LAUNCH_CHECK(ctx);
+  }
+  tmark(ctx);
+  if (vc.on_chip) {
+    unsigned long long off = 0;
+    CUDA_TRY(ctx, cudaMemcpyAsync(&sweeps, vc.cs.sweeps_out, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(&off, vc.cs.offers_out, 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    offers = (double)off;
+  }
+  *out_sweeps = sweeps;
+  *out_offers = offers;
+  return PORRT_OK;
+}
+
+// plan_qmdp on a graph that already lives on the device (all d_* are device pointers; h_val = host copy of the validity table): one
+// value column per world.  out_dist (host, [Wall][V]) may be null: the table then stays on the device only (timing, device-resident
+// pipelines).  Work space: ws_table; porrt_ctx_last_phase_ms afterwards: [0] device ms from the graph preparation to the end of the
+// backups, [1] edge records / (parent, world) pairs worked through.
 static int32_t sssp_core(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_col, const double* d_xy, int64_t V, int64_t E,
                          const int32_t* d_nvid, const uint64_t* d_val, const uint64_t* h_val, int32_t n_validities, int32_t mask_words,
                          bool world_view, int Wall, const int64_t* finals_ptr, const int32_t* finals_ids, double* out_dist,
                          int32_t* out_sweeps) {
   cudaStream_t st = ctx->stream;
-  // multi-GPU (comm.cu): the worlds are independent problems on one graph -- rank r relaxes worlds [wlo, whi) and the dist
-  // rows are all-gathered (SURVEY 8(e)); the plain-graph call (n_worlds == 0) is not sharded
-  int64_t wlo = 0, whi = Wall;
-  const bool sharded = world_view && ctx->comm_world > 1;
-  if (sharded) comm_shard_range(Wall, ctx->comm_rank, ctx->comm_world, &wlo, &whi);
-  const int W = (int)(whi - wlo);
-  const bool cols = colsolve_fits(V, E, world_view ? n_validities : 1) && !ctx->force_global_sweeps;
-  // the finals of this rank's worlds: indices into the [world][node] table (column solver) or (node, local world) pairs (frontier)
-  std::vector<int64_t> zero_idx;
-  std::vector<int32_t> fin_nw;
+  // multi-GPU (comm.cu): the worlds are independent problems on one graph, sharded over the ranks and all-gathered (SURVEY 8(e));
+  // the plain-graph call (n_worlds == 0) is not sharded
+  const ColumnLayout lay = column_layout(std::vector<int32_t>((size_t)Wall, 0), world_view && ctx->comm_world > 1 ? ctx->comm_world : 1);
+  const int64_t n_pos = (int64_t)lay.poscol.size();
+  std::vector<int2> fin;
   for (int w = 0; w < Wall; ++w)
     for (int64_t k = finals_ptr[w]; k < finals_ptr[w + 1]; ++k) {
       const int32_t f = finals_ids[k];
       if (f < 0 || f >= V) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "sssp_worlds: final id out of range");
-      if (w >= wlo && w < whi) {
-        if (cols) zero_idx.push_back((int64_t)w * V + f);
-        else { fin_nw.push_back(f); fin_nw.push_back((int32_t)(w - wlo)); }
-      }
+      fin.push_back(make_int2(lay.colpos[(size_t)w], f));
     }
-  const int64_t n_fin = cols ? (int64_t)zero_idx.size() : (int64_t)fin_nw.size() / 2;
-  double* d_out;   // [Wall][V]: this rank fills rows wlo..whi, the gather the rest
-  int32_t* d_flag;
-  int64_t* d_zero = nullptr;                           // column solver
-  double *d_cost = nullptr, *d_cost_t = nullptr;
-  uint32_t *d_ce = nullptr, *d_rs = nullptr, *d_cursor = nullptr;
-  uint64_t* d_cmask = nullptr;
-  int32_t* d_fin = nullptr;                            // frontier
+  // the validity ids each world admits, as far as the column solver reads them (colsolve_fits refuses more than 256); every node of
+  // the plain graph is valid
+  std::vector<uint64_t> cmask((size_t)n_pos * 4, world_view ? 0 : ~(uint64_t)0);
+  for (int64_t p = 0; world_view && p < n_pos; ++p) {
+    const int w = lay.poscol[(size_t)p];
+    for (int v = 0; w >= 0 && v < std::min(n_validities, 256); ++v)
+      if ((h_val[(size_t)v * mask_words + w / 64] >> (w % 64)) & 1) cmask[(size_t)p * 4 + v / 64] |= (uint64_t)1 << (v % 64);
+  }
+  double* d_out;   // [n_pos][V]
+  uint64_t* d_cmask;
+  int32_t* d_poscol;
   CUDA_TRY(ctx, carve(ctx->ws_table, [&](Carve& c) {
-    d_out = c.take<double>((size_t)V * Wall);
-    d_flag = c.take<int32_t>(4);
-    if (W > 0 && cols) {
-      d_zero = c.take<int64_t>(n_fin + 1);
-      d_cost = c.take<double>(E); d_cost_t = c.take<double>(E);
-      d_ce = c.take<uint32_t>(E); d_rs = c.take<uint32_t>(V + 1); d_cursor = c.take<uint32_t>(V + 1);
-      d_cmask = c.take<uint64_t>((size_t)Wall * 4);
-    } else if (W > 0) {
-      d_fin = c.take<int32_t>(2 * n_fin + 2);
-    }
+    d_out = c.take<double>((size_t)V * n_pos); d_cmask = c.take<uint64_t>(cmask.size()); d_poscol = c.take<int32_t>(n_pos);
   }));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_cmask, cmask.data(), cmask.size() * 8, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_poscol, lay.poscol.data(), (size_t)n_pos * 4, cudaMemcpyHostToDevice, st));
+  ValueColumns vc = {};
+  vc.kind = COLSOLVE_WORLD; vc.row = d_row; vc.col = d_col; vc.xy = d_xy; vc.V = V; vc.E = E; vc.n_validities = world_view ? n_validities : 1;
+  vc.layout = &lay; vc.validities = d_val; vc.mask_words = mask_words;
+  vc.cs.V = (int32_t)V; vc.cs.ld = V; vc.cs.dist_cm = d_out; vc.cs.cmask = d_cmask; vc.cs.col_belief = d_poscol;
+  vc.cs.nvid = world_view ? d_nvid : nullptr;
   int sweeps = 0;
   double offers = 0.0;
   tstart(ctx);
-  if (W > 0 && cols) {
-    // one column per world, solved on chip; d_out is the column-major table itself
-    std::vector<uint64_t> cmask((size_t)Wall * 4, world_view ? 0 : ~(uint64_t)0);
-    if (world_view)
-      for (int w = 0; w < Wall; ++w)
-        for (int v = 0; v < n_validities; ++v)
-          if ((h_val[(size_t)v * mask_words + w / 64] >> (w % 64)) & 1) cmask[(size_t)w * 4 + v / 64] |= (uint64_t)1 << (v % 64);
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_cmask, cmask.data(), cmask.size() * 8, cudaMemcpyHostToDevice, st));
-    if (n_fin) CUDA_TRY(ctx, cudaMemcpyAsync(d_zero, zero_idx.data(), (size_t)n_fin * 8, cudaMemcpyHostToDevice, st));
-    edge_cost_kernel<<<div_up(V * 32, 256), 256, 0, st>>>(d_row, d_col, (const double2*)d_xy, V, d_cost);
-    LAUNCH_CHECK(ctx);
-    int32_t rc = colsolve_pack(ctx, d_row, d_col, nullptr, d_cost, V, E, d_rs, d_ce, d_cost_t, d_cursor, st);
-    if (rc) return rc;
-    fill_inf_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(d_out + wlo * V, V * (int64_t)W);
-    LAUNCH_CHECK(ctx);
-    if (n_fin) {
-      scatter_zero_kernel<<<div_up(n_fin, 256), 256, 0, st>>>(d_out, d_zero, n_fin);
-      LAUNCH_CHECK(ctx);
-    }
-    CUDA_TRY(ctx, cudaMemsetAsync(d_flag, 0, 16, st));
-    ColSolveArgs ca = {};
-    ca.row_start = d_rs; ca.cost = d_cost_t; ca.ce = d_ce; ca.V = (int32_t)V; ca.ld = V; ca.dist_cm = d_out; ca.cmask = d_cmask;
-    ca.nvid = world_view ? d_nvid : nullptr; ca.sweeps_out = d_flag; ca.offers_out = (unsigned long long*)(d_flag + 2);
-    rc = colsolve_level(ctx, ca, COLSOLVE_WORLD, (int)wlo, (int)whi, st);
-    if (rc) return rc;
-    tmark(ctx);
-    unsigned long long off = 0;
-    CUDA_TRY(ctx, cudaMemcpyAsync(&sweeps, d_flag, 4, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(&off, d_flag + 2, 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    offers = (double)off;
-  } else if (W > 0) {
-    // (node, world) pairs interleaved on the host -> two arrays on the device
-    std::vector<int32_t> split((size_t)n_fin * 2);
-    for (int64_t k = 0; k < n_fin; ++k) { split[(size_t)k] = fin_nw[(size_t)2 * k]; split[(size_t)(n_fin + k)] = fin_nw[(size_t)2 * k + 1]; }
-    if (n_fin) CUDA_TRY(ctx, cudaMemcpyAsync(d_fin, split.data(), (size_t)n_fin * 8, cudaMemcpyHostToDevice, st));
-    int32_t rc = sssp_frontier_run(ctx, d_row, d_col, d_xy, V, E, world_view ? d_nvid : nullptr, d_val, mask_words, (int32_t)wlo, W, d_fin,
-                                   d_fin + n_fin, n_fin, d_out + wlo * V, &sweeps, &offers, st);
-    if (rc) return rc;
-    tmark(ctx);
-  } else {
-    tmark(ctx);
+  int32_t rc = value_columns_prepare(ctx, vc, fin, st);
+  if (rc) return rc;
+  rc = value_columns_solve(ctx, vc, &sweeps, &offers, st);
+  if (rc) return rc;
+  // one copy per rank block: the worlds of rank r sit at the front of its shard
+  for (int r = 0; out_dist && r < lay.shards; ++r) {
+    int64_t a, b;
+    comm_shard_range(Wall, r, lay.shards, &a, &b);
+    if (b > a) CUDA_TRY(ctx, cudaMemcpyAsync(out_dist + a * V, d_out + (int64_t)r * lay.levels[0].per * V, (size_t)((b - a) * V) * 8, cudaMemcpyDeviceToHost, st));
   }
-  if (sharded) {
-    std::vector<int64_t> off(ctx->comm_world + 1);
-    for (int r = 0; r < ctx->comm_world; ++r) { int64_t a2, b2; comm_shard_range(Wall, r, ctx->comm_world, &a2, &b2); off[r] = a2 * V * 8; off[r + 1] = b2 * V * 8; }
-    int32_t rc = comm_all_gatherv_dev(ctx, nullptr, d_out, off.data(), st);
-    if (rc) return rc;
-  }
-  if (out_dist) CUDA_TRY(ctx, cudaMemcpyAsync(out_dist, d_out, (size_t)V * Wall * 8, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
   tfinish(ctx);
   ctx->last_ms[1] = offers; ctx->n_last = 2;
@@ -1139,50 +1300,6 @@ __global__ void type_finish_kernel(uint8_t* __restrict__ type, int64_t n) {
     if (type[i] == 255) type[i] = PORRT_NODE_UNKNOWN;
 }
 
-// ---- belief columns through the frontier relaxation (sssp_frontier.cu): roadmaps whose column does not fit in shared memory.
-// Initial values of the columns [c_lo, c_hi) of one level in the Morton-numbered table: +inf, 0 at the finals (already scattered),
-// the Observation value  sum_k p_k * (0.0 + dist[n][succ_k])  (belief_graph.rs:125-135) from the finished columns; the sign bit on
-// everything that is not an Action node (never relaxed).
-__global__ void belief_level_init_kernel(int64_t V, int B, int c_lo, int c_hi, const uint32_t* __restrict__ order, const uint8_t* __restrict__ type_cm,
-                                         const int32_t* __restrict__ nvid, const int32_t* __restrict__ node_set, const int32_t* __restrict__ col_belief,
-                                         const int64_t* __restrict__ succ_ptr, const int32_t* __restrict__ succ_col, const double* __restrict__ succ_p,
-                                         const uint64_t* __restrict__ cmask, double* __restrict__ table) {
-  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= (int64_t)(c_hi - c_lo) * V) return;
-  const int c = c_lo + (int)(t / V);
-  const int64_t pos = t - (int64_t)(c - c_lo) * V;
-  if (col_belief[c] < 0) return;                       // padding column
-  const int64_t n = order[pos];
-  const uint8_t ty = type_cm[(int64_t)c * V + n];
-  double v = table[(int64_t)c * V + pos];
-  if (ty == PORRT_NODE_OBSERVATION) {
-    const int32_t nv = nvid[n];
-    const int64_t sp = (int64_t)node_set[n] * B + col_belief[c];
-    double alt = 0.0;
-    for (int64_t k = succ_ptr[sp]; k < succ_ptr[sp + 1]; ++k) {
-      const int32_t cc = succ_col[k];
-      if (!((cmask[(int64_t)cc * 4 + (nv >> 6)] >> (nv & 63)) & 1)) continue;   // successor belief node does not exist here
-      alt = __dadd_rn(alt, __dmul_rn(succ_p[k], __dadd_rn(0.0, fabs(table[(int64_t)cc * V + pos]))));
-    }
-    if (alt < v) v = alt;
-  }
-  table[(int64_t)c * V + pos] = ty != PORRT_NODE_ACTION ? -v : v;
-}
-// finals: 0 in the Morton-numbered table; idx = column * V + node (caller's numbering)
-__global__ void scatter_zero_perm_kernel(double* __restrict__ table, const int64_t* __restrict__ idx, int64_t n, const int32_t* __restrict__ perm, int64_t V) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  const int64_t c = idx[i] / V, node = idx[i] - c * V;
-  table[c * V + perm[node]] = 0.0;
-}
-// table (Morton numbering, signs) -> dist_cm[column][node]
-__global__ void belief_unpermute_kernel(const double* __restrict__ table, const int32_t* __restrict__ perm, int64_t V, int64_t n_cols, double* __restrict__ dist_cm) {
-  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= n_cols * V) return;
-  const int64_t c = t / V, n = t - c * V;
-  dist_cm[t] = fabs(table[c * V + perm[n]]);
-}
-
 // dist_cm[colpos[b]][n] -> dist[n][b] through a 32 x 32 tile (both sides coalesced)
 __global__ void __launch_bounds__(256) belief_untranspose_kernel(const double* __restrict__ dist_cm, int64_t ld, const int32_t* __restrict__ colpos,
                                                                  int64_t V, int B, double* __restrict__ dist) {
@@ -1301,37 +1418,14 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
     if (it == set_index.end()) { it = set_index.emplace(vis, (int)sets.size()).first; sets.push_back(vis); }
     node_set[n] = it->second;
   }
-  // column order for colsolve.cu: beliefs sorted by the size of their support (observations only ever split it, so a column
-  // reads Observation values from columns that come earlier), level by level
-  std::vector<int32_t> level((size_t)B, 0), colpos((size_t)B), by_level((size_t)B);
+  // column levels: beliefs by the size of their support (observations only ever split it, so a column reads Observation values
+  // from columns of earlier levels)
+  std::vector<int32_t> level((size_t)B, 0);
   for (int b2 = 0; b2 < B; ++b2)
     for (int k = 0; k < mask_words; ++k) level[(size_t)b2] += __builtin_popcountll(support[(size_t)b2 * mask_words + k]);
-  for (int b2 = 0; b2 < B; ++b2) by_level[(size_t)b2] = b2;
-  std::stable_sort(by_level.begin(), by_level.end(), [&](int32_t x, int32_t y) { return level[(size_t)x] < level[(size_t)y]; });
-  // Column positions.  On one GPU the columns of a level are simply consecutive.  With a communicator every level is cut into
-  // `world` shards of EQUAL width (the last columns of a shard may be unused padding) so that the exchange after a level is one
-  // plain ncclAllGather instead of a group of ragged broadcasts; rank r owns the columns [lo + r * per, lo + r * per + count_r).
-  const int shards = ctx->comm_world > 1 ? ctx->comm_world : 1;
-  struct Level { int lo, per, n_real; };
-  std::vector<Level> levels;
-  std::vector<int32_t> col_belief;   // belief of a column position, -1 = padding
-  for (int c = 0; c < B;) {
-    int e = c;
-    while (e < B && level[(size_t)by_level[(size_t)e]] == level[(size_t)by_level[(size_t)c]]) ++e;
-    const int n_real = e - c, per = (n_real + shards - 1) / shards, lo = (int)col_belief.size();
-    col_belief.resize((size_t)lo + (size_t)per * shards, -1);
-    for (int r = 0; r < shards; ++r) {
-      int64_t a2, b2;
-      comm_shard_range(n_real, r, shards, &a2, &b2);
-      for (int64_t j = a2; j < b2; ++j) {
-        const int pos = lo + r * per + (int)(j - a2);
-        col_belief[(size_t)pos] = by_level[(size_t)(c + j)];
-        colpos[(size_t)by_level[(size_t)(c + j)]] = pos;
-      }
-    }
-    levels.push_back({lo, per, n_real});
-    c = e;
-  }
+  const ColumnLayout lay = column_layout(level, ctx->comm_world > 1 ? ctx->comm_world : 1);
+  const std::vector<int32_t>& colpos = lay.colpos;
+  const std::vector<int32_t>& col_belief = lay.poscol;
   const int Bp = (int)col_belief.size();   // columns incl. padding (== B on one GPU)
   // observation successor tables, one entry per (set, belief), built on the device (belief_tables.cu)
   BeliefSuccDev succ = {};
@@ -1340,19 +1434,17 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
     if (rc) return rc;
   }
   // initial distances: 0 at final belief nodes (pto.rs:261-271), +inf elsewhere -- written on the device; only the list of final
-  // belief nodes is built here (a host-side V*B table cost 30 ms + a 150 MB upload at B = 4095)
-  std::vector<int64_t> zero_idx;
+  // belief nodes, as (column position, node), is built here (a host-side V*B table cost 30 ms + a 150 MB upload at B = 4095)
+  std::vector<int2> fin;
   for (int k = 0; k < n_finals; ++k) {
     const int32_t f = finals_ids[k];
     if (f < 0 || f >= V) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "belief_vi: final id out of range");
     for (int b = 0; b < B; ++b)
       if (compat[(size_t)b * n_validities + node_vid[f]] && compatible(b, finals_masks + (size_t)k * mask_words))
-        zero_idx.push_back((int64_t)f * B + b);
+        fin.push_back(make_int2(colpos[(size_t)b], f));
   }
   t1 = now_ms(); ph[0] = t1 - t0; t0 = t1;
 
-  const bool cols = colsolve_fits(V, E, n_validities) && !ctx->force_global_sweeps && succ.levels_ok;
-  const bool sharded = ctx->comm_world > 1;
   if (n_validities > 256) return porrt_fail(ctx, PORRT_ERR_UNSUPPORTED, "belief_vi: more than 256 validity ids");
   if (!succ.levels_ok) return porrt_fail(ctx, PORRT_ERR_UNSUPPORTED, "belief_vi: an observation does not split the belief's support (the level order of the backups does not apply)");
   std::vector<uint64_t> cmask((size_t)Bp * 4, 0);
@@ -1361,32 +1453,21 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
       for (int v = 0; col_belief[(size_t)c] >= 0 && v < n_validities; ++v)
         if (compat[(size_t)col_belief[(size_t)c] * n_validities + v]) cmask[(size_t)c * 4 + v / 64] |= (uint64_t)1 << (v % 64);
   }
-  // final belief nodes as indices into the [column][node] table the backups run on
-  for (int64_t& z : zero_idx) { const int64_t f = z / B; const int b2 = (int)(z % B); z = (int64_t)colpos[(size_t)b2] * V + f; }
 
   int64_t* d_row;
-  double *d_cost, *d_xy, *d_cost_t;
-  double* d_table_m = nullptr;   // frontier path: the table in Morton numbering, [column][pos]
+  double* d_xy;
   uint64_t* d_cmask;
-  int32_t *d_col, *d_evid, *d_nvid, *d_nset, *d_col_belief, *d_changed;
-  uint32_t *d_ce, *d_rs, *d_cursor;
+  int32_t *d_col, *d_evid, *d_nvid, *d_nset, *d_col_belief;
   uint8_t* d_compat;
-  int64_t* d_zero;
   CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
     d_row = c.take<int64_t>(V + 1);
-    d_cost = c.take<double>(E);
     d_xy = c.take<double>(2 * V);
-    if (!cols) d_table_m = c.take<double>((size_t)V * Bp);
     d_cmask = c.take<uint64_t>((size_t)Bp * 4);
     d_col = c.take<int32_t>(E); d_evid = c.take<int32_t>(E);
-    d_ce = c.take<uint32_t>(E); d_rs = c.take<uint32_t>(V + 1); d_cursor = c.take<uint32_t>(V + 1);
-    d_cost_t = c.take<double>(E);
     d_nvid = c.take<int32_t>(V); d_nset = c.take<int32_t>(V); d_col_belief = c.take<int32_t>(Bp);
-    d_changed = c.take<int32_t>(4);
     d_compat = c.take<uint8_t>(compat.size());
-    d_zero = c.take<int64_t>(zero_idx.size() + 1);
   }));
-  // the column solver's table ([column][node]), the node types and the column map outlive the call (lazy result, policy walk)
+  // the table ([column][node]), the node types and the column map outlive the call (lazy result, policy walk)
   auto& R = ctx->bel;
   R.V = 0; R.on_host = false;
   double* d_dist_cm;
@@ -1408,98 +1489,33 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
   CUDA_TRY(ctx, cudaMemcpyAsync(d_colpos, colpos.data(), (size_t)B * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_col_belief, col_belief.data(), (size_t)Bp * 4, cudaMemcpyHostToDevice, st));
   CUDA_TRY(ctx, cudaMemcpyAsync(d_cmask, cmask.data(), cmask.size() * 8, cudaMemcpyHostToDevice, st));
-  SfGraph sfg = {};
-  if (!cols) {   // Morton numbering + transposed adjacency with edge validity ids (sssp_frontier.cu)
-    int32_t rc = sf_build_graph(ctx, d_row, d_col, d_evid, d_xy, V, E, &sfg, st);
-    if (rc) return rc;
-  }
-  double* d_table = cols ? d_dist_cm : d_table_m;
-  fill_inf_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(d_table, V * (int64_t)Bp);
-  LAUNCH_CHECK(ctx);
-  if (!zero_idx.empty()) {
-    CUDA_TRY(ctx, cudaMemcpyAsync(d_zero, zero_idx.data(), zero_idx.size() * 8, cudaMemcpyHostToDevice, st));
-    if (cols) scatter_zero_kernel<<<div_up((int64_t)zero_idx.size(), 256), 256, 0, st>>>(d_table, d_zero, (int64_t)zero_idx.size());
-    else scatter_zero_perm_kernel<<<div_up((int64_t)zero_idx.size(), 256), 256, 0, st>>>(d_table, d_zero, (int64_t)zero_idx.size(), sfg.perm, V);
-    LAUNCH_CHECK(ctx);
-  }
-  edge_cost_kernel<<<div_up(V * 32, 256), 256, 0, st>>>(d_row, d_col, (const double2*)d_xy, V, d_cost);
-  LAUNCH_CHECK(ctx);
-  BeliefDev gd = {d_row, d_col, d_evid, d_cost, d_nvid, d_nset, d_compat, succ.succ_ptr, succ.succ_b, succ.succ_p, V, B, n_validities};
+  BeliefDev gd = {d_row, d_col, d_evid, nullptr, d_nvid, d_nset, d_compat, succ.succ_ptr, succ.succ_b, succ.succ_p, V, B, n_validities};
   const int blocks = div_up(V * (int64_t)B, 256);
   belief_type_kernel<<<blocks, 256, 0, st>>>(gd, d_type, d_colpos, d_type_cm);
   LAUNCH_CHECK(ctx);
-  if (cols) {
-    int32_t rc = colsolve_pack(ctx, d_row, d_col, d_evid, d_cost, V, E, d_rs, d_ce, d_cost_t, d_cursor, st);
+  ValueColumns vc = {};
+  vc.kind = COLSOLVE_BELIEF; vc.row = d_row; vc.col = d_col; vc.xy = d_xy; vc.V = V; vc.E = E; vc.evid = d_evid; vc.n_validities = n_validities;
+  vc.layout = &lay;
+  ColSolveArgs& ca = vc.cs;
+  ca.V = (int32_t)V; ca.ld = V; ca.dist_cm = d_dist_cm; ca.cmask = d_cmask; ca.nvid = d_nvid; ca.type_cm = d_type_cm; ca.node_set = d_nset;
+  ca.col_belief = d_col_belief; ca.succ_ptr = succ.succ_ptr; ca.succ_col = succ.succ_col; ca.succ_p = succ.succ_p; ca.B = B;
+  {
+    int32_t rc = value_columns_prepare(ctx, vc, fin, st);
     if (rc) return rc;
-    CUDA_TRY(ctx, cudaMemsetAsync(d_changed, 0, 16, st));
   }
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
   t1 = now_ms(); ph[1] = t1 - t0; t0 = t1;
+  // porrt_ctx_last_phase_ms: [0] device ms of the backups (all levels), [1] edge records / (parent, column) pairs worked through
   int sweeps = 0;
-  if (cols) {
-    // One launch per level; the CTAs of a level solve their columns on chip to the fixed point (colsolve.cu).  With a communicator
-    // (SURVEY 8(f) rank 2) the columns of a level are sharded over the ranks and all-gathered before the next level reads them.
-    ColSolveArgs ca = {};
-    ca.row_start = d_rs; ca.cost = d_cost_t; ca.ce = d_ce; ca.V = (int32_t)V; ca.ld = V; ca.dist_cm = d_dist_cm; ca.cmask = d_cmask;
-    ca.nvid = d_nvid; ca.type_cm = d_type_cm; ca.node_set = d_nset; ca.col_belief = d_col_belief; ca.succ_ptr = succ.succ_ptr;
-    ca.succ_col = succ.succ_col; ca.succ_p = succ.succ_p; ca.B = B; ca.sweeps_out = d_changed;
-    ca.offers_out = (unsigned long long*)(d_changed + 2);
-    tstart(ctx);
-    for (const Level& L : levels) {
-      int64_t a2 = 0, b2 = L.n_real;
-      if (sharded) comm_shard_range(L.n_real, ctx->comm_rank, ctx->comm_world, &a2, &b2);
-      const int mine = L.lo + (sharded ? ctx->comm_rank * L.per : 0);
-      int32_t rc = colsolve_level(ctx, ca, COLSOLVE_BELIEF, mine, mine + (int)(b2 - a2), st);
-      if (rc) return rc;
-      if (sharded) {
-        std::vector<int64_t> off(ctx->comm_world + 1);
-        for (int r = 0; r <= ctx->comm_world; ++r) off[r] = (int64_t)(L.lo + r * L.per) * V * 8;   // equal shards: one ncclAllGather
-        rc = comm_all_gatherv_dev(ctx, nullptr, d_dist_cm, off.data(), st);
-        if (rc) return rc;
-      }
-    }
-    tmark(ctx);
-    unsigned long long offers = 0;
-    CUDA_TRY(ctx, cudaMemcpyAsync(&sweeps, d_changed, 4, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaMemcpyAsync(&offers, d_changed + 2, 8, cudaMemcpyDeviceToHost, st));
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    tfinish(ctx);   // porrt_ctx_last_phase_ms: [0] device ms of the column solver (all levels), [1] edge records it worked through
-    ctx->last_ms[1] = (double)offers; ctx->n_last = 2;
-  } else {
-    // The same levels through the frontier relaxation over global memory (sssp_frontier.cu): a level's columns get their initial
-    // values (finals, Observation values from the finished levels, sign bit on everything that is not an Action node) and are
-    // relaxed together; shards and exchange as above.  The table is kept in Morton numbering until the end.
-    double offers_total = 0.0;
-    tstart(ctx);
-    for (const Level& L : levels) {
-      int64_t a2 = 0, b2 = L.n_real;
-      if (sharded) comm_shard_range(L.n_real, ctx->comm_rank, ctx->comm_world, &a2, &b2);
-      const int mine = L.lo + (sharded ? ctx->comm_rank * L.per : 0), n_mine = (int)(b2 - a2);
-      if (n_mine > 0) {
-        belief_level_init_kernel<<<div_up((int64_t)n_mine * V, 256), 256, 0, st>>>(V, B, mine, mine + n_mine, sfg.order, d_type_cm, d_nvid, d_nset,
-                                                                                    d_col_belief, succ.succ_ptr, succ.succ_col, succ.succ_p, d_cmask, d_table_m);
-        LAUNCH_CHECK(ctx);
-        int32_t rounds = 0;
-        double offers = 0.0;
-        int32_t rc = sf_relax(ctx, sfg, d_table_m + (int64_t)mine * V, n_mine, d_cmask + (int64_t)mine * 4, &rounds, &offers, st);
-        if (rc) return rc;
-        sweeps = std::max(sweeps, (int)rounds);
-        offers_total += offers;
-      }
-      if (sharded) {
-        std::vector<int64_t> off(ctx->comm_world + 1);
-        for (int r = 0; r <= ctx->comm_world; ++r) off[r] = (int64_t)(L.lo + r * L.per) * V * 8;
-        int32_t rc = comm_all_gatherv_dev(ctx, nullptr, d_table_m, off.data(), st);
-        if (rc) return rc;
-      }
-    }
-    tmark(ctx);
-    belief_unpermute_kernel<<<div_up((int64_t)Bp * V, 256), 256, 0, st>>>(d_table_m, sfg.perm, V, Bp, d_dist_cm);
-    LAUNCH_CHECK(ctx);
-    CUDA_TRY(ctx, cudaStreamSynchronize(st));
-    tfinish(ctx);
-    ctx->last_ms[1] = offers_total; ctx->n_last = 2;
+  double offers = 0.0;
+  tstart(ctx);
+  {
+    int32_t rc = value_columns_solve(ctx, vc, &sweeps, &offers, st);
+    if (rc) return rc;
   }
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  tfinish(ctx);
+  ctx->last_ms[1] = offers; ctx->n_last = 2;
   t1 = now_ms(); ph[2] = t1 - t0; t0 = t1;
   // results: retained for porrt_extract_policy / porrt_belief_result; to the caller if asked for
   R.V = V; R.B = B; R.n_worlds = nw; R.n_validities = n_validities;

@@ -1,7 +1,8 @@
-// sssp_frontier.cu -- world-view shortest paths on roadmaps that do not fit the on-chip column solver (colsolve.cu): a
-// label-correcting FRONTIER relaxation over the value table in global memory.
+// sssp_frontier.cu -- value columns on roadmaps that do not fit the on-chip column solver (colsolve.cu): a label-correcting
+// FRONTIER relaxation over the value table in global memory.  graph.cu's value-column driver runs it for world and belief columns.
 //
-// Reference: dijkstra over PTOGraphWorldView, one problem per world (pto_graph.rs:245-303, qmdp_policy_extractor.rs:23-35).
+// Reference: dijkstra over PTOGraphWorldView, one problem per world (pto_graph.rs:245-303, qmdp_policy_extractor.rs:23-35), and
+// conditional_dijkstra's Action nodes, one problem per belief of a level (belief_graph.rs:89-182).
 //
 // At PRM scale (1e6 nodes, 5.3e7 directed edges, 64 worlds) a Bellman-Ford sweep touches E * W = 3.4e9 (edge, world) pairs and the
 // roadmap's diameter is several hundred hops: the order-free Jacobi sweeps of round 1 were never run at that size.  Here only
@@ -92,17 +93,6 @@ __global__ void sf_fill_kernel(const int64_t* __restrict__ row_ptr, const int32_
   }
 }
 
-// dist[w][pos] = +inf, or -inf where the node is invalid in world wlo + w (PTOGraphWorldView::parents filters by the parent node)
-__global__ void sf_init_kernel(const int32_t* __restrict__ node_vid, const uint64_t* __restrict__ validities, int mask_words,
-                               const uint32_t* __restrict__ order, int64_t V, int W, int wlo, double* __restrict__ dist) {
-  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= V * W) return;
-  const int w = (int)(t / V);
-  const int64_t pos = t - (int64_t)w * V;
-  const int wg = wlo + w;
-  const bool ok = node_vid ? ((validities[(int64_t)node_vid[order[pos]] * mask_words + (wg >> 6)] >> (wg & 63)) & 1) != 0 : true;
-  dist[t] = ok ? INFINITY : -INFINITY;
-}
 struct SfArgs {
   const int64_t* row_t; const int32_t* col_t; const double* cost_t;
   const uint16_t* evid_t;         // validity id of the transposed record's edge (nullable)
@@ -252,14 +242,6 @@ __global__ void sf_sum_kernel(const double* __restrict__ x, int64_t n, double* _
   if ((threadIdx.x & 31) == 0) atomicAdd(out, s);   // only the order of magnitude matters (a schedule parameter, not a result)
 }
 
-__global__ void sf_out_kernel(const double* __restrict__ dist /* [W][V] Morton numbering */, const int32_t* __restrict__ perm, int64_t V, int W,
-                              double* __restrict__ out /* [W][V] caller's numbering */) {
-  const int64_t t = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= V * W) return;
-  const int w = (int)(t / V);
-  const int64_t u = t - (int64_t)w * V;
-  out[t] = fabs(dist[(int64_t)w * V + perm[u]]);
-}
 // ---- seeding: every entry that holds a finite value (finals, Observation values) is a source
 __global__ void sf_seed_all_kernel(SfArgs a) {
   const int64_t v = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
@@ -281,13 +263,6 @@ __global__ void sf_seed_all_kernel(SfArgs a) {
     base = __shfl_sync(0xffffffffu, base, 0);
     if (any) a.list[0][base + __popc(fm & ((1u << lane) - 1u))] = (int32_t)v;
   }
-}
-__global__ void sf_zero_finals_kernel(const int32_t* __restrict__ fin_node, const int32_t* __restrict__ fin_world, int64_t n,
-                                      const int32_t* __restrict__ perm, int64_t V, double* __restrict__ dist) {
-  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
-  if (i >= n) return;
-  double* d = dist + (int64_t)fin_world[i] * V + perm[fin_node[i]];
-  *d = (__double_as_longlong(*d) < 0) ? -0.0 : 0.0;   // (several finals may name the same entry: same value)
 }
 }  // namespace
 
@@ -347,9 +322,9 @@ int32_t sf_build_graph(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_co
   return PORRT_OK;
 }
 
-// The frontier state of sf_relax over V nodes and W columns in ws_state; with `table`, a [W][V] value table behind it.  Every user of
-// ws_state carves through this layout, so sf_relax never moves a table its caller placed there.
-static void sf_state_layout(Carve& c, SfArgs& a, int64_t V, int32_t W, double** table) {
+// The frontier state of sf_relax over V nodes and W columns, at the front of ws_state.  Its size grows with W, so state for fewer
+// columns fits in the space reserved for more.
+static void sf_state_layout(Carve& c, SfArgs& a, int64_t V, int32_t W) {
   const int words = (W + 63) / 64;
   a.pair_cap = (int32_t)std::min<int64_t>(V * (int64_t)W, std::max<int64_t>(4 << 20, 4 * V));
   a.dirty[0] = c.take<unsigned long long>((size_t)V * words); a.dirty[1] = c.take<unsigned long long>((size_t)V * words);
@@ -361,19 +336,23 @@ static void sf_state_layout(Carve& c, SfArgs& a, int64_t V, int32_t W, double** 
   a.min_far = c.take<unsigned long long>(4);
   a.pair_count = c.take<int32_t>(4);
   a.pairs = c.take<int2>(a.pair_cap);
-  if (table) *table = c.take<double>((size_t)V * W);
+}
+void sf_state_reserve(Carve& c, int64_t V, int32_t W) {
+  SfArgs unused = {};
+  sf_state_layout(c, unused, V, W);
 }
 
 // Relaxes W value columns to their fixed point.  dist[w * V + pos] (Morton numbering) holds the initial values on entry -- +inf, the
 // sources' values, the sign bit on every entry that must not be relaxed -- and the result on exit (signs kept).  cmask (nullable):
-// [W][4] validity ids an edge must carry to be admissible in column w (needs g.evid_t).  Work space: ws_state.
+// [W][4] validity ids an edge must carry to be admissible in column w (needs g.evid_t).  Work space: ws_state, within
+// sf_state_reserve(V, W).
 int32_t sf_relax(porrt_ctx* ctx, const SfGraph& g, double* dist, int32_t W, const uint64_t* cmask, int32_t* out_rounds, double* out_offers,
                  cudaStream_t st) {
   const int64_t V = g.V;
   const int words = (W + 63) / 64;
   if (W <= 0) { if (out_rounds) *out_rounds = 0; if (out_offers) *out_offers = 0.0; return PORRT_OK; }
   SfArgs a = {};
-  CUDA_TRY(ctx, carve(ctx->ws_state, [&](Carve& c) { sf_state_layout(c, a, V, W, nullptr); }));
+  CUDA_TRY(ctx, carve(ctx->ws_state, [&](Carve& c) { sf_state_layout(c, a, V, W); }));
   a.row_t = g.row_t; a.col_t = g.col_t; a.cost_t = g.cost_t; a.evid_t = g.evid_t; a.cmask = cmask; a.V = V; a.W = W; a.words = words;
   a.dist = dist; a.delta = g.delta;
   CUDA_TRY(ctx, cudaMemsetAsync(a.dirty[0], 0, 2 * (((size_t)V * words * 8 + 15) & ~(size_t)15), st));
@@ -408,31 +387,5 @@ int32_t sf_relax(porrt_ctx* ctx, const SfGraph& g, double* dist, int32_t W, cons
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
     *out_offers = (double)off;
   }
-  return PORRT_OK;
-}
-
-// plan_qmdp's world columns.  All pointers are device pointers.  fin_node / fin_world: the finals of the worlds [wlo, wlo + W) as
-// (node, local world) pairs.  out_wv receives rows [0, W) of the [world][node] table.  Work space: ws_state (the value table behind
-// sf_relax's state) and sf_build_graph's.
-int32_t sssp_frontier_run(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_col, const double* d_xy, int64_t V, int64_t E,
-                          const int32_t* d_node_vid, const uint64_t* d_validities, int32_t mask_words, int32_t wlo, int32_t W,
-                          const int32_t* d_fin_node, const int32_t* d_fin_world, int64_t n_fin, double* d_out_wv, int32_t* out_rounds,
-                          double* out_offers, cudaStream_t st) {
-  SfGraph g;
-  int32_t rc = sf_build_graph(ctx, d_row, d_col, nullptr, d_xy, V, E, &g, st);
-  if (rc) return rc;
-  double* dist;
-  SfArgs unused = {};
-  CUDA_TRY(ctx, carve(ctx->ws_state, [&](Carve& c) { sf_state_layout(c, unused, V, W, &dist); }));
-  sf_init_kernel<<<div_up(V * (int64_t)W, 256), 256, 0, st>>>(d_node_vid, d_validities, mask_words, g.order, V, W, wlo, dist);
-  LAUNCH_CHECK(ctx);
-  if (n_fin > 0) {
-    sf_zero_finals_kernel<<<div_up(n_fin, 256), 256, 0, st>>>(d_fin_node, d_fin_world, n_fin, g.perm, V, dist);
-    LAUNCH_CHECK(ctx);
-  }
-  rc = sf_relax(ctx, g, dist, W, nullptr, out_rounds, out_offers, st);
-  if (rc) return rc;
-  sf_out_kernel<<<div_up(V * (int64_t)W, 256), 256, 0, st>>>(dist, g.perm, V, W, d_out_wv);
-  LAUNCH_CHECK(ctx);
   return PORRT_OK;
 }

@@ -6,9 +6,9 @@
 Every rank holds two contexts on its GPU: `ctx` with an NCCL communicator (sharded porrt_prm_build / porrt_sssp_worlds,
 porrt_comm_all_gather_dev) and `solo` without one (the single-GPU result).  Checks, all bit-exact:
   1. sharded PRM build == single-GPU PRM build == the oracle's PRM (CSR in the reference's insertion order), on every rank
-  2. sharded plan_qmdp dist rows == single-GPU == oracle
+  2. sharded plan_qmdp dist rows == single-GPU == oracle, through both value-backup schedules (on chip / frontier)
   3. all-gathered per-shard edge validity ids / world masks == the whole batch evaluated on one GPU
-  4. belief-space value backups with the columns of every level sharded over the ranks == single GPU == oracle
+  4. belief-space value backups with the columns of every level sharded over the ranks == single GPU == oracle, both schedules
 --big adds timings at the c5 shape (8192^2 map, V = 1e6 PRM build) and prints them as JSON on rank 0.
 The oracle is used here as the checker only.
 """
@@ -86,12 +86,14 @@ def main():
     keep = nvid >= 0
     nvid = np.where(keep, nvid, 0).astype(np.int32)
     vw = smap.world_validities_words()
-    for n_fin_worlds in (8, 3):
+    for force, n_fin_worlds in ((f, k) for f in (0, 1) for k in (8, 3)):   # force: the sharded run on the frontier relaxation
         finals = [list(range(k, n, 97 + 13 * k))[:5] for k in range(n_fin_worlds)]
+        ctx.set_option(P.OPT_FORCE_GLOBAL_SWEEPS, force)
         a, _ = P.dijkstra_worlds(ctx, got.row_ptr, got.col, got.states, nvid, vw, finals)
         b, _ = P.dijkstra_worlds(solo, got.row_ptr, got.col, got.states, nvid, vw, finals)
         np.testing.assert_array_equal(a, b)
         assert np.isfinite(a).any()
+    ctx.set_option(P.OPT_FORCE_GLOBAL_SWEEPS, 0)
     report["qmdp_worlds"] = 8
 
     # ---- 3. per-shard edge validity + device all-gather
@@ -125,16 +127,20 @@ def main():
         assert pto.grow_graph((0.0, -0.9), O.SquareGoal(goals, 0.05), 0.1, 2.0, nmin, 100000) == 0
         bxy, bnvid, brp, bcol, bev = pto.graph.export(0)
         fin_ids, fin_bits = pto.reach.finals()
-        plans = []
+        bms = []
         for c in (ctx, solo):
             bm = P.MapShelfDomain(c, socc, [-1.0, -1.0], [1.0, 1.0])
             bm.add_zones(szones, 0.5)
-            plans.append(P.plan_belief_space(bm, brp, bcol, bev, bxy, bnvid, [1.0 / Z] * Z, fin_ids, P.words_from_bits(fin_bits)))
-        np.testing.assert_array_equal(plans[0].dist, plans[1].dist)
-        np.testing.assert_array_equal(plans[0].type, plans[1].type)
-        np.testing.assert_array_equal(plans[0].policy_node, plans[1].policy_node)
+            bms.append(bm)
         pto.build_belief_graph([1.0 / Z] * Z)
-        np.testing.assert_array_equal(plans[0].dist.reshape(-1), pto.compute_expected_costs_to_goals())
+        for force in (0, 1):                       # the sharded run on chip, then on the frontier relaxation
+            ctx.set_option(P.OPT_FORCE_GLOBAL_SWEEPS, force)
+            plans = [P.plan_belief_space(bm, brp, bcol, bev, bxy, bnvid, [1.0 / Z] * Z, fin_ids, P.words_from_bits(fin_bits)) for bm in bms]
+            np.testing.assert_array_equal(plans[0].dist, plans[1].dist)
+            np.testing.assert_array_equal(plans[0].type, plans[1].type)
+            np.testing.assert_array_equal(plans[0].policy_node, plans[1].policy_node)
+            np.testing.assert_array_equal(plans[0].dist.reshape(-1), pto.compute_expected_costs_to_goals())
+        ctx.set_option(P.OPT_FORCE_GLOBAL_SWEEPS, 0)
     report["belief_vi_sharded_levels"] = True
     for m in (pmap, smap):      # the belief problems replaced the ctx maps
         m.add_zones(zones, 0.3)
