@@ -240,12 +240,12 @@ __global__ void colsolve_fill_kernel(const int64_t* __restrict__ row_ptr, const 
 }
 
 template <int C, int MODE>
-cudaError_t launch_one(const ColSolveArgs& a, int col_lo, int col_hi, size_t smem, cudaStream_t st) {
-  static bool configured = false;   // per instantiation
-  if (!configured) {
+cudaError_t launch_one(const porrt_ctx* ctx, const ColSolveArgs& a, int col_lo, int col_hi, size_t smem, cudaStream_t st) {
+  static bool configured[16] = {};   // per instantiation and device: the attribute holds for the current device only
+  if (!configured[ctx->device & 15]) {
     cudaError_t e = cudaFuncSetAttribute(colsolve_push_kernel<C, MODE>, cudaFuncAttributeMaxDynamicSharedMemorySize, COLSOLVE_SMEM_MAX);
     if (e != cudaSuccess) return e;
-    configured = true;
+    configured[ctx->device & 15] = true;
   }
   const int n_cta = (col_hi - col_lo + C - 1) / C;
   colsolve_push_kernel<C, MODE><<<n_cta, COLSOLVE_THREADS, smem, st>>>(a, col_lo, col_hi);
@@ -289,17 +289,17 @@ int32_t colsolve_level(porrt_ctx* ctx, const ColSolveArgs& a, int mode, int col_
   cudaError_t e;
   if (mode == COLSOLVE_BELIEF) {
     switch (Cc) {
-      case 1: e = launch_one<1, COLSOLVE_BELIEF>(a, col_lo, col_hi, smem, st); break;
-      case 2: e = launch_one<2, COLSOLVE_BELIEF>(a, col_lo, col_hi, smem, st); break;
-      case 4: e = launch_one<4, COLSOLVE_BELIEF>(a, col_lo, col_hi, smem, st); break;
-      default: e = launch_one<6, COLSOLVE_BELIEF>(a, col_lo, col_hi, smem, st); break;
+      case 1: e = launch_one<1, COLSOLVE_BELIEF>(ctx, a, col_lo, col_hi, smem, st); break;
+      case 2: e = launch_one<2, COLSOLVE_BELIEF>(ctx, a, col_lo, col_hi, smem, st); break;
+      case 4: e = launch_one<4, COLSOLVE_BELIEF>(ctx, a, col_lo, col_hi, smem, st); break;
+      default: e = launch_one<6, COLSOLVE_BELIEF>(ctx, a, col_lo, col_hi, smem, st); break;
     }
   } else {
     switch (Cc) {
-      case 1: e = launch_one<1, COLSOLVE_WORLD>(a, col_lo, col_hi, smem, st); break;
-      case 2: e = launch_one<2, COLSOLVE_WORLD>(a, col_lo, col_hi, smem, st); break;
-      case 4: e = launch_one<4, COLSOLVE_WORLD>(a, col_lo, col_hi, smem, st); break;
-      default: e = launch_one<6, COLSOLVE_WORLD>(a, col_lo, col_hi, smem, st); break;
+      case 1: e = launch_one<1, COLSOLVE_WORLD>(ctx, a, col_lo, col_hi, smem, st); break;
+      case 2: e = launch_one<2, COLSOLVE_WORLD>(ctx, a, col_lo, col_hi, smem, st); break;
+      case 4: e = launch_one<4, COLSOLVE_WORLD>(ctx, a, col_lo, col_hi, smem, st); break;
+      default: e = launch_one<6, COLSOLVE_WORLD>(ctx, a, col_lo, col_hi, smem, st); break;
     }
   }
   ctx->launches += 1;
