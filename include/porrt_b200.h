@@ -431,6 +431,35 @@ int32_t porrt_pto_grow_batch(porrt_ctx* ctx, int32_t n_roadmaps, const uint64_t*
 int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
                                 int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks);
 
+/* ------------------------------------------------------------------ RRT* tree growth on the device (pto_grow.cu, DESIGN.md 3.9)
+ * RRT::grow_tree (rrt.rs:102-174) with sample() (:176-181) on the uploaded map, as ONE call per batch of trees; tree t samples with
+ * Pcg64::seed_from_u64(sampler_seeds[t]), one continuous stream in [low, up): iteration i % 100 == 0 takes goal_example(0) and draws
+ * nothing.  The 1-NN is unfiltered; the radius is heuristic_radius(nodes before the new one); the neighbours are the radius hits in
+ * kd pre-order whose edge hit -> new is valid, else [nearest] unchecked; the parent is the first minimum of dist + norm2; every other
+ * neighbour is rewired when that is strictly shorter (no propagation).  A node is final when some goal has norm1 < goal_max_dist;
+ * loop: i < n_iter_min || (no finals && i < n_iter_max).  The start is not checked: node 0, parent -1, dist 0.
+ * out_sizes[3 n] = iterations, nodes, finals per tree; out_status[t] = 0 when tree t has a final, 1 when it has none, PORRT_ERR_PANIC
+ * when a state check, or the first edge check in kd order among the hits within the radius, panics: then out_panic_code[t]
+ * (nullable [n]) is its PORRT_PANIC_* code and out_sizes[3 t] that iteration.  A panic stops only its own tree; the call returns
+ * PORRT_OK.  out_counters (nullable [4 n]): porrt_pto_grow_batch's window counters.  Argument errors as porrt_pto_grow_batch (no map,
+ * overlapping goal masks, low >= up; n_trees outside 1 .. PORRT_PTO_MAX_ROADMAPS or more trees than free memory holds at their
+ * starting size: PORRT_ERR_INVALID_ARG; out of memory while growing: PORRT_ERR_CUDA).  The trees stay on the device until
+ * porrt_rrt_fetch_tree; RRT and PTO growth keep separate state, neither changes what the other's fetch returns. */
+int32_t porrt_rrt_grow_batch(porrt_ctx* ctx, int32_t n_trees, const uint64_t* sampler_seeds, const double start[2], const double low[2],
+                             const double up[2], const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
+                             double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes,
+                             int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters);
+/* porrt_rrt_grow_batch for one seed (the batch of one through the same code): out_sizes[3], *out_status, out_counters[4]; a panic
+ * also returns PORRT_ERR_PANIC */
+int32_t porrt_rrt_grow(porrt_ctx* ctx, uint64_t sampler_seed, const double start[2], const double low[2], const double up[2],
+                       const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist, double max_step,
+                       double search_radius, int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status,
+                       int32_t* out_panic_code, int64_t* out_counters);
+/* tree t of the last RRT growth on this ctx, every pointer nullable: states xy[2V], parent[V] (-1 at the root) and dist_from_root[V]
+ * as they stand after the last rewire, final node ids in the order they were found.  PORRT_ERR_INVALID_ARG when nothing has been
+ * grown, t is out of range, or tree t panicked. */
+int32_t porrt_rrt_fetch_tree(porrt_ctx* ctx, int32_t t, double* out_xy, int32_t* out_parent, double* out_dist, int64_t* out_final_ids);
+
 /* ------------------------------------------------------------------ multi-GPU (SURVEY.md 8(e))
  * The reference is single-threaded and has no distributed code; what shards are its independent units (edge checks,
  * radius / NN queries, the worlds of plan_qmdp).  One process and one ctx per GPU; map and vertex set replicated.

@@ -949,6 +949,82 @@ class PTOBatch:
         return _roadmap_finals(self._fetcher(r), self.sizes[r], self.fns)
 
 
+class RRT:
+    """src/rrt.rs RRT::grow_tree on the device (porrt_rrt_grow): `fns` is an uploaded Map / MapShelfDomain, the sampler is seeded
+    with `seed`.  The tree stays on the device until tree() asks.  After grow_tree: n_it, sizes = (iterations, nodes, finals),
+    counters = (windows, iterations re-speculated, conflicts by nearest neighbour, conflicts by radius / kd slot)."""
+
+    def __init__(self, fns, low, up, seed=0):
+        self.fns, self.ctx = fns, fns.ctx
+        self.low, self.up, self.seed = _f64(low), _f64(up), int(seed)
+        self.n_it, self.sizes, self.counters = 0, (0, 0, 0), (0, 0, 0, 0)
+
+    def grow_tree(self, start, goal, max_step, search_radius, n_iter_min, n_iter_max):
+        """-> 0 when the tree has a final node, 1 when it has none (rrt.rs: "No path found!"); PorrtError where a state or edge check
+        panics (e.code == 5, e.panic_code = its code, n_it = its iteration)"""
+        self.fns._need()
+        c = self.ctx
+        sizes, counters = np.zeros(3, np.int64), np.zeros(4, np.int64)
+        status, panic = C.c_int32(), C.c_int32()
+        rc = c.lib.porrt_rrt_grow(c.h, self.seed, _p(_f64(start)), _p(self.low), _p(self.up), _p(goal.goals), _p(goal.masks), len(goal.goals),
+                                  goal.max_dist, float(max_step), float(search_radius), int(n_iter_min), int(n_iter_max), _p(sizes),
+                                  C.byref(status), C.byref(panic), _p(counters))
+        self.n_it, self.sizes, self.counters = int(sizes[0]), tuple(int(x) for x in sizes), tuple(int(x) for x in counters)
+        if rc:
+            err = PorrtError(rc, (c.lib.porrt_last_error(c.h) or b"").decode())
+            err.panic_code = panic.value
+            raise err
+        return int(status.value)
+
+    def tree(self):
+        """-> states[V, 2], parent[V] (-1 at the root), dist_from_root[V], final node ids in the order they were found"""
+        return _fetch_tree(self.ctx, 0, self.sizes)
+
+
+class RRTBatch:
+    """RRT::grow_tree for one tree per seed in `seeds`, all in one device call (porrt_rrt_grow_batch); map, start, goal and parameters
+    are shared.  Tree t is what RRT(fns, low, up, seeds[t]) grows, counters included.  After grow_tree the attributes n_it[R],
+    sizes[R, 3], counters[R, 4] and panic_code[R] hold one row per tree; tree(t) reads tree t.  The batch replaces the context's
+    last RRT growth; PTO growth on the same context is kept apart."""
+
+    def __init__(self, fns, low, up, seeds):
+        self.fns, self.ctx = fns, fns.ctx
+        self.low, self.up = _f64(low), _f64(up)
+        self.seeds = np.ascontiguousarray(np.asarray(seeds, dtype=np.uint64).reshape(-1))
+        R = len(self.seeds)
+        self.n_it, self.panic_code = np.zeros(R, np.int64), np.zeros(R, np.int32)
+        self.sizes, self.counters = np.zeros((R, 3), np.int64), np.zeros((R, 4), np.int64)
+
+    def __len__(self):
+        return len(self.seeds)
+
+    def grow_tree(self, start, goal, max_step, search_radius, n_iter_min, n_iter_max):
+        """-> status[R]: 0 when tree t has a final node, 1 when it has none, 5 (PORRT_ERR_PANIC) where its growth panics (its code in
+        panic_code[t], its iteration in n_it[t]).  Raises PorrtError when the call as a whole fails (bad arguments, no map,
+        overlapping goal masks, low >= up, too many trees)."""
+        self.fns._need()
+        c = self.ctx
+        R = len(self.seeds)
+        status = np.zeros(R, np.int32)
+        rc = c.lib.porrt_rrt_grow_batch(c.h, R, _p(self.seeds), _p(_f64(start)), _p(self.low), _p(self.up), _p(goal.goals), _p(goal.masks),
+                                        len(goal.goals), goal.max_dist, float(max_step), float(search_radius), int(n_iter_min),
+                                        int(n_iter_max), _p(self.sizes), _p(status), _p(self.panic_code), _p(self.counters))
+        self.n_it = self.sizes[:, 0].copy()
+        c.check(rc)
+        return status
+
+    def tree(self, t):
+        """RRT.tree of tree t"""
+        return _fetch_tree(self.ctx, t, self.sizes[t])
+
+
+def _fetch_tree(ctx, t, sizes):
+    _, V, F = (int(x) for x in sizes)
+    xy, parent, dist, finals = np.empty((V, 2)), np.empty(V, np.int32), np.empty(V), np.empty(F, np.int64)
+    ctx.check(ctx.lib.porrt_rrt_fetch_tree(ctx.h, int(t), _p(xy), _p(parent), _p(dist), _p(finals)))
+    return xy, parent, dist, finals
+
+
 # the arrays of a device-grown roadmap; fetch(xy, node_vid, row_ptr, col, edge_vid, reach, final_ids, final_masks) is
 # porrt_pto_fetch or porrt_pto_fetch_roadmap, sizes = (iterations, V, E, finals)
 def _roadmap_graph_arrays(fetch, sizes):

@@ -224,6 +224,8 @@ struct porrt_ctx {
 
   // ---- last PTO growth (pto_grow.cu): the roadmap stays on the device until porrt_pto_fetch
   struct PtoGrow* pto = nullptr;
+  // ---- last RRT growth (pto_grow.cu, the same machinery): the trees stay on the device until porrt_rrt_fetch_tree
+  struct PtoGrow* rrt = nullptr;
 
   // ---- multi-GPU (comm.cu): NCCL communicator bound at run time; world 1 = no communicator
   void* comm = nullptr;

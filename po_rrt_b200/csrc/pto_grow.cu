@@ -21,6 +21,9 @@
 // porrt_pto_grow_batch grows R roadmaps that differ only in their sampler seed through the same kernels: each keeps its own state
 // (PtoRoad, control block r), the kernels find roadmap r's pointers in device arrays of descriptors, a speculate launch covers
 // every window slot of every roadmap and a commit launch is one CTA per roadmap.  porrt_pto_grow is the batch of one.
+//
+// porrt_rrt_grow_batch grows RRT::grow_tree (rrt.rs:102-174) trees through the same speculation and host loop, with its own commit
+// (choose-parent and rewire run in order there; DESIGN.md 3.9).  porrt_rrt_grow is its batch of one.
 #include <algorithm>
 #include <cmath>
 #include <climits>
@@ -52,24 +55,26 @@ struct PtoRoad {   // one roadmap of a batch: its state, its samples, its specul
   DevBuf samples, worlds;                     // iteration i (1-based) at [i - 1]
   DevBuf spec;                                // per-slot speculation results + hit lists [PG_WMAX * node_cap]
   DevBuf csr_row, csr_col, csr_vid;           // the assembled roadmap
+  DevBuf tparent, dist;                       // RRT trees only: the tree parent (-1 at the root) and dist_from_root [node_cap]
   int64_t node_cap = 0, edge_cap = 0;
-  // the last result (porrt_pto_fetch_roadmap)
+  // the last result (porrt_pto_fetch_roadmap / porrt_rrt_fetch_tree)
   bool have = false;
   int64_t V = 0, E = 0, n_finals = 0;
-  DevBuf* bufs[23] = {&xy, &node_vid, &reach, &child, &parent, &depth, &key, &final_idx, &gain, &epoch, &edge_off, &ecnt, &fin_ids,
-                      &fin_goal, &fin_acc, &log_nbr, &log_vid, &samples, &worlds, &spec, &csr_row, &csr_col, &csr_vid};
+  DevBuf* bufs[25] = {&xy, &node_vid, &reach, &child, &parent, &depth, &key, &final_idx, &gain, &epoch, &edge_off, &ecnt, &fin_ids,
+                      &fin_goal, &fin_acc, &log_nbr, &log_vid, &samples, &worlds, &spec, &csr_row, &csr_col, &csr_vid, &tparent, &dist};
   PtoRoad() = default;
   PtoRoad(const PtoRoad&) = delete;           // bufs points into this object
   size_t bytes() const { size_t s = 0; for (DevBuf* b : bufs) s += b->cap; return s; }
   void release() { for (DevBuf* b : bufs) b->release(); }
 };
 
-struct PtoGrow {
+struct PtoGrow {    // the state of the last PTO growth (ctx->pto) or of the last RRT growth (ctx->rrt), one road per seed
   std::vector<std::unique_ptr<PtoRoad>> roads;   // the roadmaps of the last batch; a single growth is the batch of one
   DevBuf radius;                                 // heuristic_radius(n) at [n]
   DevBuf goals, goal_masks;
   DevBuf ctl;                                    // control blocks, roadmap r at [r * C_N]
   DevBuf pg_desc, spec_desc, caps;               // PgDev / SpecDev of every roadmap; node cap, edge cap, samples drawn of each
+  DevBuf tree_desc;                              // RrtDev of every tree (RRT growth only)
   DevBuf work;                                   // CSR assembly work space, one roadmap at a time
   PinBuf ctl_host;                               // every control block, as the last look saw it
   std::vector<char> desc_host;                   // what pg_desc + spec_desc hold
@@ -79,15 +84,18 @@ struct PtoGrow {
   std::vector<uint64_t> goal_masks_host;
 };
 
-void pto_grow_release(porrt_ctx* ctx) {
-  PtoGrow* g = ctx->pto;
+static void grow_state_release(PtoGrow*& g) {
   if (!g) return;
   for (auto& r : g->roads) r->release();
-  DevBuf* all[] = {&g->radius, &g->goals, &g->goal_masks, &g->ctl, &g->pg_desc, &g->spec_desc, &g->caps, &g->work};
+  DevBuf* all[] = {&g->radius, &g->goals, &g->goal_masks, &g->ctl, &g->pg_desc, &g->spec_desc, &g->caps, &g->work, &g->tree_desc};
   for (DevBuf* b : all) b->release();
   g->ctl_host.release();
   delete g;
-  ctx->pto = nullptr;
+  g = nullptr;
+}
+void pto_grow_release(porrt_ctx* ctx) {   // the PTO and the RRT growth state
+  grow_state_release(ctx->pto);
+  grow_state_release(ctx->rrt);
 }
 
 // ------------------------------------------------------------------------------------------------ device
@@ -482,6 +490,168 @@ __global__ void pto_ctl_to_host_kernel(const int32_t* __restrict__ d, int n, vol
 }
 __global__ void pto_set_i64_kernel(int64_t* p, const int32_t* ctl, int idx) { *p = ctl[idx]; }
 
+// ------------------------------------------------------------------------------------------------ RRT* trees (DESIGN.md 3.9)
+// RRT::grow_tree (rrt.rs:102-174) runs through the same windows.  pto_speculate_kernel serves it unchanged: every node's reach word
+// is 1 (bit 0: committed), every world index is 0, so its 1-NN is the unfiltered one, and the radius table is shifted by one
+// (radius[n] = heuristic_radius(n - 1)), so radius[V + 1] is RRT's heuristic_radius(nodes before the new one).  Choose-parent and
+// rewire read and write only the tree parent and dist_from_root, which no geometric answer depends on: they run in the commit.
+struct RrtDev {    // one tree's own arrays, beside its PgDev (whose parent[] is the kd parent)
+  int32_t* tparent; double* dist;
+};
+
+// (value, index) arg-min over the block: the smallest value, the smallest index among equal values (blockDim.x = PG_COMMIT_THREADS)
+__device__ __forceinline__ void rrt_block_argmin(double& v, int32_t& k, double* shv, int32_t* shk) {
+  for (int o = 16; o; o >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, v, o);
+    const int32_t ok = __shfl_xor_sync(0xffffffffu, k, o);
+    if (ov < v || (ov == v && ok < k)) { v = ov; k = ok; }
+  }
+  __syncthreads();
+  if ((threadIdx.x & 31) == 0) { shv[threadIdx.x >> 5] = v; shk[threadIdx.x >> 5] = k; }
+  __syncthreads();
+  v = shv[0]; k = shk[0];
+  for (int w = 1; w < PG_COMMIT_THREADS / 32; ++w)
+    if (shv[w] < v || (shv[w] == v && shk[w] < k)) { v = shv[w]; k = shk[w]; }
+}
+
+// ---- commit: one CTA per tree walks its window in order, each iteration in the order of rrt.rs:110-172
+__global__ void __launch_bounds__(PG_COMMIT_THREADS) rrt_commit_kernel(const PgDev* __restrict__ gs, const SpecDev* __restrict__ ss,
+                                                                       const RrtDev* __restrict__ ts) {
+  const PgDev& g = gs[blockIdx.x];
+  const SpecDev& s = ss[blockIdx.x];
+  const RrtDev& t = ts[blockIdx.x];
+  __shared__ double sh_v[PG_COMMIT_THREADS / 32];
+  __shared__ int32_t sh_k[PG_COMMIT_THREADS / 32];
+  __shared__ int32_t conflict_nn, conflict_rad, panic_idx, sh_goal;
+  __shared__ double sh_dnew;
+  int32_t* ctl = g.ctl;
+  if (ctl[C_DONE]) return;
+  const int tid = threadIdx.x;
+  const int32_t it0 = ctl[C_IT], V0 = ctl[C_V], W = ctl[C_W];
+  const int32_t Weff = min(W, ctl[C_DRAWN] - it0);
+  if (Weff <= 0) return;                                     // waiting for samples
+  const int32_t wid = ctl[C_WINDOWS];
+  int32_t V = V0, nfin = ctl[C_NFIN], committed = 0, done = 0, stall = 0;
+  bool cut = false;
+  for (int b = 0; b < Weff; ++b) {
+    const int i = it0 + 1 + b;
+    const int32_t sv = s.svid[b];
+    const double2 q = s.q[b];
+    if (b > 0) {                                             // conditions (a)-(c); every node added in the window is committed
+      if (tid == 0) { conflict_nn = 0; conflict_rad = 0; }
+      __syncthreads();
+      const double2 smp = g.samples[i - 1];
+      const double dlim = s.nn_d[b] * (1.0 + 1e-14);
+      const double r = g.radius[V + 1];
+      for (int32_t j = V0 + tid; j < V; j += PG_COMMIT_THREADS) {
+        const double2 x = g.xy[j];
+        if (pg_norm2(x, smp) <= dlim) conflict_nn = 1;                   // (a)
+        if (sv >= 0 && pg_norm2(x, q) <= r) conflict_rad = 1;            // (b)
+      }
+      if (sv >= 0 && tid == 0 && g.child[s.slot[b]] >= 0) conflict_rad = 1;   // (c)
+      __syncthreads();
+      if (conflict_nn || conflict_rad) {
+        if (tid == 0) {
+          ctl[C_RESPEC] += Weff - b;
+          if (conflict_nn) ctl[C_CONF_NN] += 1; else ctl[C_CONF_RAD] += 1;
+        }
+        cut = true;
+        break;
+      }
+    }
+    if (sv < -1) { if (tid == 0) ctl[C_PANIC] = sv; done = 2; committed = b; break; }   // the state check panics
+    if (sv >= 0) {
+      if (V + 1 > ctl[C_NODE_CAP]) { stall = 1; break; }     // the host grows the buffers
+      const int32_t k_hits = s.n_hits[b];
+      const int32_t nw = V;
+      const double r = g.radius[V + 1];                        // heuristic_radius(nodes before the new one)
+      const int32_t* hid = s.hit_id + (size_t)b * s.hcap;
+      const double* hd = s.hit_d + (size_t)b * s.hcap;
+      const int32_t* hv = s.hit_vid + (size_t)b * s.hcap;
+      if (tid == 0) panic_idx = INT_MAX;
+      __syncthreads();
+      // 1. neighbours = the hits within the exact radius whose edge hit -> new is valid, kd order; 2. choose-parent: the first
+      // minimum of dist[c] + norm2(c, new) (Iterator::min_by); a thread visits its k in increasing order, so strict < keeps the first
+      double bv = INFINITY;
+      int32_t bk = INT_MAX;
+      for (int32_t k = tid; k < k_hits; k += PG_COMMIT_THREADS) {
+        if (hd[k] > r) continue;
+        const int32_t v = hv[k];
+        if (v < -1) atomicMin(&panic_idx, k);
+        if (v < 0) continue;
+        const double c = __dadd_rn(t.dist[hid[k]], hd[k]);
+        if (c < bv) { bv = c; bk = k; }
+      }
+      rrt_block_argmin(bv, bk, sh_v, sh_k);                    // ends with __syncthreads: panic_idx is final
+      if (panic_idx < INT_MAX) { if (tid == 0) ctl[C_PANIC] = hv[panic_idx]; done = 2; committed = b; break; }   // an edge check panics
+      if (tid == 0) {
+        int32_t par;
+        double dn;
+        if (bk == INT_MAX) { par = s.nn[b]; dn = __dadd_rn(t.dist[par], pg_norm2(g.xy[par], q)); }   // no neighbour: [nearest], unchecked
+        else { par = hid[bk]; dn = bv; }
+        t.tparent[nw] = par; t.dist[nw] = dn;
+        sh_dnew = dn;
+      }
+      __syncthreads();
+      // 3. rewire every other neighbour c when dist[new] + norm2(new, c) < dist[c]; the neighbours are distinct nodes
+      if (bk != INT_MAX) {
+        const double dnew = sh_dnew;
+        for (int32_t k = tid; k < k_hits; k += PG_COMMIT_THREADS) {
+          if (k == bk || hd[k] > r || hv[k] < 0) continue;
+          const int32_t c = hid[k];
+          const double nd = __dadd_rn(dnew, pg_norm2(q, g.xy[c]));
+          if (nd < t.dist[c]) { t.dist[c] = nd; t.tparent[c] = nw; }
+        }
+      }
+      // 4. the node: kd slot, kd parent, depth and key; 5. the goal test (a final node: some goal with norm1 < max_dist)
+      if (tid == 0) {
+        g.xy[nw] = q; g.reach[(size_t)nw * g.words] = 1ull;
+        const int32_t slot = s.slot[b], p = slot >> 1;
+        g.child[2 * nw] = g.child[2 * nw + 1] = -1;
+        g.child[slot] = nw; g.parent[nw] = p;
+        const int32_t dp = g.depth[p];
+        g.depth[nw] = dp + 1;
+        g.key[nw] = dp < 64 ? (g.key[p] | ((uint64_t)(slot & 1) << (63 - dp))) : g.key[p];
+        int32_t hit = -1;
+        for (int32_t k = 0; k < g.n_goals && hit < 0; ++k) {
+          const double2 gl = g.goals[k];
+          if (__dadd_rn(fabs(__dsub_rn(gl.x, q.x)), fabs(__dsub_rn(gl.y, q.y))) < g.goal_max_dist) hit = k;
+        }
+        if (hit >= 0) g.fin_ids[nfin] = nw;
+        sh_goal = hit;
+      }
+      __syncthreads();
+      if (sh_goal >= 0) ++nfin;
+      ++V;
+    }
+    committed = b + 1;
+    // the loop condition: i < n_iter_min || (no finals && i < n_iter_max)
+    if (!((int64_t)i < g.n_iter_min || (nfin == 0 && (int64_t)i < g.n_iter_max))) { done = 1; break; }
+    __syncthreads();
+  }
+  __syncthreads();
+  if (tid == 0) {
+    ctl[C_V] = V; ctl[C_NFIN] = nfin; ctl[C_IT] = it0 + committed;
+    ctl[C_WINDOWS] = wid + 1;
+    if (done) ctl[C_DONE] = done;
+    ctl[C_STALL] = stall;
+    ctl[C_W] = cut ? max(PG_WMIN, 2 * committed) : (stall ? W : min(PG_WMAX, 2 * W));
+  }
+}
+
+// start: node 0 with tree parent -1 and dist 0; RRT does not check the start.  One thread per tree.
+__global__ void rrt_init_kernel(const PgDev* __restrict__ gs, const RrtDev* __restrict__ ts, double2 start, int n) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  const PgDev& g = gs[r];
+  const RrtDev& t = ts[r];
+  int32_t* ctl = g.ctl;
+  ctl[C_V] = 1; ctl[C_IT] = 0; ctl[C_W] = PG_WMIN * 2; ctl[C_DONE] = 0; ctl[C_PANIC] = 0;
+  ctl[C_STALL] = 0; ctl[C_NFIN] = 0; ctl[C_E] = 0; ctl[C_WINDOWS] = 0; ctl[C_RESPEC] = 0; ctl[C_CONF_NN] = 0; ctl[C_CONF_RAD] = 0;
+  g.xy[0] = start; g.reach[0] = 1ull; g.child[0] = g.child[1] = -1; g.parent[0] = -1; g.depth[0] = 0; g.key[0] = 0ull;
+  t.tparent[0] = -1; t.dist[0] = 0.0;
+}
+
 // ------------------------------------------------------------------------------------------------ host
 static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double max_step, double goal_max_dist, int n_goals,
                     int64_t nmin, int64_t nmax) {
@@ -511,29 +681,45 @@ static void spec_layout(Carve& c, SpecDev& s, int64_t h) {
 }
 static size_t spec_bytes(int64_t h) { SpecDev s; return carve_size([&](Carve& c) { spec_layout(c, s, h); }); }
 static SpecDev spec_dev(PtoRoad* r) { SpecDev s = {}; Carve c{(uintptr_t)r->spec.p}; spec_layout(c, s, r->node_cap); return s; }
-static size_t node_bytes(int words) { return 72 + 16 * (size_t)words; }   // every per-node array below, per node
+// the per-node arrays of a roadmap (PTO) or of a tree (RRT: no validity ids, reachability gains, edge log or finality, but a tree
+// parent and dist_from_root), with their bytes per node
+struct NodeArray { DevBuf* b; size_t per; };
+static std::vector<NodeArray> node_arrays(PtoRoad* g, int words, bool rrt) {
+  const size_t w8 = (size_t)words * 8;
+  if (rrt)
+    return {{&g->xy, 16}, {&g->reach, w8}, {&g->child, 8}, {&g->parent, 4}, {&g->depth, 4}, {&g->key, 8}, {&g->fin_ids, 4},
+            {&g->tparent, 4}, {&g->dist, 8}};
+  return {{&g->xy, 16}, {&g->node_vid, 4}, {&g->reach, w8}, {&g->child, 8}, {&g->parent, 4}, {&g->depth, 4}, {&g->key, 8},
+          {&g->final_idx, 4}, {&g->gain, w8}, {&g->epoch, 4}, {&g->edge_off, 8}, {&g->ecnt, 4}, {&g->fin_ids, 4}, {&g->fin_goal, 4}};
+}
+static size_t node_bytes(int words, bool rrt) {   // every per-node array, per node
+  PtoRoad r;
+  size_t s = 0;
+  for (const NodeArray& a : node_arrays(&r, words, rrt)) s += a.per;
+  return s;
+}
 
 // every per-node array holds node_cap entries, kept across growth (DevBuf::grow_keep)
-static int32_t pg_grow_nodes(porrt_ctx* ctx, PtoRoad* g, int words, int64_t want, int64_t V_now) {
+static int32_t pg_grow_nodes(porrt_ctx* ctx, PtoRoad* g, int words, bool rrt, int64_t want, int64_t V_now) {
   if (want <= g->node_cap) return PORRT_OK;
   const int64_t cap = std::max<int64_t>(want, 2 * g->node_cap);
   cudaStream_t st = ctx->stream;
-  const size_t w8 = (size_t)words * 8;
-  struct { DevBuf* b; size_t per; } arr[] = {{&g->xy, 16}, {&g->node_vid, 4}, {&g->reach, w8}, {&g->child, 8}, {&g->parent, 4},
-      {&g->depth, 4}, {&g->key, 8}, {&g->final_idx, 4}, {&g->gain, w8}, {&g->epoch, 4}, {&g->edge_off, 8}, {&g->ecnt, 4},
-      {&g->fin_ids, 4}, {&g->fin_goal, 4}};
-  for (auto& a : arr) CUDA_TRY(ctx, a.b->grow_keep((size_t)(cap + 1) * a.per, (size_t)(V_now + 1) * a.per, st));
+  for (const NodeArray& a : node_arrays(g, words, rrt))
+    CUDA_TRY(ctx, a.b->grow_keep((size_t)(cap + 1) * a.per, (size_t)(V_now + 1) * a.per, st));
   CUDA_TRY(ctx, g->spec.ensure(spec_bytes(cap)));
   g->node_cap = cap;
   return PORRT_OK;
 }
 
-// heuristic_radius(n) for every n a window can reach (host libm, DESIGN.md 4)
-static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, int64_t node_cap, double max_step, double search_radius) {
+// heuristic_radius(n) for every n a window can reach (host libm, DESIGN.md 4); shifted by one for RRT, which takes the radius of the
+// node count before add (rrt.rs:125) where PTO takes it after: radius[n] = heuristic_radius(n - 1), so radius[V + 1] serves both
+static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, int64_t node_cap, double max_step, double search_radius, bool rrt) {
   const int64_t rn = node_cap + PG_WMAX + 2;
   if (rn <= g->radius_n) return PORRT_OK;
   std::vector<double> r((size_t)rn);
-  for (int64_t n = 0; n < rn; ++n) r[(size_t)n] = n == 0 ? 0.0 : heuristic_radius(n, max_step, search_radius, 2);
+  const int64_t shift = rrt ? 1 : 0;
+  for (int64_t n = 0; n < rn; ++n)
+    r[(size_t)n] = n - shift <= 0 ? 0.0 : heuristic_radius(n - shift, max_step, search_radius, 2);
   CUDA_TRY(ctx, g->radius.ensure((size_t)rn * 8));
   CUDA_TRY(ctx, cudaMemcpyAsync(g->radius.p, r.data(), (size_t)rn * 8, cudaMemcpyHostToDevice, ctx->stream));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));
@@ -541,7 +727,7 @@ static int32_t pg_radius_table(porrt_ctx* ctx, PtoGrow* g, int64_t node_cap, dou
   return PORRT_OK;
 }
 
-// one host sample stream per roadmap: pto.rs:141-149, the continuous and the discrete sampler seeded alike
+// one host sample stream per roadmap: pto.rs:141-149, the continuous and the discrete sampler seeded alike (RRT: the continuous one)
 struct PgStream {
   Pcg64 cont, disc;
   int64_t drawn;
@@ -549,13 +735,15 @@ struct PgStream {
   std::vector<int32_t> wld;
 };
 
-// PTO::grow_graph for n roadmaps that differ only in their sampler seed.  Every roadmap runs the host decisions and the windows the
-// single growth would run: each look grows its buffers and draws its samples by the same rules, then PG_BATCH windows of every
-// roadmap that is still running go out in one speculate and one commit launch per window.
-static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const uint64_t* seeds, const double start[2], const double low[2],
-                             const double up[2], const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
-                             double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes,
-                             int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters) {
+// PTO::grow_graph (rrt == false) or RRT::grow_tree (rrt == true) for n roadmaps / trees that differ only in their sampler seed.
+// Every one runs the host decisions and the windows the single growth would run: each look grows its buffers and draws its samples
+// by the same rules, then PG_BATCH windows of every one that is still running go out in one speculate and one commit launch per
+// window.  The two differ in the sample rule, the radius table, the init and commit kernels and what is kept at the end.
+// out_sizes: 4 per roadmap (iterations, nodes, directed edges, finals), 3 per tree (iterations, nodes, finals).
+static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, const uint64_t* seeds, const double start[2],
+                         const double low[2], const double up[2], const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals,
+                         double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
+                         int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters) {
   CTX_CHECK(ctx);
   if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
   if (!start || !low || !up || (n_goals > 0 && (!goals_xy || !goal_masks)) || n_goals < 0 || n_iter_min < 0 || n_iter_max < 0 ||
@@ -563,15 +751,17 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": bad arguments");
   if (n < 1 || n > PORRT_PTO_MAX_ROADMAPS)
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": n_roadmaps must be in 1 .. " + std::to_string(PORRT_PTO_MAX_ROADMAPS));
-  if (!ctx->pto) ctx->pto = new PtoGrow();
-  PtoGrow* g = ctx->pto;
+  PtoGrow*& state = rrt ? ctx->rrt : ctx->pto;
+  if (!state) state = new PtoGrow();
+  PtoGrow* g = state;
   g->n_have = 0;
   for (auto& r : g->roads) r->have = false;
-  for (int64_t k = 0; k < 4 * (int64_t)n; ++k) out_sizes[k] = 0;
+  const int n_sizes = rrt ? 3 : 4;
+  for (int64_t k = 0; k < n_sizes * (int64_t)n; ++k) out_sizes[k] = 0;
   for (int32_t r = 0; r < n; ++r) out_status[r] = 0;
   if (out_panic_code) for (int32_t r = 0; r < n; ++r) out_panic_code[r] = 0;
   if (out_counters) for (int64_t k = 0; k < 4 * (int64_t)n; ++k) out_counters[k] = 0;
-  const int words = ctx->mask_words, n_worlds = ctx->n_worlds;
+  const int words = rrt ? 1 : ctx->mask_words, n_worlds = ctx->n_worlds;   // a tree's reach word is its committed bit
   // SquareGoal::new (common.rs:304-350): world_to_goal, asserting that no world has two goals (:320)
   std::vector<double> world_goal((size_t)n_worlds * 2, 0.0);
   if (n_goals > 0 && porrt_square_goal_examples(goals_xy, goal_masks, n_goals, n_worlds, world_goal.data()) == PORRT_ERR_PANIC)
@@ -587,14 +777,14 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
   const int64_t cap0 = std::min<int64_t>(bound, 4096) + PG_BATCH * PG_WMAX + 1;
   const int64_t draw0 = runs ? std::min(n_iter_min + 4096, bound) : 0;
   {  // every roadmap must fit at its starting size: what the buffers below take, growth factors included
-    const double per = 1.5 * (double)(cap0 + 1) * node_bytes(words) + 1.25 * spec_bytes(cap0) + 2 * 1.25 * 64.0 * cap0 +
+    const double per = 1.5 * (double)(cap0 + 1) * node_bytes(words, rrt) + 1.25 * spec_bytes(cap0) + (rrt ? 0.0 : 2 * 1.25 * 64.0 * cap0) +
                        1.5 * 20.0 * draw0 + 1e5;
     size_t free_b = 0, total_b = 0;
     CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
     double held = 0;
     for (auto& r : g->roads) held += (double)r->bytes();
     if ((double)n * per > (double)free_b + held)
-      return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": " + std::to_string(n) + " roadmaps need about " +
+      return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": " + std::to_string(n) + (rrt ? " trees" : " roadmaps") + " need about " +
                         std::to_string((int64_t)(n * per / 1e6)) + " MB to start, the device has " +
                         std::to_string((int64_t)((free_b + held) / 1e6)) + " MB");
   }
@@ -609,13 +799,14 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
   for (auto& rp : g->roads) {
     PtoRoad* r = rp.get();
     r->node_cap = 0;
-    if ((rc = pg_grow_nodes(ctx, r, words, cap0, 0))) return rc;
+    if ((rc = pg_grow_nodes(ctx, r, words, rrt, cap0, 0))) return rc;
+    if (rrt) continue;
     r->edge_cap = std::max<int64_t>(r->edge_cap, 16 * r->node_cap);
     CUDA_TRY(ctx, r->log_nbr.ensure((size_t)r->edge_cap * 4));
     CUDA_TRY(ctx, r->log_vid.ensure((size_t)r->edge_cap * 4));
     CUDA_TRY(ctx, r->fin_acc.ensure((size_t)words * 8));
   }
-  if ((rc = pg_radius_table(ctx, g, cap0, max_step, search_radius))) return rc;
+  if ((rc = pg_radius_table(ctx, g, cap0, max_step, search_radius, rrt))) return rc;
   CUDA_TRY(ctx, g->goals.ensure((size_t)std::max(n_goals, 1) * 16));
   CUDA_TRY(ctx, g->goal_masks.ensure((size_t)std::max(n_goals, 1) * words * 8));
   CUDA_TRY(ctx, g->ctl.ensure((size_t)n * C_N * 4 + 64));
@@ -623,24 +814,28 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
   CUDA_TRY(ctx, g->caps.ensure((size_t)n * 3 * 4));
   CUDA_TRY(ctx, g->pg_desc.ensure((size_t)n * sizeof(PgDev)));
   CUDA_TRY(ctx, g->spec_desc.ensure((size_t)n * sizeof(SpecDev)));
+  if (rrt) CUDA_TRY(ctx, g->tree_desc.ensure((size_t)n * sizeof(RrtDev)));
   if (n_goals > 0) {
     CUDA_TRY(ctx, cudaMemcpyAsync(g->goals.p, goals_xy, (size_t)n_goals * 16, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(g->goal_masks.p, goal_masks, (size_t)n_goals * words * 8, cudaMemcpyHostToDevice, st));
   }
   int32_t* ctl = g->ctl.as<int32_t>();
   // the descriptors, re-uploaded whenever a buffer moved
-  std::vector<char> desc((size_t)n * (sizeof(PgDev) + sizeof(SpecDev)));
+  std::vector<char> desc((size_t)n * (sizeof(PgDev) + sizeof(SpecDev) + (rrt ? sizeof(RrtDev) : 0)));
   g->desc_host.clear();
   auto upload_desc = [&]() -> int32_t {
     PgDev* pd = (PgDev*)desc.data();
     SpecDev* sd = (SpecDev*)(desc.data() + (size_t)n * sizeof(PgDev));
+    RrtDev* td = (RrtDev*)(desc.data() + (size_t)n * (sizeof(PgDev) + sizeof(SpecDev)));
     for (int32_t r = 0; r < n; ++r) {
       pd[r] = pg_dev(ctx, g, g->roads[r].get(), ctl + (size_t)r * C_N, max_step, goal_max_dist, n_goals, n_iter_min, n_iter_max);
       sd[r] = spec_dev(g->roads[r].get());
+      if (rrt) td[r] = RrtDev{g->roads[r]->tparent.as<int32_t>(), g->roads[r]->dist.as<double>()};
     }
     if (desc == g->desc_host) return PORRT_OK;
     CUDA_TRY(ctx, cudaMemcpyAsync(g->pg_desc.p, pd, (size_t)n * sizeof(PgDev), cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(g->spec_desc.p, sd, (size_t)n * sizeof(SpecDev), cudaMemcpyHostToDevice, st));
+    if (rrt) CUDA_TRY(ctx, cudaMemcpyAsync(g->tree_desc.p, td, (size_t)n * sizeof(RrtDev), cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));   // desc is rewritten at the next look
     g->desc_host = desc;
     return PORRT_OK;
@@ -663,7 +858,8 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
   std::vector<PgStream> hs;
   hs.reserve((size_t)n);
   for (int32_t r = 0; r < n; ++r) hs.push_back(PgStream{Pcg64::seed_from_u64(seeds[r]), Pcg64::seed_from_u64(seeds[r]), 0, {}, {}});
-  // pto.rs:141-149: one discrete draw per iteration, a continuous draw only when i % 100 != 0 (then goal_example(world))
+  // pto.rs:141-149: one discrete draw per iteration, a continuous draw only when i % 100 != 0 (then goal_example(world));
+  // rrt.rs:176-181: no world, a continuous draw only when i % 100 != 0 (then goal_example(0))
   auto draw = [&](int32_t r, int64_t upto) -> int32_t {
     PgStream& h = hs[(size_t)r];
     PtoRoad* d = g->roads[r].get();
@@ -673,7 +869,7 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
     h.smp.resize((size_t)m * 2); h.wld.resize((size_t)m);
     for (int64_t k = 0; k < m; ++k) {
       const int64_t i = h.drawn + k + 1;
-      const int32_t w = (int32_t)h.disc.below((uint64_t)n_worlds);
+      const int32_t w = rrt ? 0 : (int32_t)h.disc.below((uint64_t)n_worlds);
       h.wld[(size_t)k] = w;
       if (i % 100 == 0) { h.smp[2 * k] = world_goal[2 * (size_t)w]; h.smp[2 * k + 1] = world_goal[2 * (size_t)w + 1]; }
       else { h.smp[2 * k] = h.cont.range_f64(low[0], up[0]); h.smp[2 * k + 1] = h.cont.range_f64(low[1], up[1]); }
@@ -696,7 +892,8 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
     return PORRT_OK;
   };
   if ((rc = upload_desc())) return rc;
-  pto_init_kernel<<<n, 64, 0, st>>>(ctx->map, g->pg_desc.as<PgDev>(), make_double2(start[0], start[1]));
+  if (rrt) rrt_init_kernel<<<div_up(n, 128), 128, 0, st>>>(g->pg_desc.as<PgDev>(), g->tree_desc.as<RrtDev>(), make_double2(start[0], start[1]), n);
+  else pto_init_kernel<<<n, 64, 0, st>>>(ctx->map, g->pg_desc.as<PgDev>(), make_double2(start[0], start[1]));
   LAUNCH_CHECK(ctx);
   if (runs) for (int32_t r = 0; r < n; ++r) if ((rc = draw(r, n_iter_min + 4096))) return rc;
   if ((rc = upload_caps())) return rc;
@@ -714,8 +911,8 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
         running = true;
         const int64_t V = fr[C_V], it = fr[C_IT];
         // room for the next batch of windows: nodes (every commit adds at most one), edges (the commit stalls when they run out)
-        if (V + PG_BATCH * PG_WMAX + 1 > d->node_cap && (rc = pg_grow_nodes(ctx, d, words, V + PG_BATCH * PG_WMAX + 1, V))) return rc;
-        if (fr[C_STALL] || (int64_t)fr[C_E] + 64 * PG_BATCH * PG_WMAX > d->edge_cap) {
+        if (V + PG_BATCH * PG_WMAX + 1 > d->node_cap && (rc = pg_grow_nodes(ctx, d, words, rrt, V + PG_BATCH * PG_WMAX + 1, V))) return rc;
+        if (!rrt && (fr[C_STALL] || (int64_t)fr[C_E] + 64 * PG_BATCH * PG_WMAX > d->edge_cap)) {
           const int64_t want = std::max<int64_t>(2 * d->edge_cap, (int64_t)fr[C_E] + V + 1 + 64 * PG_BATCH * PG_WMAX);
           CUDA_TRY(ctx, d->log_nbr.grow_keep((size_t)want * 4, (size_t)fr[C_E] * 4, st));
           CUDA_TRY(ctx, d->log_vid.grow_keep((size_t)want * 4, (size_t)fr[C_E] * 4, st));
@@ -727,7 +924,7 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
       node_cap = std::max(node_cap, d->node_cap);
     }
     if (!running) break;
-    if ((rc = pg_radius_table(ctx, g, node_cap, max_step, search_radius))) return rc;
+    if ((rc = pg_radius_table(ctx, g, node_cap, max_step, search_radius, rrt))) return rc;
     if ((rc = upload_caps())) return rc;
     if ((rc = upload_desc())) return rc;
     const PgDev* pd = g->pg_desc.as<PgDev>();
@@ -736,9 +933,33 @@ static int32_t pto_grow_impl(porrt_ctx* ctx, const char* who, int32_t n, const u
       if (ctx->map.kind == PORRT_DOMAIN_SHELF) pto_speculate_kernel<PORRT_DOMAIN_SHELF><<<dim3(PG_WMAX, n), PG_SPEC_THREADS, 0, st>>>(ctx->map, pd, sd);
       else pto_speculate_kernel<PORRT_DOMAIN_DOOR><<<dim3(PG_WMAX, n), PG_SPEC_THREADS, 0, st>>>(ctx->map, pd, sd);
       LAUNCH_CHECK(ctx);
-      pto_commit_kernel<<<n, PG_COMMIT_THREADS, 0, st>>>(pd, sd);
+      if (rrt) rrt_commit_kernel<<<n, PG_COMMIT_THREADS, 0, st>>>(pd, sd, g->tree_desc.as<RrtDev>());
+      else pto_commit_kernel<<<n, PG_COMMIT_THREADS, 0, st>>>(pd, sd);
       LAUNCH_CHECK(ctx);
     }
+  }
+  if (rrt) {   // per tree: outputs; the tree stays where it grew
+    for (int32_t r = 0; r < n; ++r) {
+      const int32_t* fr = f + (size_t)r * C_N;
+      int64_t* sz = out_sizes + 3 * (size_t)r;
+      sz[0] = fr[C_IT];
+      if (out_counters) {
+        int64_t* c = out_counters + 4 * (size_t)r;
+        c[0] = fr[C_WINDOWS]; c[1] = fr[C_RESPEC]; c[2] = fr[C_CONF_NN]; c[3] = fr[C_CONF_RAD];
+      }
+      if (fr[C_DONE] == 2) {
+        out_status[r] = PORRT_ERR_PANIC;
+        if (out_panic_code) out_panic_code[r] = fr[C_PANIC];
+        sz[0] = fr[C_IT] + 1;                                  // the iteration whose check panicked
+        continue;
+      }
+      PtoRoad* d = g->roads[r].get();
+      d->have = true; d->V = fr[C_V]; d->E = 0; d->n_finals = fr[C_NFIN];
+      sz[1] = d->V; sz[2] = d->n_finals;
+      out_status[r] = d->n_finals > 0 ? 0 : 1;
+    }
+    g->n_have = n;
+    return PORRT_OK;
   }
   // per roadmap: outputs, then the children CSR from the edge log (graph.cu's late-list kernels, carrying the validity ids)
   // CSR assembly work space of a roadmap of V nodes and E edges (late_list_csr_dev), one roadmap at a time
@@ -813,8 +1034,8 @@ PORRT_API int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const do
   if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
   if (!out_complete) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_grow: bad arguments");
   int32_t status = 0, panic = 0;
-  const int32_t rc = pto_grow_impl(ctx, "porrt_pto_grow", 1, &sampler_seed, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
-                                   max_step, search_radius, n_iter_min, n_iter_max, out_sizes, &status, &panic, out_counters);
+  const int32_t rc = grow_impl(ctx, "porrt_pto_grow", false, 1, &sampler_seed, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
+                               max_step, search_radius, n_iter_min, n_iter_max, out_sizes, &status, &panic, out_counters);
   *out_complete = rc == PORRT_OK && status == 0 ? 1 : 0;
   if (rc) return rc;
   if (out_panic_code) *out_panic_code = panic;
@@ -828,8 +1049,8 @@ PORRT_API int32_t porrt_pto_grow_batch(porrt_ctx* ctx, int32_t n_roadmaps, const
                                        int32_t n_goals, double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min,
                                        int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code,
                                        int64_t* out_counters) {
-  return pto_grow_impl(ctx, "porrt_pto_grow_batch", n_roadmaps, sampler_seeds, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
-                       max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
+  return grow_impl(ctx, "porrt_pto_grow_batch", false, n_roadmaps, sampler_seeds, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
+                   max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
 }
 
 PORRT_API int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr,
@@ -868,4 +1089,50 @@ PORRT_API int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out
 PORRT_API int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
                                   int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks) {
   return porrt_pto_fetch_roadmap(ctx, 0, out_xy, out_node_vid, out_row_ptr, out_col, out_edge_vid, out_reach, out_final_ids, out_final_masks);
+}
+
+PORRT_API int32_t porrt_rrt_grow_batch(porrt_ctx* ctx, int32_t n_trees, const uint64_t* sampler_seeds, const double start[2],
+                                       const double low[2], const double up[2], const double* goals_xy, const uint64_t* goal_masks,
+                                       int32_t n_goals, double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min,
+                                       int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code,
+                                       int64_t* out_counters) {
+  return grow_impl(ctx, "porrt_rrt_grow_batch", true, n_trees, sampler_seeds, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
+                   max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
+}
+
+PORRT_API int32_t porrt_rrt_grow(porrt_ctx* ctx, uint64_t sampler_seed, const double start[2], const double low[2], const double up[2],
+                                 const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
+                                 double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes,
+                                 int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters) {
+  CTX_CHECK(ctx);
+  if (!out_status) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_grow: bad arguments");
+  int32_t panic = 0;
+  const int32_t rc = grow_impl(ctx, "porrt_rrt_grow", true, 1, &sampler_seed, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
+                               max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, &panic, out_counters);
+  if (rc) return rc;
+  if (out_panic_code) *out_panic_code = panic;
+  if (*out_status != PORRT_ERR_PANIC) return PORRT_OK;
+  return porrt_fail(ctx, PORRT_ERR_PANIC, "porrt_rrt_grow: a state / edge check hit a reference panic (code " + std::to_string(panic) + ")");
+}
+
+PORRT_API int32_t porrt_rrt_fetch_tree(porrt_ctx* ctx, int32_t t, double* out_xy, int32_t* out_parent, double* out_dist,
+                                       int64_t* out_final_ids) {
+  CTX_CHECK(ctx);
+  PtoGrow* rg = ctx->rrt;
+  if (!rg || rg->n_have == 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_fetch_tree: no tree grown on this ctx");
+  if (t < 0 || t >= rg->n_have)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_fetch_tree: tree " + std::to_string(t) + " of " + std::to_string(rg->n_have));
+  const PtoRoad* g = rg->roads[t].get();
+  if (!g->have) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_fetch_tree: tree " + std::to_string(t) + " panicked");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const int64_t V = g->V, F = g->n_finals;
+  std::vector<int32_t> ids((size_t)F);
+  if (out_xy) CUDA_TRY(ctx, cudaMemcpyAsync(out_xy, g->xy.p, (size_t)V * 16, cudaMemcpyDeviceToHost, st));
+  if (out_parent) CUDA_TRY(ctx, cudaMemcpyAsync(out_parent, g->tparent.p, (size_t)V * 4, cudaMemcpyDeviceToHost, st));
+  if (out_dist) CUDA_TRY(ctx, cudaMemcpyAsync(out_dist, g->dist.p, (size_t)V * 8, cudaMemcpyDeviceToHost, st));
+  if (out_final_ids && F) CUDA_TRY(ctx, cudaMemcpyAsync(ids.data(), g->fin_ids.p, (size_t)F * 4, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  if (out_final_ids) for (int64_t k = 0; k < F; ++k) out_final_ids[k] = ids[(size_t)k];
+  return PORRT_OK;
 }

@@ -46,6 +46,22 @@ def shelf_map(size=200, n_rects=12, n_zones=2, seed=5):
     return occ, zones
 
 
+def pixel_centres(size):
+    """(x, y) of every pixel centre of a size x size map on [-1, 1]^2; row 0 is the top (largest y), as Map::to_pixel reads it"""
+    c = (np.arange(size) + 0.5) / size * 2.0 - 1.0
+    return np.meshgrid(c, c[::-1])
+
+
+def rrt_map(size=1024, n_rects=4096, seed=7, clear=((-0.8, -0.8), (0.8, 0.8)), clear_r=0.06):
+    """Single-world stand-in for the RRT* config's map (BASELINE config 1): free grid with obstacle rectangles (0) on [-1, 1]^2, no
+    zones, and a free disc of radius clear_r around each point of `clear` (the start and the goal)."""
+    occ, _ = door_map(size=size, n_rects=n_rects, n_zones=0, seed=seed)
+    x, y = pixel_centres(size)
+    for px, py in clear:
+        occ[(x - px) ** 2 + (y - py) ** 2 <= clear_r ** 2] = 255
+    return occ
+
+
 def edges(n, seed=2, max_len=0.1, low=-1.0, up=1.0):
     """a uniform in [low,up)^2; b = a + l*(cos t, sin t), l ~ U[0,max_len], clamped into [low, up - 2^-20]"""
     rng = np.random.default_rng(seed)
