@@ -133,7 +133,10 @@ int32_t porrt_visibility_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, ui
 
 /* ------------------------------------------------------------------ nearest neighbours (nearest_neighbor.rs)
  * The vertex set replaces the KdTree's contents: vertex i has id i (KdTree::add(state, id) with ids 0..n-1).
- * cell_size <= 0 picks one from the vertex density. */
+ * cell_size <= 0 picks one from the vertex density.  A NaN or infinite coordinate, or a bounding box whose width or height
+ * overflows a double, is refused with PORRT_ERR_INVALID_ARG (here, and by the rebuild that follows porrt_vertices_append).
+ * porrt_vertices_set_dev with an explicit bbox_lo / bbox_hi checks only the box: the coordinates are not scanned, and the caller
+ * guarantees that they are finite and inside it (a NaN vertex would be binned into the first cell and never be found). */
 int32_t porrt_vertices_set(porrt_ctx* ctx, const double* xy, int64_t n, double cell_size);
 int32_t porrt_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, double cell_size,
                                const double bbox_lo[2], const double bbox_hi[2]);

@@ -213,12 +213,16 @@ int bits_for(uint64_t max_value) {
 }
 
 // ================================================================================================ cell grid
-__global__ void bbox_kernel(const double2* __restrict__ xy, int64_t n, double* __restrict__ out /* minx,miny,maxx,maxy as ordered u64 */) {
+// out[4] counts the NaN coordinates: fmin / fmax skip them, and a NaN vertex would be binned into cell 0 and never hit anything
+__global__ void bbox_kernel(const double2* __restrict__ xy, int64_t n, double* __restrict__ out /* minx,miny,maxx,maxy as ordered u64, n_nan */) {
   double mnx = INFINITY, mny = INFINITY, mxx = -INFINITY, mxy = -INFINITY;
+  bool nan = false;
   for (int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x; i < n; i += (int64_t)gridDim.x * blockDim.x) {
     double2 p = xy[i];
+    nan |= p.x != p.x || p.y != p.y;
     mnx = fmin(mnx, p.x); mny = fmin(mny, p.y); mxx = fmax(mxx, p.x); mxy = fmax(mxy, p.y);
   }
+  if (__any_sync(0xffffffffu, nan) && (threadIdx.x & 31) == 0) atomicAdd((unsigned long long*)out + 4, 1ull);
   for (int o = 16; o; o >>= 1) {
     mnx = fmin(mnx, __shfl_xor_sync(0xffffffffu, mnx, o)); mny = fmin(mny, __shfl_xor_sync(0xffffffffu, mny, o));
     mxx = fmax(mxx, __shfl_xor_sync(0xffffffffu, mxx, o)); mxy = fmax(mxy, __shfl_xor_sync(0xffffffffu, mxy, o));
@@ -270,14 +274,15 @@ int32_t nn_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, dou
   double blo[2], bhi[2];
   if (lo && hi) { blo[0] = lo[0]; blo[1] = lo[1]; bhi[0] = hi[0]; bhi[1] = hi[1]; }
   else {
-    CUDA_TRY(ctx, ctx->ws_query.ensure(32));
-    unsigned long long init[4] = {~0ull, ~0ull, 0ull, 0ull};
-    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws_query.p, init, 32, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, ctx->ws_query.ensure(40));
+    unsigned long long init[5] = {~0ull, ~0ull, 0ull, 0ull, 0ull};
+    CUDA_TRY(ctx, cudaMemcpyAsync(ctx->ws_query.p, init, 40, cudaMemcpyHostToDevice, st));
     bbox_kernel<<<ctx->sm_count * 4, 256, 0, st>>>((const double2*)xy_dev, n, ctx->ws_query.as<double>());
     LAUNCH_CHECK(ctx);
-    unsigned long long enc[4];
-    CUDA_TRY(ctx, cudaMemcpyAsync(enc, ctx->ws_query.p, 32, cudaMemcpyDeviceToHost, st));
+    unsigned long long enc[5];
+    CUDA_TRY(ctx, cudaMemcpyAsync(enc, ctx->ws_query.p, 40, cudaMemcpyDeviceToHost, st));
     CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    if (enc[4]) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "vertices_set: non-finite coordinates");
     double dec[4];
     for (int k = 0; k < 4; ++k) {
       unsigned long long b = (enc[k] & 0x8000000000000000ull) ? (enc[k] & 0x7fffffffffffffffull) : ~enc[k];
@@ -288,6 +293,8 @@ int32_t nn_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, dou
   if (!(blo[0] <= bhi[0]) || !(blo[1] <= bhi[1]) || !std::isfinite(blo[0]) || !std::isfinite(bhi[0]) || !std::isfinite(blo[1]) || !std::isfinite(bhi[1]))
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "vertices_set: non-finite coordinates");
   double ex = bhi[0] - blo[0], ey = bhi[1] - blo[1];
+  // a span beyond DBL_MAX (corners near -DBL_MAX and +DBL_MAX) has no finite cell count: the sizing loop below would never end
+  if (!std::isfinite(ex) || !std::isfinite(ey)) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "vertices_set: bounding box span overflows");
   double cell = cell_size;
   if (!(cell > 0.0)) cell = std::sqrt(std::max(ex * ey, 1e-300) * 2.0 / (double)n);  // ~2 vertices per cell
   if (!(cell > 0.0) || !std::isfinite(cell)) cell = 1.0;
