@@ -32,6 +32,7 @@ extern "C" {
 #define PORRT_ERR_UNSUPPORTED 6
 #define PORRT_ERR_NO_VERTICES 7 /* NN call before porrt_vertices_set */
 #define PORRT_ERR_COMM 8        /* NCCL not loadable / communicator error (multi-GPU paths only) */
+#define PORRT_ERR_INTERNAL 9    /* a result the library's own invariants rule out (see porrt_last_error) */
 
 /* per-element validity codes (int32): >= 0 is a validity id into the world-validity table */
 #define PORRT_INVALID (-1)            /* Option::None: obstacle                          map_io.rs:491,511 */
@@ -462,6 +463,30 @@ int32_t porrt_rrt_grow(porrt_ctx* ctx, uint64_t sampler_seed, const double start
  * as they stand after the last rewire, final node ids in the order they were found.  PORRT_ERR_INVALID_ARG when nothing has been
  * grown, t is out of range, or tree t panicked. */
 int32_t porrt_rrt_fetch_tree(porrt_ctx* ctx, int32_t t, double* out_xy, int32_t* out_parent, double* out_dist, int64_t* out_final_ids);
+/* porrt_rrt_grow_batch with one query per tree: tree t starts at starts[2 t ..], heads for goals goal_ptr[t] .. goal_ptr[t + 1] of
+ * goals_xy[2 * goal_ptr[n]] / goal_masks[goal_ptr[n] * mask_words] with goal_max_dist[t], and samples with sampler_seeds[t].  Map,
+ * bounds, max_step, search_radius and the iteration bounds are shared.  Tree t equals porrt_rrt_grow(sampler_seeds[t], starts[t], its
+ * goals, goal_max_dist[t], ...) bit for bit, counters included; outputs, per-tree panics and porrt_rrt_fetch_tree as porrt_rrt_grow_batch.
+ * PORRT_ERR_INVALID_ARG for porrt_rrt_grow_batch's argument errors and for goal_ptr[0] != 0, a goal_ptr that decreases, a start that is
+ * not finite or a goal_max_dist that is negative or NaN; PORRT_ERR_PANIC when the goal masks of one query overlap (SquareGoal::new,
+ * common.rs:320; porrt_last_error names the query). */
+int32_t porrt_rrt_grow_queries(porrt_ctx* ctx, int32_t n_trees, const uint64_t* sampler_seeds, const double* starts, const double low[2],
+                               const double up[2], const int64_t* goal_ptr, const double* goals_xy, const uint64_t* goal_masks,
+                               const double* goal_max_dist, double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
+                               int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters);
+/* RRT::plan's second half (get_best_solution, rrt.rs:183-193, and RRTTree::get_path_to, :48-60) for every tree of the last RRT growth
+ * on this ctx (porrt_rrt_grow, _batch or _queries), on the device in one launch; only the paths are copied back.
+ *  - path to a final f: the chain of tree parents as they stand after the last rewire, root first, as states;
+ *  - its cost: accumulated root first from 0.0, c[root] = 0, c[v] = c[parent[v]] + norm2(state[parent[v]], state[v]) with the no-FMA
+ *    norm2 of common.rs:203-213 (not dist_from_root, which a rewire does not propagate to descendants);
+ *  - the winner: the smallest (cost, number of states), lexicographically; among equal pairs the final found first.
+ * Per tree t: out_final[t] = the winning final's node id, out_cost[t] its cost, its path at out_path_xy[2 * out_path_ptr[t] ..
+ * 2 * out_path_ptr[t + 1]] (out_path_ptr[n + 1]).  A tree without a final ("No path found!"), a root-only tree and a panicked tree give
+ * -1, +inf and an empty path.  cap (in states) smaller than the total path length: PORRT_ERR_CAPACITY with *out_total set (and
+ * out_final, out_cost, out_path_ptr filled).  PORRT_ERR_INVALID_ARG when nothing has been grown; PORRT_ERR_INTERNAL when a parent walk
+ * is longer than the tree's node count (a cycle). */
+int32_t porrt_rrt_best_paths(porrt_ctx* ctx, int32_t* out_final, double* out_cost, int64_t* out_path_ptr, double* out_path_xy, int64_t cap,
+                             int64_t* out_total);
 
 /* ------------------------------------------------------------------ multi-GPU (SURVEY.md 8(e))
  * The reference is single-threaded and has no distributed code; what shards are its independent units (edge checks,

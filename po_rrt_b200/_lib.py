@@ -102,6 +102,8 @@ SIGNATURES = {
     "porrt_rrt_grow_batch": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, i32, f64, f64, f64, i64, i64, vp, vp, vp, vp]),
     "porrt_rrt_grow": (i32, [vp, C.c_uint64, vp, vp, vp, vp, vp, i32, f64, f64, f64, i64, i64, vp, pp(i32), pp(i32), vp]),
     "porrt_rrt_fetch_tree": (i32, [vp, i32, vp, vp, vp, vp]),
+    "porrt_rrt_grow_queries": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp, f64, f64, i64, i64, vp, vp, vp, vp]),
+    "porrt_rrt_best_paths": (i32, [vp, vp, vp, vp, vp, i64, pp(i64)]),
     "porrt_comm_unique_id": (i32, [vp]),
     "porrt_comm_init": (i32, [vp, vp, i32, i32]),
     "porrt_comm_destroy": (i32, [vp]),

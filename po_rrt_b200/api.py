@@ -970,6 +970,8 @@ class RRT:
                                   goal.max_dist, float(max_step), float(search_radius), int(n_iter_min), int(n_iter_max), _p(sizes),
                                   C.byref(status), C.byref(panic), _p(counters))
         self.n_it, self.sizes, self.counters = int(sizes[0]), tuple(int(x) for x in sizes), tuple(int(x) for x in counters)
+        if rc in (0, 5):
+            c._rrt_trees = 1
         if rc:
             err = PorrtError(rc, (c.lib.porrt_last_error(c.h) or b"").decode())
             err.panic_code = panic.value
@@ -979,6 +981,17 @@ class RRT:
     def tree(self):
         """-> states[V, 2], parent[V] (-1 at the root), dist_from_root[V], final node ids in the order they were found"""
         return _fetch_tree(self.ctx, 0, self.sizes)
+
+    def best_path(self):
+        """get_best_solution + get_path_to (rrt.rs:183-193, :48-60) on the device: -> (path[L, 2] root first, cost) of the final
+        with the smallest (cost, path length), or None when the tree has no final (porrt_rrt_best_paths)"""
+        return _best_paths(self.ctx)[0]
+
+    def plan(self, start, goal, max_step, search_radius, n_iter_min, n_iter_max):
+        """rrt.rs:183-193 plan: grow_tree, then the best path -> (path[L, 2], cost), or None ("No path found!"); PorrtError where
+        the growth panics"""
+        self.grow_tree(start, goal, max_step, search_radius, n_iter_min, n_iter_max)
+        return self.best_path()
 
 
 class RRTBatch:
@@ -1011,11 +1024,56 @@ class RRTBatch:
                                         int(n_iter_max), _p(self.sizes), _p(status), _p(self.panic_code), _p(self.counters))
         self.n_it = self.sizes[:, 0].copy()
         c.check(rc)
+        c._rrt_trees = R
+        return status
+
+    def grow_queries(self, starts, goals, max_step, search_radius, n_iter_min, n_iter_max):
+        """grow_tree with one query per tree (porrt_rrt_grow_queries): tree t starts at starts[t] and heads for goals[t] (a
+        SquareGoal) with sampler seed seeds[t]; tree t is what RRT(fns, low, up, seeds[t]).grow_tree(starts[t], goals[t], ...) grows,
+        counters included.  -> status[R] as grow_tree; raises PorrtError when the call as a whole fails (grow_tree's errors, a start
+        that is not finite, a negative or NaN max_dist, goal masks that overlap within one query)."""
+        self.fns._need()
+        c = self.ctx
+        R = len(self.seeds)
+        starts, goals = _f64(starts, 2), list(goals)
+        if len(starts) != R or len(goals) != R:
+            raise ValueError("one start and one goal per seed")
+        ptr = np.zeros(R + 1, np.int64)
+        ptr[1:] = np.cumsum([len(g.goals) for g in goals])
+        gxy = np.ascontiguousarray(np.concatenate([g.goals for g in goals]))
+        gmask = np.ascontiguousarray(np.concatenate([g.masks for g in goals]))
+        gmd = np.array([g.max_dist for g in goals], np.float64)
+        status = np.zeros(R, np.int32)
+        rc = c.lib.porrt_rrt_grow_queries(c.h, R, _p(self.seeds), _p(starts), _p(self.low), _p(self.up), _p(ptr), _p(gxy), _p(gmask),
+                                          _p(gmd), float(max_step), float(search_radius), int(n_iter_min), int(n_iter_max),
+                                          _p(self.sizes), _p(status), _p(self.panic_code), _p(self.counters))
+        self.n_it = self.sizes[:, 0].copy()
+        c.check(rc)
+        c._rrt_trees = R
         return status
 
     def tree(self, t):
         """RRT.tree of tree t"""
         return _fetch_tree(self.ctx, t, self.sizes[t])
+
+    def best_paths(self):
+        """RRT.best_path of every tree, in one device call: a list of (path[L, 2], cost) or None"""
+        return _best_paths(self.ctx)
+
+
+def _best_paths(ctx):
+    """porrt_rrt_best_paths on the last RRT growth of ctx -> [(path[L, 2], cost) or None per tree]"""
+    n = getattr(ctx, "_rrt_trees", 0)          # the trees of the context's last RRT growth (set by the growth calls)
+    fin, cost, ptr, total = np.empty(max(n, 1), np.int32), np.empty(max(n, 1)), np.empty(n + 1, np.int64), C.c_int64()
+    cap = 64 * n
+    while True:
+        xy = np.empty((max(cap, 1), 2))
+        rc = ctx.lib.porrt_rrt_best_paths(ctx.h, _p(fin), _p(cost), _p(ptr), _p(xy), cap, C.byref(total))
+        if rc == ERR_CAPACITY and total.value > cap:
+            cap = total.value
+            continue
+        ctx.check(rc)
+        return [None if fin[t] < 0 else (xy[ptr[t]:ptr[t + 1]].copy(), float(cost[t])) for t in range(n)]
 
 
 def _fetch_tree(ctx, t, sizes):

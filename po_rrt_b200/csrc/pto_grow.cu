@@ -23,7 +23,9 @@
 // every window slot of every roadmap and a commit launch is one CTA per roadmap.  porrt_pto_grow is the batch of one.
 //
 // porrt_rrt_grow_batch grows RRT::grow_tree (rrt.rs:102-174) trees through the same speculation and host loop, with its own commit
-// (choose-parent and rewire run in order there; DESIGN.md 3.9).  porrt_rrt_grow is its batch of one.
+// (choose-parent and rewire run in order there; DESIGN.md 3.9).  porrt_rrt_grow is its batch of one; porrt_rrt_grow_queries gives
+// every tree its own start and goals.  porrt_rrt_best_paths runs get_best_solution + get_path_to (rrt.rs:183-193, :48-60) on every
+// tree of the last RRT growth in one launch.
 #include <algorithm>
 #include <cmath>
 #include <climits>
@@ -75,6 +77,8 @@ struct PtoGrow {    // the state of the last PTO growth (ctx->pto) or of the las
   DevBuf ctl;                                    // control blocks, roadmap r at [r * C_N]
   DevBuf pg_desc, spec_desc, caps;               // PgDev / SpecDev of every roadmap; node cap, edge cap, samples drawn of each
   DevBuf tree_desc;                              // RrtDev of every tree (RRT growth only)
+  DevBuf starts;                                 // every tree's start (RRT growth only)
+  DevBuf best, paths;                            // porrt_rrt_best_paths: RrtBest of every tree, the packed paths
   DevBuf work;                                   // CSR assembly work space, one roadmap at a time
   PinBuf ctl_host;                               // every control block, as the last look saw it
   std::vector<char> desc_host;                   // what pg_desc + spec_desc hold
@@ -87,7 +91,8 @@ struct PtoGrow {    // the state of the last PTO growth (ctx->pto) or of the las
 static void grow_state_release(PtoGrow*& g) {
   if (!g) return;
   for (auto& r : g->roads) r->release();
-  DevBuf* all[] = {&g->radius, &g->goals, &g->goal_masks, &g->ctl, &g->pg_desc, &g->spec_desc, &g->caps, &g->work, &g->tree_desc};
+  DevBuf* all[] = {&g->radius, &g->goals, &g->goal_masks, &g->ctl, &g->pg_desc, &g->spec_desc, &g->caps, &g->work, &g->tree_desc,
+                    &g->starts, &g->best, &g->paths};
   for (DevBuf* b : all) b->release();
   g->ctl_host.release();
   delete g;
@@ -640,7 +645,7 @@ __global__ void __launch_bounds__(PG_COMMIT_THREADS) rrt_commit_kernel(const PgD
 }
 
 // start: node 0 with tree parent -1 and dist 0; RRT does not check the start.  One thread per tree.
-__global__ void rrt_init_kernel(const PgDev* __restrict__ gs, const RrtDev* __restrict__ ts, double2 start, int n) {
+__global__ void rrt_init_kernel(const PgDev* __restrict__ gs, const RrtDev* __restrict__ ts, const double2* __restrict__ starts, int n) {
   const int r = blockIdx.x * blockDim.x + threadIdx.x;
   if (r >= n) return;
   const PgDev& g = gs[r];
@@ -648,13 +653,90 @@ __global__ void rrt_init_kernel(const PgDev* __restrict__ gs, const RrtDev* __re
   int32_t* ctl = g.ctl;
   ctl[C_V] = 1; ctl[C_IT] = 0; ctl[C_W] = PG_WMIN * 2; ctl[C_DONE] = 0; ctl[C_PANIC] = 0;
   ctl[C_STALL] = 0; ctl[C_NFIN] = 0; ctl[C_E] = 0; ctl[C_WINDOWS] = 0; ctl[C_RESPEC] = 0; ctl[C_CONF_NN] = 0; ctl[C_CONF_RAD] = 0;
-  g.xy[0] = start; g.reach[0] = 1ull; g.child[0] = g.child[1] = -1; g.parent[0] = -1; g.depth[0] = 0; g.key[0] = 0ull;
+  g.xy[0] = starts[r]; g.reach[0] = 1ull; g.child[0] = g.child[1] = -1; g.parent[0] = -1; g.depth[0] = 0; g.key[0] = 0ull;
   t.tparent[0] = -1; t.dist[0] = 0.0;
 }
 
+// ---- get_best_solution + get_path_to (rrt.rs:183-193, :48-60) on every tree of the last growth
+struct RrtBest { int32_t final_id, len, cycle; double cost; };   // final_id -1: no path; len: states on the path; cycle: a parent loop
+
+// One CTA per tree.  The cost of a node is accumulated root first, c[root] = 0, c[v] = c[parent] + norm2(parent, v) (no FMA), so a
+// final's cost is the reference's sum over its path in path order.  Every node on a final's path gets its depth (one walk per final;
+// threads that share an ancestor write the same depth), then the costs are filled in level by level.  The winner is the smallest
+// (cost, length, order found).  Scratch: the tree's speculation block (tmp_id = depth, tmp_d = cost), free once the growth ended.
+__global__ void __launch_bounds__(PG_COMMIT_THREADS) rrt_best_kernel(const PgDev* __restrict__ gs, const SpecDev* __restrict__ ss,
+                                                                     const RrtDev* __restrict__ ts, RrtBest* __restrict__ out) {
+  const PgDev& g = gs[blockIdx.x];
+  const SpecDev& s = ss[blockIdx.x];
+  const RrtDev& t = ts[blockIdx.x];
+  __shared__ double sh_v[PG_COMMIT_THREADS / 32];
+  __shared__ int32_t sh_k[PG_COMMIT_THREADS / 32], sh_l[PG_COMMIT_THREADS / 32];
+  __shared__ int32_t cycle, max_depth;
+  const int tid = threadIdx.x;
+  const int32_t V = g.ctl[C_V], F = g.ctl[C_DONE] == 2 ? 0 : g.ctl[C_NFIN];   // a panicked tree has no path
+  int32_t* depth = s.tmp_id;
+  double* cost = s.tmp_d;
+  if (tid == 0) { cycle = 0; max_depth = 0; }
+  for (int32_t v = tid; v < V; v += PG_COMMIT_THREADS) depth[v] = -1;
+  __syncthreads();
+  for (int32_t k = tid; k < F; k += PG_COMMIT_THREADS) {
+    int32_t L = 0;
+    for (int32_t v = g.fin_ids[k]; v >= 0 && L <= V; v = t.tparent[v]) ++L;
+    if (L > V) { cycle = 1; continue; }                       // more steps than nodes: the parents loop
+    int32_t d = L - 1;
+    for (int32_t v = g.fin_ids[k]; v >= 0; v = t.tparent[v]) depth[v] = d--;
+    atomicMax(&max_depth, L - 1);
+  }
+  __syncthreads();
+  if (cycle) {
+    if (tid == 0) out[blockIdx.x] = RrtBest{-1, 0, 1, INFINITY};
+    return;
+  }
+  if (tid == 0 && F > 0) cost[0] = 0.0;
+  for (int32_t lv = 1; lv <= max_depth; ++lv) {
+    __syncthreads();
+    for (int32_t v = tid; v < V; v += PG_COMMIT_THREADS)
+      if (depth[v] == lv) { const int32_t p = t.tparent[v]; cost[v] = __dadd_rn(cost[p], pg_norm2(g.xy[p], g.xy[v])); }
+  }
+  __syncthreads();
+  // the smallest (cost, length); a thread visits its finals in the order found, so strict < keeps the first of equal pairs
+  double bv = INFINITY;
+  int32_t bl = INT_MAX, bk = INT_MAX;
+  for (int32_t k = tid; k < F; k += PG_COMMIT_THREADS) {
+    const int32_t f = g.fin_ids[k], l = depth[f] + 1;
+    const double c = cost[f];
+    if (c < bv || (c == bv && l < bl)) { bv = c; bl = l; bk = k; }
+  }
+  // block-wide arg-min of (cost, length, k)
+  for (int o = 16; o; o >>= 1) {
+    const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+    const int32_t ol = __shfl_xor_sync(0xffffffffu, bl, o), ok = __shfl_xor_sync(0xffffffffu, bk, o);
+    if (ov < bv || (ov == bv && (ol < bl || (ol == bl && ok < bk)))) { bv = ov; bl = ol; bk = ok; }
+  }
+  if ((tid & 31) == 0) { sh_v[tid >> 5] = bv; sh_l[tid >> 5] = bl; sh_k[tid >> 5] = bk; }
+  __syncthreads();
+  if (tid == 0) {
+    for (int w = 1; w < PG_COMMIT_THREADS / 32; ++w)
+      if (sh_v[w] < bv || (sh_v[w] == bv && (sh_l[w] < bl || (sh_l[w] == bl && sh_k[w] < bk)))) { bv = sh_v[w]; bl = sh_l[w]; bk = sh_k[w]; }
+    out[blockIdx.x] = bk == INT_MAX ? RrtBest{-1, 0, 0, INFINITY} : RrtBest{g.fin_ids[bk], bl, 0, bv};
+  }
+}
+
+// the winner's path of tree t, root first, at out_xy[ptr[t] ..]: node v sits at its depth.  One thread per tree.
+__global__ void rrt_path_kernel(const PgDev* __restrict__ gs, const RrtDev* __restrict__ ts, const RrtBest* __restrict__ best,
+                                const int64_t* __restrict__ ptr, double2* __restrict__ out_xy, int n) {
+  const int r = blockIdx.x * blockDim.x + threadIdx.x;
+  if (r >= n) return;
+  double2* o = out_xy + ptr[r];
+  int32_t d = best[r].len - 1;
+  for (int32_t v = best[r].final_id; d >= 0; v = ts[r].tparent[v]) o[d--] = gs[r].xy[v];
+}
+
 // ------------------------------------------------------------------------------------------------ host
-static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double max_step, double goal_max_dist, int n_goals,
-                    int64_t nmin, int64_t nmax) {
+// what one roadmap / tree starts from and heads for: its start, goals [g0, g1) of the call's goal arrays, their max_dist
+struct PgQuery { double start[2]; int64_t g0, g1; double goal_max_dist; };
+
+static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double max_step, const PgQuery& q, int64_t nmin, int64_t nmax) {
   PgDev d = {};
   d.xy = r->xy.as<double2>(); d.node_vid = r->node_vid.as<int32_t>(); d.reach = r->reach.as<uint64_t>(); d.child = r->child.as<int32_t>();
   d.parent = r->parent.as<int32_t>(); d.depth = r->depth.as<int32_t>(); d.key = r->key.as<uint64_t>(); d.final_idx = r->final_idx.as<int32_t>();
@@ -662,9 +744,10 @@ static PgDev pg_dev(porrt_ctx* ctx, PtoGrow* g, PtoRoad* r, int32_t* ctl, double
   d.fin_ids = r->fin_ids.as<int32_t>(); d.fin_goal = r->fin_goal.as<int32_t>(); d.fin_acc = r->fin_acc.as<uint64_t>();
   d.log_nbr = r->log_nbr.as<int32_t>(); d.log_vid = r->log_vid.as<int32_t>();
   d.samples = r->samples.as<double2>(); d.worlds = r->worlds.as<int32_t>(); d.radius = g->radius.as<double>();
-  d.goals = g->goals.as<double2>(); d.goal_masks = g->goal_masks.as<uint64_t>(); d.validities = ctx->d_validities.as<uint64_t>();
+  d.goals = g->goals.as<double2>() + q.g0; d.goal_masks = g->goal_masks.as<uint64_t>() + (size_t)q.g0 * g->words;
+  d.validities = ctx->d_validities.as<uint64_t>();
   d.ctl = ctl;
-  d.words = g->words; d.n_worlds = ctx->n_worlds; d.n_goals = n_goals; d.goal_max_dist = goal_max_dist; d.max_step = max_step;
+  d.words = g->words; d.n_worlds = ctx->n_worlds; d.n_goals = (int32_t)(q.g1 - q.g0); d.goal_max_dist = q.goal_max_dist; d.max_step = max_step;
   d.n_iter_min = nmin; d.n_iter_max = nmax;
   return d;
 }
@@ -735,22 +818,24 @@ struct PgStream {
   std::vector<int32_t> wld;
 };
 
-// PTO::grow_graph (rrt == false) or RRT::grow_tree (rrt == true) for n roadmaps / trees that differ only in their sampler seed.
-// Every one runs the host decisions and the windows the single growth would run: each look grows its buffers and draws its samples
+// PTO::grow_graph (rrt == false) or RRT::grow_tree (rrt == true) for n roadmaps / trees, r with sampler seed seeds[r] and query
+// qs[r] over the call's goals_xy / goal_masks [n_goals] (qs == nullptr: bad arguments).  PTO roadmaps share one start: pto_init_kernel
+// takes qs[0]'s, and every PTO caller passes the same query for every roadmap.  Every one runs the host decisions and the windows the single growth would run: each look grows its buffers and draws its samples
 // by the same rules, then PG_BATCH windows of every one that is still running go out in one speculate and one commit launch per
 // window.  The two differ in the sample rule, the radius table, the init and commit kernels and what is kept at the end.
 // out_sizes: 4 per roadmap (iterations, nodes, directed edges, finals), 3 per tree (iterations, nodes, finals).
-static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, const uint64_t* seeds, const double start[2],
-                         const double low[2], const double up[2], const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals,
-                         double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
+static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, const uint64_t* seeds, const PgQuery* qs,
+                         const double low[2], const double up[2], const double* goals_xy, const uint64_t* goal_masks, int64_t n_goals,
+                         double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
                          int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code, int64_t* out_counters) {
   CTX_CHECK(ctx);
   if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
-  if (!start || !low || !up || (n_goals > 0 && (!goals_xy || !goal_masks)) || n_goals < 0 || n_iter_min < 0 || n_iter_max < 0 ||
+  if (!low || !up || (n_goals > 0 && (!goals_xy || !goal_masks)) || n_goals < 0 || n_iter_min < 0 || n_iter_max < 0 ||
       !out_sizes || !out_status || !seeds)
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": bad arguments");
   if (n < 1 || n > PORRT_PTO_MAX_ROADMAPS)
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": n_roadmaps must be in 1 .. " + std::to_string(PORRT_PTO_MAX_ROADMAPS));
+  if (!qs) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": bad arguments");
   PtoGrow*& state = rrt ? ctx->rrt : ctx->pto;
   if (!state) state = new PtoGrow();
   PtoGrow* g = state;
@@ -762,10 +847,21 @@ static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, c
   if (out_panic_code) for (int32_t r = 0; r < n; ++r) out_panic_code[r] = 0;
   if (out_counters) for (int64_t k = 0; k < 4 * (int64_t)n; ++k) out_counters[k] = 0;
   const int words = rrt ? 1 : ctx->mask_words, n_worlds = ctx->n_worlds;   // a tree's reach word is its committed bit
-  // SquareGoal::new (common.rs:304-350): world_to_goal, asserting that no world has two goals (:320)
-  std::vector<double> world_goal((size_t)n_worlds * 2, 0.0);
-  if (n_goals > 0 && porrt_square_goal_examples(goals_xy, goal_masks, n_goals, n_worlds, world_goal.data()) == PORRT_ERR_PANIC)
-    return porrt_fail(ctx, PORRT_ERR_PANIC, "SquareGoal: validities shouldn't overlap (common.rs:320)");
+  // SquareGoal::new (common.rs:304-350): world_to_goal of every goal set, asserting that no world has two goals (:320); wg[r] is
+  // roadmap r's table (one per run of equal goal slices)
+  std::vector<std::vector<double>> world_goals;
+  std::vector<size_t> wg((size_t)n);
+  for (int32_t r = 0; r < n; ++r) {
+    const PgQuery& q = qs[r];
+    if (r == 0 || q.g0 != qs[r - 1].g0 || q.g1 != qs[r - 1].g1) {
+      world_goals.emplace_back((size_t)n_worlds * 2, 0.0);
+      const size_t m = (size_t)ctx->mask_words;
+      if (q.g1 > q.g0 && porrt_square_goal_examples(goals_xy + 2 * q.g0, goal_masks + (size_t)q.g0 * m, (int32_t)(q.g1 - q.g0), n_worlds,
+                                                    world_goals.back().data()) == PORRT_ERR_PANIC)
+        return porrt_fail(ctx, PORRT_ERR_PANIC, "SquareGoal: validities shouldn't overlap (common.rs:320)");
+    }
+    wg[(size_t)r] = world_goals.size() - 1;
+  }
   for (int d = 0; d < 2; ++d)
     if (!(low[d] < up[d]) || !std::isfinite(low[d]) || !std::isfinite(up[d]))
       return porrt_fail(ctx, PORRT_ERR_PANIC, "ContinuousSampler: low < up required (rand asserts it)");
@@ -807,14 +903,15 @@ static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, c
     CUDA_TRY(ctx, r->fin_acc.ensure((size_t)words * 8));
   }
   if ((rc = pg_radius_table(ctx, g, cap0, max_step, search_radius, rrt))) return rc;
-  CUDA_TRY(ctx, g->goals.ensure((size_t)std::max(n_goals, 1) * 16));
-  CUDA_TRY(ctx, g->goal_masks.ensure((size_t)std::max(n_goals, 1) * words * 8));
+  CUDA_TRY(ctx, g->goals.ensure((size_t)std::max<int64_t>(n_goals, 1) * 16));
+  CUDA_TRY(ctx, g->goal_masks.ensure((size_t)std::max<int64_t>(n_goals, 1) * words * 8));
   CUDA_TRY(ctx, g->ctl.ensure((size_t)n * C_N * 4 + 64));
   CUDA_TRY(ctx, g->ctl_host.ensure((size_t)n * C_N * 4));
   CUDA_TRY(ctx, g->caps.ensure((size_t)n * 3 * 4));
   CUDA_TRY(ctx, g->pg_desc.ensure((size_t)n * sizeof(PgDev)));
   CUDA_TRY(ctx, g->spec_desc.ensure((size_t)n * sizeof(SpecDev)));
   if (rrt) CUDA_TRY(ctx, g->tree_desc.ensure((size_t)n * sizeof(RrtDev)));
+  if (rrt) CUDA_TRY(ctx, g->starts.ensure((size_t)n * 16));
   if (n_goals > 0) {
     CUDA_TRY(ctx, cudaMemcpyAsync(g->goals.p, goals_xy, (size_t)n_goals * 16, cudaMemcpyHostToDevice, st));
     CUDA_TRY(ctx, cudaMemcpyAsync(g->goal_masks.p, goal_masks, (size_t)n_goals * words * 8, cudaMemcpyHostToDevice, st));
@@ -828,7 +925,7 @@ static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, c
     SpecDev* sd = (SpecDev*)(desc.data() + (size_t)n * sizeof(PgDev));
     RrtDev* td = (RrtDev*)(desc.data() + (size_t)n * (sizeof(PgDev) + sizeof(SpecDev)));
     for (int32_t r = 0; r < n; ++r) {
-      pd[r] = pg_dev(ctx, g, g->roads[r].get(), ctl + (size_t)r * C_N, max_step, goal_max_dist, n_goals, n_iter_min, n_iter_max);
+      pd[r] = pg_dev(ctx, g, g->roads[r].get(), ctl + (size_t)r * C_N, max_step, qs[r], n_iter_min, n_iter_max);
       sd[r] = spec_dev(g->roads[r].get());
       if (rrt) td[r] = RrtDev{g->roads[r]->tparent.as<int32_t>(), g->roads[r]->dist.as<double>()};
     }
@@ -863,6 +960,7 @@ static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, c
   auto draw = [&](int32_t r, int64_t upto) -> int32_t {
     PgStream& h = hs[(size_t)r];
     PtoRoad* d = g->roads[r].get();
+    const std::vector<double>& world_goal = world_goals[wg[(size_t)r]];
     upto = std::min(upto, bound);
     if (upto <= h.drawn) return PORRT_OK;
     const int64_t m = upto - h.drawn;
@@ -892,8 +990,14 @@ static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, c
     return PORRT_OK;
   };
   if ((rc = upload_desc())) return rc;
-  if (rrt) rrt_init_kernel<<<div_up(n, 128), 128, 0, st>>>(g->pg_desc.as<PgDev>(), g->tree_desc.as<RrtDev>(), make_double2(start[0], start[1]), n);
-  else pto_init_kernel<<<n, 64, 0, st>>>(ctx->map, g->pg_desc.as<PgDev>(), make_double2(start[0], start[1]));
+  std::vector<double> starts;                 // read by the copy below until the first look synchronises
+  if (rrt) {
+    for (int32_t r = 0; r < n; ++r) starts.insert(starts.end(), qs[r].start, qs[r].start + 2);
+    CUDA_TRY(ctx, cudaMemcpyAsync(g->starts.p, starts.data(), (size_t)n * 16, cudaMemcpyHostToDevice, st));
+    rrt_init_kernel<<<div_up(n, 128), 128, 0, st>>>(g->pg_desc.as<PgDev>(), g->tree_desc.as<RrtDev>(), g->starts.as<double2>(), n);
+  } else {
+    pto_init_kernel<<<n, 64, 0, st>>>(ctx->map, g->pg_desc.as<PgDev>(), make_double2(qs[0].start[0], qs[0].start[1]));
+  }
   LAUNCH_CHECK(ctx);
   if (runs) for (int32_t r = 0; r < n; ++r) if ((rc = draw(r, n_iter_min + 4096))) return rc;
   if ((rc = upload_caps())) return rc;
@@ -1026,6 +1130,12 @@ static int32_t grow_impl(porrt_ctx* ctx, const char* who, bool rrt, int32_t n, c
   return PORRT_OK;
 }
 
+// one start and one goal set for every roadmap / tree; empty (grow_impl refuses it) when there is no start or n is out of range
+static std::vector<PgQuery> shared_queries(int32_t n, const double start[2], int32_t n_goals, double goal_max_dist) {
+  if (!start || n < 1 || n > PORRT_PTO_MAX_ROADMAPS) return {};
+  return std::vector<PgQuery>((size_t)n, PgQuery{{start[0], start[1]}, 0, n_goals, goal_max_dist});
+}
+
 PORRT_API int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const double low[2], const double up[2], uint64_t sampler_seed,
                                  const double* goals_xy, const uint64_t* goal_masks, int32_t n_goals, double goal_max_dist,
                                  double max_step, double search_radius, int64_t n_iter_min, int64_t n_iter_max,
@@ -1034,8 +1144,9 @@ PORRT_API int32_t porrt_pto_grow(porrt_ctx* ctx, const double start[2], const do
   if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
   if (!out_complete) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_pto_grow: bad arguments");
   int32_t status = 0, panic = 0;
-  const int32_t rc = grow_impl(ctx, "porrt_pto_grow", false, 1, &sampler_seed, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
-                               max_step, search_radius, n_iter_min, n_iter_max, out_sizes, &status, &panic, out_counters);
+  const std::vector<PgQuery> qs = shared_queries(1, start, n_goals, goal_max_dist);
+  const int32_t rc = grow_impl(ctx, "porrt_pto_grow", false, 1, &sampler_seed, qs.empty() ? nullptr : qs.data(), low, up, goals_xy, goal_masks,
+                               n_goals, max_step, search_radius, n_iter_min, n_iter_max, out_sizes, &status, &panic, out_counters);
   *out_complete = rc == PORRT_OK && status == 0 ? 1 : 0;
   if (rc) return rc;
   if (out_panic_code) *out_panic_code = panic;
@@ -1049,8 +1160,9 @@ PORRT_API int32_t porrt_pto_grow_batch(porrt_ctx* ctx, int32_t n_roadmaps, const
                                        int32_t n_goals, double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min,
                                        int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code,
                                        int64_t* out_counters) {
-  return grow_impl(ctx, "porrt_pto_grow_batch", false, n_roadmaps, sampler_seeds, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
-                   max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
+  const std::vector<PgQuery> qs = shared_queries(n_roadmaps, start, n_goals, goal_max_dist);
+  return grow_impl(ctx, "porrt_pto_grow_batch", false, n_roadmaps, sampler_seeds, qs.empty() ? nullptr : qs.data(), low, up, goals_xy,
+                   goal_masks, n_goals, max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
 }
 
 PORRT_API int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr,
@@ -1096,8 +1208,9 @@ PORRT_API int32_t porrt_rrt_grow_batch(porrt_ctx* ctx, int32_t n_trees, const ui
                                        int32_t n_goals, double goal_max_dist, double max_step, double search_radius, int64_t n_iter_min,
                                        int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status, int32_t* out_panic_code,
                                        int64_t* out_counters) {
-  return grow_impl(ctx, "porrt_rrt_grow_batch", true, n_trees, sampler_seeds, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
-                   max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
+  const std::vector<PgQuery> qs = shared_queries(n_trees, start, n_goals, goal_max_dist);
+  return grow_impl(ctx, "porrt_rrt_grow_batch", true, n_trees, sampler_seeds, qs.empty() ? nullptr : qs.data(), low, up, goals_xy,
+                   goal_masks, n_goals, max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
 }
 
 PORRT_API int32_t porrt_rrt_grow(porrt_ctx* ctx, uint64_t sampler_seed, const double start[2], const double low[2], const double up[2],
@@ -1107,8 +1220,9 @@ PORRT_API int32_t porrt_rrt_grow(porrt_ctx* ctx, uint64_t sampler_seed, const do
   CTX_CHECK(ctx);
   if (!out_status) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_grow: bad arguments");
   int32_t panic = 0;
-  const int32_t rc = grow_impl(ctx, "porrt_rrt_grow", true, 1, &sampler_seed, start, low, up, goals_xy, goal_masks, n_goals, goal_max_dist,
-                               max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, &panic, out_counters);
+  const std::vector<PgQuery> qs = shared_queries(1, start, n_goals, goal_max_dist);
+  const int32_t rc = grow_impl(ctx, "porrt_rrt_grow", true, 1, &sampler_seed, qs.empty() ? nullptr : qs.data(), low, up, goals_xy, goal_masks,
+                               n_goals, max_step, search_radius, n_iter_min, n_iter_max, out_sizes, out_status, &panic, out_counters);
   if (rc) return rc;
   if (out_panic_code) *out_panic_code = panic;
   if (*out_status != PORRT_ERR_PANIC) return PORRT_OK;
@@ -1134,5 +1248,81 @@ PORRT_API int32_t porrt_rrt_fetch_tree(porrt_ctx* ctx, int32_t t, double* out_xy
   if (out_final_ids && F) CUDA_TRY(ctx, cudaMemcpyAsync(ids.data(), g->fin_ids.p, (size_t)F * 4, cudaMemcpyDeviceToHost, st));
   CUDA_TRY(ctx, cudaStreamSynchronize(st));
   if (out_final_ids) for (int64_t k = 0; k < F; ++k) out_final_ids[k] = ids[(size_t)k];
+  return PORRT_OK;
+}
+
+PORRT_API int32_t porrt_rrt_grow_queries(porrt_ctx* ctx, int32_t n_trees, const uint64_t* sampler_seeds, const double* starts,
+                                         const double low[2], const double up[2], const int64_t* goal_ptr, const double* goals_xy,
+                                         const uint64_t* goal_masks, const double* goal_max_dist, double max_step, double search_radius,
+                                         int64_t n_iter_min, int64_t n_iter_max, int64_t* out_sizes, int32_t* out_status,
+                                         int32_t* out_panic_code, int64_t* out_counters) {
+  CTX_CHECK(ctx);
+  if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
+  const char* who = "porrt_rrt_grow_queries";
+  if (n_trees < 1 || n_trees > PORRT_PTO_MAX_ROADMAPS)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": n_trees must be in 1 .. " + std::to_string(PORRT_PTO_MAX_ROADMAPS));
+  if (!starts || !goal_ptr || !goal_max_dist) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": bad arguments");
+  if (goal_ptr[0] != 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": goal_ptr[0] must be 0");
+  std::vector<PgQuery> qs((size_t)n_trees);
+  for (int32_t t = 0; t < n_trees; ++t) {
+    const std::string q = std::string(who) + ": query " + std::to_string(t);
+    const int64_t g0 = goal_ptr[t], g1 = goal_ptr[t + 1];
+    if (g1 < g0 || g1 - g0 > INT32_MAX) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, q + ": goal_ptr is not monotone");
+    if (!std::isfinite(starts[2 * t]) || !std::isfinite(starts[2 * t + 1]))
+      return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, q + ": the start is not finite");
+    if (!(goal_max_dist[t] >= 0.0)) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, q + ": goal_max_dist is negative or NaN");
+    qs[(size_t)t] = PgQuery{{starts[2 * t], starts[2 * t + 1]}, g0, g1, goal_max_dist[t]};
+  }
+  if (goal_ptr[n_trees] > 0 && (!goals_xy || !goal_masks)) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, std::string(who) + ": bad arguments");
+  std::vector<double> examples((size_t)ctx->n_worlds * 2);   // SquareGoal::new of every query (common.rs:320)
+  for (int32_t t = 0; t < n_trees; ++t) {
+    const PgQuery& q = qs[(size_t)t];
+    if (q.g1 > q.g0 && porrt_square_goal_examples(goals_xy + 2 * q.g0, goal_masks + (size_t)q.g0 * ctx->mask_words, (int32_t)(q.g1 - q.g0),
+                                                  ctx->n_worlds, examples.data()) == PORRT_ERR_PANIC)
+      return porrt_fail(ctx, PORRT_ERR_PANIC, std::string(who) + ": query " + std::to_string(t) +
+                                              ": SquareGoal: validities shouldn't overlap (common.rs:320)");
+  }
+  return grow_impl(ctx, who, true, n_trees, sampler_seeds, qs.data(), low, up, goals_xy, goal_masks, goal_ptr[n_trees], max_step,
+                   search_radius, n_iter_min, n_iter_max, out_sizes, out_status, out_panic_code, out_counters);
+}
+
+PORRT_API int32_t porrt_rrt_best_paths(porrt_ctx* ctx, int32_t* out_final, double* out_cost, int64_t* out_path_ptr, double* out_path_xy,
+                                       int64_t cap, int64_t* out_total) {
+  CTX_CHECK(ctx);
+  PtoGrow* rg = ctx->rrt;
+  if (!rg || rg->n_have == 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_best_paths: no tree grown on this ctx");
+  if (!out_final || !out_cost || !out_path_ptr || !out_total || cap < 0 || (cap > 0 && !out_path_xy))
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_rrt_best_paths: bad arguments");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const int32_t n = rg->n_have;
+  CUDA_TRY(ctx, rg->best.ensure((size_t)n * sizeof(RrtBest) + (size_t)(n + 1) * 8));
+  RrtBest* best_dev = rg->best.as<RrtBest>();
+  int64_t* ptr_dev = (int64_t*)(best_dev + n);
+  rrt_best_kernel<<<n, PG_COMMIT_THREADS, 0, st>>>(rg->pg_desc.as<PgDev>(), rg->spec_desc.as<SpecDev>(), rg->tree_desc.as<RrtDev>(), best_dev);
+  LAUNCH_CHECK(ctx);
+  std::vector<RrtBest> best((size_t)n);
+  CUDA_TRY(ctx, cudaMemcpyAsync(best.data(), best_dev, (size_t)n * sizeof(RrtBest), cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  out_path_ptr[0] = 0;
+  for (int32_t t = 0; t < n; ++t) {
+    if (best[(size_t)t].cycle)
+      return porrt_fail(ctx, PORRT_ERR_INTERNAL, "porrt_rrt_best_paths: the tree parents of tree " + std::to_string(t) + " form a cycle");
+    out_final[t] = best[(size_t)t].final_id;
+    out_cost[t] = best[(size_t)t].cost;
+    out_path_ptr[t + 1] = out_path_ptr[t] + best[(size_t)t].len;
+  }
+  const int64_t total = out_path_ptr[n];
+  *out_total = total;
+  if (total > cap)
+    return porrt_fail(ctx, PORRT_ERR_CAPACITY, "porrt_rrt_best_paths: " + std::to_string(total) + " path states, cap " + std::to_string(cap));
+  if (total == 0) return PORRT_OK;
+  CUDA_TRY(ctx, rg->paths.ensure((size_t)total * 16));
+  CUDA_TRY(ctx, cudaMemcpyAsync(ptr_dev, out_path_ptr, (size_t)(n + 1) * 8, cudaMemcpyHostToDevice, st));
+  rrt_path_kernel<<<div_up(n, 128), 128, 0, st>>>(rg->pg_desc.as<PgDev>(), rg->tree_desc.as<RrtDev>(), best_dev, ptr_dev,
+                                                  rg->paths.as<double2>(), n);
+  LAUNCH_CHECK(ctx);
+  CUDA_TRY(ctx, cudaMemcpyAsync(out_path_xy, rg->paths.p, (size_t)total * 16, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
   return PORRT_OK;
 }
