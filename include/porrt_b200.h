@@ -72,6 +72,8 @@ const char* porrt_last_error(porrt_ctx* ctx);
 #define PORRT_OPT_FORCE_THREAD_PER_QUERY_NN 3  /* value != 0: radius / 1-NN / k-NN queries skip the tile kernels and run the
                                              thread-per-query ring search (used by itself for batches < 2048 queries and for
                                              the queries the tiles cannot serve) */
+#define PORRT_OPT_PRM_PATHS_CHUNK_COLUMNS 4  /* value > 0: porrt_prm_plan_paths solves at most `value` goal columns per chunk (the
+                                             chunks are otherwise sized by PORRT_PRM_PATHS_TABLE_BYTES); 0 restores that */
 int32_t porrt_ctx_set_option(porrt_ctx* ctx, int32_t option, int64_t value);
 /* number of kernels this ctx has launched so far (bench.py's gpu_launches) */
 int64_t porrt_ctx_launch_count(porrt_ctx* ctx);
@@ -203,6 +205,37 @@ int32_t porrt_sssp_worlds(porrt_ctx* ctx, int64_t V, const int64_t* row_ptr, con
  * Both calls: porrt_ctx_last_phase_ms = [device ms of the backups, edge records / (parent, world) pairs worked through]. */
 int32_t porrt_sssp_worlds_prm(porrt_ctx* ctx, const int64_t* finals_ptr, const int32_t* finals_ids, double* out_dist,
                               int32_t* out_sweeps);
+
+/* PRM::plan_path (prm.rs:111-122) with extract_path (pto_graph.rs:305-359) for n (start, goal) pairs, on the roadmap the last
+ * porrt_prm_build on this ctx left on the device (its CSR and the vertex coordinates in id order); only the paths are copied back.
+ * Per query q, with start = starts_xy[2q ..] and goal = goals_xy[2q ..]:
+ *  - s = KdTree::nearest_neighbor(start), g = KdTree::nearest_neighbor(goal): over all vertices, unfiltered; ties on norm2 go as the
+ *    reference's nn_inner breaks them (strict <, near side first), so an exact tie between distinct vertices is decided by the
+ *    kd order, not by the lowest id;
+ *  - cost = dijkstra(graph, [g]) on the plain graph (no world view): the column porrt_sssp_worlds gives with n_worlds = 0 and the
+ *    finals {g}; out_cost[q] = cost[s];
+ *  - the path: from s, while cost[node] != 0.0, move to the first parent p in stored order (for a PRM the parents of a node are its
+ *    CSR row) that minimises cost[p] + norm2(state[p], state[node]) (Iterator::min_by; the no-FMA norm2 of common.rs:203-213);
+ *    the states of the visited nodes, s first, are out_path_xy[2 * out_path_ptr[q] .. 2 * out_path_ptr[q + 1]] (out_path_ptr[n + 1]).
+ *    s == g gives one state and cost 0.
+ * out_status[q]: PORRT_PATH_FOUND; PORRT_PATH_NONE when cost[s] is +inf (empty path, cost +inf: the oracle's plan_path returns no
+ * path there); PORRT_PATH_CYCLE when the walk makes V steps without reaching a node of cost 0.0 -- an edge too short to lower an f64
+ * cost, e.g. duplicate samples joined by a zero-length edge, where the reference never returns (empty path, out_cost = cost[s]).
+ * out_start_node / out_goal_node (nullable [n]) = s and g.  The goal columns are solved in chunks of at most
+ * PORRT_PRM_PATHS_TABLE_BYTES of table each; results do not depend on the order or grouping of the queries, the chunking, the
+ * column schedule (PORRT_OPT_FORCE_GLOBAL_SWEEPS) or the 1-NN kernels (PORRT_OPT_FORCE_THREAD_PER_QUERY_NN).  On a ctx with a
+ * communicator every rank answers its own queries, with no collective.
+ * cap (in states) smaller than the total path length: PORRT_ERR_CAPACITY with *out_total set (and the node ids, out_cost, out_status
+ * and out_path_ptr filled).  n == 0 is valid.  PORRT_ERR_INVALID_ARG for n < 0, a null required pointer, a coordinate that is not
+ * finite, no PRM built on this ctx, a last PRM result that is porrt_mmprm_plan's grouped build, and a vertex set replaced or extended
+ * (porrt_vertices_set, _set_dev, _append) since the build. */
+#define PORRT_PATH_FOUND 0
+#define PORRT_PATH_NONE 1
+#define PORRT_PATH_CYCLE 2
+#define PORRT_PRM_PATHS_TABLE_BYTES 1073741824   /* 1 GiB: one chunk's goal columns (8 V bytes each; 134 columns at 1e6 nodes) */
+int32_t porrt_prm_plan_paths(porrt_ctx* ctx, const double* starts_xy, const double* goals_xy, int64_t n, int32_t* out_start_node,
+                             int32_t* out_goal_node, double* out_cost, int32_t* out_status, int64_t* out_path_ptr, double* out_path_xy,
+                             int64_t cap, int64_t* out_total);
 
 /* PTO::build_belief_graph + compute_expected_costs_to_goals (pto.rs:185-275, belief_graph.rs:89-182) on the IMPLICIT
  * belief graph (belief node id = node * B + belief):

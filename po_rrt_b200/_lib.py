@@ -60,6 +60,7 @@ SIGNATURES = {
     "porrt_prm_build": (i32, [vp, vp, i64, f64, f64, vp, vp, i64, pp(i64), vp]),
     "porrt_prm_fetch": (i32, [vp, vp, vp, i64]),
     "porrt_sssp_worlds_prm": (i32, [vp, vp, vp, vp, pp(i32)]),
+    "porrt_prm_plan_paths": (i32, [vp, vp, vp, i64, vp, vp, vp, vp, vp, vp, i64, pp(i64)]),
     "porrt_sssp_worlds": (i32, [vp, i64, vp, vp, vp, vp, vp, i32, i32, i32, vp, vp, vp, pp(i32)]),
     "porrt_policy_decompose": (i32, [vp, i64, vp, vp, vp, vp, i32, pp(i32)]),
     "porrt_policy_expected_cost": (i32, [vp, vp, vp, i64, vp, i32, i32, pp(f64)]),

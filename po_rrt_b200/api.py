@@ -23,6 +23,8 @@ ERR_CAPACITY = 4
 OPT_FORCE_LARGE_MAP_PATH = 1
 OPT_FORCE_GLOBAL_SWEEPS = 2
 OPT_FORCE_THREAD_PER_QUERY_NN = 3
+OPT_PRM_PATHS_CHUNK_COLUMNS = 4
+PATH_FOUND, PATH_NONE, PATH_CYCLE = 0, 1, 2   # PORRT_PATH_* (porrt_prm_plan_paths)
 PTO_MAX_ROADMAPS = 65535   # PORRT_PTO_MAX_ROADMAPS
 
 
@@ -414,6 +416,34 @@ class PRM:
             self.ctx.check(self.ctx.lib.porrt_prm_fetch(self.ctx.h, None, _p(col), len(col)))
         self.states, self.row_ptr, self.col = xy, row_ptr, col[:n_edges.value]
         return self
+
+    def plan_paths(self, starts, goals):
+        """PRM::plan_path (prm.rs:111-122) for every (start, goal) row, on the roadmap the last PRM build of this context left on the
+        device (porrt_prm_plan_paths; only the paths come back).  -> (paths: a list of [L, 2] arrays, cost[n], status[n] (PATH_*),
+        start_node[n], goal_node[n]); a query whose status is not PATH_FOUND has an empty path"""
+        s, g = _f64(starts, 2), _f64(goals, 2)
+        if len(s) != len(g):
+            raise ValueError("plan_paths: %d starts, %d goals" % (len(s), len(g)))
+        n = len(s)
+        sn, gn, st = np.empty(max(n, 1), np.int32), np.empty(max(n, 1), np.int32), np.empty(max(n, 1), np.int32)
+        cost, ptr, total = np.empty(max(n, 1)), np.empty(n + 1, np.int64), C.c_int64()
+        cap = 64 * n
+        while True:
+            xy = np.empty((max(cap, 1), 2))
+            rc = self.ctx.lib.porrt_prm_plan_paths(self.ctx.h, _p(s), _p(g), n, _p(sn), _p(gn), _p(cost), _p(st), _p(ptr), _p(xy), cap,
+                                                   C.byref(total))
+            if rc == ERR_CAPACITY and total.value > cap:
+                cap = total.value
+                continue
+            self.ctx.check(rc)
+            paths = [xy[ptr[q]:ptr[q + 1]].copy() for q in range(n)]
+            return paths, cost[:n].copy(), st[:n].copy(), sn[:n].copy(), gn[:n].copy()
+
+    def plan_path(self, start, goal):
+        """PRM::plan_path for one query, as the oracle's PRM.plan_path returns it: the path [L, 2], or an empty (0, 2) array when
+        there is none (status PATH_NONE or PATH_CYCLE)"""
+        paths, _, status, _, _ = self.plan_paths([start], [goal])
+        return paths[0] if status[0] == PATH_FOUND else np.zeros((0, 2))
 
 
 def dijkstra_worlds(ctx, row_ptr, col, xy, node_vid, validities_words, finals_per_world):

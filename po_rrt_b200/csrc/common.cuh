@@ -138,6 +138,7 @@ struct porrt_ctx {
 
   // ---- vertices / cell grid (nn.cu)
   int64_t n_vertices = 0;          // vertices in d_vxy (upload order), including appended ones
+  int64_t vertex_gen = 0;          // bumped by every porrt_vertices_set / _set_dev / _append: a PRM query knows its roadmap's set
   bool grid_stale = false;         // porrt_vertices_append: the cell grid below is rebuilt on the device before the next query
   double cell_request = 0.0;       // cell size asked for by the last porrt_vertices_set (<= 0: from the density)
   double cell = 0, inv_cell = 0, org_x = 0, org_y = 0;
@@ -216,6 +217,9 @@ struct porrt_ctx {
   const int32_t* prm_col = nullptr;
   const void* radii_ptr = nullptr; int64_t radii_lo = 0, radii_n = 0; double radii_ms = 0, radii_sr = 0;   // what pin_radii holds: heuristic_radius(k + 1) for k in [radii_lo, radii_n)
   DevBuf d_prm_row, d_prm_col;         // dedicated: the retained CSR must survive later calls that reuse the shared scratch
+  bool prm_grouped = false;            // the last PRM result is porrt_mmprm_plan's grouped build (its vertex set mixes modes)
+  int64_t prm_vertex_gen = -1;         // vertex_gen when the last PRM build bound its vertex set
+  int64_t prm_paths_chunk = 0;         // PORRT_OPT_PRM_PATHS_CHUNK_COLUMNS (tests): > 0 caps porrt_prm_plan_paths' columns per chunk
 
   // ---- last multi-modal PRM result (mmprm.cu): the explicit belief graph, kept for porrt_mmprm_fetch_graph
   struct MmPrm_ {
@@ -239,9 +243,12 @@ struct porrt_ctx {
   DevBuf ws_main;     // the entry points' inputs and work blocks: porrt_radius_query, knn_host, porrt_state_validity, porrt_visibility,
                       // porrt_transition_valid, the shortcut and Reparent refiners, porrt_sssp_worlds(_prm) and porrt_belief_vi (held
                       // while graph.cu's value-column driver runs, which carves from ws_state),
-                      // porrt_conditional_dijkstra_graph, the PRM build's per-node arrays; edge_pipeline's chunk slots
-  DevBuf ws_owner;    // map upload: the occupancy image; PRM build: the owner of each candidate, then the packed neighbour lists
-  DevBuf ws_vid;      // map upload: the zone image; PRM build: the candidates' validity ids, then the late lists and cursors
+                      // porrt_conditional_dijkstra_graph, the PRM build's per-node arrays; edge_pipeline's chunk slots;
+                      // porrt_prm_plan_paths' queries and per-query results (held while the 1-NN, the kd rank and sssp_core run)
+  DevBuf ws_owner;    // map upload: the occupancy image; PRM build: the owner of each candidate, then the packed neighbour lists;
+                      // porrt_prm_plan_paths: the paths in query order
+  DevBuf ws_vid;      // map upload: the zone image; PRM build: the candidates' validity ids, then the late lists and cursors;
+                      // porrt_prm_plan_paths: the paths in chunk order, as the walks write them
   DevBuf ws_table;    // map upload: zone statistics; the radius id lists of porrt_radius_query and the PRM build
                       // (nn_radius_count_fill_dev's ids_buf); sssp_core's world table, world masks and column map;
                       // belief_download_full's [node][belief] table
@@ -401,6 +408,8 @@ int32_t nn_tile_knn(porrt_ctx* ctx, const GridDev& g, const double* q_dev, int64
 // nn.cu helpers used by graph.cu
 int32_t nn_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, double cell_size, const double* lo, const double* hi);
 int32_t nn_flush_appended(porrt_ctx* ctx);   // re-bins the vertex set if porrt_vertices_append left it stale
+int32_t nn_knn_dev(porrt_ctx* ctx, const double* q_dev, int64_t m, int k, const uint64_t* reach_dev, const uint32_t* world_dev,
+                   int32_t* ids_dev, double* dist_dev, int32_t* ties_dev);   // knn_host's kernels on device inputs / outputs
 int32_t nn_radius_count_fill_dev(porrt_ctx* ctx, const double* q_dev, const double* radius_dev, int64_t m,
                                  const uint32_t* prefix_dev, const uint64_t* reach_dev, const uint32_t* world_dev,
                                  int64_t* offsets_dev /* [m+1] */, DevBuf* ids_buf, int64_t* total_out,

@@ -167,6 +167,18 @@ __global__ void kd_init_kernel(int64_t n, int32_t* __restrict__ cur, int32_t* __
   size[i] = 0; node_depth[i] = i == root ? 0 : -1; rank[i] = i == root ? (int32_t)root : 0;
 }
 
+// kd_preorder_rank_dev's work space in ctx->kd_buf.  After a rank, child[2 i + side] (0x7fffffff = none) and parent[i] (i > 0) are
+// the links of the tree; node_depth may have been reused as a buffer by then.
+struct KdWork { int32_t *cur, *child, *size, *parent, *node_depth, *exits, *up, *remaining; uint8_t* side; };
+static void kd_work_layout(Carve& c, int64_t n, KdWork& w) {
+  w.cur = c.take<int32_t>(n); w.child = c.take<int32_t>(2 * n); w.size = c.take<int32_t>(n); w.parent = c.take<int32_t>(n);
+  w.node_depth = c.take<int32_t>(n);
+  w.exits = c.take<int32_t>(n);     // two-phase start only
+  w.up = c.take<int32_t>(n);
+  w.remaining = c.take<int32_t>(2);
+  w.side = c.take<uint8_t>(n);
+}
+
 // xy_dev: n vertices (device); out_rank_dev[n]; work space ctx->kd_buf
 int32_t kd_preorder_rank_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, int32_t* out_rank_dev, const uint32_t* root_of_dev,
                              cudaStream_t st_in, std::string* err, int64_t* n_launch) {
@@ -180,16 +192,11 @@ int32_t kd_preorder_rank_dev(porrt_ctx* ctx, const double* xy_dev, int64_t n, in
 #define KD_TRY(expr) do { cudaError_t _e = (expr); if (_e != cudaSuccess) return fail(#expr, _e); } while (0)
 #define KD_LAUNCHED() do { ++launches; KD_TRY(cudaGetLastError()); } while (0)
   if (n <= 0) return PORRT_OK;
-  int32_t *cur, *child, *size, *parent, *node_depth, *exits, *up, *remaining;
-  uint8_t* side;
-  KD_TRY(carve(ctx->kd_buf, [&](Carve& c) {
-    cur = c.take<int32_t>(n); child = c.take<int32_t>(2 * n); size = c.take<int32_t>(n); parent = c.take<int32_t>(n);
-    node_depth = c.take<int32_t>(n);
-    exits = c.take<int32_t>(n);     // two-phase start only
-    up = c.take<int32_t>(n);
-    remaining = c.take<int32_t>(2);
-    side = c.take<uint8_t>(n);
-  }));
+  KdWork w;
+  KD_TRY(carve(ctx->kd_buf, [&](Carve& c) { kd_work_layout(c, n, w); }));
+  int32_t *cur = w.cur, *child = w.child, *size = w.size, *parent = w.parent, *node_depth = w.node_depth, *exits = w.exits, *up = w.up;
+  int32_t* remaining = w.remaining;
+  uint8_t* side = w.side;
   int32_t* max_depth = remaining + 1;
   const int blocks = div_up(n, 256);
   kd_init_kernel<<<blocks, 256, 0, st>>>(n, cur, child, size, node_depth, out_rank_dev, root_of_dev);
@@ -757,6 +764,7 @@ int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, doub
   ph[7] = (double)total;
   if (out_phase_ms) memcpy(out_phase_ms, ph, sizeof(ph));
   ctx->prm_n = n; ctx->prm_edges = n_edges; ctx->prm_row_ptr = d_row_ptr; ctx->prm_col = d_col;  // retained for porrt_prm_fetch
+  ctx->prm_grouped = gb != nullptr; ctx->prm_vertex_gen = ctx->vertex_gen;                        // and for porrt_prm_plan_paths
   return status;
 }
 
@@ -1025,12 +1033,13 @@ static int32_t value_columns_solve(porrt_ctx* ctx, ValueColumns& vc, int32_t* ou
 
 // plan_qmdp on a graph that already lives on the device (all d_* are device pointers; h_val = host copy of the validity table): one
 // value column per world.  out_dist (host, [Wall][V]) may be null: the table then stays on the device only (timing, device-resident
-// pipelines).  Work space: ws_table; porrt_ctx_last_phase_ms afterwards: [0] device ms from the graph preparation to the end of the
-// backups, [1] edge records / (parent, world) pairs worked through.
+// pipelines).  out_table_dev (nullable): the device table, [world][node] for an unsharded call (valid until ws_table is carved again).
+// Work space: ws_table; porrt_ctx_last_phase_ms afterwards: [0] device ms from the graph preparation to the end of the backups,
+// [1] edge records / (parent, world) pairs worked through.
 static int32_t sssp_core(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_col, const double* d_xy, int64_t V, int64_t E,
                          const int32_t* d_nvid, const uint64_t* d_val, const uint64_t* h_val, int32_t n_validities, int32_t mask_words,
                          bool world_view, int Wall, const int64_t* finals_ptr, const int32_t* finals_ids, double* out_dist,
-                         int32_t* out_sweeps) {
+                         int32_t* out_sweeps, const double** out_table_dev = nullptr) {
   cudaStream_t st = ctx->stream;
   // multi-GPU (comm.cu): the worlds are independent problems on one graph, sharded over the ranks and all-gathered (SURVEY 8(e));
   // the plain-graph call (n_worlds == 0) is not sharded
@@ -1081,6 +1090,7 @@ static int32_t sssp_core(porrt_ctx* ctx, const int64_t* d_row, const int32_t* d_
   tfinish(ctx);
   ctx->last_ms[1] = offers; ctx->n_last = 2;
   if (out_sweeps) *out_sweeps = sweeps;
+  if (out_table_dev) *out_table_dev = d_out;
   return PORRT_OK;
 }
 
@@ -1146,6 +1156,282 @@ PORRT_API int32_t porrt_sssp_worlds_prm(porrt_ctx* ctx, const int64_t* finals_pt
   LAUNCH_CHECK(ctx);
   return sssp_core(ctx, ctx->prm_row_ptr, ctx->prm_col, ctx->d_vxy.as<double>(), V, E, d_nvid, d_val, val.data(), nv + 1, ctx->mask_words, true,
                    ctx->n_worlds, finals_ptr, finals_ids, out_dist, out_sweeps);
+}
+
+// ================================================================================================ PRM path queries
+// PRM::plan_path (prm.rs:111-122) for a batch of (start, goal) pairs on the roadmap the last PRM build left on the device
+// (DESIGN 3.4): the 1-NN of all 2n points (tile / ring kernels of nn.cu, kd replay where norm2 ties), one value column per distinct
+// goal node through the value-column driver (sssp_core, plain graph), solved in chunks of PORRT_PRM_PATHS_TABLE_BYTES, and after each
+// chunk extract_path (pto_graph.rs:305-359) for the queries whose goal is in it: a length pass, then a pass that writes the states.
+
+// norm2 (common.rs:203-213) with the reference's operand order and no FMA
+__device__ __forceinline__ double pq_norm2(double2 a, double2 b) {
+  const double dx = __dsub_rn(b.x, a.x), dy = __dsub_rn(b.y, a.y);
+  return __dsqrt_rn(__dadd_rn(__dmul_rn(dx, dx), __dmul_rn(dy, dy)));
+}
+
+// nn_inner (nearest_neighbor.rs:58-88) replayed without a stack on the kd links kd_preorder_rank_dev leaves in kd_buf (child
+// 0x7fffffff = none; kd node i = vertex i): strict <, near side first, the far side's test evaluated with dmin as it stands after the
+// near side.  The split axis is the depth parity, tracked on the way (node_depth is not kept by the rank).  One thread per query of
+// list[n]: out[i] = the reference's nearest vertex of query list[i].
+__global__ void prm_nn_replay_kernel(const double2* __restrict__ xy, const int32_t* __restrict__ child, const int32_t* __restrict__ parent,
+                                     const double2* __restrict__ q, const int32_t* __restrict__ list, int32_t n, int32_t* __restrict__ out) {
+  const int32_t i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= n) return;
+  const double2 p = q[list[i]];
+  double dmin = INFINITY;
+  int32_t nearest = 0, cur = 0, from = -1, depth = 0;   // from: the child we just came back from (-1: entering cur)
+  for (;;) {
+    const double2 v = xy[cur];
+    const bool ax = depth & 1;
+    const double qa = ax ? p.y : p.x, na = ax ? v.y : v.x;
+    const int32_t l = child[2 * (int64_t)cur], r = child[2 * (int64_t)cur + 1];
+    const bool near_left = qa < na;
+    const int32_t first = near_left ? l : r, second = near_left ? r : l;
+    int32_t next = -1;
+    if (from < 0) {
+      const double d = pq_norm2(v, p);
+      if (d < dmin) { dmin = d; nearest = cur; }
+      const bool c1 = near_left ? __dsub_rn(qa, dmin) < na : __dadd_rn(qa, dmin) >= na;
+      if (c1 && first != 0x7fffffff) next = first;
+    }
+    if (next < 0 && (from < 0 || from == first)) {
+      const bool c2 = near_left ? __dadd_rn(qa, dmin) >= na : __dsub_rn(qa, dmin) < na;
+      if (c2 && second != 0x7fffffff) next = second;
+    }
+    if (next >= 0) { cur = next; from = -1; ++depth; continue; }
+    if (cur == 0) break;
+    from = cur; cur = parent[cur]; --depth;
+  }
+  out[i] = nearest;
+}
+
+// The queries of one chunk of goal columns.  Query slots are positions in the order sorted by (goal column, query index): the chunk's
+// queries are the slots [s0, s0 + n_slots), and every per-slot array below is indexed by slot.
+struct PrmWalk {
+  const int64_t* row; const int32_t* col; const double2* xy;
+  const double* table; int64_t V;     // the chunk's columns, [column - c0][node]
+  int32_t c0;
+  const int32_t* start; const int32_t* gcol;   // [slot] start node, goal column
+  int32_t* len; int32_t* status; double* cost;  // [slot] pass 1
+  const int64_t* stage_off; double2* stage;     // [slot] pass 2: where the slot's states go
+};
+
+// extract_path, one warp per query: the lanes stride over the node's CSR row (= its parents, in stored order) and a warp arg-min over
+// (value, position) keeps the first minimum (Iterator::min_by).  PATHS = false: length and status (a cycle is found by Brent's
+// method: the walk is a function of the node, so it repeats a node iff it would make V steps without reaching cost 0.0);
+// PATHS = true: the states of the FOUND queries.
+template <bool PATHS>
+__global__ void __launch_bounds__(256) prm_walk_kernel(PrmWalk w, int32_t s0, int32_t n_slots) {
+  const int lane = threadIdx.x & 31;
+  const int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (k >= n_slots) return;                    // whole warps leave together
+  const int32_t slot = s0 + (int32_t)k;
+  const double* cost = w.table + (int64_t)(w.gcol[slot] - w.c0) * w.V;
+  int32_t node = w.start[slot];
+  double c = cost[node];
+  if (PATHS && w.status[slot] != PORRT_PATH_FOUND) return;
+  if (!PATHS && isinf(c)) {
+    if (lane == 0) { w.len[slot] = 0; w.status[slot] = PORRT_PATH_NONE; w.cost[slot] = c; }
+    return;
+  }
+  double2* out = PATHS ? w.stage + w.stage_off[slot] : nullptr;
+  if (PATHS && lane == 0) out[0] = w.xy[node];
+  int64_t n_states = 1;
+  int32_t tortoise = node;
+  int64_t power = 1, lam = 0;
+  bool cycle = false;
+  while (c != 0.0) {
+    const double2 x = w.xy[node];
+    const int64_t e1 = w.row[node + 1];
+    double bv = INFINITY;
+    int64_t be = INT64_MAX;
+    for (int64_t e = w.row[node] + lane; e < e1; e += 32) {
+      const int32_t p = w.col[e];
+      const double v = __dadd_rn(cost[p], pq_norm2(w.xy[p], x));
+      if (v < bv || (v == bv && e < be)) { bv = v; be = e; }
+    }
+#pragma unroll
+    for (int o = 16; o; o >>= 1) {
+      const double ov = __shfl_xor_sync(0xffffffffu, bv, o);
+      const int64_t oe = __shfl_xor_sync(0xffffffffu, be, o);
+      if (ov < bv || (ov == bv && oe < be)) { bv = ov; be = oe; }
+    }
+    if (be == INT64_MAX) break;                // no parent: cannot happen at a finite non-zero cost (the oracle stops there too)
+    node = w.col[be];
+    c = cost[node];
+    if (PATHS && lane == 0) out[n_states] = w.xy[node];
+    ++n_states;
+    if (!PATHS) {
+      if (node == tortoise) { cycle = true; break; }
+      if (++lam == power) { tortoise = node; power <<= 1; lam = 0; }
+    }
+  }
+  if (!PATHS && lane == 0) {
+    w.len[slot] = cycle ? 0 : (int32_t)n_states;
+    w.status[slot] = cycle ? PORRT_PATH_CYCLE : PORRT_PATH_FOUND;
+    w.cost[slot] = w.table[(int64_t)(w.gcol[slot] - w.c0) * w.V + w.start[slot]];
+  }
+}
+
+// the paths from slot order (stage) into query order (out): one warp per slot
+__global__ void prm_path_gather_kernel(const double2* __restrict__ stage, const int64_t* __restrict__ stage_off,
+                                       const int64_t* __restrict__ dst_off, const int32_t* __restrict__ len, int32_t n_slots,
+                                       double2* __restrict__ out) {
+  const int64_t k = ((int64_t)blockIdx.x * blockDim.x + threadIdx.x) >> 5;
+  if (k >= n_slots) return;
+  const double2* src = stage + stage_off[k];
+  double2* dst = out + dst_off[k];
+  for (int32_t j = threadIdx.x & 31; j < len[k]; j += 32) dst[j] = src[j];
+}
+
+PORRT_API int32_t porrt_prm_plan_paths(porrt_ctx* ctx, const double* starts_xy, const double* goals_xy, int64_t n, int32_t* out_start_node,
+                                       int32_t* out_goal_node, double* out_cost, int32_t* out_status, int64_t* out_path_ptr,
+                                       double* out_path_xy, int64_t cap, int64_t* out_total) {
+  CTX_CHECK(ctx);
+  if (n < 0 || cap < 0 || !out_path_ptr || !out_total || (n > 0 && (!starts_xy || !goals_xy || !out_cost || !out_status)) ||
+      (cap > 0 && !out_path_xy) || n > 0x3fffffff)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "prm_plan_paths: bad arguments");
+  if (ctx->prm_n <= 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "prm_plan_paths: no PRM built on this ctx (porrt_prm_build first)");
+  if (ctx->prm_grouped)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "prm_plan_paths: the last PRM result is porrt_mmprm_plan's grouped build");
+  if (ctx->prm_vertex_gen != ctx->vertex_gen)
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "prm_plan_paths: the vertex set was replaced or extended since the PRM build");
+  for (int64_t i = 0; i < 2 * n; ++i)
+    if (!std::isfinite(starts_xy[i]) || !std::isfinite(goals_xy[i]))
+      return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "prm_plan_paths: a start or goal coordinate is not finite");
+  out_path_ptr[0] = 0;
+  *out_total = 0;
+  if (n == 0) return PORRT_OK;
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  const int64_t V = ctx->prm_n, E = ctx->prm_edges, m = 2 * n;
+  const double2* d_vxy = ctx->d_vxy.as<double2>();
+
+  // 1. the 1-NN of the 2n points (starts, then goals).  Two nearest by (d2, id): the reference compares norm2 = sqrt(d2), and distinct
+  // d2 can round to the same norm2, so a tie is a second nearest at the winner's norm2 (an exact d2 tie is one too)
+  double *d_q, *d_dist, *d_cost;
+  int32_t *d_ids, *d_rank, *d_list, *d_rep, *d_start, *d_gcol, *d_len, *d_status;
+  int64_t *d_stage_off, *d_dst_off;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_q = c.take<double>((size_t)m * 2); d_dist = c.take<double>((size_t)m * 2); d_ids = c.take<int32_t>((size_t)m * 2);
+    d_rank = c.take<int32_t>(V); d_list = c.take<int32_t>(m); d_rep = c.take<int32_t>(m);
+    d_start = c.take<int32_t>(n); d_gcol = c.take<int32_t>(n); d_len = c.take<int32_t>(n); d_status = c.take<int32_t>(n);
+    d_cost = c.take<double>(n); d_stage_off = c.take<int64_t>(n); d_dst_off = c.take<int64_t>(n);
+  }));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_q, starts_xy, (size_t)n * 16, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_q + 2 * n, goals_xy, (size_t)n * 16, cudaMemcpyHostToDevice, st));
+  ctx->reach_words = 1;
+  int32_t rc = nn_knn_dev(ctx, d_q, m, 2, nullptr, nullptr, d_ids, d_dist, nullptr);
+  if (rc) return rc;
+  std::vector<int32_t> ids((size_t)m * 2);
+  std::vector<double> dist((size_t)m * 2);
+  CUDA_TRY(ctx, cudaMemcpyAsync(ids.data(), d_ids, (size_t)m * 8, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(dist.data(), d_dist, (size_t)m * 16, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  std::vector<int32_t> node((size_t)m), tied;
+  for (int64_t t = 0; t < m; ++t) {
+    node[(size_t)t] = ids[(size_t)t * 2];
+    if (ids[(size_t)t * 2 + 1] >= 0 && dist[(size_t)t * 2 + 1] == dist[(size_t)t * 2]) tied.push_back((int32_t)t);
+  }
+  if (!tied.empty()) {   // the kd-tree of the vertex set, then nn_inner for the tied points only
+    rc = kd_preorder_rank_dev(ctx, (const double*)d_vxy, V, d_rank, nullptr);
+    if (rc) return rc;
+    KdWork kw;
+    CUDA_TRY(ctx, carve(ctx->kd_buf, [&](Carve& c) { kd_work_layout(c, V, kw); }));   // the same layout: the rank's links
+    const int32_t nt = (int32_t)tied.size();
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_list, tied.data(), (size_t)nt * 4, cudaMemcpyHostToDevice, st));
+    prm_nn_replay_kernel<<<div_up(nt, 128), 128, 0, st>>>(d_vxy, kw.child, kw.parent, (const double2*)d_q, d_list, nt, d_rep);
+    LAUNCH_CHECK(ctx);
+    std::vector<int32_t> rep((size_t)nt);
+    CUDA_TRY(ctx, cudaMemcpyAsync(rep.data(), d_rep, (size_t)nt * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    for (int32_t i = 0; i < nt; ++i) node[(size_t)tied[(size_t)i]] = rep[(size_t)i];
+  }
+  if (out_start_node) memcpy(out_start_node, node.data(), (size_t)n * 4);
+  if (out_goal_node) memcpy(out_goal_node, node.data() + n, (size_t)n * 4);
+
+  // 2. one column per distinct goal node (ascending); slots sorted by (goal column, query index)
+  std::vector<int32_t> goals(node.begin() + n, node.end());
+  std::sort(goals.begin(), goals.end());
+  goals.erase(std::unique(goals.begin(), goals.end()), goals.end());
+  const int64_t G = (int64_t)goals.size();
+  std::vector<int32_t> qcol((size_t)n), slot_q((size_t)n);
+  for (int64_t q = 0; q < n; ++q) {
+    qcol[(size_t)q] = (int32_t)(std::lower_bound(goals.begin(), goals.end(), node[(size_t)(n + q)]) - goals.begin());
+    slot_q[(size_t)q] = (int32_t)q;
+  }
+  std::stable_sort(slot_q.begin(), slot_q.end(), [&](int32_t a, int32_t b) { return qcol[(size_t)a] < qcol[(size_t)b]; });
+  std::vector<int32_t> slot_start((size_t)n), slot_gcol((size_t)n);
+  for (int64_t k = 0; k < n; ++k) {
+    slot_start[(size_t)k] = node[(size_t)slot_q[(size_t)k]];
+    slot_gcol[(size_t)k] = qcol[(size_t)slot_q[(size_t)k]];
+  }
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_start, slot_start.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_gcol, slot_gcol.data(), (size_t)n * 4, cudaMemcpyHostToDevice, st));
+
+  // 3. chunks of columns; after each, the walks of its queries: lengths, the host lays out the stage, then the states
+  int64_t per = std::max<int64_t>(1, (int64_t)PORRT_PRM_PATHS_TABLE_BYTES / (V * 8));
+  if (ctx->prm_paths_chunk > 0) per = std::min(per, ctx->prm_paths_chunk);
+  std::vector<int32_t> len((size_t)n), status((size_t)n);
+  std::vector<int64_t> stage_off((size_t)n);
+  std::vector<double> cost((size_t)n);
+  int64_t staged = 0;
+  for (int64_t c0 = 0, s0 = 0; c0 < G; c0 += per) {
+    const int64_t c1 = std::min(G, c0 + per);
+    int64_t s1 = s0;
+    while (s1 < n && slot_gcol[(size_t)s1] < c1) ++s1;
+    std::vector<int64_t> fptr((size_t)(c1 - c0) + 1);
+    for (int64_t j = 0; j <= c1 - c0; ++j) fptr[(size_t)j] = j;
+    const double* d_table = nullptr;
+    int32_t sweeps = 0;
+    rc = sssp_core(ctx, ctx->prm_row_ptr, ctx->prm_col, (const double*)d_vxy, V, E, nullptr, nullptr, nullptr, 1, 1, false, (int)(c1 - c0),
+                   fptr.data(), goals.data() + c0, nullptr, &sweeps, &d_table);
+    if (rc) return rc;
+    PrmWalk w = {ctx->prm_row_ptr, ctx->prm_col, d_vxy, d_table, V, (int32_t)c0, d_start, d_gcol, d_len, d_status, d_cost, d_stage_off, nullptr};
+    const int32_t ns = (int32_t)(s1 - s0);
+    prm_walk_kernel<false><<<div_up((int64_t)ns * 32, 256), 256, 0, st>>>(w, (int32_t)s0, ns);
+    LAUNCH_CHECK(ctx);
+    CUDA_TRY(ctx, cudaMemcpyAsync(len.data() + s0, d_len + s0, (size_t)ns * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    const int64_t chunk0 = staged;
+    for (int64_t k = s0; k < s1; ++k) { stage_off[(size_t)k] = staged; staged += len[(size_t)k]; }
+    if (staged > chunk0) {
+      CUDA_TRY(ctx, ctx->ws_vid.grow_keep((size_t)staged * 16, (size_t)chunk0 * 16, st));
+      CUDA_TRY(ctx, cudaMemcpyAsync(d_stage_off + s0, stage_off.data() + s0, (size_t)ns * 8, cudaMemcpyHostToDevice, st));
+      w.stage = ctx->ws_vid.as<double2>();
+      prm_walk_kernel<true><<<div_up((int64_t)ns * 32, 256), 256, 0, st>>>(w, (int32_t)s0, ns);
+      LAUNCH_CHECK(ctx);
+    }
+    s0 = s1;
+  }
+  CUDA_TRY(ctx, cudaMemcpyAsync(status.data(), d_status, (size_t)n * 4, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(cost.data(), d_cost, (size_t)n * 8, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+
+  // 4. results in query order; the paths leave in one copy
+  std::vector<int64_t> dst_off((size_t)n);
+  for (int64_t k = 0; k < n; ++k) {
+    const int32_t q = slot_q[(size_t)k];
+    out_status[q] = status[(size_t)k];
+    out_cost[q] = cost[(size_t)k];
+    out_path_ptr[q + 1] = len[(size_t)k];
+  }
+  for (int64_t q = 0; q < n; ++q) out_path_ptr[q + 1] += out_path_ptr[q];
+  for (int64_t k = 0; k < n; ++k) dst_off[(size_t)k] = out_path_ptr[slot_q[(size_t)k]];
+  const int64_t total = out_path_ptr[n];
+  *out_total = total;
+  if (total > cap)
+    return porrt_fail(ctx, PORRT_ERR_CAPACITY, "prm_plan_paths: " + std::to_string(total) + " path states, cap " + std::to_string(cap));
+  if (total == 0) return PORRT_OK;
+  CUDA_TRY(ctx, ctx->ws_owner.ensure((size_t)total * 16));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_dst_off, dst_off.data(), (size_t)n * 8, cudaMemcpyHostToDevice, st));
+  prm_path_gather_kernel<<<div_up(n * 32, 256), 256, 0, st>>>(ctx->ws_vid.as<double2>(), d_stage_off, d_dst_off, d_len, (int32_t)n,
+                                                               ctx->ws_owner.as<double2>());
+  LAUNCH_CHECK(ctx);
+  CUDA_TRY(ctx, cudaMemcpyAsync(out_path_xy, ctx->ws_owner.p, (size_t)total * 16, cudaMemcpyDeviceToHost, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  return PORRT_OK;
 }
 
 // ================================================================================================ belief-space VI

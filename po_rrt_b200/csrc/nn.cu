@@ -332,6 +332,7 @@ PORRT_API int32_t porrt_vertices_set_dev(porrt_ctx* ctx, const double* xy_dev, i
   CTX_CHECK(ctx);
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   if (!xy_dev) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "vertices_set_dev: null");
+  ++ctx->vertex_gen;
   if (n > 0 && xy_dev != ctx->d_vxy.as<double>()) {   // the library keeps its own copy in upload order (porrt_edge_validity_indexed reads it)
     CUDA_TRY(ctx, ctx->d_vxy.ensure((size_t)n * 16));
     CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_vxy.p, xy_dev, (size_t)n * 16, cudaMemcpyDeviceToDevice, ctx->stream));
@@ -343,6 +344,7 @@ PORRT_API int32_t porrt_vertices_set(porrt_ctx* ctx, const double* xy, int64_t n
   CTX_CHECK(ctx);
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   if (!xy || n <= 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "vertices_set: bad arguments");
+  ++ctx->vertex_gen;
   CUDA_TRY(ctx, ctx->d_vxy.ensure((size_t)n * 16));
   CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_vxy.p, xy, (size_t)n * 16, cudaMemcpyHostToDevice, ctx->stream));
   ctx->cell_request = cell_size;
@@ -359,6 +361,7 @@ PORRT_API int32_t porrt_vertices_append(porrt_ctx* ctx, const double* xy, int64_
   CUDA_TRY(ctx, cudaSetDevice(ctx->device));
   const int64_t n = ctx->n_vertices;
   if (n + m > 0x7fffffff) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "vertices_append: too many vertices");
+  ++ctx->vertex_gen;
   CUDA_TRY(ctx, ctx->d_vxy.grow_keep((size_t)(n + m) * 16, (size_t)n * 16, ctx->stream));
   CUDA_TRY(ctx, cudaMemcpyAsync(ctx->d_vxy.as<char>() + (size_t)n * 16, xy, (size_t)m * 16, cudaMemcpyHostToDevice, ctx->stream));
   CUDA_TRY(ctx, cudaStreamSynchronize(ctx->stream));   // xy is the caller's (possibly pageable) memory
@@ -1071,6 +1074,35 @@ __global__ void __launch_bounds__(KNN_THREADS) knn_warp_kernel(GridDev g, const 
   }
 }
 
+// k nearest of m queries already on the device (q_dev [2m]), results left on the device: ids_dev / dist_dev [m * k], ties_dev [m]
+// (k == 1 only, nullable).  The caller has flushed appended vertices (nn_flush_appended) and set ctx->reach_words.
+int32_t nn_knn_dev(porrt_ctx* ctx, const double* q_dev, int64_t m, int k, const uint64_t* reach_dev, const uint32_t* world_dev,
+                   int32_t* ids_dev, double* dist_dev, int32_t* ties_dev) {
+  cudaStream_t st = ctx->stream;
+  GridDev g = grid_dev(ctx);
+  int64_t m_run = m;
+  const int32_t* list = nullptr;
+  if (nn_tile_usable(ctx, m)) {   // TMA-staged tiles, thread per query; whoever needs a wider ring comes back in the list
+    int32_t fb_n = 0;
+    int32_t rc = nn_tile_knn(ctx, g, q_dev, m, k, reach_dev, world_dev, ids_dev, dist_dev, k == 1 ? ties_dev : nullptr, &list, &fb_n);
+    if (rc) return rc;
+    m_run = fb_n;
+  }
+  if (m_run > 0 && list && m_run <= 65536) {   // few hard queries left by the tiles: a warp each
+    const int blocks = div_up(m_run * 32, KNN_THREADS);
+    if (k == 1) knn_warp_kernel<1><<<blocks, KNN_THREADS, 0, st>>>(g, (const double2*)q_dev, m_run, 1, reach_dev, world_dev, ids_dev, dist_dev, ties_dev, list);
+    else if (k <= 8) knn_warp_kernel<8><<<blocks, KNN_THREADS, 0, st>>>(g, (const double2*)q_dev, m_run, k, reach_dev, world_dev, ids_dev, dist_dev, nullptr, list);
+    else knn_warp_kernel<32><<<blocks, KNN_THREADS, 0, st>>>(g, (const double2*)q_dev, m_run, k, reach_dev, world_dev, ids_dev, dist_dev, nullptr, list);
+    LAUNCH_CHECK(ctx);
+  } else if (m_run > 0) {
+    if (k == 1) knn_kernel<1><<<div_up(m_run, KNN_THREADS), KNN_THREADS, 0, st>>>(g, (const double2*)q_dev, m_run, 1, reach_dev, world_dev, ids_dev, dist_dev, ties_dev, list);
+    else if (k <= 8) knn_kernel<8><<<div_up(m_run, KNN_THREADS), KNN_THREADS, 0, st>>>(g, (const double2*)q_dev, m_run, k, reach_dev, world_dev, ids_dev, dist_dev, nullptr, list);
+    else knn_kernel<32><<<div_up(m_run, KNN_THREADS), KNN_THREADS, 0, st>>>(g, (const double2*)q_dev, m_run, k, reach_dev, world_dev, ids_dev, dist_dev, nullptr, list);
+    LAUNCH_CHECK(ctx);
+  }
+  return PORRT_OK;
+}
+
 static int32_t knn_host(porrt_ctx* ctx, const double* q_xy, int64_t m, int k, const uint64_t* reach_mask, int32_t reach_words,
                         const uint32_t* world, int32_t* out_ids, double* out_dist, int32_t* out_ties) {
   if (ctx->n_vertices <= 0) return porrt_fail(ctx, PORRT_ERR_NO_VERTICES, "no vertex set");
@@ -1099,28 +1131,9 @@ static int32_t knn_host(porrt_ctx* ctx, const double* q_xy, int64_t m, int k, co
   CUDA_TRY(ctx, cudaMemcpyAsync(d_q, q_xy, (size_t)m * 16, cudaMemcpyHostToDevice, st));
   if (d_world) CUDA_TRY(ctx, cudaMemcpyAsync(d_world, world, (size_t)m * 4, cudaMemcpyHostToDevice, st));
   if (d_reach) CUDA_TRY(ctx, cudaMemcpyAsync(d_reach, reach_mask, reach_bytes, cudaMemcpyHostToDevice, st));
-  GridDev g = grid_dev(ctx);
   tstart(ctx);  // phases: [kernel, D2H]
-  int64_t m_run = m;
-  const int32_t* list = nullptr;
-  if (nn_tile_usable(ctx, m)) {   // TMA-staged tiles, thread per query; whoever needs a wider ring comes back in the list
-    int32_t fb_n = 0;
-    int32_t rc = nn_tile_knn(ctx, g, d_q, m, k, d_reach, d_world, d_ids, d_dist, k == 1 ? d_ties : nullptr, &list, &fb_n);
-    if (rc) return rc;
-    m_run = fb_n;
-  }
-  if (m_run > 0 && list && m_run <= 65536) {   // few hard queries left by the tiles: a warp each
-    const int blocks = div_up(m_run * 32, KNN_THREADS);
-    if (k == 1) knn_warp_kernel<1><<<blocks, KNN_THREADS, 0, st>>>(g, (const double2*)d_q, m_run, 1, d_reach, d_world, d_ids, d_dist, d_ties, list);
-    else if (k <= 8) knn_warp_kernel<8><<<blocks, KNN_THREADS, 0, st>>>(g, (const double2*)d_q, m_run, k, d_reach, d_world, d_ids, d_dist, nullptr, list);
-    else knn_warp_kernel<32><<<blocks, KNN_THREADS, 0, st>>>(g, (const double2*)d_q, m_run, k, d_reach, d_world, d_ids, d_dist, nullptr, list);
-    LAUNCH_CHECK(ctx);
-  } else if (m_run > 0) {
-    if (k == 1) knn_kernel<1><<<div_up(m_run, KNN_THREADS), KNN_THREADS, 0, st>>>(g, (const double2*)d_q, m_run, 1, d_reach, d_world, d_ids, d_dist, d_ties, list);
-    else if (k <= 8) knn_kernel<8><<<div_up(m_run, KNN_THREADS), KNN_THREADS, 0, st>>>(g, (const double2*)d_q, m_run, k, d_reach, d_world, d_ids, d_dist, nullptr, list);
-    else knn_kernel<32><<<div_up(m_run, KNN_THREADS), KNN_THREADS, 0, st>>>(g, (const double2*)d_q, m_run, k, d_reach, d_world, d_ids, d_dist, nullptr, list);
-    LAUNCH_CHECK(ctx);
-  }
+  int32_t rc = nn_knn_dev(ctx, d_q, m, k, d_reach, d_world, d_ids, d_dist, d_ties);
+  if (rc) return rc;
   tmark(ctx);
   CUDA_TRY(ctx, cudaMemcpyAsync(out_ids, d_ids, (size_t)m * k * 4, cudaMemcpyDeviceToHost, st));
   if (out_dist) CUDA_TRY(ctx, cudaMemcpyAsync(out_dist, d_dist, (size_t)m * k * 8, cudaMemcpyDeviceToHost, st));
