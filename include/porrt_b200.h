@@ -74,6 +74,9 @@ const char* porrt_last_error(porrt_ctx* ctx);
                                              the queries the tiles cannot serve) */
 #define PORRT_OPT_PRM_PATHS_CHUNK_COLUMNS 4  /* value > 0: porrt_prm_plan_paths solves at most `value` goal columns per chunk (the
                                              chunks are otherwise sized by PORRT_PRM_PATHS_TABLE_BYTES); 0 restores that */
+#define PORRT_OPT_REPARENT_BRUTE_MAX_NODES 5  /* value >= 0: porrt_refine_policy_reparent finds the radius / 2 candidates of trees of at
+                                             most `value` nodes with the all-pairs sweep and of larger trees with the kd search (the
+                                             same hits in the same order either way); value < 0 restores the default, 4096 */
 int32_t porrt_ctx_set_option(porrt_ctx* ctx, int32_t option, int64_t value);
 /* number of kernels this ctx has launched so far (bench.py's gpu_launches) */
 int64_t porrt_ctx_launch_count(porrt_ctx* ctx);

@@ -494,13 +494,14 @@ API void* orc_pto_extract_policy(void* p) {
   if (!extract_policy(pto->belief_graph, pto->expected_costs, h->p)) { delete h; return nullptr; }
   return h;
 }
-// refine_solution(PartialShortCut(n)) on the PTO's last extracted policy (main.rs:442: PartialShortCut(1500))
-API void* orc_pto_refine_shortcut(void* p, uint64_t n_iterations) {
+// refine_solution(PartialShortCut(n)) on the PTO's last extracted policy (main.rs:442: PartialShortCut(1500)); every piece's sampler
+// starts from `seed` (the reference's is seed 0)
+API void* orc_pto_refine_shortcut(void* p, uint64_t n_iterations, uint64_t seed) {
   PTO* pto = (PTO*)p;
   Policy pol;
   if (!extract_policy(pto->belief_graph, pto->expected_costs, pol)) return nullptr;
   PolicyHandle* h = new PolicyHandle();
-  if (!refiner_refine_shortcut(*pto->fns, pol, pto->belief_graph, (size_t)n_iterations, h->p)) { delete h; return nullptr; }
+  if (!refiner_refine_shortcut(*pto->fns, pol, pto->belief_graph, (size_t)n_iterations, h->p, seed)) { delete h; return nullptr; }
   return h;
 }
 // Policy::decompose + compute_expected_costs_to_goals on a policy given as arrays (common.rs:85-153; the reference's tests :425-489)
@@ -559,13 +560,14 @@ API void orc_refiner_transition_valid_batch(void* mp, const double* from, const 
   for (uint64_t v = 0; v < n_validities; ++v) row[v] = compat_row[v] != 0;
   for (int64_t i = 0; i < n; ++i) out[i] = refiner_is_transition_valid(*m, {from[2 * i], from[2 * i + 1]}, {to[2 * i], to[2 * i + 1]}, row);
 }
-API int64_t orc_refiner_partial_shortcut(void* mp, double* states, uint64_t L, const uint8_t* compat_row, uint64_t n_validities, uint64_t n_iterations) {
+API int64_t orc_refiner_partial_shortcut(void* mp, double* states, uint64_t L, const uint8_t* compat_row, uint64_t n_validities, uint64_t n_iterations,
+                                          uint64_t seed) {
   GridMap* m = (GridMap*)mp;
   std::vector<bool> row(n_validities);
   for (uint64_t v = 0; v < n_validities; ++v) row[v] = compat_row[v] != 0;
   std::vector<State> st(L);
   for (uint64_t k = 0; k < L; ++k) st[k] = {states[2 * k], states[2 * k + 1]};
-  const int64_t rc = refiner_partial_shortcut(*m, st, row, (size_t)n_iterations);
+  const int64_t rc = refiner_partial_shortcut(*m, st, row, (size_t)n_iterations, seed);
   for (uint64_t k = 0; k < L; ++k) { states[2 * k] = st[k][0]; states[2 * k + 1] = st[k][1]; }
   return rc;
 }

@@ -940,11 +940,11 @@ int64_t refiner_is_transition_valid(const GridMap& m, const State& from, const S
   return compat_row[(size_t)v] ? 1 : 0;            // :417
 }
 
-int64_t refiner_partial_shortcut(const GridMap& m, std::vector<State>& states, const std::vector<bool>& compat_row, size_t n_iterations) {
+int64_t refiner_partial_shortcut(const GridMap& m, std::vector<State>& states, const std::vector<bool>& compat_row, size_t n_iterations, uint64_t seed) {
   auto interpolate = [](double a, double b, double lambda) { return a * (1.0 - lambda) + b * lambda; };   // :159-161
   if (states.size() <= 2) return 0;                // :163-165
   const size_t joint_dim = 2;                      // tree.nodes.first().state.len()
-  DiscreteSampler sampler;                         // :169 DiscreteSampler::new()
+  DiscreteSampler sampler(seed);                   // :169 DiscreteSampler::new() (seed 0)
   int64_t commits = 0;
   for (size_t it = 0; it < n_iterations; ++it) {
     const size_t joint = (size_t)sampler.sample(joint_dim);                                   // :172
@@ -1038,7 +1038,7 @@ std::vector<std::vector<bool>> refiner_compat(const GridMap& m, const BeliefGrap
 void refiner_recompose(const std::vector<Tree>& trees, const std::vector<std::vector<size_t>>& skeleton, const BeliefGraph& g, Policy& out);
 }  // namespace
 
-bool refiner_refine_shortcut(const GridMap& m, const Policy& policy, const BeliefGraph& g, size_t n_iterations, Policy& out) {
+bool refiner_refine_shortcut(const GridMap& m, const Policy& policy, const BeliefGraph& g, size_t n_iterations, Policy& out, uint64_t seed) {
   const std::vector<std::vector<bool>> compat = refiner_compat(m, g);
   std::vector<std::pair<size_t, std::vector<size_t>>> path_pieces;
   std::vector<std::vector<size_t>> skeleton;
@@ -1057,7 +1057,7 @@ bool refiner_refine_shortcut(const GridMap& m, const Policy& policy, const Belie
     tree.leaf = tree.nodes.size() - 1;
     std::vector<State> states;                                                                                         // partial_shortcut :158-206
     for (const TreeNode& n : tree.nodes) states.push_back(n.state);
-    if (refiner_partial_shortcut(m, states, compat[tree.belief_state_id], n_iterations) < 0) return false;
+    if (refiner_partial_shortcut(m, states, compat[tree.belief_state_id], n_iterations, seed) < 0) return false;
     for (size_t k = 0; k < states.size(); ++k) tree.nodes[k].state = states[k];
     trees.push_back(tree);
   }

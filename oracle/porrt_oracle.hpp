@@ -195,15 +195,17 @@ bool extract_policy(const BeliefGraph& g, const std::vector<double>& costs, Poli
 // with the transition's validity.  Returns 1 / 0, or the (negative) panic code the reference would hit first.
 int64_t refiner_is_transition_valid(const GridMap& m, const State& from, const State& to, const std::vector<bool>& compat_row);
 // partial_shortcut (pto_policy_refiner.rs:158-206) on one path piece: `states` is modified in place; returns the number of
-// committed shortcuts, or a negative panic code.  The sampler is a fresh DiscreteSampler::new() (seed 0) like in the reference.
-int64_t refiner_partial_shortcut(const GridMap& m, std::vector<State>& states, const std::vector<bool>& compat_row, size_t n_iterations);
+// committed shortcuts, or a negative panic code.  The sampler is a fresh DiscreteSampler(seed); the reference's DiscreteSampler::new()
+// is seed 0.
+int64_t refiner_partial_shortcut(const GridMap& m, std::vector<State>& states, const std::vector<bool>& compat_row, size_t n_iterations,
+                                 uint64_t seed = 0);
 // Policy::decompose (common.rs:85-129): path pieces (belief id of the piece's first node, policy node ids) + skeleton (successor pieces)
 void policy_decompose(const Policy& p, std::vector<std::pair<size_t, std::vector<size_t>>>& pieces, std::vector<std::vector<size_t>>& skeleton);
 // Policy::compute_expected_costs_to_goals (common.rs:131-153)
 double policy_expected_costs(const Policy& p, const BeliefGraph& g);
 // PTOPolicyRefiner::refine_solution(RefinmentStrategy::PartialShortCut(n)) (pto_policy_refiner.rs:85-133,135-206,324-393): decompose,
 // build_path_piece + partial_shortcut per piece, recompose.  Returns false on a reference panic.
-bool refiner_refine_shortcut(const GridMap& m, const Policy& policy, const BeliefGraph& g, size_t n_iterations, Policy& out);
+bool refiner_refine_shortcut(const GridMap& m, const Policy& policy, const BeliefGraph& g, size_t n_iterations, Policy& out, uint64_t seed = 0);
 // refine_solution(RefinmentStrategy::Reparent(radius)) (pto_policy_refiner.rs:85-133,208-322): build_tree + reparent(radius / 2) per
 // piece, recompose.  The pop order among equal priorities follows priority-queue 1.0.5's heap (restated; parity unpinned).
 bool refiner_refine_reparent(const GridMap& m, const Policy& policy, const BeliefGraph& g, double radius, Policy& out);

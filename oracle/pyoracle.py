@@ -70,11 +70,11 @@ _SIGS = {
     "orc_pto_set_validities": (None, [vp, vp, u64, u64]), "orc_pto_build_belief_graph": (C.c_int, [vp, vp, u64]),
     "orc_pto_n_beliefs": (i64, [vp]), "orc_pto_beliefs": (None, [vp, vp]),
     "orc_pto_compute_expected_costs": (C.c_int, [vp, vp]), "orc_pto_final_belief_nodes": (i64, [vp, vp, i64]),
-    "orc_pto_extract_policy": (vp, [vp]), "orc_pto_plan_qmdp": (C.c_int, [vp, vp]), "orc_pto_refine_shortcut": (vp, [vp, C.c_uint64]), "orc_pto_refine_reparent": (vp, [vp, f64]), "orc_policy_decompose_count": (i64, [vp, u64]),
+    "orc_pto_extract_policy": (vp, [vp]), "orc_pto_plan_qmdp": (C.c_int, [vp, vp]), "orc_pto_refine_shortcut": (vp, [vp, C.c_uint64, C.c_uint64]), "orc_pto_refine_reparent": (vp, [vp, f64]), "orc_policy_decompose_count": (i64, [vp, u64]),
     "orc_policy_expected_cost": (f64, [vp, vp, vp, u64, vp, u64, u64]),
     "orc_pto_react_qmdp": (i64, [vp, vp, vp, f64, vp, vp, i64]),
     "orc_refiner_transition_valid_batch": (None, [vp, vp, vp, i64, vp, u64, vp]),
-    "orc_refiner_partial_shortcut": (i64, [vp, vp, u64, vp, u64, u64]),
+    "orc_refiner_partial_shortcut": (i64, [vp, vp, u64, vp, u64, u64, u64]),
     "orc_tamp_new": (vp, [vp, vp, vp, u64]), "orc_tamp_free": (None, [vp]),
     "orc_tamp_plan": (C.c_int, [vp, vp, vp, u64, f64, f64, u64, vp]), "orc_tamp_belief_graph": (vp, [vp]),
     "orc_tamp_policy": (vp, [vp]), "orc_tamp_sizes": (None, [vp, vp]),
@@ -242,11 +242,12 @@ class GridMap:
         lib().orc_refiner_transition_valid_batch(self.h, P(frm), P(to), len(frm), P(row), len(row), P(out))
         return out
 
-    def refiner_partial_shortcut(self, states, compat_row, n_iterations):
-        """pto_policy_refiner.rs:158-206 partial_shortcut on one path piece -> (new states, commits or panic code)"""
+    def refiner_partial_shortcut(self, states, compat_row, n_iterations, seed=0):
+        """pto_policy_refiner.rs:158-206 partial_shortcut on one path piece -> (new states, commits or panic code); the trials are
+        drawn from DiscreteSampler(seed) (the reference's DiscreteSampler::new() is seed 0)"""
         st = f64a(states).copy()
         row = np.ascontiguousarray(np.asarray(compat_row, dtype=np.uint8))
-        rc = lib().orc_refiner_partial_shortcut(self.h, P(st), len(st), P(row), len(row), int(n_iterations))
+        rc = lib().orc_refiner_partial_shortcut(self.h, P(st), len(st), P(row), len(row), int(n_iterations), int(seed))
         return st, int(rc)
 
     def visible_zones(self, xy):
@@ -653,9 +654,10 @@ class PTO:
             raise RuntimeError("reference panic in extract_policy")
         return Policy(h)
 
-    def refine_policy_shortcut(self, n_iterations):
-        """PTOPolicyRefiner::refine_solution(RefinmentStrategy::PartialShortCut(n)) on extract_policy()'s result"""
-        h = lib().orc_pto_refine_shortcut(self.h, n_iterations)
+    def refine_policy_shortcut(self, n_iterations, seed=0):
+        """PTOPolicyRefiner::refine_solution(RefinmentStrategy::PartialShortCut(n)) on extract_policy()'s result; every piece's
+        trials come from DiscreteSampler(seed) (the reference's is seed 0)"""
+        h = lib().orc_pto_refine_shortcut(self.h, n_iterations, int(seed))
         if not h:
             raise RuntimeError("reference panic in refine_solution")
         return Policy(h)

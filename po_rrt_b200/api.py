@@ -24,6 +24,7 @@ OPT_FORCE_LARGE_MAP_PATH = 1
 OPT_FORCE_GLOBAL_SWEEPS = 2
 OPT_FORCE_THREAD_PER_QUERY_NN = 3
 OPT_PRM_PATHS_CHUNK_COLUMNS = 4
+OPT_REPARENT_BRUTE_MAX_NODES = 5
 PATH_FOUND, PATH_NONE, PATH_CYCLE = 0, 1, 2   # PORRT_PATH_* (porrt_prm_plan_paths)
 PTO_MAX_ROADMAPS = 65535   # PORRT_PTO_MAX_ROADMAPS
 

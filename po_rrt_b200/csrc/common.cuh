@@ -220,6 +220,7 @@ struct porrt_ctx {
   bool prm_grouped = false;            // the last PRM result is porrt_mmprm_plan's grouped build (its vertex set mixes modes)
   int64_t prm_vertex_gen = -1;         // vertex_gen when the last PRM build bound its vertex set
   int64_t prm_paths_chunk = 0;         // PORRT_OPT_PRM_PATHS_CHUNK_COLUMNS (tests): > 0 caps porrt_prm_plan_paths' columns per chunk
+  int64_t reparent_brute_max = 4096;   // PORRT_OPT_REPARENT_BRUTE_MAX_NODES (tests): reparent trees up to this size take the all-pairs sweep
 
   // ---- last multi-modal PRM result (mmprm.cu): the explicit belief graph, kept for porrt_mmprm_fetch_graph
   struct MmPrm_ {

@@ -554,6 +554,7 @@ PORRT_API int32_t porrt_ctx_set_option(porrt_ctx* ctx, int32_t option, int64_t v
     case PORRT_OPT_FORCE_GLOBAL_SWEEPS: ctx->force_global_sweeps = value != 0; return PORRT_OK;
     case PORRT_OPT_FORCE_THREAD_PER_QUERY_NN: ctx->force_thread_per_query_nn = value != 0; return PORRT_OK;
     case PORRT_OPT_PRM_PATHS_CHUNK_COLUMNS: ctx->prm_paths_chunk = value > 0 ? value : 0; return PORRT_OK;
+    case PORRT_OPT_REPARENT_BRUTE_MAX_NODES: ctx->reparent_brute_max = value >= 0 ? value : 4096; return PORRT_OK;
     default: return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_ctx_set_option: unknown option");
   }
 }

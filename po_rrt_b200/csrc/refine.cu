@@ -171,8 +171,8 @@ PORRT_API int32_t porrt_partial_shortcut_batch(porrt_ctx* ctx, double* states_xy
   if (n_pieces < 0 || n_iterations < 0 || (n_pieces > 0 && (!states_xy || !piece_ptr || !compat_rows)))
     return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_partial_shortcut_batch: bad arguments");
   if (out_waves) *out_waves = 0;
+  if (out_commits) std::fill(out_commits, out_commits + n_pieces, 0);   // every entry, also when a later piece is refused
   for (int p = 0; p < n_pieces; ++p) {
-    if (out_commits) out_commits[p] = 0;
     if (piece_ptr[p + 1] < piece_ptr[p] || piece_ptr[p] < 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "porrt_partial_shortcut_batch: piece_ptr must be non-decreasing");
     if (piece_ptr[p + 1] - piece_ptr[p] > SHORTCUT_MAX_STATES) return porrt_fail(ctx, PORRT_ERR_UNSUPPORTED, "porrt_partial_shortcut_batch: a piece has more than 1024 states");
   }
@@ -575,7 +575,7 @@ PORRT_API int32_t porrt_refine_policy_reparent(porrt_ctx* ctx, const int32_t* po
       node_xy.insert(node_xy.end(), T.xy.begin(), T.xy.end());
       // small trees: all pairs against the nodes laid out in kd pre-order (the search visits node, left subtree, right subtree and
       // prunes only what cannot hit, so its hits come in that order) -- a contiguous sweep instead of ~n/2 pointer hops per query
-      const bool brute = T.size() <= 4096;
+      const bool brute = (int64_t)T.size() <= ctx->reparent_brute_max;   // 4096 unless PORRT_OPT_REPARENT_BRUTE_MAX_NODES says otherwise
       if (brute) {
         order.clear(); oxy.clear();
         kd_stack.assign(1, 0);
