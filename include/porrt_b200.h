@@ -471,6 +471,27 @@ int32_t porrt_pto_grow_batch(porrt_ctx* ctx, int32_t n_roadmaps, const uint64_t*
 int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
                                 int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks);
 
+/* ------------------------------------------------------------------ belief planning of a PTO batch (graph.cu, DESIGN.md 3.10)
+ * PTO::plan_belief_space (pto.rs:152-182) on each of the R roadmaps of the last porrt_pto_grow_batch / porrt_pto_grow, where they
+ * lie on the device: beliefs[B * n_worlds] as porrt_reachable_belief_states returns them (belief 0 = the start belief), the finals
+ * and their masks the growth's own.  Roadmap r's policy and expected cost equal, bit for bit, porrt_pto_fetch_roadmap(r) ->
+ * porrt_visibility -> porrt_belief_vi -> porrt_extract_policy.  The policies are packed back to back: roadmap r's nodes (node,
+ * belief, parent, leaf, in creation order) are [out_policy_ptr[r], out_policy_ptr[r + 1]) of out_node / out_belief / out_parent /
+ * out_is_leaf; out_policy_ptr has R + 1 entries.  out_status[r] is the code the single path returns for roadmap r: PORRT_ERR_PANIC
+ * when its growth panicked, when observe() would panic at one of its nodes or when extract_policy's asserts fire (a walk that never
+ * ends included), PORRT_ERR_UNSUPPORTED where porrt_belief_vi refuses, PORRT_ERR_CUDA when its table does not fit in device memory;
+ * a failing roadmap has an empty policy and out_expected_cost[r] = NaN, and does not fail the call.  Roadmaps whose final set is
+ * incomplete are planned like any other.  cap (policy nodes) smaller than the total: PORRT_ERR_CAPACITY with *out_total,
+ * out_status, out_expected_cost and out_policy_ptr filled.  The whole call fails with PORRT_ERR_INVALID_ARG when nothing has been
+ * grown, when n_worlds or the mask width differs from the map's, for B <= 0 or a null required pointer; with PORRT_ERR_PANIC on
+ * a belief hash collision (as porrt_belief_vi).  out_sweeps (nullable [R]): porrt_belief_vi's out_sweeps per roadmap;
+ * out_phase_ms (nullable [4]): shared host setup, per-roadmap preparation, device ms of the value backups (CUDA events), policy
+ * walks.  Nothing is retained: porrt_belief_result, porrt_extract_policy and the refiners still read the last porrt_belief_vi. */
+int32_t porrt_pto_plan_batch(porrt_ctx* ctx, const double* beliefs, int32_t B, int32_t n_worlds, int32_t* out_status,
+                             double* out_expected_cost, int64_t* out_policy_ptr /* [R + 1] */, int32_t* out_node, int32_t* out_belief,
+                             int32_t* out_parent, uint8_t* out_is_leaf, int64_t cap, int64_t* out_total,
+                             int32_t* out_sweeps /* nullable [R] */, double* out_phase_ms /* nullable [4] */);
+
 /* ------------------------------------------------------------------ RRT* tree growth on the device (pto_grow.cu, DESIGN.md 3.9)
  * RRT::grow_tree (rrt.rs:102-174) with sample() (:176-181) on the uploaded map, as ONE call per batch of trees; tree t samples with
  * Pcg64::seed_from_u64(sampler_seeds[t]), one continuous stream in [low, up): iteration i % 100 == 0 takes goal_example(0) and draws

@@ -100,6 +100,7 @@ SIGNATURES = {
     "porrt_pto_fetch": (i32, [vp, vp, vp, vp, vp, vp, vp, vp, vp]),
     "porrt_pto_grow_batch": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, i32, f64, f64, f64, i64, i64, vp, vp, vp, vp]),
     "porrt_pto_fetch_roadmap": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, vp, vp]),
+    "porrt_pto_plan_batch": (i32, [vp, vp, i32, i32, vp, vp, vp, vp, vp, vp, vp, i64, pp(i64), vp, vp]),
     "porrt_rrt_grow_batch": (i32, [vp, i32, vp, vp, vp, vp, vp, vp, i32, f64, f64, f64, i64, i64, vp, vp, vp, vp]),
     "porrt_rrt_grow": (i32, [vp, C.c_uint64, vp, vp, vp, vp, vp, i32, f64, f64, f64, i64, i64, vp, pp(i32), pp(i32), vp]),
     "porrt_rrt_fetch_tree": (i32, [vp, i32, vp, vp, vp, vp]),

@@ -979,6 +979,43 @@ class PTOBatch:
         """PTO.finals of roadmap r"""
         return _roadmap_finals(self._fetcher(r), self.sizes[r], self.fns)
 
+    def plan_belief_space(self, start_belief, beliefs=None):
+        """plan_belief_space(copy=None) of every roadmap of the last grow_graph, in one device call (porrt_pto_plan_batch) on the
+        roadmaps where they lie -> a list of one BeliefPlan per roadmap: beliefs, policy_node / policy_belief / policy_parent /
+        policy_leaf, expected_cost, sweeps and status (0, or the PorrtError code the single path raises for that roadmap: 5 where
+        its growth panicked, observe() would panic or extract_policy's asserts fire, 6 where porrt_belief_vi refuses, 2 where its
+        table does not fit in device memory; its policy is then empty and expected_cost NaN).  Nothing is retained: the table
+        of each roadmap is gone after the call (fetch_table() is not available), and the context's last plan_belief_space is
+        kept.  The call's phase times are in self.plan_phase_ms."""
+        fns, c = self.fns, self.ctx
+        fns._need()
+        bel = fns.reachable_belief_states(start_belief) if beliefs is None else _f64(beliefs, fns.n_worlds())
+        R = len(self.seeds)
+        status, cost = np.zeros(R, np.int32), np.zeros(R)
+        ptr, sweeps, total, phase = np.zeros(R + 1, np.int64), np.zeros(R, np.int32), C.c_int64(), np.zeros(4)
+        cap = 1024 * R
+        while True:
+            node, belief, parent = (np.empty(max(cap, 1), np.int32) for _ in range(3))
+            leaf = np.empty(max(cap, 1), np.uint8)
+            rc = c.lib.porrt_pto_plan_batch(c.h, _p(bel), len(bel), fns.n_worlds(), _p(status), _p(cost), _p(ptr), _p(node), _p(belief),
+                                            _p(parent), _p(leaf), cap, C.byref(total), _p(sweeps), _p(phase))
+            if rc == ERR_CAPACITY and total.value > cap:
+                cap = total.value
+                continue
+            c.check(rc)
+            break
+        self.plan_phase_ms = phase
+        plans = []
+        for r in range(R):
+            plan = BeliefPlan()
+            lo, hi = int(ptr[r]), int(ptr[r + 1])
+            plan.beliefs = bel
+            plan.policy_node, plan.policy_belief = node[lo:hi].copy(), belief[lo:hi].copy()
+            plan.policy_parent, plan.policy_leaf = parent[lo:hi].copy(), leaf[lo:hi].copy()
+            plan.expected_cost, plan.sweeps, plan.status = float(cost[r]), int(sweeps[r]), int(status[r])
+            plans.append(plan)
+        return plans
+
 
 class RRT:
     """src/rrt.rs RRT::grow_tree on the device (porrt_rrt_grow): `fns` is an uploaded Map / MapShelfDomain, the sampler is seeded

@@ -52,8 +52,9 @@ __device__ __forceinline__ void lds_cols(const double* p, double (&out)[C]) {
 // patterns); an improvement marks u dirty.  Fixed entries carry the sign bit, i.e. compare below every offer, and are never written.
 // The fixed point is the one of the pull sweeps: every value ever stored is the reference's left-to-right sum along some
 // admissible path, and the final value of v is always pushed after v's last improvement.
+// The kernel's whole body, shared with the batched kernel below (one CTA works on the roadmap whose arguments `a` are).
 template <int C, int MODE>
-__global__ void __launch_bounds__(COLSOLVE_THREADS, 1) colsolve_push_kernel(ColSolveArgs a, int col_lo, int col_hi) {
+__device__ __forceinline__ void colsolve_push_body(const ColSolveArgs& a, int col_lo, int col_hi) {
   extern __shared__ __align__(16) unsigned char smem_raw[];
   double* sd = reinterpret_cast<double*>(smem_raw);                 // [V][C]
   uint8_t* s_adm = smem_raw + (size_t)a.V * C * 8;                  // [256]
@@ -202,6 +203,18 @@ __global__ void __launch_bounds__(COLSOLVE_THREADS, 1) colsolve_push_kernel(ColS
   }
 }
 
+template <int C, int MODE>
+__global__ void __launch_bounds__(COLSOLVE_THREADS, 1) colsolve_push_kernel(ColSolveArgs a, int col_lo, int col_hi) {
+  colsolve_push_body<C, MODE>(a, col_lo, col_hi);
+}
+
+// Belief columns of several roadmaps in one launch: blockIdx.y picks the roadmap, whose arguments the kernel reads from a device
+// array of descriptors (the level's columns and the belief tables are the same for all of them; graph.cu, porrt_pto_plan_batch).
+template <int C>
+__global__ void __launch_bounds__(COLSOLVE_THREADS, 1) colsolve_push_batch_kernel(const ColSolveArgs* __restrict__ descs, int col_lo, int col_hi) {
+  colsolve_push_body<C, COLSOLVE_BELIEF>(descs[blockIdx.y], col_lo, col_hi);
+}
+
 __global__ void colsolve_count_kernel(const int32_t* __restrict__ col, int64_t E, uint32_t* __restrict__ cnt) {
   const int64_t e = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
   if (e < E) atomicAdd(&cnt[col[e]], 1u);
@@ -301,6 +314,43 @@ int32_t colsolve_level(porrt_ctx* ctx, const ColSolveArgs& a, int mode, int col_
       case 4: e = launch_one<4, COLSOLVE_WORLD>(ctx, a, col_lo, col_hi, smem, st); break;
       default: e = launch_one<6, COLSOLVE_WORLD>(ctx, a, col_lo, col_hi, smem, st); break;
     }
+  }
+  ctx->launches += 1;
+  CUDA_TRY(ctx, e);
+  return PORRT_OK;
+}
+
+// colsolve_level for the belief columns [col_lo, col_hi) of n_roads roadmaps at once (descs_dev: their arguments, device): a grid of
+// (CTAs per roadmap, roadmaps).  Columns per CTA and shared memory are what colsolve_level chooses for one roadmap of the largest
+// V of the launch, V_max nodes; the roadmaps side by side fill the SMs where one roadmap's level cannot.
+int32_t colsolve_level_batch(porrt_ctx* ctx, const ColSolveArgs* descs_dev, int n_roads, int32_t V_max, int col_lo, int col_hi,
+                             cudaStream_t st) {
+  const int n = col_hi - col_lo;
+  if (n <= 0 || n_roads <= 0) return PORRT_OK;
+  const int cap = (int)((COLSOLVE_SMEM_MAX - 280 - COLSOLVE_QCAP * 2 - (size_t)V_max) / ((size_t)V_max * 8));
+  const int cmax = cap >= 6 ? 6 : cap >= 4 ? 4 : cap >= 2 ? 2 : 1;
+  const int waves = (n + cmax * ctx->sm_count - 1) / (cmax * ctx->sm_count);
+  const int want = (n + waves * ctx->sm_count - 1) / (waves * ctx->sm_count);
+  const int C = std::min(want <= 1 ? 1 : want <= 2 ? 2 : want <= 4 ? 4 : 6, cmax);
+  const size_t smem = (size_t)V_max * C * 8 + 256 + (size_t)((V_max + 3) / 4) * 4 + COLSOLVE_QCAP * 2 + 16;
+  static bool configured[4][16] = {};   // per instantiation and device
+  const int ci = C == 1 ? 0 : C == 2 ? 1 : C == 4 ? 2 : 3;
+  const dim3 grid((unsigned)((n + C - 1) / C), (unsigned)n_roads);
+  auto launch = [&](auto kernel) -> cudaError_t {
+    if (!configured[ci][ctx->device & 15]) {
+      const cudaError_t e = cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, COLSOLVE_SMEM_MAX);
+      if (e != cudaSuccess) return e;
+      configured[ci][ctx->device & 15] = true;
+    }
+    kernel<<<grid, COLSOLVE_THREADS, smem, st>>>(descs_dev, col_lo, col_hi);
+    return cudaGetLastError();
+  };
+  cudaError_t e;
+  switch (C) {
+    case 1: e = launch(colsolve_push_batch_kernel<1>); break;
+    case 2: e = launch(colsolve_push_batch_kernel<2>); break;
+    case 4: e = launch(colsolve_push_batch_kernel<4>); break;
+    default: e = launch(colsolve_push_batch_kernel<6>); break;
   }
   ctx->launches += 1;
   CUDA_TRY(ctx, e);

@@ -38,3 +38,5 @@ bool colsolve_fits(int64_t V, int64_t E, int32_t n_validities);
 int32_t colsolve_pack(porrt_ctx* ctx, const int64_t* row_ptr_dev, const int32_t* col_dev, const int32_t* evid_dev, const double* cost_dev,
                       int64_t V, int64_t E, uint32_t* row_start_t, uint32_t* ce_t, double* cost_t, uint32_t* cursor_tmp, cudaStream_t st);
 int32_t colsolve_level(porrt_ctx* ctx, const ColSolveArgs& a, int mode, int col_lo, int col_hi, cudaStream_t st);
+int32_t colsolve_level_batch(porrt_ctx* ctx, const ColSolveArgs* descs_dev, int n_roads, int32_t V_max, int col_lo, int col_hi,
+                             cudaStream_t st);

@@ -427,6 +427,14 @@ int32_t late_list_csr_dev(porrt_ctx* ctx, const int64_t* seg_off, int64_t n, con
                           int64_t* row_ptr, int32_t* col, int32_t* vid);
 // pto_grow.cu
 void pto_grow_release(porrt_ctx* ctx);
+struct PtoRoadDev {   // one roadmap of the last PTO growth, device pointers (have = false: its growth panicked)
+  bool have;
+  int64_t V, E, n_finals;
+  const double* xy; const int32_t* node_vid;                        // [2V], [V]
+  const int64_t* row_ptr; const int32_t* col; const int32_t* edge_vid;   // children CSR, as porrt_pto_fetch_roadmap returns it
+  const int32_t* fin_ids; const int32_t* fin_goal;                  // finals in add order, the goal each one hit
+};
+bool pto_roads(const porrt_ctx* ctx, std::vector<PtoRoadDev>& out, std::vector<uint64_t>* goal_masks, int* words);
 int32_t prm_build_impl(porrt_ctx* ctx, const double* samples_xy, int64_t n, double max_step, double search_radius,
                        const double* ms_arr, const double* sr_arr, int64_t* out_row_ptr, int32_t* out_col, int64_t cap,
                        int64_t* out_n_edges, double* out_phase_ms, const int64_t* group_ptr = nullptr, int32_t n_groups = 0);

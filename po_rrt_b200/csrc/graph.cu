@@ -1548,6 +1548,85 @@ PORRT_API int32_t porrt_reachable_belief_states(porrt_ctx* ctx, const double* st
   return PORRT_OK;
 }
 
+// ---- the host part of porrt_belief_vi that depends only on the beliefs and the map, shared with porrt_pto_plan_batch, which plans
+// many roadmaps on the same beliefs
+struct BeliefHost {
+  int B = 0, nw = 0, mask_words = 1, n_validities = 0;
+  std::vector<uint64_t> support;   // [B][mask_words] the worlds each belief holds possible
+  std::vector<uint8_t> compat;     // [B][n_validities]
+  std::vector<uint64_t> bhash;     // [B]
+  std::vector<int32_t> level;      // [B] support size
+  ColumnLayout lay;
+  // is_compatible(belief, mask) (common.rs:256-264) = "no world with positive probability outside the mask": one AND-NOT per
+  // word on the belief's support bits
+  bool compatible(int b, const uint64_t* mask) const {
+    for (int k = 0; k < mask_words; ++k)
+      if (support[(size_t)b * mask_words + k] & ~mask[k]) return false;
+    return true;
+  }
+};
+
+// compute_compatibility (common.rs:266-276), belief ids by hash (belief_graph.rs:75-87; collisions are a reference panic) and the
+// column levels: beliefs by the size of their support (observations only ever split it, so a column reads Observation values from
+// columns of earlier levels), cut into `shards` shards
+static int32_t belief_host_prepare(porrt_ctx* ctx, const double* beliefs, int B, int nw, const uint64_t* validities, int n_validities,
+                                   int mask_words, int shards, BeliefHost& h) {
+  h.B = B; h.nw = nw; h.mask_words = mask_words; h.n_validities = n_validities;
+  h.support.assign((size_t)B * mask_words, 0);
+  for (int b = 0; b < B; ++b)
+    for (int w = 0; w < nw; ++w)
+      if (beliefs[(size_t)b * nw + w] > 0.0) h.support[(size_t)b * mask_words + w / 64] |= (uint64_t)1 << (w % 64);
+  h.compat.resize((size_t)B * n_validities);
+  for (int b = 0; b < B; ++b)
+    for (int v = 0; v < n_validities; ++v) h.compat[(size_t)b * n_validities + v] = h.compatible(b, validities + (size_t)v * mask_words);
+  std::unordered_map<uint64_t, int> hash_to_id;
+  h.bhash.resize((size_t)B);
+  for (int b = 0; b < B; ++b) { h.bhash[b] = belief_hash(beliefs + (size_t)b * nw, nw); hash_to_id[h.bhash[b]] = b; }
+  if ((int)hash_to_id.size() != B) return porrt_fail(ctx, PORRT_ERR_PANIC, "collision when hashing the belief states! (belief_graph.rs:84)");
+  h.level.assign((size_t)B, 0);
+  for (int b2 = 0; b2 < B; ++b2)
+    for (int k = 0; k < mask_words; ++k) h.level[(size_t)b2] += __builtin_popcountll(h.support[(size_t)b2 * mask_words + k]);
+  h.lay = column_layout(h.level, shards);
+  return PORRT_OK;
+}
+
+// observe_impl is a function of the node's set of visible zones only: one observation successor table per distinct set.
+// node_set[n] = the index of node n's set in `sets`; sets not seen before are appended (set_index: set -> index).
+static void visible_zone_sets(const porrt_ctx* ctx, const uint64_t* visible_zone_mask, int64_t V, std::map<uint64_t, int>& set_index,
+                              std::vector<uint64_t>& sets, int32_t* node_set) {
+  const uint64_t zone_bits = ctx->n_zones >= 64 ? ~(uint64_t)0 : (((uint64_t)1 << ctx->n_zones) - 1);
+  for (int64_t n = 0; n < V; ++n) {
+    const uint64_t vis = visible_zone_mask[n] & zone_bits;
+    auto it = set_index.find(vis);
+    if (it == set_index.end()) { it = set_index.emplace(vis, (int)sets.size()).first; sets.push_back(vis); }
+    node_set[n] = it->second;
+  }
+}
+
+// the final belief nodes (pto.rs:261-271) as (column position, node); false when a final id is out of range
+static bool belief_finals(const BeliefHost& h, const int32_t* node_vid, int64_t V, const int32_t* finals_ids, const uint64_t* finals_masks,
+                          int32_t n_finals, std::vector<int2>& fin) {
+  for (int k = 0; k < n_finals; ++k) {
+    const int32_t f = finals_ids[k];
+    if (f < 0 || f >= V) return false;
+    for (int b = 0; b < h.B; ++b)
+      if (h.compat[(size_t)b * h.n_validities + node_vid[f]] && h.compatible(b, finals_masks + (size_t)k * h.mask_words))
+        fin.push_back(make_int2(h.lay.colpos[(size_t)b], f));
+  }
+  return true;
+}
+
+// the validity ids (< 256) each column position admits, colsolve.cu's cmask
+static std::vector<uint64_t> column_masks(const BeliefHost& h) {
+  const std::vector<int32_t>& col_belief = h.lay.poscol;
+  const int Bp = (int)col_belief.size();
+  std::vector<uint64_t> cmask((size_t)Bp * 4, 0);
+  for (int c = 0; c < Bp; ++c)
+    for (int v = 0; col_belief[(size_t)c] >= 0 && v < h.n_validities; ++v)
+      if (h.compat[(size_t)col_belief[(size_t)c] * h.n_validities + v]) cmask[(size_t)c * 4 + v / 64] |= (uint64_t)1 << (v % 64);
+  return cmask;
+}
+
 struct BeliefDev {
   const int64_t* row_ptr; const int32_t* col; const int32_t* edge_vid; const double* cost;
   const int32_t* node_vid; const int32_t* node_set;
@@ -1673,72 +1752,36 @@ PORRT_API int32_t porrt_belief_vi(porrt_ctx* ctx, int64_t V, const int64_t* row_
   for (int64_t u = 0; u < V; ++u)
     if (node_vid[u] < 0 || node_vid[u] >= n_validities) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "belief_vi: node validity id out of range");
   const int nw = n_worlds;
-  // compute_compatibility (common.rs:266-276)
-  // is_compatible(belief, mask) (common.rs:256-264) = "no world with positive probability outside the mask": one AND-NOT per
-  // word on the belief's support bits
-  std::vector<uint64_t> support((size_t)B * mask_words, 0);
-  for (int b = 0; b < B; ++b)
-    for (int w = 0; w < nw; ++w)
-      if (beliefs[(size_t)b * nw + w] > 0.0) support[(size_t)b * mask_words + w / 64] |= (uint64_t)1 << (w % 64);
-  auto compatible = [&](int b, const uint64_t* mask) {
-    for (int k = 0; k < mask_words; ++k)
-      if (support[(size_t)b * mask_words + k] & ~mask[k]) return false;
-    return true;
-  };
-  std::vector<uint8_t> compat((size_t)B * n_validities);
-  for (int b = 0; b < B; ++b)
-    for (int v = 0; v < n_validities; ++v) compat[(size_t)b * n_validities + v] = compatible(b, validities + (size_t)v * mask_words);
-  // belief ids by hash (belief_graph.rs:75-87); collisions are a reference panic
-  std::unordered_map<uint64_t, int> hash_to_id;
-  std::vector<uint64_t> bhash(B);
-  for (int b = 0; b < B; ++b) { bhash[b] = belief_hash(beliefs + (size_t)b * nw, nw); hash_to_id[bhash[b]] = b; }
-  if ((int)hash_to_id.size() != B) return porrt_fail(ctx, PORRT_ERR_PANIC, "collision when hashing the belief states! (belief_graph.rs:84)");
-  // observation successor tables, one per distinct set of visible zones (observe_impl is a function of that set only)
+  BeliefHost h;
+  {
+    int32_t rc = belief_host_prepare(ctx, beliefs, B, nw, validities, n_validities, mask_words, ctx->comm_world > 1 ? ctx->comm_world : 1, h);
+    if (rc) return rc;
+  }
+  const std::vector<uint8_t>& compat = h.compat;
   std::map<uint64_t, int> set_index;
   std::vector<int32_t> node_set((size_t)V);
   std::vector<uint64_t> sets;
-  const uint64_t zone_bits = ctx->n_zones >= 64 ? ~(uint64_t)0 : (((uint64_t)1 << ctx->n_zones) - 1);
-  for (int64_t n = 0; n < V; ++n) {
-    const uint64_t vis = visible_zone_mask[n] & zone_bits;
-    auto it = set_index.find(vis);
-    if (it == set_index.end()) { it = set_index.emplace(vis, (int)sets.size()).first; sets.push_back(vis); }
-    node_set[n] = it->second;
-  }
-  // column levels: beliefs by the size of their support (observations only ever split it, so a column reads Observation values
-  // from columns of earlier levels)
-  std::vector<int32_t> level((size_t)B, 0);
-  for (int b2 = 0; b2 < B; ++b2)
-    for (int k = 0; k < mask_words; ++k) level[(size_t)b2] += __builtin_popcountll(support[(size_t)b2 * mask_words + k]);
-  const ColumnLayout lay = column_layout(level, ctx->comm_world > 1 ? ctx->comm_world : 1);
+  visible_zone_sets(ctx, visible_zone_mask, V, set_index, sets, node_set.data());
+  const ColumnLayout& lay = h.lay;
   const std::vector<int32_t>& colpos = lay.colpos;
   const std::vector<int32_t>& col_belief = lay.poscol;
   const int Bp = (int)col_belief.size();   // columns incl. padding (== B on one GPU)
   // observation successor tables, one entry per (set, belief), built on the device (belief_tables.cu)
   BeliefSuccDev succ = {};
   {
-    int32_t rc = belief_succ_tables(ctx, beliefs, B, nw, sets, bhash, level, colpos, &succ, st);
+    int32_t rc = belief_succ_tables(ctx, beliefs, B, nw, sets, h.bhash, h.level, colpos, &succ, st);
     if (rc) return rc;
   }
   // initial distances: 0 at final belief nodes (pto.rs:261-271), +inf elsewhere -- written on the device; only the list of final
   // belief nodes, as (column position, node), is built here (a host-side V*B table cost 30 ms + a 150 MB upload at B = 4095)
   std::vector<int2> fin;
-  for (int k = 0; k < n_finals; ++k) {
-    const int32_t f = finals_ids[k];
-    if (f < 0 || f >= V) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "belief_vi: final id out of range");
-    for (int b = 0; b < B; ++b)
-      if (compat[(size_t)b * n_validities + node_vid[f]] && compatible(b, finals_masks + (size_t)k * mask_words))
-        fin.push_back(make_int2(colpos[(size_t)b], f));
-  }
+  if (!belief_finals(h, node_vid, V, finals_ids, finals_masks, n_finals, fin))
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "belief_vi: final id out of range");
   t1 = now_ms(); ph[0] = t1 - t0; t0 = t1;
 
   if (n_validities > 256) return porrt_fail(ctx, PORRT_ERR_UNSUPPORTED, "belief_vi: more than 256 validity ids");
   if (!succ.levels_ok) return porrt_fail(ctx, PORRT_ERR_UNSUPPORTED, "belief_vi: an observation does not split the belief's support (the level order of the backups does not apply)");
-  std::vector<uint64_t> cmask((size_t)Bp * 4, 0);
-  {
-    for (int c = 0; c < Bp; ++c)
-      for (int v = 0; col_belief[(size_t)c] >= 0 && v < n_validities; ++v)
-        if (compat[(size_t)col_belief[(size_t)c] * n_validities + v]) cmask[(size_t)c * 4 + v / 64] |= (uint64_t)1 << (v % 64);
-  }
+  const std::vector<uint64_t> cmask = column_masks(h);
 
   int64_t* d_row;
   double* d_xy;
@@ -1865,30 +1908,354 @@ bool porrt_ctx::BeliefState_::fetch_column(porrt_ctx* ctx, int b) {
 }
 
 // ================================================================================================ policy extraction
+// The walk over the implicit V x B belief graph of a belief table R (value columns fetched as the walk visits them); an Observation
+// child keeps its parent's state, so its cost is norm2(state n, state n).  *expected_cost: the value of the root (node 0, belief 0).
+static int32_t belief_policy_walk(porrt_ctx* ctx, porrt_ctx::BeliefState_& R, const double* beliefs, const char* name,
+                                  std::vector<PolicyNode>& pol, double* expected_cost) {
+  const int B = R.B;
+  R.fetch_failed = false;
+  const int32_t rc = get_best_expected_children(
+      ctx, name, R.V * (int64_t)B, beliefs, R.n_worlds,
+      [&](int64_t id, auto&& fn) { R.for_children(ctx, id, fn); },
+      [&](int64_t id) { return (int32_t)(id % B); },
+      [&](int64_t a, int64_t c) { return norm2(&R.xy[2 * (size_t)(a / B)], &R.xy[2 * (size_t)(c / B)], 2); },
+      [&](int64_t id) { return R.value(ctx, id); }, pol);
+  *expected_cost = R.value(ctx, 0);
+  // a failed fetch read as 0: it outranks any assert the walk tested on such a value
+  if (R.fetch_failed) return porrt_fail(ctx, PORRT_ERR_CUDA, std::string(name) + ": fetching a value column failed");
+  return rc;
+}
+
 PORRT_API int32_t porrt_extract_policy(porrt_ctx* ctx, int32_t* out_node, int32_t* out_belief, int32_t* out_parent,
                                        uint8_t* out_is_leaf, int64_t cap, int64_t* out_n, double* out_expected_cost) {
   CTX_CHECK(ctx);
   auto& R = ctx->bel;
   if (R.V <= 0) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "extract_policy: run porrt_belief_vi first");
   const int B = R.B;
-  // the walk over the implicit V x B belief graph; an Observation child keeps its parent's state, so its cost is norm2(state n, state n)
-  R.fetch_failed = false;
   std::vector<PolicyNode> pol;
-  const int32_t rc = get_best_expected_children(
-      ctx, "extract_policy", R.V * (int64_t)B, R.beliefs.data(), R.n_worlds,
-      [&](int64_t id, auto&& fn) { R.for_children(ctx, id, fn); },
-      [&](int64_t id) { return (int32_t)(id % B); },
-      [&](int64_t a, int64_t c) { return norm2(&R.xy[2 * (size_t)(a / B)], &R.xy[2 * (size_t)(c / B)], 2); },
-      [&](int64_t id) { return R.value(ctx, id); }, pol);
-  const double expected_cost = R.value(ctx, 0);
-  // a failed fetch read as 0: it outranks any assert the walk tested on such a value
-  if (R.fetch_failed) return porrt_fail(ctx, PORRT_ERR_CUDA, "extract_policy: fetching a value column failed");
+  double expected_cost;
+  const int32_t rc = belief_policy_walk(ctx, R, R.beliefs.data(), "extract_policy", pol, &expected_cost);
   if (rc) return rc;
   if (out_n) *out_n = (int64_t)pol.size();
   if (out_expected_cost) *out_expected_cost = expected_cost;
   if ((int64_t)pol.size() > cap || !out_node || !out_belief || !out_parent || !out_is_leaf) return porrt_fail(ctx, PORRT_ERR_CAPACITY, "extract_policy: cap too small");
   for (size_t k = 0; k < pol.size(); ++k) {
     out_node[k] = (int32_t)(pol[k].id / B); out_belief[k] = (int32_t)(pol[k].id % B); out_parent[k] = pol[k].parent; out_is_leaf[k] = pol[k].leaf;
+  }
+  return PORRT_OK;
+}
+
+// ================================================================================================ belief planning of a PTO batch
+// porrt_belief_vi + porrt_extract_policy on every roadmap of the last PTO growth, where the roadmaps lie (PtoRoadDev).  Shared by
+// all roadmaps and built once: the belief algebra (belief_host_prepare), the column masks and one set of observation successor
+// tables over the union of the roadmaps' visible-zone sets.  Per roadmap: node types, the transposed adjacency and the initial
+// table, all from the resident CSR.  Then every level is ONE launch over all roadmaps whose columns fit on chip (grid y = roadmap);
+// a roadmap that does not fit, or every roadmap under PORRT_OPT_FORCE_GLOBAL_SWEEPS, takes value_columns_solve's frontier schedule
+// on its own.  The roadmaps go through in chunks whose tables fit in the device's free memory.  Each policy is walked by
+// belief_policy_walk over its roadmap's table, fetching the columns it visits.  Nothing outlives the call: ctx->bel is untouched.
+namespace {
+struct PlanRoad {   // one roadmap of porrt_pto_plan_batch: the host copies the walk reads, and where its table lies in the chunk
+  std::vector<int64_t> row; std::vector<int32_t> col, evid, nvid, node_set; std::vector<double> xy;
+  std::vector<int2> fin;                  // final belief nodes as (column position, node)
+  bool on_chip = false;
+  size_t bytes = 0;                       // its share of the chunk (plan_road_layout)
+  double* dist_cm = nullptr; uint8_t *type = nullptr, *type_cm = nullptr; int32_t *d_node_set = nullptr, *sweeps = nullptr;
+  double *cost = nullptr, *cost_t = nullptr; uint32_t *ce = nullptr, *rs = nullptr, *cursor = nullptr; int2* d_fin = nullptr;
+  std::vector<PolicyNode> pol;
+};
+struct DevScratch {   // device memory of one call, freed when it returns
+  void* p = nullptr;
+  ~DevScratch() { if (p) cudaFree(p); }
+};
+}  // namespace
+
+// the table ([column][node]), node types, set index and sweep counter of a roadmap, and the column solver's inputs if it is on chip
+static void plan_road_layout(Carve& c, PlanRoad& d, int64_t V, int64_t E, int B, int Bp) {
+  d.dist_cm = c.take<double>((size_t)V * Bp); d.type = c.take<uint8_t>((size_t)V * B); d.type_cm = c.take<uint8_t>((size_t)V * Bp);
+  d.d_node_set = c.take<int32_t>(V); d.sweeps = c.take<int32_t>(4);
+  if (d.on_chip) {
+    d.cost = c.take<double>(E); d.cost_t = c.take<double>(E); d.ce = c.take<uint32_t>(E);
+    d.rs = c.take<uint32_t>(V + 1); d.cursor = c.take<uint32_t>(V + 1); d.d_fin = c.take<int2>(d.fin.size());
+  }
+}
+
+PORRT_API int32_t porrt_pto_plan_batch(porrt_ctx* ctx, const double* beliefs, int32_t B, int32_t n_worlds, int32_t* out_status,
+                                       double* out_expected_cost, int64_t* out_policy_ptr, int32_t* out_node, int32_t* out_belief,
+                                       int32_t* out_parent, uint8_t* out_is_leaf, int64_t cap, int64_t* out_total, int32_t* out_sweeps,
+                                       double* out_phase_ms) {
+  CTX_CHECK(ctx);
+  if (!ctx->has_map) return porrt_fail(ctx, PORRT_ERR_NO_MAP, "no map uploaded");
+  std::vector<PtoRoadDev> roads;
+  std::vector<uint64_t> goal_masks;
+  int words = 0;
+  if (!pto_roads(ctx, roads, &goal_masks, &words)) return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "pto_plan_batch: no roadmap grown on this ctx");
+  if (!beliefs || B <= 0 || n_worlds != ctx->n_worlds || words != ctx->mask_words || !out_status || !out_expected_cost ||
+      !out_policy_ptr || !out_total || cap < 0 || (cap > 0 && (!out_node || !out_belief || !out_parent || !out_is_leaf)))
+    return porrt_fail(ctx, PORRT_ERR_INVALID_ARG, "pto_plan_batch: bad arguments");
+  CUDA_TRY(ctx, cudaSetDevice(ctx->device));
+  cudaStream_t st = ctx->stream;
+  double t0 = now_ms(), t1, ph[4] = {0};
+  const int R = (int)roads.size(), nw = n_worlds, mw = ctx->mask_words, nval = ctx->n_validities;
+  for (int r = 0; r < R; ++r) {
+    out_status[r] = roads[(size_t)r].have ? PORRT_OK : PORRT_ERR_PANIC;
+    out_expected_cost[r] = std::numeric_limits<double>::quiet_NaN();
+    if (out_sweeps) out_sweeps[r] = 0;
+  }
+  BeliefHost h;
+  {
+    int32_t rc = belief_host_prepare(ctx, beliefs, B, nw, ctx->validities.data(), nval, mw, 1, h);
+    if (rc) return rc;
+  }
+  const int Bp = (int)h.lay.poscol.size();
+  const std::vector<uint64_t> cmask = column_masks(h);
+
+  // ---- the roadmaps' graphs and finals on the host (the policy walk reads them), visibility of all nodes in one launch
+  std::vector<PlanRoad> pr((size_t)R);
+  std::vector<int64_t> vis_off((size_t)R + 1, 0);
+  for (int r = 0; r < R; ++r) vis_off[(size_t)r + 1] = vis_off[(size_t)r] + (roads[(size_t)r].have ? roads[(size_t)r].V : 0);
+  const int64_t Vsum = vis_off[(size_t)R];
+  double* d_vxy;
+  uint64_t *d_vmask, *d_cmask;
+  int32_t *d_vstatus, *d_col_belief, *d_colpos;
+  uint8_t* d_compat;
+  CUDA_TRY(ctx, carve(ctx->ws_main, [&](Carve& c) {
+    d_vxy = c.take<double>(2 * (size_t)Vsum); d_vmask = c.take<uint64_t>(Vsum); d_vstatus = c.take<int32_t>(Vsum);
+    d_cmask = c.take<uint64_t>((size_t)Bp * 4); d_col_belief = c.take<int32_t>(Bp); d_colpos = c.take<int32_t>(B);
+    d_compat = c.take<uint8_t>(h.compat.size());
+  }));
+  std::vector<std::vector<int32_t>> fin_ids((size_t)R), fin_goal((size_t)R);
+  for (int r = 0; r < R; ++r) {
+    const PtoRoadDev& g = roads[(size_t)r];
+    if (!g.have) continue;
+    PlanRoad& d = pr[(size_t)r];
+    d.row.resize((size_t)g.V + 1); d.col.resize((size_t)g.E); d.evid.resize((size_t)g.E); d.nvid.resize((size_t)g.V);
+    d.xy.resize(2 * (size_t)g.V);
+    fin_ids[(size_t)r].resize((size_t)g.n_finals); fin_goal[(size_t)r].resize((size_t)g.n_finals);
+    CUDA_TRY(ctx, cudaMemcpyAsync(d.row.data(), g.row_ptr, (size_t)(g.V + 1) * 8, cudaMemcpyDeviceToHost, st));
+    if (g.E) {
+      CUDA_TRY(ctx, cudaMemcpyAsync(d.col.data(), g.col, (size_t)g.E * 4, cudaMemcpyDeviceToHost, st));
+      CUDA_TRY(ctx, cudaMemcpyAsync(d.evid.data(), g.edge_vid, (size_t)g.E * 4, cudaMemcpyDeviceToHost, st));
+    }
+    CUDA_TRY(ctx, cudaMemcpyAsync(d.nvid.data(), g.node_vid, (size_t)g.V * 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(d.xy.data(), g.xy, (size_t)g.V * 16, cudaMemcpyDeviceToHost, st));
+    if (g.n_finals) {
+      CUDA_TRY(ctx, cudaMemcpyAsync(fin_ids[(size_t)r].data(), g.fin_ids, (size_t)g.n_finals * 4, cudaMemcpyDeviceToHost, st));
+      CUDA_TRY(ctx, cudaMemcpyAsync(fin_goal[(size_t)r].data(), g.fin_goal, (size_t)g.n_finals * 4, cudaMemcpyDeviceToHost, st));
+    }
+    CUDA_TRY(ctx, cudaMemcpyAsync(d_vxy + 2 * vis_off[(size_t)r], g.xy, (size_t)g.V * 16, cudaMemcpyDeviceToDevice, st));
+  }
+  std::vector<uint64_t> vmask((size_t)Vsum);
+  std::vector<int32_t> vstatus((size_t)Vsum);
+  if (Vsum) {
+    int32_t rc = porrt_visibility_dev(ctx, d_vxy, Vsum, d_vmask, d_vstatus);
+    if (rc) return rc;
+    CUDA_TRY(ctx, cudaMemcpyAsync(vmask.data(), d_vmask, (size_t)Vsum * 8, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaMemcpyAsync(vstatus.data(), d_vstatus, (size_t)Vsum * 4, cudaMemcpyDeviceToHost, st));
+  }
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+
+  // ---- per roadmap: where observe() would panic, which visible-zone sets it has (into the union), its finals
+  const uint64_t zone_bits = ctx->n_zones >= 64 ? ~(uint64_t)0 : (((uint64_t)1 << ctx->n_zones) - 1);
+  std::map<uint64_t, int> set_index;
+  std::vector<uint64_t> sets;
+  for (int r = 0; r < R; ++r) {
+    if (out_status[r]) continue;
+    const int64_t V = roads[(size_t)r].V;
+    const uint64_t* m = vmask.data() + vis_off[(size_t)r];
+    const int32_t* sv = vstatus.data() + vis_off[(size_t)r];
+    bool panic = false, wide = false;
+    for (int64_t n = 0; n < V; ++n) { panic |= sv[n] != 0; wide |= __builtin_popcountll(m[n] & zone_bits) > 20; }
+    if (panic) { out_status[r] = PORRT_ERR_PANIC; continue; }          // observe() would panic at one of its nodes
+    if (wide) { out_status[r] = PORRT_ERR_UNSUPPORTED; continue; }     // belief_succ_tables refuses more than 20 visible zones
+    if (nval > 256) { out_status[r] = PORRT_ERR_UNSUPPORTED; continue; }
+    PlanRoad& d = pr[(size_t)r];
+    d.node_set.resize((size_t)V);
+    visible_zone_sets(ctx, m, V, set_index, sets, d.node_set.data());
+    const int F = (int)fin_ids[(size_t)r].size();
+    std::vector<uint64_t> fmask((size_t)F * mw);
+    for (int k = 0; k < F; ++k) memcpy(fmask.data() + (size_t)k * mw, goal_masks.data() + (size_t)fin_goal[(size_t)r][(size_t)k] * mw, (size_t)mw * 8);
+    if (!belief_finals(h, d.nvid.data(), V, fin_ids[(size_t)r].data(), fmask.data(), F, d.fin)) out_status[r] = PORRT_ERR_INVALID_ARG;
+  }
+  // ---- the observation successor tables over the union of the sets.  An entry (set, belief) is read only by the roadmaps that
+  // have the set, so a roadmap is refused for a successor that does not split its belief only if one of ITS sets has one: when the
+  // union's tables report such a successor, each roadmap's own sets are checked, and the union is built again.
+  BeliefSuccDev succ = {};
+  bool any = false;
+  for (int r = 0; r < R; ++r) any |= out_status[r] == PORRT_OK;
+  if (any) {
+    int32_t rc = belief_succ_tables(ctx, beliefs, B, nw, sets, h.bhash, h.level, h.lay.colpos, &succ, st);
+    if (rc) return rc;
+    if (!succ.levels_ok) {
+      for (int r = 0; r < R; ++r) {
+        if (out_status[r]) continue;
+        std::vector<char> has(sets.size(), 0);
+        std::vector<uint64_t> own;
+        for (int32_t k : pr[(size_t)r].node_set) if (!has[(size_t)k]) { has[(size_t)k] = 1; own.push_back(sets[(size_t)k]); }
+        rc = belief_succ_tables(ctx, beliefs, B, nw, own, h.bhash, h.level, h.lay.colpos, &succ, st);
+        if (rc) return rc;
+        if (!succ.levels_ok) out_status[r] = PORRT_ERR_UNSUPPORTED;
+      }
+      rc = belief_succ_tables(ctx, beliefs, B, nw, sets, h.bhash, h.level, h.lay.colpos, &succ, st);
+      if (rc) return rc;
+    }
+  }
+  // the walks read the successor tables on the host, like porrt_belief_vi's retained copies
+  porrt_ctx::BeliefState_ W;
+  W.B = B; W.n_worlds = nw; W.n_validities = nval; W.compat = h.compat; W.colpos = h.lay.colpos; W.on_host = false;
+  if (any) {
+    W.succ_ptr.resize(sets.size() * (size_t)B + 1); W.succ_belief.resize((size_t)succ.n_succ);
+    CUDA_TRY(ctx, cudaMemcpyAsync(W.succ_ptr.data(), succ.succ_ptr, W.succ_ptr.size() * 8, cudaMemcpyDeviceToHost, st));
+    if (succ.n_succ) CUDA_TRY(ctx, cudaMemcpyAsync(W.succ_belief.data(), succ.succ_b, (size_t)succ.n_succ * 4, cudaMemcpyDeviceToHost, st));
+  }
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_cmask, cmask.data(), cmask.size() * 8, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_col_belief, h.lay.poscol.data(), (size_t)Bp * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_colpos, h.lay.colpos.data(), (size_t)B * 4, cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaMemcpyAsync(d_compat, h.compat.data(), h.compat.size(), cudaMemcpyHostToDevice, st));
+  CUDA_TRY(ctx, cudaStreamSynchronize(st));
+  t1 = now_ms(); ph[0] = t1 - t0; t0 = t1;
+
+  // ---- chunks of roadmaps whose tables fit in the free device memory (an eighth of it and 256 MB kept for the frontier schedule's
+  // work space); a roadmap that does not fit on its own fails with PORRT_ERR_CUDA, as porrt_belief_vi's allocation would
+  size_t free_b = 0, total_b = 0;
+  CUDA_TRY(ctx, cudaMemGetInfo(&free_b, &total_b));
+  const size_t keep = free_b / 8 + ((size_t)256 << 20);
+  const size_t budget = free_b > keep ? free_b - keep : 0;
+  std::vector<std::vector<int>> chunks;
+  size_t chunk_max = 0, in_chunk = 0;
+  for (int r = 0; r < R; ++r) {
+    if (out_status[r]) continue;
+    PlanRoad& d = pr[(size_t)r];
+    const PtoRoadDev& g = roads[(size_t)r];
+    d.on_chip = colsolve_fits(g.V, g.E, nval) && !ctx->force_global_sweeps;
+    // its pieces, its descriptor, and the alignment in front of it inside the chunk
+    d.bytes = carve_size([&](Carve& c) { plan_road_layout(c, d, g.V, g.E, B, Bp); c.take<ColSolveArgs>(1); }) + 16;
+    if (d.bytes > budget) {
+      out_status[r] = porrt_fail(ctx, PORRT_ERR_CUDA, "pto_plan_batch: roadmap " + std::to_string(r) + "'s belief table does not fit in device memory");
+      continue;
+    }
+    if (chunks.empty() || in_chunk + d.bytes > budget) { chunks.emplace_back(); in_chunk = 0; }
+    chunks.back().push_back(r);
+    in_chunk += d.bytes;
+    chunk_max = std::max(chunk_max, in_chunk);
+  }
+  DevScratch mem;
+  if (chunk_max) CUDA_TRY(ctx, cudaMalloc(&mem.p, chunk_max + sizeof(ColSolveArgs) + 16));   // + the descriptor array's spare entry
+  cudaEvent_t ev[2] = {nullptr, nullptr};
+  CUDA_TRY(ctx, cudaEventCreate(&ev[0]));
+  CUDA_TRY(ctx, cudaEventCreate(&ev[1]));
+  struct EvGuard { cudaEvent_t* e; ~EvGuard() { cudaEventDestroy(e[0]); cudaEventDestroy(e[1]); } } ev_guard{ev};
+  for (const std::vector<int>& chunk : chunks) {
+    // ---- per roadmap: node types, and for the column solver the transposed adjacency and the initial table, from the resident CSR
+    Carve c{(uintptr_t)mem.p};
+    std::vector<int> on_chip;
+    int32_t V_max = 0;
+    for (int r : chunk) {
+      PlanRoad& d = pr[(size_t)r];
+      const PtoRoadDev& g = roads[(size_t)r];
+      plan_road_layout(c, d, g.V, g.E, B, Bp);
+      CUDA_TRY(ctx, cudaMemcpyAsync(d.d_node_set, d.node_set.data(), (size_t)g.V * 4, cudaMemcpyHostToDevice, st));
+      CUDA_TRY(ctx, cudaMemsetAsync(d.sweeps, 0, 16, st));
+      BeliefDev gd = {g.row_ptr, g.col, g.edge_vid, nullptr, g.node_vid, d.d_node_set, d_compat, succ.succ_ptr, succ.succ_b, succ.succ_p,
+                      g.V, B, nval};
+      belief_type_kernel<<<div_up(g.V * (int64_t)B, 256), 256, 0, st>>>(gd, d.type, d_colpos, d.type_cm);
+      LAUNCH_CHECK(ctx);
+      if (!d.on_chip) continue;
+      on_chip.push_back(r);
+      V_max = std::max(V_max, (int32_t)g.V);
+      edge_cost_kernel<<<div_up(g.V * 32, 256), 256, 0, st>>>(g.row_ptr, g.col, (const double2*)g.xy, g.V, d.cost);
+      LAUNCH_CHECK(ctx);
+      int32_t rc = colsolve_pack(ctx, g.row_ptr, g.col, g.edge_vid, d.cost, g.V, g.E, d.rs, d.ce, d.cost_t, d.cursor, st);
+      if (rc) return rc;
+      fill_inf_kernel<<<ctx->sm_count * 8, 256, 0, st>>>(d.dist_cm, g.V * (int64_t)Bp);
+      LAUNCH_CHECK(ctx);
+      if (!d.fin.empty()) {
+        CUDA_TRY(ctx, cudaMemcpyAsync(d.d_fin, d.fin.data(), d.fin.size() * sizeof(int2), cudaMemcpyHostToDevice, st));
+        scatter_zero_kernel<<<div_up((int64_t)d.fin.size(), 256), 256, 0, st>>>(d.dist_cm, d.d_fin, (int64_t)d.fin.size(), nullptr, g.V, 0, Bp);
+        LAUNCH_CHECK(ctx);
+      }
+    }
+    // the column solver's arguments of every on-chip roadmap, in launch order (blockIdx.y)
+    std::vector<ColSolveArgs> descs(on_chip.size());
+    for (size_t k = 0; k < on_chip.size(); ++k) {
+      const int r = on_chip[k];
+      const PlanRoad& d = pr[(size_t)r];
+      ColSolveArgs& a = descs[k];
+      a = ColSolveArgs{};
+      a.row_start = d.rs; a.cost = d.cost_t; a.ce = d.ce; a.V = (int32_t)roads[(size_t)r].V; a.ld = roads[(size_t)r].V; a.dist_cm = d.dist_cm;
+      a.cmask = d_cmask; a.nvid = roads[(size_t)r].node_vid; a.type_cm = d.type_cm; a.node_set = d.d_node_set; a.col_belief = d_col_belief;
+      a.succ_ptr = succ.succ_ptr; a.succ_col = succ.succ_col; a.succ_p = succ.succ_p; a.B = B; a.sweeps_out = d.sweeps;
+    }
+    ColSolveArgs* d_descs = c.take<ColSolveArgs>(descs.size() + 1);
+    if (!descs.empty()) CUDA_TRY(ctx, cudaMemcpyAsync(d_descs, descs.data(), descs.size() * sizeof(ColSolveArgs), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    t1 = now_ms(); ph[1] += t1 - t0; t0 = t1;
+
+    // ---- the levels: one launch for all on-chip roadmaps per level, then the others one at a time on the frontier schedule
+    CUDA_TRY(ctx, cudaEventRecord(ev[0], st));
+    if (!descs.empty())
+      for (const ColumnLayout::Level& L : h.lay.levels) {
+        int32_t rc = colsolve_level_batch(ctx, d_descs, (int)descs.size(), V_max, L.lo, L.lo + L.n_real, st);
+        if (rc) return rc;
+      }
+    for (int r : chunk) {
+      PlanRoad& d = pr[(size_t)r];
+      if (d.on_chip) continue;
+      const PtoRoadDev& g = roads[(size_t)r];
+      ValueColumns vc = {};
+      vc.kind = COLSOLVE_BELIEF; vc.row = g.row_ptr; vc.col = g.col; vc.xy = g.xy; vc.V = g.V; vc.E = g.E; vc.evid = g.edge_vid;
+      vc.n_validities = nval; vc.layout = &h.lay;
+      ColSolveArgs& ca = vc.cs;
+      ca.V = (int32_t)g.V; ca.ld = g.V; ca.dist_cm = d.dist_cm; ca.cmask = d_cmask; ca.nvid = g.node_vid; ca.type_cm = d.type_cm;
+      ca.node_set = d.d_node_set; ca.col_belief = d_col_belief; ca.succ_ptr = succ.succ_ptr; ca.succ_col = succ.succ_col;
+      ca.succ_p = succ.succ_p; ca.B = B;
+      int32_t rc = value_columns_prepare(ctx, vc, d.fin, st);
+      if (rc) return rc;
+      int32_t sweeps = 0;
+      double offers = 0.0;
+      rc = value_columns_solve(ctx, vc, &sweeps, &offers, st);
+      if (rc) return rc;
+      if (out_sweeps) out_sweeps[r] = sweeps;
+    }
+    CUDA_TRY(ctx, cudaEventRecord(ev[1], st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    float ms = 0.f;
+    CUDA_TRY(ctx, cudaEventElapsedTime(&ms, ev[0], ev[1]));
+    ph[2] += ms;
+    for (int r : on_chip)
+      if (out_sweeps) CUDA_TRY(ctx, cudaMemcpyAsync(&out_sweeps[r], pr[(size_t)r].sweeps, 4, cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(ctx, cudaStreamSynchronize(st));
+    t0 = now_ms();
+
+    // ---- the policy walks, each over its own roadmap's table
+    for (int r : chunk) {
+      PlanRoad& d = pr[(size_t)r];
+      W.V = roads[(size_t)r].V;
+      W.row_ptr = std::move(d.row); W.col = std::move(d.col); W.edge_vid = std::move(d.evid); W.xy = std::move(d.xy);
+      W.node_vid = std::move(d.nvid); W.node_obs_set = std::move(d.node_set);
+      W.d_dist_cm = d.dist_cm; W.d_type_cm = d.type_cm;
+      W.col_dist.assign((size_t)B, std::vector<double>()); W.col_type.assign((size_t)B, std::vector<uint8_t>());
+      double cost = 0.0;
+      const int32_t rc = belief_policy_walk(ctx, W, beliefs, "pto_plan_batch", d.pol, &cost);
+      if (rc) { out_status[r] = rc; d.pol.clear(); }
+      else out_expected_cost[r] = cost;
+    }
+    t1 = now_ms(); ph[3] += t1 - t0; t0 = t1;
+  }
+
+  // ---- the policies, back to back
+  int64_t total = 0;
+  for (int r = 0; r < R; ++r) { out_policy_ptr[r] = total; total += (int64_t)pr[(size_t)r].pol.size(); }
+  out_policy_ptr[R] = total;
+  *out_total = total;
+  if (out_phase_ms) memcpy(out_phase_ms, ph, sizeof(ph));
+  if (total > cap) return porrt_fail(ctx, PORRT_ERR_CAPACITY, "pto_plan_batch: cap too small");
+  for (int r = 0; r < R; ++r) {
+    const std::vector<PolicyNode>& pol = pr[(size_t)r].pol;
+    const int64_t at = out_policy_ptr[r];
+    for (size_t k = 0; k < pol.size(); ++k) {
+      out_node[at + (int64_t)k] = (int32_t)(pol[k].id / B); out_belief[at + (int64_t)k] = (int32_t)(pol[k].id % B);
+      out_parent[at + (int64_t)k] = pol[k].parent; out_is_leaf[at + (int64_t)k] = pol[k].leaf;
+    }
   }
   return PORRT_OK;
 }

@@ -1198,6 +1198,26 @@ PORRT_API int32_t porrt_pto_fetch_roadmap(porrt_ctx* ctx, int32_t r, double* out
   return PORRT_OK;
 }
 
+// The roadmaps of the last PTO growth as they lie on the device, for graph.cu's porrt_pto_plan_batch; false when nothing has been grown.
+bool pto_roads(const porrt_ctx* ctx, std::vector<PtoRoadDev>& out, std::vector<uint64_t>* goal_masks, int* words) {
+  const PtoGrow* pg = ctx->pto;
+  if (!pg || pg->n_have == 0) return false;
+  out.assign((size_t)pg->n_have, PtoRoadDev{});
+  for (int32_t r = 0; r < pg->n_have; ++r) {
+    const PtoRoad* g = pg->roads[(size_t)r].get();
+    PtoRoadDev& d = out[(size_t)r];
+    d.have = g->have;
+    if (!g->have) continue;
+    d.V = g->V; d.E = g->E; d.n_finals = g->n_finals;
+    d.xy = g->xy.as<double>(); d.node_vid = g->node_vid.as<int32_t>();
+    d.row_ptr = g->csr_row.as<int64_t>(); d.col = g->csr_col.as<int32_t>(); d.edge_vid = g->csr_vid.as<int32_t>();
+    d.fin_ids = g->fin_ids.as<int32_t>(); d.fin_goal = g->fin_goal.as<int32_t>();
+  }
+  *goal_masks = pg->goal_masks_host;
+  *words = pg->words;
+  return true;
+}
+
 PORRT_API int32_t porrt_pto_fetch(porrt_ctx* ctx, double* out_xy, int32_t* out_node_vid, int64_t* out_row_ptr, int32_t* out_col,
                                   int32_t* out_edge_vid, uint64_t* out_reach, int64_t* out_final_ids, uint64_t* out_final_masks) {
   return porrt_pto_fetch_roadmap(ctx, 0, out_xy, out_node_vid, out_row_ptr, out_col, out_edge_vid, out_reach, out_final_ids, out_final_masks);
